@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — the hot path of BASELINE.json on synthetic corpora of the named shapes.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--workload c2|c1|c3|c5] [--files F]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--workload c2|c1|c3|c5] [--files F] [--dump-outputs DIR]
   python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
   python bench.py --impl reference ...        # the UNMODIFIED reference binary (zlib L6 / zlib inflate / OpenSSL MD5) on host cores
 
@@ -465,6 +465,46 @@ def fill_device(torch, d_raw, sh: Shard):
     del d_unit
 
 
+DUMP_ROWS = 1 << 16    # --dump-outputs: rows kept of every per-chunk, per-record and per-file array
+DUMP_BYTES = 1 << 20   # and bytes kept of the packed and of the inflated buffer
+
+
+def dump_rows(n):
+    """A fixed, seeded choice of at most DUMP_ROWS of n rows, in order (all n when there are few)."""
+    if n <= DUMP_ROWS:
+        return np.arange(n)
+    return np.sort(np.random.default_rng([596, n]).choice(n, DUMP_ROWS, replace=False))
+
+
+def step_outputs(torch, state, d_packed, d_back, U):
+    """What the last device step handed its caller, as float arrays for --dump-outputs (values below 2^24 as float32, byte
+    offsets as float64): the deflate result of every chunk, the packed stream offsets, the inflated length and status of every
+    record and the MD5 of every source and every inflated file (rows chosen by dump_rows), and the packed and the inflated
+    bytes at DUMP_BYTES fixed, seeded positions."""
+    res = state["res"]
+    r = dump_rows(len(res))
+    out = {f"deflate_{k}": res[k][r].astype(np.float32) for k in ("len0", "len1", "raw0", "btype")}
+    out["packed_off"] = state["poff"][dump_rows(len(state["poff"]))].astype(np.float64)
+    r = dump_rows(len(state["rl"]))
+    out["inflate_len"] = state["rl"][r].astype(np.float32)
+    out["inflate_status"] = state["st"][r].astype(np.float32)
+    for key, name in (("dg1", "md5_src"), ("dg2", "md5_out")):
+        if state[key] is not None:
+            out[name] = state[key][dump_rows(len(state[key]))].astype(np.float32)
+    for name, buf, size in (("packed_bytes", d_packed, int(state["poff"][-1])), ("inflated_bytes", d_back, U)):
+        pos = np.sort(np.random.default_rng([596, size]).integers(0, size, DUMP_BYTES))
+        out[name] = buf[torch.from_numpy(pos).to(buf.device)].cpu().numpy().astype(np.float32)
+    return out
+
+
+def write_dump(path, arrays):
+    total = sum(a.nbytes for a in arrays.values())
+    assert total <= 64 << 20, f"--dump-outputs: {total} bytes"
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), a)
+
+
 # ---------------------------------------------------------------------------------------------------------------------
 def main():
     ap = argparse.ArgumentParser()
@@ -487,7 +527,11 @@ def main():
     ap.add_argument("--md5", default="auto", choices=["auto", "on", "off"],
                     help="auto: on for c2/c1/c5 (compress+decompress+MD5 verify), off for c3 (BASELINE.json config 3 is deflate+inflate only: "
                          "the MD5 of ONE file is a single serial chain, one lane, ~0.13 GB/s)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed device steps, write what the last one computed on rank 0 "
+                    "(see step_outputs) to DIR/<name>.npy, so that two builds can be compared output for output on the same inputs")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps: at least one timed step")
     if args.warmup < 3:
         args.warmup = 3  # timing rule: W >= 3
     if args.files == 0:
@@ -708,6 +752,8 @@ def main():
     launches = ctx.launches - launches0
     prof = ctx.profile_read(True)
     ctx.profile_enable(False)
+    if args.dump_outputs and rank == 0:
+        write_dump(args.dump_outputs, step_outputs(torch, state, d_packed, d_back, U))
 
     # e2e (host buffers only: the device-resident copies of the shard are not needed any more — at 32 GB per GPU, C5 over two
     # GPUs, they and the workers' arenas do not fit side by side)

@@ -1,5 +1,6 @@
 """ctypes loader for oracle/liboracle.so — the CHECKER. Only tests/, smoke() and bench.py's CPU legs use this."""
 import ctypes as C
+import hashlib
 import os
 import subprocess
 
@@ -95,3 +96,50 @@ def ref_inflate_chunk(comp, cap=1 << 21) -> bytes:
     n = lib().oracle_ref_inflate_chunk(p, a.size, out.ctypes.data, cap)
     assert n >= 0
     return out[:n].tobytes()
+
+
+def ref_decompress(arch_dir, out_dir) -> dict:
+    """`main decompress <arch_dir> <out_dir>` of the reference (decompression.cpp:45-178) restated: every *.zwz is read
+    record by record with per-archive, per-path state. A record whose sequence id is the expected one is inflated
+    (ref_inflate_chunk) and appended to <out_dir>/<path>, followed by any waiting records that are now in order; other records
+    wait in a min-heap. When the record just read is the last one, was in order and nothing waits, the file is closed and
+    the MD5 of what was written is compared with the stored one (decompression.cpp:132-146). Returns the verdict counts
+    {"match": m, "mismatch": k}. tests/test_oracle.py pins this to what the reference binary wrote for tests/golden/."""
+    import heapq
+
+    import zwz_format
+    verdicts = {"match": 0, "mismatch": 0}
+    for name in sorted(f for f in os.listdir(arch_dir) if f.endswith(".zwz")):
+        files = {}   # path -> [output file, its path, expected sequence id, heap of (sequence id, payload)]
+        for r in zwz_format.parse(open(os.path.join(arch_dir, name), "rb").read()):
+            if r.path not in files:
+                dst = os.path.join(out_dir, r.path)
+                os.makedirs(os.path.dirname(dst), exist_ok=True)
+                files[r.path] = [open(dst, "wb"), dst, 0, []]
+            st = files[r.path]
+            if r.seq != st[2]:
+                heapq.heappush(st[3], (r.seq, r.payload))
+                continue
+            st[0].write(ref_inflate_chunk(r.payload))
+            st[2] += 1
+            while st[3] and st[3][0][0] == st[2]:
+                st[0].write(ref_inflate_chunk(heapq.heappop(st[3])[1]))
+                st[2] += 1
+            if r.last and st[2] == r.seq + 1 and not st[3]:
+                st[0].close()
+                ok = ref_md5_hex(open(st[1], "rb").read()) == r.md5.decode()
+                verdicts["match" if ok else "mismatch"] += 1
+        for st in files.values():
+            st[0].close()
+    return verdicts
+
+
+def md5_tree(root) -> dict:
+    """{relative path: {"size", "md5"}} of every file under root (the form of tests/golden/manifest.json)."""
+    out = {}
+    for d, _, names in os.walk(root):
+        for f in names:
+            p = os.path.join(d, f)
+            b = open(p, "rb").read()
+            out[os.path.relpath(p, root)] = {"size": len(b), "md5": hashlib.md5(b).hexdigest()}
+    return out

@@ -70,6 +70,33 @@ def test_global_totals_match_shards():
         assert tuple(tot) == bench.global_totals(wl, files, world)
 
 
+def test_dump_outputs_sampled_seeded_and_bounded(tmp_path):
+    """--dump-outputs of a step with C2's 370 000 chunks, records and files: float arrays, the same rows and byte positions on
+    every run, bytes read where the sample says, at most 64 MB in all."""
+    import torch
+    n, U = 370_000, 40 << 20
+    rng = np.random.default_rng(1)
+    res = np.zeros(n, dtype=zwz_b200.RESULT_DTYPE)
+    res["len0"] = rng.integers(8, 60000, n)
+    res["raw0"] = 65535
+    poff = np.concatenate([[0], np.cumsum(res["len0"])]).astype(np.uint64)
+    state = {"res": res, "poff": poff, "rl": res["raw0"].copy(), "st": np.zeros(n, dtype=np.uint32),
+             "dg1": rng.integers(0, 256, (n, 16), dtype=np.uint8), "dg2": rng.integers(0, 256, (n, 16), dtype=np.uint8)}
+    packed = torch.from_numpy(rng.integers(0, 256, int(poff[-1]), dtype=np.uint8))
+    back = torch.from_numpy(rng.integers(0, 256, U, dtype=np.uint8))
+    a = bench.step_outputs(torch, state, packed, back, U)
+    b = bench.step_outputs(torch, state, packed, back, U)
+    assert a.keys() == b.keys() and all(np.array_equal(a[k], b[k]) for k in a)
+    assert all(v.dtype in (np.float32, np.float64) for v in a.values())
+    assert sum(v.nbytes for v in a.values()) <= 64 << 20
+    r = bench.dump_rows(n)
+    assert len(r) == bench.DUMP_ROWS and np.array_equal(a["md5_out"], state["dg2"][r]) and np.array_equal(a["deflate_len0"], res["len0"][r])
+    pos = np.sort(np.random.default_rng([596, U]).integers(0, U, bench.DUMP_BYTES))
+    assert np.array_equal(a["inflated_bytes"], back.numpy()[pos])
+    bench.write_dump(str(tmp_path / "d"), a)
+    assert np.array_equal(np.load(tmp_path / "d" / "packed_off.npy"), a["packed_off"])
+
+
 def test_sample_of_periodic():
     sh = bench.Shard(np.arange(1000, dtype=np.uint8), 5000, [0, 5000], "x")
     assert np.array_equal(sh.host_bytes(990, 1010), np.concatenate([np.arange(990, 1000), np.arange(0, 10)]).astype(np.uint8))

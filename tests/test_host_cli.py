@@ -1,4 +1,6 @@
-"""The C++ host (`main compress|decompress <src> <dst>`) against the UNMODIFIED reference binary (oracle/_ref/main_ref).
+"""The C++ host (`main compress|decompress <src> <dst>`) against the reference: the archives its unmodified binary wrote for
+the edge-case tree (tests/golden/), and its reader restated (oracle_lib.ref_decompress, pinned to what the binary wrote when
+it read those archives, tests/test_oracle.py).
 
 `[emu]`: the host sources linked against the SIMT-emulator build of the C ABI (CPU, here). `[cuda]`: the shipped `main`
 over libzwz_cuda.so on the B200. Criteria from BASELINE.json:
@@ -17,15 +19,13 @@ import subprocess
 
 import pytest
 
+import oracle_lib as O
 import zwz_format
 from tools import corpus
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-MAIN_REF = os.path.join(ROOT, "oracle", "_ref", "main_ref")
 GOLD = os.path.join(ROOT, "tests", "golden")
 HOST = os.path.join(ROOT, "parallel-data-compression-and-decompression_b200", "host")
-
-needs_ref = pytest.mark.skipif(not os.path.exists(MAIN_REF), reason="oracle/_ref/main_ref not built (needs /root/reference once)")
 
 
 @pytest.fixture(params=[pytest.param("emu", id="emu"), pytest.param("cuda", id="cuda", marks=pytest.mark.gpu)])
@@ -67,7 +67,14 @@ def edge_tree(tmp_path):
     return str(src), specs
 
 
-@needs_ref
+def reference_archives_of(src, name):
+    """The archives the reference binary wrote for the edge-case tree (edge_r1: one rank, edge_r2: two), once it is checked
+    that `src` is that very tree."""
+    man = json.load(open(os.path.join(GOLD, "manifest.json")))
+    assert O.md5_tree(src) == man["inputs"]
+    return os.path.join(GOLD, name)
+
+
 def test_reference_decompresses_our_archive(main_bin, edge_tree, tmp_path):
     src, specs = edge_tree
     arch = str(tmp_path / "arch")
@@ -76,12 +83,10 @@ def test_reference_decompresses_our_archive(main_bin, edge_tree, tmp_path):
     assert os.listdir(arch) == ["compressed_0.zwz"]                       # compression.cpp:151-159
     assert os.path.exists(os.path.join(os.path.dirname(src), "sorted_files_by_size.txt"))  # file_sort.cpp:33
     out = str(tmp_path / "out")
-    dlog = run([MAIN_REF, "decompress", arch, out])
-    assert dlog.count("MD5 match for file") == len(specs) and "MD5 mismatch" not in dlog
+    assert O.ref_decompress(arch, out) == {"match": len(specs), "mismatch": 0}
     same_tree(src, out)  # lossless even for the incompressible 65 535-byte chunk the reference itself truncates
 
 
-@needs_ref
 def test_record_layout_and_md5(main_bin, edge_tree, tmp_path):
     src, specs = edge_tree
     arch = str(tmp_path / "arch")
@@ -108,17 +113,14 @@ def test_record_layout_and_md5(main_bin, edge_tree, tmp_path):
     assert len(by["empty.bin"]) == 1
 
 
-@needs_ref
 def test_we_decompress_reference_archives_byte_exact(main_bin, edge_tree, tmp_path):
     src, specs = edge_tree
-    arch = str(tmp_path / "arch_ref")
-    run([MAIN_REF, "compress", src, arch])
+    arch = reference_archives_of(src, "edge_r1")
     ref_out, our_out = str(tmp_path / "ref_out"), str(tmp_path / "our_out")
-    rlog = run([MAIN_REF, "decompress", arch, ref_out])
+    rv = O.ref_decompress(arch, ref_out)
     olog = run([main_bin, "decompress", arch, our_out])
     same_tree(ref_out, our_out)
-    for key in ("MD5 match for file", "MD5 mismatch for file"):
-        assert rlog.count(key) == olog.count(key)
+    assert (olog.count("MD5 match for file"), olog.count("MD5 mismatch for file")) == (rv["match"], rv["mismatch"])
     assert olog.count("MD5 mismatch for file") == 1   # the reference's own truncated record (SURVEY.md §5.1)
 
 
@@ -139,10 +141,9 @@ def test_we_decompress_golden_archives(main_bin, name, tmp_path):
     assert log.count("MD5 mismatch for file") == man[name]["verdicts"]["mismatch"]
 
 
-@needs_ref
 def test_self_launch_one_process_per_gpu(main_bin, edge_tree, tmp_path):
     """`ZWZ_GPUS=2 main compress` forks rank 1 itself (no MPI launcher): two archives with the reference's deal, and the
-    reference reads them back to the source tree."""
+    reference's reader reads them back to the source tree."""
     src, specs = edge_tree
     arch, out = str(tmp_path / "arch"), str(tmp_path / "out")
     log = run([main_bin, "compress", src, arch], {"ZWZ_GPUS": "2"})
@@ -155,7 +156,7 @@ def test_self_launch_one_process_per_gpu(main_bin, edge_tree, tmp_path):
             if rec.path not in paths:
                 paths.append(rec.path)
         assert sorted(paths) == sorted(s.relpath for s in order[r::2])
-    run([MAIN_REF, "decompress", arch, out])
+    O.ref_decompress(arch, out)
     same_tree(src, out)
 
 
@@ -177,15 +178,10 @@ def test_strict_mode_names_the_records_zlib_would_have_rejected(main_bin, tmp_pa
     same_tree(out1, out2)
 
 
-@needs_ref
 def test_two_ranks_same_deal_as_reference(main_bin, edge_tree, tmp_path):
     """`mpirun -n 2` analogue: rank r takes sorted files r, r+2, ... and writes compressed_<r>.zwz (compression.cpp:31-41,157)."""
     src, specs = edge_tree
-    ours, ref = str(tmp_path / "ours"), str(tmp_path / "ref")
-    bc = tmp_path / "bc"
-    bc.mkdir()
-    for r in (0, 1):
-        run([MAIN_REF, "compress", src, ref], {"ZWZ_STUB_SIZE": "2", "ZWZ_STUB_RANK": str(r), "ZWZ_STUB_DIR": str(bc)})
+    ours, ref = str(tmp_path / "ours"), reference_archives_of(src, "edge_r2")
     procs = [subprocess.Popen([main_bin, "compress", src, ours], env={**os.environ, "ZWZ_WORLD": "2", "ZWZ_RANK": str(r)},
                               stdout=subprocess.PIPE, stderr=subprocess.STDOUT) for r in (0, 1)]
     for p in procs:
@@ -197,8 +193,7 @@ def test_two_ranks_same_deal_as_reference(main_bin, edge_tree, tmp_path):
         pr = [r.path for r in zwz_format.parse(open(os.path.join(ref, a), "rb").read()) if r.seq == 0]
         assert po == pr, a
     out = str(tmp_path / "out")
-    dlog = run([MAIN_REF, "decompress", ours, out])
-    assert dlog.count("MD5 match for file") == len(specs)
+    assert O.ref_decompress(ours, out)["match"] == len(specs)
     same_tree(src, out)
 
 
@@ -324,13 +319,12 @@ def test_multi_rank_decompress(main_bin, tmp_path, launch):
     same_tree(src, out)
 
 
-@needs_ref
 @pytest.mark.parametrize("launch", ["self", "ranks"])
 def test_one_file_cut_over_the_ranks_lands_in_one_archive(main_bin, tmp_path, launch):
     """BASELINE config 3 / SURVEY.md §8(e): the reference's deal is file-granular (compression.cpp:31-41) and its reader wants
     all records of a path in ONE archive (decompression.cpp:52-55). A file that is cut into segments is deflated by several
     ranks here; the owner hands out archive offsets and sequence ids through the segment ledger and every rank writes its
-    records into the owner's archive. The unmodified reference reads the result back."""
+    records into the owner's archive. The reference's reader reads the result back."""
     src = tmp_path / "w" / "src"
     src.mkdir(parents=True)
     specs = [corpus.FileSpec("big/huge.log", 5_300_000, "T", 997), corpus.FileSpec("big/second.bin", 2_500_000, "S", 996),
@@ -361,8 +355,7 @@ def test_one_file_cut_over_the_ranks_lands_in_one_archive(main_bin, tmp_path, la
             assert rs[-1].md5.decode() == hashlib.md5(open(os.path.join(str(src), pth), "rb").read()).hexdigest()
     order = sorted(specs, key=lambda s_: -s_.size)
     assert owner == {s_.relpath: i % 3 for i, s_ in enumerate(order)}       # the reference's deal decides the archive
-    dlog = run([MAIN_REF, "decompress", arch, out])
-    assert dlog.count("MD5 match for file") == len(specs) and "mismatch" not in dlog
+    assert O.ref_decompress(arch, out) == {"match": len(specs), "mismatch": 0}
     same_tree(str(src), out)
 
 
