@@ -23,11 +23,22 @@ from typing import Optional, Tuple
 import numpy as np
 
 __all__ = ["Context", "ZwzError", "load_library", "library_path", "CHUNK_SIZE", "deflate_bound", "chunk_table",
-           "STREAM_END", "STREAM_TRUNCATED", "STREAM_BAD", "STREAM_OUTPUT_FULL", "RESULT_DTYPE"]
+           "STREAM_END", "STREAM_TRUNCATED", "STREAM_BAD", "STREAM_OUTPUT_FULL", "RESULT_DTYPE",
+           "FORMAT_ZLIB", "FORMAT_GZIP", "FORMAT_RAW", "BGZF_BLOCK"]
 
 CHUNK_SIZE = 65535  # process.hpp:12
 STREAM_END, STREAM_TRUNCATED, STREAM_BAD, STREAM_OUTPUT_FULL = 0, 1, 2, 3
 INFLATE_NO_ADLER = 1
+# stream formats (ZWZ_FORMAT_*): the wrapper around the DEFLATE body. The ``format=`` keywords take these names.
+FORMAT_ZLIB, FORMAT_GZIP, FORMAT_RAW = 0, 1, 2
+BGZF_BLOCK = 65280  # largest chunk in gzip format: one BGZF member each
+_FORMATS = {"zlib": FORMAT_ZLIB, "gzip": FORMAT_GZIP, "raw": FORMAT_RAW}
+
+
+def _format(name: str) -> int:
+    if name not in _FORMATS:
+        raise ValueError(f"format must be one of {sorted(_FORMATS)}, not {name!r}")
+    return _FORMATS[name]
 
 RESULT_DTYPE = np.dtype([("len0", "<u4"), ("len1", "<u4"), ("raw0", "<u4"), ("btype", "<u4")])
 
@@ -80,6 +91,15 @@ def _declare(L):
     L.zwz_md5_hex.argtypes = [vp, vp]
     L.zwz_md5_hex.restype = None
     L.zwz_adler32_batch_device.argtypes = [vp, vp, vp, vp, u32, vp, vp]
+    L.zwz_crc32_batch_device.argtypes = [vp, vp, vp, vp, u32, vp, vp]
+    L.zwz_deflate_batch_device_ex.argtypes = [vp, vp, vp, vp, u32, vp, vp, vp, i32, i32, vp]
+    L.zwz_deflate_batch_ex.argtypes = [vp, vp, vp, vp, u32, vp, u64, vp, vp, i32, i32]
+    L.zwz_gzip_bound.argtypes = [vp, u32]
+    L.zwz_gzip_bound.restype = u64
+    L.zwz_gzip_files.argtypes = [vp, vp, vp, u32, i32, vp, u64, vp]
+    L.zwz_gunzip_bound.argtypes = [vp, vp, u32]
+    L.zwz_gunzip_bound.restype = u64
+    L.zwz_gunzip_files.argtypes = [vp, vp, vp, u32, vp, u64, vp, vp]
     L.zwz_compress_files.argtypes = [vp, vp, vp, u32, i32, vp, u64, vp, vp, vp]
     L.zwz_decompress_records.argtypes = [vp, vp, vp, vp, vp, vp, u32, u32, vp, u64, vp, vp, vp, vp, u32]
     L.zwz_ctx_tune.argtypes = [vp, i32, u64]
@@ -221,8 +241,9 @@ class Context:
         self._check(self.lib.zwz_sync(self.h))
 
     # ---- deflate: compression.cpp:119-134 ----
-    def deflate_batch(self, raw, off, length, level: int = 0):
-        """Host buffers. Returns (packed uint8 array, packed_off[n+1] u64, results[n] RESULT_DTYPE)."""
+    def deflate_batch(self, raw, off, length, level: int = 0, format: str = "zlib"):
+        """Host buffers. Returns (packed uint8 array, packed_off[n+1] u64, results[n] RESULT_DTYPE). format: "zlib", "gzip" (one
+        BGZF member per chunk, chunks <= BGZF_BLOCK) or "raw"."""
         raw = _u8(raw)
         off = np.ascontiguousarray(off, dtype=np.uint64)
         length = np.ascontiguousarray(length, dtype=np.uint32)
@@ -231,18 +252,18 @@ class Context:
         out = np.empty(max(cap, 1), dtype=np.uint8)
         poff = np.zeros(n + 1, dtype=np.uint64)
         res = np.zeros(n, dtype=RESULT_DTYPE)
-        self._check(self.lib.zwz_deflate_batch(self.h, _ptr(raw), _ptr(off), _ptr(length), n, _ptr(out), cap, poff.ctypes.data,
-                                               _ptr(res), level))
+        self._check(self.lib.zwz_deflate_batch_ex(self.h, _ptr(raw), _ptr(off), _ptr(length), n, _ptr(out), cap, poff.ctypes.data,
+                                                  _ptr(res), level, _format(format)))
         return out[:int(poff[n])], poff, res
 
-    def deflate_batch_device(self, d_raw: int, off, length, d_out: int, out_off, level: int = 0, stream: int = 0):
+    def deflate_batch_device(self, d_raw: int, off, length, d_out: int, out_off, level: int = 0, stream: int = 0, format: str = "zlib"):
         off = np.ascontiguousarray(off, dtype=np.uint64)
         length = np.ascontiguousarray(length, dtype=np.uint32)
         out_off = np.ascontiguousarray(out_off, dtype=np.uint64)
         n = len(off)
         res = np.zeros(n, dtype=RESULT_DTYPE)
-        self._check(self.lib.zwz_deflate_batch_device(self.h, d_raw, _ptr(off), _ptr(length), n, d_out, _ptr(out_off), _ptr(res), level,
-                                                      stream or None))
+        self._check(self.lib.zwz_deflate_batch_device_ex(self.h, d_raw, _ptr(off), _ptr(length), n, d_out, _ptr(out_off), _ptr(res), level,
+                                                         _format(format), stream or None))
         return res
 
     def pack_streams_device(self, d_slots: int, slot_off, res, d_packed: int, stream: int = 0) -> np.ndarray:
@@ -255,8 +276,9 @@ class Context:
         return poff
 
     # ---- inflate: decompression.cpp:11-37 ----
-    def inflate_batch(self, comp, off, length, raw_off, flags: int = 0):
-        """Host buffers. raw_off[n+1] gives every stream's output window. Returns (raw_out, raw_len[n], status[n])."""
+    def inflate_batch(self, comp, off, length, raw_off, flags: int = 0, format: str = "zlib"):
+        """Host buffers. raw_off[n+1] gives every stream's output window. Returns (raw_out, raw_len[n], status[n]).
+        format: "zlib", "gzip" (one member per stream, as zlib with windowBits 31) or "raw"."""
         comp = _u8(comp)
         off = np.ascontiguousarray(off, dtype=np.uint64)
         length = np.ascontiguousarray(length, dtype=np.uint32)
@@ -265,10 +287,11 @@ class Context:
         out = np.zeros(max(int(raw_off[n]) if n else 0, 1), dtype=np.uint8)
         rl = np.zeros(n, dtype=np.uint32)
         st = np.zeros(n, dtype=np.uint32)
-        self._check(self.lib.zwz_inflate_batch(self.h, _ptr(comp), _ptr(off), _ptr(length), n, _ptr(out), _ptr(raw_off), _ptr(rl), _ptr(st), flags))
+        self._check(self.lib.zwz_inflate_batch(self.h, _ptr(comp), _ptr(off), _ptr(length), n, _ptr(out), _ptr(raw_off), _ptr(rl), _ptr(st),
+                                               flags | (_format(format) << 8)))
         return out, rl, st
 
-    def inflate_batch_device(self, d_comp: int, off, length, d_raw_out: int, raw_off, flags: int = 0, stream: int = 0):
+    def inflate_batch_device(self, d_comp: int, off, length, d_raw_out: int, raw_off, flags: int = 0, stream: int = 0, format: str = "zlib"):
         off = np.ascontiguousarray(off, dtype=np.uint64)
         length = np.ascontiguousarray(length, dtype=np.uint32)
         raw_off = np.ascontiguousarray(raw_off, dtype=np.uint64)
@@ -276,7 +299,7 @@ class Context:
         rl = np.zeros(n, dtype=np.uint32)
         st = np.zeros(n, dtype=np.uint32)
         self._check(self.lib.zwz_inflate_batch_device(self.h, d_comp, _ptr(off), _ptr(length), n, d_raw_out, _ptr(raw_off), _ptr(rl), _ptr(st),
-                                                      flags, stream or None))
+                                                      flags | (_format(format) << 8), stream or None))
         return rl, st
 
     def decompress_records(self, comp, off, length, rec_cap, rec_file, nf: int, out_cap: int, want_md5: bool = True, flags: int = 0):
@@ -328,17 +351,18 @@ class Context:
                                                     out_cap, _ptr(foff), _ptr(rl), _ptr(st), _ptr(dg) if want_md5 else None, flags))
         return foff, rl, st, dg
 
-    def deflate_batch_into(self, raw_ptr: int, off, length, out_ptr: int, out_cap: int, level: int = 0):
+    def deflate_batch_into(self, raw_ptr: int, off, length, out_ptr: int, out_cap: int, level: int = 0, format: str = "zlib"):
         """zwz_deflate_batch on raw addresses. Returns (packed_off[n+1], results[n])."""
         off = np.ascontiguousarray(off, dtype=np.uint64)
         length = np.ascontiguousarray(length, dtype=np.uint32)
         n = len(off)
         poff = np.zeros(n + 1, dtype=np.uint64)
         res = np.zeros(n, dtype=RESULT_DTYPE)
-        self._check(self.lib.zwz_deflate_batch(self.h, raw_ptr, _ptr(off), _ptr(length), n, out_ptr, out_cap, poff.ctypes.data, _ptr(res), level))
+        self._check(self.lib.zwz_deflate_batch_ex(self.h, raw_ptr, _ptr(off), _ptr(length), n, out_ptr, out_cap, poff.ctypes.data, _ptr(res), level,
+                                                  _format(format)))
         return poff, res
 
-    def inflate_batch_into(self, comp_ptr: int, off, length, out_ptr: int, raw_off, flags: int = 0):
+    def inflate_batch_into(self, comp_ptr: int, off, length, out_ptr: int, raw_off, flags: int = 0, format: str = "zlib"):
         """zwz_inflate_batch on raw addresses (raw_off[n+1] relative to out_ptr). Returns (raw_len[n], status[n])."""
         off = np.ascontiguousarray(off, dtype=np.uint64)
         length = np.ascontiguousarray(length, dtype=np.uint32)
@@ -346,7 +370,8 @@ class Context:
         n = len(off)
         rl = np.zeros(n, dtype=np.uint32)
         st = np.zeros(n, dtype=np.uint32)
-        self._check(self.lib.zwz_inflate_batch(self.h, comp_ptr, _ptr(off), _ptr(length), n, out_ptr, _ptr(raw_off), _ptr(rl), _ptr(st), flags))
+        self._check(self.lib.zwz_inflate_batch(self.h, comp_ptr, _ptr(off), _ptr(length), n, out_ptr, _ptr(raw_off), _ptr(rl), _ptr(st),
+                                               flags | (_format(format) << 8)))
         return rl, st
 
     # ---- MD5: verification.cpp:13-27 ----
@@ -393,6 +418,43 @@ class Context:
         out = np.zeros(n, dtype=np.uint32)
         self._check(self.lib.zwz_adler32_batch_device(self.h, d_data, _ptr(off), _ptr(length), n, _ptr(out), stream or None))
         return out
+
+    def crc32_batch_device(self, d_data: int, off, length, stream: int = 0) -> np.ndarray:
+        """CRC-32 (RFC 1952, what zlib.crc32 computes) of every range d_data[off[i] .. off[i]+length[i]), one warp each."""
+        off = np.ascontiguousarray(off, dtype=np.uint64)
+        length = np.ascontiguousarray(length, dtype=np.uint32)
+        n = len(off)
+        out = np.zeros(n, dtype=np.uint32)
+        self._check(self.lib.zwz_crc32_batch_device(self.h, d_data, _ptr(off), _ptr(length), n, _ptr(out), stream or None))
+        return out
+
+    # ---- whole files <-> BGZF .gz files ----
+    def gzip_files(self, data, file_off, level: int = 0):
+        """File i = data[file_off[i] .. file_off[i+1]) -> its BGZF .gz file out[gz_off[i] .. gz_off[i+1]) (readable by gzip -d,
+        zcat, Python's gzip, htslib). Returns (out uint8 array, gz_off[nf+1] u64)."""
+        data = _u8(data)
+        file_off = np.ascontiguousarray(file_off, dtype=np.uint64)
+        nf = len(file_off) - 1
+        cap = int(self.lib.zwz_gzip_bound(_ptr(file_off), nf))
+        out = np.empty(max(cap, 1), dtype=np.uint8)
+        gz_off = np.zeros(nf + 1, dtype=np.uint64)
+        self._check(self.lib.zwz_gzip_files(self.h, _ptr(data), _ptr(file_off), nf, level, _ptr(out), cap, _ptr(gz_off)))
+        return out[:int(gz_off[nf])], gz_off
+
+    def gunzip_files(self, gz, gz_off, out_cap: Optional[int] = None):
+        """BGZF file i = gz[gz_off[i] .. gz_off[i+1]) -> (out uint8 array, out_off[nf+1] u64, status[nf]): file i's bytes are
+        out[out_off[i] .. out_off[i+1]), status[i] STREAM_END when the whole file decoded cleanly. out_cap defaults to
+        zwz_gunzip_bound (a smaller one raises ZwzError with ZWZ_E_CAPACITY)."""
+        gz = _u8(gz)
+        gz_off = np.ascontiguousarray(gz_off, dtype=np.uint64)
+        nf = len(gz_off) - 1
+        if out_cap is None:
+            out_cap = int(self.lib.zwz_gunzip_bound(_ptr(gz), _ptr(gz_off), nf))
+        out = np.empty(max(out_cap, 1), dtype=np.uint8)
+        out_off = np.zeros(nf + 1, dtype=np.uint64)
+        st = np.zeros(max(nf, 1), dtype=np.uint32)
+        self._check(self.lib.zwz_gunzip_files(self.h, _ptr(gz), _ptr(gz_off), nf, _ptr(out), out_cap, _ptr(out_off), _ptr(st)))
+        return out[:int(out_off[nf])], out_off, st[:nf]
 
 
 def md5_hex(digests: np.ndarray):

@@ -4,6 +4,8 @@
 // left in HBM scratch by lz_match_kernel and the raw chunk. Output: one complete zlib stream (78 9C, one final DEFLATE
 // block — stored, fixed or dynamic, whichever is smallest — and the big-endian Adler-32), or two stored streams when
 // even the smallest encoding would not fit the reader's 65 535-byte payload array (decompression.cpp:116).
+// job.format selects the wrapper around the same DEFLATE body: ZLIB as above, GZIP one BGZF member (18-byte header with
+// the BC extra subfield, little-endian CRC-32 and ISIZE), RAW the bare blocks. Only the zlib form has the split rule.
 //
 // Per warp:
 //   parse   32 positions per step. Every lane decides locally "match here or literal" with zlib-style lazy evaluation
@@ -296,25 +298,53 @@ ZWZ_DEV_NOINLINE uint32_t enc_adler_global(const uint8_t *p, uint32_t n) {
     return (b << 16) | a;
 }
 
-// one complete zlib stream with a single stored block; returns its size
-ZWZ_DEV_NOINLINE uint32_t enc_stored_stream(uint8_t *out, const uint8_t *src, uint32_t n, uint32_t adler) {
+// wrapper bytes in front of the DEFLATE body, and in front plus behind it
+ZWZ_DEV uint32_t enc_head_bytes(uint32_t format) { return format == ZWZ_FORMAT_GZIP ? 18u : (format == ZWZ_FORMAT_ZLIB ? 2u : 0u); }
+ZWZ_DEV uint32_t enc_wrap_bytes(uint32_t format) { return format == ZWZ_FORMAT_GZIP ? 26u : (format == ZWZ_FORMAT_ZLIB ? 6u : 0u); }
+
+// BSIZE of a BGZF member header (bytes 16-17): the member's length minus 1
+ZWZ_DEV void enc_bgzf_bsize(uint8_t *out, uint32_t member_bytes) {
+    out[16] = (uint8_t) (member_bytes - 1u);
+    out[17] = (uint8_t) ((member_bytes - 1u) >> 8);
+}
+
+// one complete stream in `format` with a single stored block (check = Adler-32 for zlib, CRC-32 for gzip); returns its size
+ZWZ_DEV_NOINLINE uint32_t enc_stored_stream(uint8_t *out, const uint8_t *src, uint32_t n, uint32_t check, uint32_t format) {
     const unsigned lane = lane_id();
+    const uint32_t h = enc_head_bytes(format);
     if (lane == 0) {
-        out[0] = 0x78;
-        out[1] = 0x9c;
-        out[2] = 0x01;
-        out[3] = (uint8_t) n;
-        out[4] = (uint8_t) (n >> 8);
-        out[5] = (uint8_t) ~n;
-        out[6] = (uint8_t) (~n >> 8);
-        out[7 + n] = (uint8_t) (adler >> 24);
-        out[8 + n] = (uint8_t) (adler >> 16);
-        out[9 + n] = (uint8_t) (adler >> 8);
-        out[10 + n] = (uint8_t) adler;
+        if (format == ZWZ_FORMAT_ZLIB) {
+            out[0] = 0x78;
+            out[1] = 0x9c;
+        } else if (format == ZWZ_FORMAT_GZIP) {
+            uint32_t *w = (uint32_t *) out; // the slot start: 4-byte aligned
+            w[0] = 0x04088b1fu;             // 1f 8b 08 04 | MTIME 0 | XFL 0, OS ff | XLEN 6 | 'B' 'C' 2 0
+            w[1] = 0u;
+            w[2] = 0x0006ff00u;
+            w[3] = 0x00024342u;
+            enc_bgzf_bsize(out, n + 31u);
+        }
+        out[h] = 0x01;
+        out[h + 1u] = (uint8_t) n;
+        out[h + 2u] = (uint8_t) (n >> 8);
+        out[h + 3u] = (uint8_t) ~n;
+        out[h + 4u] = (uint8_t) (~n >> 8);
+        uint8_t *t = out + h + 5u + n;
+        if (format == ZWZ_FORMAT_ZLIB) {
+            t[0] = (uint8_t) (check >> 24);
+            t[1] = (uint8_t) (check >> 16);
+            t[2] = (uint8_t) (check >> 8);
+            t[3] = (uint8_t) check;
+        } else if (format == ZWZ_FORMAT_GZIP) {
+            for (int i = 0; i < 4; ++i) {
+                t[i] = (uint8_t) (check >> (8 * i));
+                t[4 + i] = (uint8_t) (n >> (8 * i));
+            }
+        }
     }
     __syncwarp();
-    inf_copy_plain(out + 7u, src, n);
-    return n + 11u;
+    inf_copy_plain(out + h + 5u, src, n);
+    return n + 5u + enc_wrap_bytes(format);
 }
 
 // histogram of the tokens [t0, t1) into freq[0..320) (literal/length at 0, distance at 288); returns their extra bits
@@ -557,6 +587,43 @@ ZWZ_DEV_NOINLINE void enc_emit_block(BitSink *kp, const uint32_t *m, uint32_t t0
     *kp = k;
 }
 
+// The wrapper around the Huffman-coded body (out of line: the format costs the encoder's main loop no registers).
+// Header: zlib 78 9C; gzip the 18-byte BGZF header with BSIZE left 0 (set by enc_wrap_tail); raw none.
+ZWZ_DEV_NOINLINE void enc_wrap_head(BitSink *kp, uint32_t format) {
+    EncWarpSmem &S = enc_smem();
+    const unsigned lane = lane_id();
+    BitSink k = *kp;
+    if (format == ZWZ_FORMAT_ZLIB) {
+        sink_put(S, k, lane == 0 ? 0x9c78ull : 0ull, lane == 0 ? 16u : 0u); // RFC 1950 header 78 9C
+    } else if (format == ZWZ_FORMAT_GZIP) {
+        // 1f 8b 08 04 | MTIME 0 | XFL 0, OS ff | XLEN 6 | 'B' 'C' 2 0 | BSIZE
+        const uint32_t w = lane == 0 ? 0x04088b1fu : (lane == 2u ? 0x0006ff00u : (lane == 3u ? 0x00024342u : 0u));
+        sink_put(S, k, w, lane < 4u ? 32u : (lane == 4u ? 16u : 0u));
+    }
+    *kp = k;
+}
+// Trailer: pad to a byte boundary, then Adler-32 big-endian (zlib) or CRC-32 and ISIZE little-endian (gzip). A gzip member's
+// length is known here: BSIZE goes into its header (whose words the sink has written by now: a member has >= 28 bytes).
+ZWZ_DEV_NOINLINE void enc_wrap_tail(BitSink *kp, uint32_t format, uint32_t check, uint32_t n) {
+    EncWarpSmem &S = enc_smem();
+    const unsigned lane = lane_id();
+    BitSink k = *kp;
+    const uint32_t padbits = (8u - ((k.nwords * 32u + k.fill) & 7u)) & 7u;
+    const uint32_t be = ((check & 0xffu) << 24) | ((check & 0xff00u) << 8) | ((check >> 8) & 0xff00u) | (check >> 24);
+    uint64_t v = 0;
+    uint32_t nb = lane == 0 ? padbits : 0u;
+    if (lane == 1u && format != ZWZ_FORMAT_RAW) {
+        v = format == ZWZ_FORMAT_ZLIB ? be : check;
+        nb = 32u;
+    } else if (lane == 2u && format == ZWZ_FORMAT_GZIP) {
+        v = n;
+        nb = 32u;
+    }
+    sink_put(S, k, v, nb);
+    if (format == ZWZ_FORMAT_GZIP && lane == 0) enc_bgzf_bsize((uint8_t *) k.outw, k.nwords * 4u + (k.fill >> 3));
+    *kp = k;
+}
+
 #define ZWZ_DE_STORED_MIN 512u // literal tokens in a row before a stored region is considered
 
 // Stored-region candidates come for free from the match kernel's tile flags: a 1 024-byte stretch with matches in at most
@@ -729,8 +796,8 @@ ZWZ_DEV void enc_chunk(EncWarpSmem &S, const DeflateJob &job, uint32_t c) {
         uint32_t nu;
         const float hb = enc_entropy_bits(0u, &nu);
         const float bound_bytes = hb * 0.125f + 7.f + (float) (nu >> 2);
-        if (bound_bytes * 0.9995f >= (float) (n + 11u) - (float) (n >> 8) && n + 11u <= ZWZ_CHUNK) {
-            uint32_t l0 = enc_stored_stream(out, src, n, job.adler[c]);
+        if (bound_bytes * 0.9995f >= (float) (n + 11u) - (float) (n >> 8) && (job.format != ZWZ_FORMAT_ZLIB || n + 11u <= ZWZ_CHUNK)) {
+            uint32_t l0 = enc_stored_stream(out, src, n, job.adler[c], job.format);
             if (lane == 0) {
                 job.res[4u * c + 0u] = l0;
                 job.res[4u * c + 1u] = 0u;
@@ -851,7 +918,10 @@ ZWZ_DEV void enc_chunk(EncWarpSmem &S, const DeflateJob &job, uint32_t c) {
     // one Huffman symbol per byte to decode — for our inflate and for the reference's zlib alike — and buys nothing.
     // First an exact-safe shortcut: no prefix code beats the empirical entropy, so if even the entropy bound cannot save
     // n/256 bytes the three Huffman constructions below are skipped altogether.
-    const uint32_t sto_bytes = n + 11u;
+    // The estimates are compared with the zlib-wrapped stored size in every format, so that the choice (and the body) does not
+    // depend on the wrapper; the 65 535-byte record limit applies to zlib streams only.
+    const uint32_t sto_bytes = n + 5u + enc_wrap_bytes(job.format);
+    const uint32_t zsto_bytes = n + 11u;
     const uint32_t sto_slack = n >> 8;
     bool force_stored = false;
     {
@@ -877,10 +947,11 @@ ZWZ_DEV void enc_chunk(EncWarpSmem &S, const DeflateJob &job, uint32_t c) {
         // + zlib wrapper and block header, + ~2 bits per used symbol for a dynamic header (a small random sample sits ~23
         // bytes under 8 bits/byte of empirical entropy; its code-length header costs several times that)
         float bound_bytes = (hl_bits + (float) extra_bits) * 0.125f + 7.f + (float) (nused >> 2);
-        force_stored = bound_bytes * 0.9995f >= (float) sto_bytes - (float) sto_slack && sto_bytes <= ZWZ_CHUNK && n >= 512u;
+        force_stored = bound_bytes * 0.9995f >= (float) zsto_bytes - (float) sto_slack && (job.format != ZWZ_FORMAT_ZLIB || zsto_bytes <= ZWZ_CHUNK) &&
+                       n >= 512u;
     }
     if (force_stored) {
-        uint32_t l0 = enc_stored_stream(out, src, n, job.adler[c]);
+        uint32_t l0 = enc_stored_stream(out, src, n, job.adler[c], job.format);
         if (lane == 0) {
             job.res[4u * c + 0u] = l0;
             job.res[4u * c + 1u] = 0u;
@@ -902,7 +973,7 @@ ZWZ_DEV void enc_chunk(EncWarpSmem &S, const DeflateJob &job, uint32_t c) {
     const uint32_t cap_words = ((n + ZWZ_DEFLATE_MARGIN + 15u) & ~15u) >> 2; // zwz_deflate_bound(n) / 4
     BitSink k;
     sink_init(S, k, (uint32_t *) out, cap_words);
-    sink_put(S, k, lane == 0 ? 0x9c78ull : 0ull, lane == 0 ? 16u : 0u); // RFC 1950 header 78 9C
+    enc_wrap_head(&k, job.format);
     __syncwarp();
     const uint32_t nreg = enc_find_stored_regions(m, n, ntok);
     if (nreg == 0u) {
@@ -917,28 +988,23 @@ ZWZ_DEV void enc_chunk(EncWarpSmem &S, const DeflateJob &job, uint32_t c) {
         }
         if (t < ntok) enc_emit_range(&k, m, t, ntok, 0, true, false);
     }
-    // pad to a byte boundary, Adler-32 big-endian
     const uint32_t adler = job.adler[c];
-    {
-        uint32_t padbits = (8u - ((k.nwords * 32u + k.fill) & 7u)) & 7u;
-        uint32_t be = ((adler & 0xffu) << 24) | ((adler & 0xff00u) << 8) | ((adler >> 8) & 0xff00u) | (adler >> 24);
-        sink_put(S, k, lane == 1u ? (uint64_t) be : 0ull, lane == 0 ? padbits : (lane == 1u ? 32u : 0u));
-    }
+    enc_wrap_tail(&k, job.format, adler, n);
     const uint32_t huff_bytes = sink_finish(S, k);
     __syncwarp();
 
     uint32_t len0 = huff_bytes, len1 = 0, raw0 = n, btype = 2u;
-    if (sto_bytes <= huff_bytes + sto_slack || huff_bytes > ZWZ_CHUNK || huff_bytes > cap_words * 4u) { // see the policy above
+    if (sto_bytes <= huff_bytes + sto_slack || (job.format == ZWZ_FORMAT_ZLIB && huff_bytes > ZWZ_CHUNK) || huff_bytes > cap_words * 4u) { // see the policy above
         btype = 0u;
-        if (sto_bytes > ZWZ_CHUNK) {
+        if (job.format == ZWZ_FORMAT_ZLIB && sto_bytes > ZWZ_CHUNK) {
             // split rule: two stored streams over the halves (each needs its own Adler-32)
             raw0 = 32768u;
             uint32_t a0 = enc_adler_global(src, raw0);
             uint32_t a1 = enc_adler_global(src + raw0, n - raw0);
-            len0 = enc_stored_stream(out, src, raw0, a0);
-            len1 = enc_stored_stream(out + len0, src + raw0, n - raw0, a1);
+            len0 = enc_stored_stream(out, src, raw0, a0, ZWZ_FORMAT_ZLIB);
+            len1 = enc_stored_stream(out + len0, src + raw0, n - raw0, a1, ZWZ_FORMAT_ZLIB);
         } else {
-            len0 = enc_stored_stream(out, src, n, adler);
+            len0 = enc_stored_stream(out, src, n, adler, job.format);
         }
     }
     if (lane == 0) {

@@ -1,4 +1,6 @@
-// inflate.cuh — batched zlib-wrapped DEFLATE decoder, one warp per stream.
+// inflate.cuh — batched DEFLATE decoder, one warp per stream: zlib-wrapped (the .zwz records), gzip members or raw DEFLATE,
+// chosen by the format field of the flags (ZWZ_INFLATE_FORMAT). The wrapper is parsed and checked here; the block decoders
+// below it are the same for all three.
 //
 // Replaces decompression.cpp:11-37 (inflateInit / inflate(Z_NO_FLUSH) loop / inflateEnd, return codes ignored).
 // Output contract = the bytes zlib 1.3 would have written for the same input (see oracle/zwz_oracle.c for the rules):
@@ -20,6 +22,7 @@
 // Algorithmic bytes per stream: N_comp read + N_raw written (SURVEY.md §8(d)).
 #pragma once
 #include "zwz_common.cuh"
+#include "crc32.cuh"
 
 namespace zwz {
 
@@ -248,6 +251,56 @@ ZWZ_DEV void infb_seek_bits(InfBits &b, uint64_t bit_pos) {
 #include "inflate_fast.cuh"
 namespace zwz {
 
+// CRC-32 of p[0, n) by the calling warp. The slice table goes into the warp's literal/length decode table, which is dead
+// before the first block header and after the last block: the shared-memory layout stays that of the zlib path.
+ZWZ_DEV_NOINLINE uint32_t inf_crc32(const uint8_t *p, uint32_t n) {
+    ZWZ_DYN_SMEM(inf_raw);
+    uint32_t *tab = ((InflateWarpSmem *) inf_raw)[warp_id()].lit;
+    __syncwarp();
+    crc32_load_table(tab, lane_id(), 32u);
+    __syncwarp();
+    return crc32_warp(p, n, tab);
+}
+
+// RFC 1952 member header as zlib 1.3 reads it with windowBits 31 (inflate.c HEAD, FLAGS .. HCRC): the header length << 2 with
+// ZWZ_STREAM_END, or the status zlib ends with (a header cut short is TRUNCATED, a wrong ID or CM, reserved FLG bits or a header
+// CRC mismatch BAD). Byte-serial and warp-uniform; the zero-terminated FNAME / FCOMMENT are scanned 32 bytes a step.
+ZWZ_DEV_NOINLINE uint32_t inf_gzip_header(const uint8_t *comp, uint32_t comp_len) {
+    const unsigned lane = lane_id();
+    if (comp_len < 2u) return ZWZ_STREAM_TRUNCATED;
+    if (comp[0] != 0x1fu || comp[1] != 0x8bu) return ZWZ_STREAM_BAD;
+    if (comp_len < 4u) return ZWZ_STREAM_TRUNCATED;
+    const uint32_t flg = comp[3];
+    if (comp[2] != 8u || (flg & 0xe0u)) return ZWZ_STREAM_BAD;
+    uint32_t p = 10u; // ID1 ID2 CM FLG MTIME(4) XFL OS
+    if (comp_len < p) return ZWZ_STREAM_TRUNCATED;
+    if (flg & 0x04u) { // FEXTRA: XLEN, then XLEN bytes
+        if (comp_len < p + 2u) return ZWZ_STREAM_TRUNCATED;
+        p += 2u + ((uint32_t) comp[p] | ((uint32_t) comp[p + 1u] << 8));
+        if (comp_len < p) return ZWZ_STREAM_TRUNCATED;
+    }
+    for (uint32_t f = 0x08u; f <= 0x10u; f <<= 1) { // FNAME, FCOMMENT
+        if (!(flg & f)) continue;
+        for (;;) {
+            if (p >= comp_len) return ZWZ_STREAM_TRUNCATED;
+            const uint32_t q = p + lane;
+            const unsigned z = __ballot_sync(ZWZ_FULL, q < comp_len && comp[q] == 0u);
+            if (z) {
+                p += (uint32_t) __ffs((int) z);
+                break;
+            }
+            p += 32u;
+        }
+    }
+    if (flg & 0x02u) { // FHCRC: low 16 bits of the CRC-32 of everything before it
+        if (comp_len < p + 2u) return ZWZ_STREAM_TRUNCATED;
+        const uint32_t want = (uint32_t) comp[p] | ((uint32_t) comp[p + 1u] << 8);
+        if ((inf_crc32(comp, p) & 0xffffu) != want) return ZWZ_STREAM_BAD;
+        p += 2u;
+    }
+    return (p << 2) | ZWZ_STREAM_END;
+}
+
 // One warp decodes stream `sid`.
 ZWZ_DEV void inflate_stream(InflateWarpSmem &S, const uint8_t *__restrict__ comp, uint32_t comp_len, uint8_t *out, uint32_t cap,
                             uint32_t flags, uint32_t &raw_len_out, uint32_t &status_out) {
@@ -266,6 +319,7 @@ ZWZ_DEV void inflate_stream(InflateWarpSmem &S, const uint8_t *__restrict__ comp
     uint32_t mybyte = 0;
     uint32_t status = ZWZ_STREAM_END;
     bool overflow = false;
+    const uint32_t format = (flags >> 8) & 0xffu;
 
 #define INF_FLUSH_LITS()                                                         \
     do {                                                                         \
@@ -278,13 +332,18 @@ ZWZ_DEV void inflate_stream(InflateWarpSmem &S, const uint8_t *__restrict__ comp
 #define INF_FAST() (B.widx <= B.nfull)
 #define INF_NEED(nbits_) (INF_FAST() || infb_used(B) + (uint64_t) (nbits_) <= total_bits)
 
-    // ---- RFC 1950 header (inflate.c HEAD) ----
-    infb_refill(B);
-    if (!INF_NEED(16)) {
-        status = ZWZ_STREAM_TRUNCATED;
-        goto done;
-    }
-    {
+    if (format == ZWZ_FORMAT_GZIP) {
+        const uint32_t h = inf_gzip_header(comp, comp_len);
+        status = h & 3u;
+        if (status != ZWZ_STREAM_END) goto done;
+        infb_seek(B, h >> 2);
+    } else if (format == ZWZ_FORMAT_ZLIB) {
+        // ---- RFC 1950 header (inflate.c HEAD) ----
+        infb_refill(B);
+        if (!INF_NEED(16)) {
+            status = ZWZ_STREAM_TRUNCATED;
+            goto done;
+        }
         uint32_t cmf = (uint32_t) B.hold & 0xffu, flg = ((uint32_t) B.hold >> 8) & 0xffu;
         if (((cmf << 8) + flg) % 31u != 0u || (cmf & 15u) != 8u || (cmf >> 4) + 8u > 15u || (flg & 0x20u)) {
             status = ZWZ_STREAM_BAD;
@@ -598,8 +657,8 @@ ZWZ_DEV void inflate_stream(InflateWarpSmem &S, const uint8_t *__restrict__ comp
         }
         if (last) break;
     }
-    // ---- RFC 1950 trailer (inflate.c CHECK) ----
-    {
+    // ---- RFC 1950 trailer (inflate.c CHECK), RFC 1952 trailer (CHECK, LENGTH); raw streams have none ----
+    if (format != ZWZ_FORMAT_RAW) {
         INF_FLUSH_LITS();
         __syncwarp();
         uint64_t used = infb_used(B);
@@ -608,10 +667,23 @@ ZWZ_DEV void inflate_stream(InflateWarpSmem &S, const uint8_t *__restrict__ comp
             status = ZWZ_STREAM_TRUNCATED;
             goto done;
         }
-        if (!(flags & 1u) && !overflow) {
-            uint32_t want = ((uint32_t) comp[bpos] << 24) | ((uint32_t) comp[bpos + 1] << 16) | ((uint32_t) comp[bpos + 2] << 8) | comp[bpos + 3];
-            const uint32_t have = inf_adler32(out, pos); // a = 1 + sum(byte), b = n + sum((n - j) * byte_j)  (mod 65521)
-            if (have != want) status = ZWZ_STREAM_BAD;
+        if (format == ZWZ_FORMAT_ZLIB) {
+            if (!(flags & 1u) && !overflow) {
+                uint32_t want = ((uint32_t) comp[bpos] << 24) | ((uint32_t) comp[bpos + 1] << 16) | ((uint32_t) comp[bpos + 2] << 8) | comp[bpos + 3];
+                const uint32_t have = inf_adler32(out, pos); // a = 1 + sum(byte), b = n + sum((n - j) * byte_j)  (mod 65521)
+                if (have != want) status = ZWZ_STREAM_BAD;
+            }
+        } else {
+            const uint32_t want = (uint32_t) comp[bpos] | ((uint32_t) comp[bpos + 1] << 8) | ((uint32_t) comp[bpos + 2] << 16) | ((uint32_t) comp[bpos + 3] << 24);
+            if (!(flags & 1u) && !overflow && inf_crc32(out, pos) != want) {
+                status = ZWZ_STREAM_BAD;
+            } else if ((uint64_t) bpos + 8u > comp_len) {
+                status = ZWZ_STREAM_TRUNCATED;
+            } else {
+                const uint32_t isize = (uint32_t) comp[bpos + 4] | ((uint32_t) comp[bpos + 5] << 8) | ((uint32_t) comp[bpos + 6] << 16) |
+                                       ((uint32_t) comp[bpos + 7] << 24);
+                if (isize != pos) status = ZWZ_STREAM_BAD; // pos counts past the capacity too
+            }
         }
     }
 done:

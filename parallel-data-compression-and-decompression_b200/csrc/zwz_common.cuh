@@ -49,7 +49,8 @@ struct DeflateJob {
     const uint32_t *raw_len;   // [n]   <= 65535
     const uint64_t *scr_off;   // [n]   offset (in uint32 units) of this chunk's match/token scratch
     uint32_t *scratch;         // 4 bytes per raw byte (+ pad)
-    uint32_t *adler;           // [n]   written by the match kernel, read by the encoder
+    uint32_t *adler;           // [n]   check value: Adler-32 written by the match kernel, in GZIP format overwritten by the CRC-32
+                               //       of crc32_kernel; read by the encoder
     uint32_t *nmatch;          // [n]   positions that found a match (match kernel -> encoder: incompressibility shortcut)
     uint8_t *out;              // output slots
     const uint64_t *out_off;   // [n]   multiple of 4, capacity >= zwz_deflate_bound(len)
@@ -58,6 +59,7 @@ struct DeflateJob {
     uint32_t depth;            // hash-chain candidates examined per position
     uint32_t nice;             // stop searching at this length
     uint32_t *work_counter;    // persistent-CTA work queue
+    uint32_t format;           // ZWZ_FORMAT_*: the wrapper deflate_encode_kernel puts around the body
 };
 
 // ---- unaligned little-endian loads built from aligned 32-bit words -------------------------------------------------

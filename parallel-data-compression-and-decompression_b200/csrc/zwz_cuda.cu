@@ -8,6 +8,7 @@
 
 #include "zwz_common.cuh"
 #include "md5.cuh"
+#include "crc32.cuh"
 #include "inflate.cuh"
 #include "inflate_lanes.cuh"
 #include "deflate_match.cuh"
@@ -285,6 +286,7 @@ int zwz_init(int device, zwz_ctx **out) {
     zwz_rt::preload_kernel((const void *) zwz::pack_streams_kernel);
     zwz_rt::preload_kernel((const void *) zwz::gather_records_kernel);
     zwz_rt::preload_kernel((const void *) zwz::adler32_kernel);
+    zwz_rt::preload_kernel((const void *) zwz::crc32_kernel);
     if (const char *e = getenv("ZWZ_ARENA_SYNC")) ctx->arena_async = !(*e && *e != '0');
     if (const char *e = getenv("ZWZ_TRACE")) ctx->trace = *e && *e != '0';
     if (const char *e = getenv("ZWZ_INFLATE_MODE")) ctx->inflate_mode = !strcmp(e, "warp") ? 1 : (!strcmp(e, "lanes") ? 2 : (!strcmp(e, "careful") ? 3 : 0));
@@ -413,7 +415,13 @@ int zwz_sync(zwz_ctx *ctx) {
 // ======================================================================================================================
 int zwz_deflate_batch_device(zwz_ctx *ctx, const uint8_t *d_raw, const uint64_t *off, const uint32_t *len, uint32_t n, uint8_t *d_out,
                              const uint64_t *out_off, zwz_deflate_result *res, int level, void *stream_v) {
+    return zwz_deflate_batch_device_ex(ctx, d_raw, off, len, n, d_out, out_off, res, level, ZWZ_FORMAT_ZLIB, stream_v);
+}
+
+int zwz_deflate_batch_device_ex(zwz_ctx *ctx, const uint8_t *d_raw, const uint64_t *off, const uint32_t *len, uint32_t n, uint8_t *d_out,
+                                const uint64_t *out_off, zwz_deflate_result *res, int level, int format, void *stream_v) {
     if (!ctx) return ZWZ_E_ARG;
+    if (format < ZWZ_FORMAT_ZLIB || format > ZWZ_FORMAT_RAW) return fail(ctx, ZWZ_E_ARG, "unknown stream format");
     if (n == 0) return ZWZ_OK;
     if (!off || !len || !out_off || !res || !d_out) return fail(ctx, ZWZ_E_ARG, "null argument");
     zwz_rt::set_device(ctx->device);
@@ -421,6 +429,7 @@ int zwz_deflate_batch_device(zwz_ctx *ctx, const uint8_t *d_raw, const uint64_t 
     uint64_t total_raw = 0;
     for (uint32_t i = 0; i < n; ++i) {
         if (len[i] > ZWZ_CHUNK_SIZE) return fail(ctx, ZWZ_E_ARG, "chunk longer than 65535 bytes");
+        if (format == ZWZ_FORMAT_GZIP && len[i] > ZWZ_BGZF_BLOCK) return fail(ctx, ZWZ_E_ARG, "gzip chunk longer than ZWZ_BGZF_BLOCK bytes");
         if (out_off[i] & 3u) return fail(ctx, ZWZ_E_ARG, "out_off must be a multiple of 4");
         total_raw += len[i];
     }
@@ -514,6 +523,7 @@ int zwz_deflate_batch_device(zwz_ctx *ctx, const uint8_t *d_raw, const uint64_t 
         job.depth = lp.depth;
         job.nice = lp.nice;
         job.work_counter = nullptr;
+        job.format = (uint32_t) format;
         const uint32_t *d_order = (const uint32_t *) ((const uint64_t *) dm + 3 * (size_t) n) + n + b;
         uint32_t *d_counters = (uint32_t *) ctx->counter.p + s * 8; // [0..3] match classes, [4] encoder
         for (int cls = 0; cls < 4; ++cls) {
@@ -538,6 +548,13 @@ int zwz_deflate_batch_device(zwz_ctx *ctx, const uint8_t *d_raw, const uint64_t 
         }
         if ((rc = check_launch(ctx, "lz_match_kernel"))) return rc;
         ctx->launches--; // check_launch counted one more
+        if (format == ZWZ_FORMAT_GZIP) { // the CRC-32 replaces the Adler-32 the match kernel left in job.adler
+            {
+                ProfSpan ps(ctx, ZWZ_PROF_ADLER, st);
+                ZWZ_LAUNCH(zwz::crc32_kernel, (job.n + 7) / 8, 256, 0, st, d_raw, job.raw_off, job.raw_len, job.adler, job.n);
+            }
+            if ((rc = check_launch(ctx, "crc32_kernel"))) return rc;
+        }
         uint32_t grid2 = std::min<uint32_t>((job.n + ZWZ_DE_WARPS - 1) / ZWZ_DE_WARPS, (uint32_t) ctx->sm_count * 8u);
         {
             ProfSpan ps(ctx, ZWZ_PROF_ENCODE, st);
@@ -560,7 +577,7 @@ static int slot_acquire(zwz_ctx *ctx, zwz::DigestSlot **out);
 static int slot_queue_md5(zwz_ctx *ctx, zwz::DigestSlot &sl, const uint64_t *off, const uint64_t *len, uint32_t n, uint8_t *digest, uint64_t *ticket);
 
 static int deflate_host_impl(zwz_ctx *ctx, const uint8_t *raw, const uint64_t *off, const uint32_t *len, uint32_t n, uint8_t *out, uint64_t out_cap,
-                             uint64_t *packed_off, zwz_deflate_result *res, int level, const uint64_t *md5_off, const uint64_t *md5_len,
+                             uint64_t *packed_off, zwz_deflate_result *res, int level, int format, const uint64_t *md5_off, const uint64_t *md5_len,
                              uint32_t md5_n, uint8_t *digest, uint64_t *ticket) {
     if (!ctx) return ZWZ_E_ARG;
     if (ticket) *ticket = 0;
@@ -605,8 +622,8 @@ static int deflate_host_impl(zwz_ctx *ctx, const uint8_t *raw, const uint64_t *o
             if (!ok) s->digest_dst = nullptr;
         }
     } disarm{sl};
-    if ((rc = zwz_deflate_batch_device(ctx, (const uint8_t *) sl->data.p, roff.data(), len, n, (uint8_t *) ctx->bulk_out.p, slot.data(), res,
-                                       level, nullptr)))
+    if ((rc = zwz_deflate_batch_device_ex(ctx, (const uint8_t *) sl->data.p, roff.data(), len, n, (uint8_t *) ctx->bulk_out.p, slot.data(), res,
+                                          level, format, nullptr)))
         return rc;
     tr.mark("md5+deflate");
     for (uint32_t i = 0; i < n; ++i) packed_off[i + 1] = packed_off[i] + res[i].len0 + res[i].len1;
@@ -671,7 +688,12 @@ int zwz_pack_streams_device(zwz_ctx *ctx, const uint8_t *d_slots, const uint64_t
 
 int zwz_deflate_batch(zwz_ctx *ctx, const uint8_t *raw, const uint64_t *off, const uint32_t *len, uint32_t n, uint8_t *out, uint64_t out_cap,
                       uint64_t *packed_off, zwz_deflate_result *res, int level) {
-    return deflate_host_impl(ctx, raw, off, len, n, out, out_cap, packed_off, res, level, nullptr, nullptr, 0, nullptr, nullptr);
+    return deflate_host_impl(ctx, raw, off, len, n, out, out_cap, packed_off, res, level, ZWZ_FORMAT_ZLIB, nullptr, nullptr, 0, nullptr, nullptr);
+}
+
+int zwz_deflate_batch_ex(zwz_ctx *ctx, const uint8_t *raw, const uint64_t *off, const uint32_t *len, uint32_t n, uint8_t *out, uint64_t out_cap,
+                         uint64_t *packed_off, zwz_deflate_result *res, int level, int format) {
+    return deflate_host_impl(ctx, raw, off, len, n, out, out_cap, packed_off, res, level, format, nullptr, nullptr, 0, nullptr, nullptr);
 }
 
 uint64_t zwz_count_chunks(const uint64_t *file_off, uint32_t nf) {
@@ -700,8 +722,8 @@ static int compress_files_impl(zwz_ctx *ctx, const uint8_t *data, const uint64_t
             if (left < ZWZ_CHUNK_SIZE) break;
         }
     }
-    return deflate_host_impl(ctx, data, coff.data(), clen.data(), (uint32_t) nc, out, out_cap, packed_off, res, level, file_off, flen.data(),
-                             digest ? nf : 0, digest, ticket);
+    return deflate_host_impl(ctx, data, coff.data(), clen.data(), (uint32_t) nc, out, out_cap, packed_off, res, level, ZWZ_FORMAT_ZLIB, file_off,
+                             flen.data(), digest ? nf : 0, digest, ticket);
 }
 
 int zwz_compress_files(zwz_ctx *ctx, const uint8_t *data, const uint64_t *file_off, uint32_t nf, int level, uint8_t *out, uint64_t out_cap,
@@ -732,6 +754,9 @@ int zwz_inflate_batch_device(zwz_ctx *ctx, const uint8_t *d_comp, const uint64_t
     if (!ctx) return ZWZ_E_ARG;
     if (n == 0) return ZWZ_OK;
     if (!off || !len || !raw_off || !raw_len || !status) return fail(ctx, ZWZ_E_ARG, "null argument");
+    const uint32_t format = (flags >> 8) & 0xffu;
+    if (format > ZWZ_FORMAT_RAW) return fail(ctx, ZWZ_E_ARG, "unknown stream format");
+    if (format != ZWZ_FORMAT_ZLIB && ctx->inflate_mode == 2) return fail(ctx, ZWZ_E_ARG, "the one-lane-per-stream decoder reads zlib streams only");
     zwz_rt::set_device(ctx->device);
     zwz_stream_t st = stream_v ? (zwz_stream_t) stream_v : ctx->stream;
     // Mapping: one warp per stream (inflate.cuh) is the product path. One lane per stream (inflate_lanes.cuh,
@@ -817,12 +842,16 @@ int zwz_inflate_batch(zwz_ctx *ctx, const uint8_t *comp, const uint64_t *off, co
     return ZWZ_OK;
 }
 
+static int gather_files(zwz_ctx *ctx, const uint64_t *slot, const uint64_t *dst, const uint32_t *len, uint32_t n, uint64_t acc, uint8_t *files_out,
+                        uint32_t nf, const uint64_t *file_off_out, uint8_t *digest, uint64_t *ticket, Trace &tr);
+
 static int decompress_records_impl(zwz_ctx *ctx, const uint8_t *comp, const uint64_t *off, const uint32_t *len, const uint32_t *rec_cap,
                                    const uint32_t *rec_file, uint32_t n, uint32_t nf, uint8_t *files_out, uint64_t out_cap, uint64_t *file_off_out,
                                    uint32_t *raw_len, uint32_t *status, uint8_t *digest, uint32_t flags, uint64_t *ticket) {
     if (!ctx) return ZWZ_E_ARG;
     if (ticket) *ticket = 0;
     if (!file_off_out) return fail(ctx, ZWZ_E_ARG, "null argument");
+    if ((flags >> 8) & 0xffu) return fail(ctx, ZWZ_E_ARG, "records are zlib streams: no format may be given");
     for (uint32_t f = 0; f <= nf; ++f) file_off_out[f] = 0;
     if (n == 0) {
         if (digest && nf) { // every file is empty
@@ -884,6 +913,15 @@ static int decompress_records_impl(zwz_ctx *ctx, const uint8_t *comp, const uint
     }
     while (f < nf) file_off_out[++f] = acc;
     if (acc > out_cap) return fail(ctx, ZWZ_E_CAPACITY, "output buffer too small");
+    return gather_files(ctx, slot.data(), dst.data(), raw_len, n, acc, files_out, nf, file_off_out, digest, ticket, tr);
+}
+
+// Concatenates the n inflated records in ctx->bulk_out (record i: len[i] bytes at slot[i], 16-byte aligned) into the output files
+// (record i at dst[i]; acc bytes in all), downloads them into files_out and, when digest != NULL, queues the MD5 of the nf files
+// (file_off_out) beside the download.
+static int gather_files(zwz_ctx *ctx, const uint64_t *slot, const uint64_t *dst, const uint32_t *len, uint32_t n, uint64_t acc, uint8_t *files_out,
+                        uint32_t nf, const uint64_t *file_off_out, uint8_t *digest, uint64_t *ticket, Trace &tr) {
+    int rc;
     const size_t m_dst = (size_t) n * 8, m_len = 2 * (size_t) n * 8, meta_bytes = m_len + (size_t) n * 4;
     // the concatenated files live in a digest slot: their MD5 runs on the second stream and may outlive this call
     zwz::DigestSlot *sl = nullptr;
@@ -895,9 +933,9 @@ static int decompress_records_impl(zwz_ctx *ctx, const uint8_t *comp, const uint
     if ((rc = reserve(ctx, ctx->pin_aux, meta_bytes, true))) return rc;
     tr.mark("reserve2");
     uint8_t *hp = (uint8_t *) ctx->pin_aux.p;
-    memcpy(hp, slot.data(), (size_t) n * 8);
-    memcpy(hp + m_dst, dst.data(), (size_t) n * 8);
-    memcpy(hp + m_len, raw_len, (size_t) n * 4);
+    memcpy(hp, slot, (size_t) n * 8);
+    memcpy(hp + m_dst, dst, (size_t) n * 8);
+    memcpy(hp + m_len, len, (size_t) n * 4);
     uint8_t *dmeta = (uint8_t *) ctx->packed.p;
     uint8_t *d_files = (uint8_t *) sl->data.p;
     if (zwz_rt::memcpy_h2d(dmeta, hp, meta_bytes, ctx->stream)) return fail(ctx, ZWZ_E_CUDA, "descriptor upload failed");
@@ -942,7 +980,179 @@ int zwz_decompress_records_async(zwz_ctx *ctx, const uint8_t *comp, const uint64
 }
 
 // ======================================================================================================================
-// MD5 / Adler-32
+// whole files <-> BGZF .gz files
+// ======================================================================================================================
+uint64_t zwz_gzip_bound(const uint64_t *file_off, uint32_t nf) {
+    uint64_t b = 0;
+    for (uint32_t i = 0; file_off && i < nf; ++i) {
+        const uint64_t S = file_off[i + 1] - file_off[i], r = S % ZWZ_BGZF_BLOCK;
+        b += (S / ZWZ_BGZF_BLOCK) * zwz_deflate_bound(ZWZ_BGZF_BLOCK) + (r ? zwz_deflate_bound((uint32_t) r) : 0) + zwz_deflate_bound(0);
+    }
+    return b;
+}
+
+int zwz_gzip_files(zwz_ctx *ctx, const uint8_t *data, const uint64_t *file_off, uint32_t nf, int level, uint8_t *out, uint64_t out_cap,
+                   uint64_t *gz_off) {
+    if (!ctx) return ZWZ_E_ARG;
+    if (!file_off || !gz_off) return fail(ctx, ZWZ_E_ARG, "null argument");
+    uint64_t nc = 0;
+    for (uint32_t i = 0; i < nf; ++i) {
+        if (file_off[i + 1] < file_off[i]) return fail(ctx, ZWZ_E_ARG, "file offsets must not decrease");
+        nc += (file_off[i + 1] - file_off[i] + ZWZ_BGZF_BLOCK - 1) / ZWZ_BGZF_BLOCK + 1;
+    }
+    if (nc > 0xffffffffull) return fail(ctx, ZWZ_E_ARG, "too many chunks in one batch");
+    // every file: full ZWZ_BGZF_BLOCK chunks, the remainder, then the empty chunk whose member is the BGZF end-of-file marker
+    std::vector<uint64_t> coff((size_t) nc), poff((size_t) nc + 1), first(nf);
+    std::vector<uint32_t> clen((size_t) nc);
+    std::vector<zwz_deflate_result> res((size_t) nc);
+    size_t k = 0;
+    for (uint32_t i = 0; i < nf; ++i) {
+        first[i] = k;
+        const uint64_t S = file_off[i + 1] - file_off[i];
+        for (uint64_t o = 0; o < S; o += ZWZ_BGZF_BLOCK, ++k) {
+            coff[k] = file_off[i] + o;
+            clen[k] = (uint32_t) std::min<uint64_t>(ZWZ_BGZF_BLOCK, S - o);
+        }
+        coff[k] = file_off[i + 1];
+        clen[k++] = 0;
+    }
+    int rc = deflate_host_impl(ctx, data, coff.data(), clen.data(), (uint32_t) nc, out, out_cap, poff.data(), res.data(), level, ZWZ_FORMAT_GZIP,
+                               nullptr, nullptr, 0, nullptr, nullptr);
+    if (rc) return rc;
+    for (uint32_t i = 0; i < nf; ++i) gz_off[i] = poff[first[i]];
+    gz_off[nf] = poff[nc];
+    return ZWZ_OK;
+}
+
+struct BgzfMember {
+    uint64_t off;
+    uint32_t len, cap;
+};
+
+// Appends the BGZF members of gz[p, end) to m, each found from the BSIZE of its BC subfield; its capacity is its ISIZE trailer.
+// A member cut short by the end of the range (header included) is appended with what is there and 65 536 bytes of capacity: its
+// inflate says how it ends. Returns ZWZ_STREAM_BAD in front of a member that is not BGZF (not gzip with a BC subfield, a BSIZE
+// shorter than header + trailer, an ISIZE above the 64 KiB of a BGZF block), else ZWZ_STREAM_END.
+static uint32_t bgzf_walk(const uint8_t *gz, uint64_t p, uint64_t end, std::vector<BgzfMember> &m) {
+    while (p < end) {
+        const uint8_t *h = gz + p;
+        const uint64_t left = end - p;
+        const uint32_t xlen = left >= 12 ? (uint32_t) h[10] | ((uint32_t) h[11] << 8) : 0u;
+        if (left < 12 || left < 12u + xlen) {
+            m.push_back({p, (uint32_t) left, 65536u});
+            return ZWZ_STREAM_END;
+        }
+        if (h[0] != 0x1f || h[1] != 0x8b || h[2] != 8 || !(h[3] & 0x04)) return ZWZ_STREAM_BAD;
+        uint32_t bsize = 0;
+        bool found = false;
+        for (uint32_t x = 0; x + 4 <= xlen;) {
+            const uint8_t *f = h + 12 + x;
+            const uint32_t slen = (uint32_t) f[2] | ((uint32_t) f[3] << 8);
+            if (f[0] == 'B' && f[1] == 'C' && slen == 2 && x + 6 <= xlen) {
+                bsize = (uint32_t) f[4] | ((uint32_t) f[5] << 8);
+                found = true;
+                break;
+            }
+            x += 4 + slen;
+        }
+        const uint64_t len = (uint64_t) bsize + 1;
+        if (!found || len < 12u + xlen + 8u) return ZWZ_STREAM_BAD;
+        if (len > left) {
+            m.push_back({p, (uint32_t) left, 65536u});
+            return ZWZ_STREAM_END;
+        }
+        const uint8_t *t = h + len - 4;
+        const uint32_t isize = (uint32_t) t[0] | ((uint32_t) t[1] << 8) | ((uint32_t) t[2] << 16) | ((uint32_t) t[3] << 24);
+        if (isize > 65536u) return ZWZ_STREAM_BAD;
+        m.push_back({p, (uint32_t) len, isize});
+        p += len;
+    }
+    return ZWZ_STREAM_END;
+}
+
+uint64_t zwz_gunzip_bound(const uint8_t *gz, const uint64_t *gz_off, uint32_t nf) {
+    std::vector<BgzfMember> m;
+    for (uint32_t i = 0; gz && gz_off && i < nf; ++i)
+        if (gz_off[i + 1] > gz_off[i]) bgzf_walk(gz, gz_off[i], gz_off[i + 1], m);
+    uint64_t b = 0;
+    for (const BgzfMember &x : m) b += x.cap;
+    return b;
+}
+
+int zwz_gunzip_files(zwz_ctx *ctx, const uint8_t *gz, const uint64_t *gz_off, uint32_t nf, uint8_t *out, uint64_t out_cap, uint64_t *out_off,
+                     uint32_t *status) {
+    if (!ctx) return ZWZ_E_ARG;
+    if (!gz_off || !out_off || (nf && !status)) return fail(ctx, ZWZ_E_ARG, "null argument");
+    for (uint32_t i = 0; i <= nf; ++i) out_off[i] = 0;
+    std::vector<BgzfMember> m;
+    std::vector<size_t> first(nf + 1);
+    std::vector<uint32_t> walk(nf);
+    uint64_t bound = 0;
+    for (uint32_t i = 0; i < nf; ++i) {
+        if (gz_off[i + 1] < gz_off[i]) return fail(ctx, ZWZ_E_ARG, "file offsets must not decrease");
+        if (gz_off[i + 1] > gz_off[i] && !gz) return fail(ctx, ZWZ_E_ARG, "null argument");
+        first[i] = m.size();
+        walk[i] = bgzf_walk(gz, gz_off[i], gz_off[i + 1], m);
+    }
+    first[nf] = m.size();
+    for (const BgzfMember &x : m) bound += x.cap;
+    if (out_cap < bound) return fail(ctx, ZWZ_E_CAPACITY, "output buffer below zwz_gunzip_bound");
+    if (m.size() > 0xffffffffull) return fail(ctx, ZWZ_E_ARG, "too many members in one batch");
+    const uint32_t n = (uint32_t) m.size();
+    if (n == 0) {
+        for (uint32_t i = 0; i < nf; ++i) status[i] = walk[i];
+        return ZWZ_OK;
+    }
+    if (!out) return fail(ctx, ZWZ_E_ARG, "null argument");
+    zwz_rt::set_device(ctx->device);
+    Trace tr(ctx, "gunzip_files");
+    uint64_t lo = ~0ull, hi = 0;
+    for (const BgzfMember &x : m) {
+        lo = std::min(lo, x.off);
+        hi = std::max(hi, x.off + x.len);
+    }
+    // every member inflates into a 16-byte aligned slot of its capacity (the gather then copies with 128-bit accesses)
+    std::vector<uint64_t> coff(n), slot(n + 1), dst(n);
+    std::vector<uint32_t> mlen(n), raw_len(n), st(n), take(n);
+    slot[0] = 0;
+    for (uint32_t j = 0; j < n; ++j) {
+        coff[j] = m[j].off - lo;
+        mlen[j] = m[j].len;
+        slot[j + 1] = slot[j] + (((uint64_t) m[j].cap + 15u) & ~15ull);
+    }
+    int rc;
+    if ((rc = reserve(ctx, ctx->bulk_in, (size_t) (hi - lo) + 64, false))) return rc;
+    if ((rc = reserve(ctx, ctx->bulk_out, (size_t) slot[n] + 64, false))) return rc;
+    tr.mark("reserve");
+    if (zwz_rt::memcpy_h2d(ctx->bulk_in.p, gz + lo, (size_t) (hi - lo), ctx->stream)) return fail(ctx, ZWZ_E_CUDA, "gz upload failed");
+    tr.mark("h2d");
+    if ((rc = zwz_inflate_batch_device(ctx, (const uint8_t *) ctx->bulk_in.p, coff.data(), mlen.data(), n, (uint8_t *) ctx->bulk_out.p, slot.data(),
+                                       raw_len.data(), st.data(), ZWZ_INFLATE_FORMAT(ZWZ_FORMAT_GZIP), nullptr)))
+        return rc;
+    tr.mark("inflate");
+    // per file: its members' bytes in order, up to and including the first member that does not end cleanly
+    uint64_t acc = 0;
+    for (uint32_t i = 0; i < nf; ++i) {
+        out_off[i] = acc;
+        status[i] = ZWZ_STREAM_END;
+        for (size_t j = first[i]; j < first[i + 1]; ++j) {
+            dst[j] = acc;
+            take[j] = 0;
+            if (status[i] != ZWZ_STREAM_END) continue;
+            uint32_t s = st[j];
+            if (s == ZWZ_STREAM_OUTPUT_FULL || raw_len[j] > m[j].cap) s = ZWZ_STREAM_BAD; // more than its ISIZE
+            take[j] = std::min(raw_len[j], m[j].cap);
+            acc += take[j];
+            status[i] = s;
+        }
+        if (status[i] == ZWZ_STREAM_END) status[i] = walk[i];
+    }
+    out_off[nf] = acc;
+    return gather_files(ctx, slot.data(), dst.data(), take.data(), n, acc, out, nf, out_off, nullptr, nullptr, tr);
+}
+
+// ======================================================================================================================
+// MD5 / Adler-32 / CRC-32
 // ======================================================================================================================
 // Queues the MD5 kernel over n files on `st`: descriptors go up from `pin`, digests (and chained states) come back into `pin`
 // at *digest_off (resp. m_state). Nothing is waited for.
@@ -1110,6 +1320,32 @@ int zwz_adler32_batch_device(zwz_ctx *ctx, const uint8_t *d_data, const uint64_t
     if ((rc = check_launch(ctx, "adler32_kernel"))) return rc;
     if (zwz_rt::memcpy_d2h(hp, dm + r_base, (size_t) n * 4, st) || zwz_rt::stream_sync(st)) return fail(ctx, ZWZ_E_CUDA, "adler kernel failed");
     memcpy(adler, hp, (size_t) n * 4);
+    return ZWZ_OK;
+}
+
+int zwz_crc32_batch_device(zwz_ctx *ctx, const uint8_t *d_data, const uint64_t *off, const uint32_t *len, uint32_t n, uint32_t *crc, void *stream_v) {
+    if (!ctx) return ZWZ_E_ARG;
+    if (n == 0) return ZWZ_OK;
+    if (!off || !len || !crc) return fail(ctx, ZWZ_E_ARG, "null argument");
+    zwz_rt::set_device(ctx->device);
+    zwz_stream_t st = stream_v ? (zwz_stream_t) stream_v : ctx->stream;
+    const size_t m_len = (size_t) n * 8, meta_bytes = m_len + (size_t) n * 4, r_base = align_up(meta_bytes, 256);
+    int rc;
+    if ((rc = reserve(ctx, ctx->pin_meta, meta_bytes, true))) return rc;
+    if ((rc = reserve(ctx, ctx->meta, r_base + (size_t) n * 4 + 256, false))) return rc;
+    uint8_t *hp = (uint8_t *) ctx->pin_meta.p;
+    memcpy(hp, off, (size_t) n * 8);
+    memcpy(hp + m_len, len, (size_t) n * 4);
+    uint8_t *dm = (uint8_t *) ctx->meta.p;
+    if (zwz_rt::memcpy_h2d(dm, hp, meta_bytes, st)) return fail(ctx, ZWZ_E_CUDA, "descriptor upload failed");
+    {
+        ProfSpan ps(ctx, ZWZ_PROF_ADLER, st);
+        ZWZ_LAUNCH(zwz::crc32_kernel, (n + 7) / 8, 256, 0, st, d_data, (const uint64_t *) dm, (const uint32_t *) (dm + m_len),
+                   (uint32_t *) (dm + r_base), n);
+    }
+    if ((rc = check_launch(ctx, "crc32_kernel"))) return rc;
+    if (zwz_rt::memcpy_d2h(hp, dm + r_base, (size_t) n * 4, st) || zwz_rt::stream_sync(st)) return fail(ctx, ZWZ_E_CUDA, "crc32 kernel failed");
+    memcpy(crc, hp, (size_t) n * 4);
     return ZWZ_OK;
 }
 
