@@ -7,8 +7,8 @@
 // x^(8n) is assembled from the table of x^(2^k) like zlib's x2nmodp.
 //
 // The 4 KB slice table is read from shared memory. Kernels of the zlib path keep their shared-memory layout: crc32_kernel
-// stages the table in a static array of its own, and inflate_kernel loads it into its literal/length table once that is
-// dead (inflate.cuh, gzip header and trailer).
+// stages the table in a static array of its own, and inflate_kernel loads it over its decoder state (tables, staged window,
+// token regions) before the first block and after the last, when that is dead (inflate.cuh, gzip header and trailer).
 #pragma once
 #include "zwz_common.cuh"
 

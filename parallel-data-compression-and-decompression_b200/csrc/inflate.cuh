@@ -12,12 +12,15 @@
 //     128 bytes already in flight); the word feeding the bit buffer comes from a register of the owning lane by shuffle;
 //   * the bit buffer and every decode decision are computed redundantly by all 32 lanes (warp-uniform control flow, no
 //     divergence, no broadcast needed), so the lanes are all there when a match has to be copied;
-//   * literal/length and distance codes resolve through shared-memory lookup tables (2^10 and 2^8 entries, one LDS per
-//     symbol); longer codes fall back to a canonical walk;
+//   * literal/length and distance codes resolve through shared-memory lookup tables (2^10 and 2^8 16-bit entries, one LDS
+//     per symbol, filled by scattering each code into its slots); longer codes fall back to a canonical walk;
 //   * literals are parked in the lane `position & 31` and stored 32 at a time; back-references are copied by the whole
 //     warp, 32 bytes per step (pattern-replicated when distance < 32).
 // Output bytes are written straight to global memory; back-references re-read them through L1/L2 (the window of one
-// 65 535-byte record fits L1+L2 trivially), so shared memory only holds the ~6 KB of tables per warp and 36 warps fit an SM.
+// 65 535-byte record fits L1+L2 trivially). Shared memory holds the decode tables, the staged window and the token regions of
+// inflate_fast.cuh: 10 336 bytes per warp, so with 1 KB reserved per CTA 20 one-warp CTAs fit an SM (registers would allow
+// 24). The decoder is latency-bound: resident warps hide it, but so do long windows, which take fewer rounds and commit more
+// per round. 20 warps with 416-bit lane ranges measured faster than 24 with 288-bit ones (profiles/inflate_smem/).
 //
 // Algorithmic bytes per stream: N_comp read + N_raw written (SURVEY.md §8(d)).
 #pragma once
@@ -26,43 +29,84 @@
 
 namespace zwz {
 
-#define ZWZ_INF_WARPS 1 // one warp per CTA: ~14 KB of shared memory each, so the CTA count per SM is what shared memory allows
+#define ZWZ_INF_WARPS 1 // one warp per CTA
+// registers <= 80 a thread, which would allow 24 resident CTAs per SM (6 warps for each of the 4 schedulers): registers never
+// bind before shared memory does
+#define ZWZ_INF_MIN_CTAS 24
 #define ZWZ_INF_LBITS 10
 #define ZWZ_INF_DBITS 8
 
-enum { INF_KIND_LIT = 0, INF_KIND_BASE = 1, INF_KIND_EOB = 2, INF_KIND_SPECIAL = 3 };
-// entry: [3:0] code length, [7:4] extra bits, [9:8] kind, [31:16] literal byte / base length / base distance.
-//        kind SPECIAL: extra-bits field 1 = code longer than the table index (canonical walk needed);
-//                      extra-bits field 0 = invalid code whose length is in [3:0] (zlib's op=64 entries)
-#define ZWZ_INF_ENTRY(nb, eb, kind, val) ((uint32_t) (nb) | ((uint32_t) (eb) << 4) | ((uint32_t) (kind) << 8) | ((uint32_t) (val) << 16))
-#define ZWZ_INF_INVALID(nb) ZWZ_INF_ENTRY((nb), 0, INF_KIND_SPECIAL, 0)
-#define ZWZ_INF_LONG ZWZ_INF_ENTRY(0, 1, INF_KIND_SPECIAL, 0)
+// Decode-table entries are 16 bits.
+// literal/length: [3:0] code length, [6:4] extra bits, [15:7] literal byte (0..255) or 253 + base length (256..511).
+//                 Extra-bits field 7 marks the other entries by their value: 0 end-of-block, 1 invalid code whose length is
+//                 in [3:0] (zlib's op=64 entries), 2 code longer than the table index (canonical walk needed).
+// distance:       [3:0] code length, [7:4] extra bits, [9:8] m, [11:10] 0 valid, 1 invalid code (length in [3:0]), 2 code
+//                 longer than the index. distance - 1 = (m << extra bits) | extra: m is the symbol for symbols 0..3 and
+//                 2 | (symbol & 1) above.
+// code-length code: [3:0] code length, [8:4] symbol.
+#define ZWZ_LL_LIT(nb, byte) ((uint32_t) (nb) | ((uint32_t) (byte) << 7))
+#define ZWZ_LL_LEN(nb, eb, base) ((uint32_t) (nb) | ((uint32_t) (eb) << 4) | (((uint32_t) (base) + 253u) << 7))
+#define ZWZ_LL_EOB(nb) ((uint32_t) (nb) | 0x70u)
+#define ZWZ_LL_INVALID(nb) ((uint32_t) (nb) | 0x70u | (1u << 7))
+#define ZWZ_LL_LONG (0x70u | (2u << 7))
+#define ZWZ_LL_IS_LIT(e) (((e) & 0x8070u) == 0u)
+#define ZWZ_LL_IS_LEN(e) ((e) >= 0x8000u)
+#define ZWZ_LL_IS_EOB(e) (((e) >> 4) == 7u)
+#define ZWZ_LL_IS_INVALID(e) (((e) >> 4) == 15u)
+#define ZWZ_LL_IS_LONG(e) (((e) >> 4) == 23u)
+#define ZWZ_D_ENTRY(nb, eb, m) ((uint32_t) (nb) | ((uint32_t) (eb) << 4) | ((uint32_t) (m) << 8))
+#define ZWZ_D_INVALID(nb) ((uint32_t) (nb) | (1u << 10))
+#define ZWZ_D_LONG (2u << 10)
+#define ZWZ_D_IS_LONG(e) (((e) >> 10) == 2u)
+#define ZWZ_D_IS_SPECIAL(e) (((e) >> 10) != 0u)
+// distance - 1 of a valid entry, given the bits that follow its code
+#define ZWZ_D_DM1(e, bits) ((((e) >> 8 & 3u) << ((e) >> 4 & 15u)) | (((bits) >> ((e) & 15u)) & ((1u << ((e) >> 4 & 15u)) - 1u)))
+
+// Token entries (u16) a lane may emit per decode window of inflate_fast.cuh; a multiple of 4. A window whose lane fills its
+// region is cut there, so the region has to hold what ZWZ_IF_SW words decode to (a literal takes one entry, a match two):
+// 80 entries over 416 bits, one per 5.2 bits. 44 or 64 entries over 480 bits cut most windows of C2-shaped data.
+#ifndef ZWZ_IF_R
+#define ZWZ_IF_R 80u
+#endif
+#define ZWZ_IF_RS (ZWZ_IF_R + 2u) // region stride in u16: an odd number of words, so equal offsets in 32 regions hit 32 banks
+#ifndef ZWZ_IF_SW
+#define ZWZ_IF_SW 13u // words of compressed data per lane and decode window (odd: conflict-free strides)
+#endif
+#define ZWZ_IF_CW (32u * ZWZ_IF_SW + 8u) // staged words: 32 ranges + the overshoot of the last token
 
 struct InflateWarpSmem {
-    uint32_t lit[1 << ZWZ_INF_LBITS];
-    uint32_t dst[1 << ZWZ_INF_DBITS];
-    uint16_t sorted_ll[288];
-    uint16_t sorted_d[32];
-    uint32_t cnt_ll[16];
-    uint32_t cnt_d[16];
-    uint32_t run[16]; // running offsets while sorting
-    uint32_t cw[32u * 15u + 8u];  // inflate_fast.cuh: staged window of compressed words (ZWZ_IF_CW), then the resolve staging area
     union {
-        struct { // block header parsing only: dead once the tables are built, when the token regions come to life
-            uint8_t lens[352]; // [0,19) code-length-code lengths; [32, 32+316) literal/length then distance lengths
-            uint32_t clt[128]; // code-length-code table (7 bits)
-            uint16_t sorted_cl[20];
-            uint32_t cnt_cl[16];
+        struct {
+            uint16_t lit[1 << ZWZ_INF_LBITS];
+            uint16_t dst[1 << ZWZ_INF_DBITS];
+            uint16_t sorted_ll[288];
+            uint16_t sorted_d[32];
+            uint32_t cnt_ll[16];
+            uint32_t cnt_d[16];
+            uint32_t run[16];            // running offsets while sorting
+            uint32_t cw[ZWZ_IF_CW];     // inflate_fast.cuh: staged window of compressed words, then the resolve staging area
+            union {
+                struct { // block header parsing only: dead once the tables are built, when the token regions come to life
+                    uint8_t lens[352]; // [0,19) code-length-code lengths; [32, 32+316) literal/length then distance lengths
+                    uint16_t clt[128]; // code-length-code table (7 bits)
+                    uint16_t sorted_cl[20];
+                    uint32_t cnt_cl[16];
+                };
+                uint16_t tok[32u * ZWZ_IF_RS]; // inflate_fast.cuh: one token region per lane
+            };
         };
-        uint16_t tok[32u * 98u];  // inflate_fast.cuh: one token region per lane (32 x ZWZ_IF_RS)
+        // gzip: CRC-32 slice table. Only used before the first block header and after the last block, when nothing above
+        // is alive, so the gzip path needs no shared memory of its own.
+        uint32_t crc[1024];
     };
 };
 #define ZWZ_INF_SMEM (ZWZ_INF_WARPS * (uint32_t) sizeof(zwz::InflateWarpSmem))
+static_assert(sizeof(InflateWarpSmem) > sizeof(uint32_t[1024]), "the CRC-32 table must not set the size of the decoder's shared memory");
 
 ZWZ_DEV uint32_t inf_litlen_entry(uint32_t sym, uint32_t nb) {
-    if (sym < 256u) return ZWZ_INF_ENTRY(nb, 0, INF_KIND_LIT, sym);
-    if (sym == 256u) return ZWZ_INF_ENTRY(nb, 0, INF_KIND_EOB, 0);
-    if (sym > 285u) return ZWZ_INF_INVALID(nb);
+    if (sym < 256u) return ZWZ_LL_LIT(nb, sym);
+    if (sym == 256u) return ZWZ_LL_EOB(nb);
+    if (sym > 285u) return ZWZ_LL_INVALID(nb);
     uint32_t k = sym - 257u, eb, base;
     if (k < 8u) {
         eb = 0;
@@ -74,21 +118,14 @@ ZWZ_DEV uint32_t inf_litlen_entry(uint32_t sym, uint32_t nb) {
         eb = (k - 4u) >> 2;
         base = 3u + ((4u + (k & 3u)) << eb);
     }
-    return ZWZ_INF_ENTRY(nb, eb, INF_KIND_BASE, base);
+    return ZWZ_LL_LEN(nb, eb, base);
 }
 ZWZ_DEV uint32_t inf_dist_entry(uint32_t sym, uint32_t nb) {
-    if (sym > 29u) return ZWZ_INF_INVALID(nb);
-    uint32_t eb, base;
-    if (sym < 4u) {
-        eb = 0;
-        base = 1u + sym;
-    } else {
-        eb = (sym - 2u) >> 1;
-        base = 1u + ((2u + (sym & 1u)) << eb);
-    }
-    return ZWZ_INF_ENTRY(nb, eb, INF_KIND_BASE, base);
+    if (sym > 29u) return ZWZ_D_INVALID(nb);
+    if (sym < 4u) return ZWZ_D_ENTRY(nb, 0, sym);
+    return ZWZ_D_ENTRY(nb, (sym >> 1) - 1u, 2u | (sym & 1u));
 }
-ZWZ_DEV uint32_t inf_cl_entry(uint32_t sym, uint32_t nb) { return ZWZ_INF_ENTRY(nb, 0, INF_KIND_LIT, sym); }
+ZWZ_DEV uint32_t inf_cl_entry(uint32_t sym, uint32_t nb) { return nb | (sym << 4); }
 
 // Canonical-code walk over `bits` (LSB first), lengths 1..maxwalk. Returns entry-maker input (sym,len) or ~0u.
 ZWZ_DEV uint32_t inf_canon_walk(uint32_t bits, const uint32_t *cnt, const uint16_t *sorted, uint32_t maxwalk, uint32_t &len_out) {
@@ -112,7 +149,7 @@ ZWZ_DEV uint32_t inf_canon_walk(uint32_t bits, const uint32_t *cnt, const uint16
 // Warp-cooperative table build. kind: 0 = code-length code (must be complete), 1 = literal/length, 2 = distance.
 // Returns (warp-uniform) 0 ok / 1 invalid set. max_len_out = longest code (0 = empty set).
 template <int KIND>
-ZWZ_DEV int inf_build(const uint8_t *lens, uint32_t n, uint32_t *cnt, uint16_t *sorted, uint32_t *run, uint32_t *table, uint32_t tbits,
+ZWZ_DEV int inf_build(const uint8_t *lens, uint32_t n, uint32_t *cnt, uint16_t *sorted, uint32_t *run, uint16_t *table, uint32_t tbits,
                       uint32_t &max_len_out) {
     const unsigned lane = lane_id();
     if (lane < 16u) cnt[lane] = 0;
@@ -157,17 +194,30 @@ ZWZ_DEV int inf_build(const uint8_t *lens, uint32_t n, uint32_t *cnt, uint16_t *
         if (L && (grp >> lane) == 1u) run[L] += (uint32_t) __popc(grp); // highest lane of each group
         __syncwarp();
     }
-    // fill: every table slot resolves its own prefix
-    uint32_t walk = max_len < tbits ? max_len : tbits;
-    for (uint32_t e = lane; e < (1u << tbits); e += 32u) {
-        uint32_t len = 0;
-        uint32_t sym = inf_canon_walk(e, cnt, sorted, walk, len);
-        uint32_t ent;
-        if (sym == 0xffffffffu)
-            ent = (max_len > tbits) ? ZWZ_INF_LONG : ZWZ_INF_INVALID(max_len ? max_len : 1u);
-        else
-            ent = KIND == 0 ? inf_cl_entry(sym, len) : (KIND == 1 ? inf_litlen_entry(sym, len) : inf_dist_entry(sym, len));
-        table[e] = ent;
+    // fill. Slots that start no code of <= tbits bits: the prefix of a longer code (or of none, in an incomplete set)
+    if (left > 0 || max_len > tbits) {
+        const uint32_t dflt = KIND == 0 ? 0u
+                                        : (max_len > tbits ? (KIND == 1 ? ZWZ_LL_LONG : ZWZ_D_LONG)
+                                                           : (KIND == 1 ? ZWZ_LL_INVALID(max_len ? max_len : 1u) : ZWZ_D_INVALID(max_len ? max_len : 1u)));
+        uint32_t *t2 = (uint32_t *) table;
+        for (uint32_t e = lane; e < (1u << (tbits - 1u)); e += 32u) t2[e] = dflt | (dflt << 16);
+        __syncwarp();
+    }
+    // then every code of <= tbits bits writes its 2^(tbits - len) slots: the bit-reversed code, followed by any bits.
+    // The (code, replica) pairs of one length are spread over the lanes, so a short code does not keep one lane busy.
+    const uint32_t top = max_len < tbits ? max_len : tbits;
+    uint32_t code = 0, idx = 0; // canonical code of the first length-l code; its place in `sorted`
+    for (uint32_t l = 1; l <= top; ++l) {
+        const uint32_t c = cnt[l], sh = tbits - l;
+        for (uint32_t t = lane; t < (c << sh); t += 32u) {
+            const uint32_t i = t >> sh;
+            const uint32_t sym = sorted[idx + i];
+            const uint32_t r = __brev(code + i) >> (32u - l);
+            table[r | ((t & ((1u << sh) - 1u)) << l)] =
+                (uint16_t) (KIND == 0 ? inf_cl_entry(sym, l) : (KIND == 1 ? inf_litlen_entry(sym, l) : inf_dist_entry(sym, l)));
+        }
+        idx += c;
+        code = (code + c) << 1;
     }
     __syncwarp();
     return 0;
@@ -251,11 +301,11 @@ ZWZ_DEV void infb_seek_bits(InfBits &b, uint64_t bit_pos) {
 #include "inflate_fast.cuh"
 namespace zwz {
 
-// CRC-32 of p[0, n) by the calling warp. The slice table goes into the warp's literal/length decode table, which is dead
-// before the first block header and after the last block: the shared-memory layout stays that of the zlib path.
+// CRC-32 of p[0, n) by the calling warp. The slice table overlays the warp's decoder state, which is dead before the first
+// block header and after the last block: the shared-memory layout stays that of the zlib path.
 ZWZ_DEV_NOINLINE uint32_t inf_crc32(const uint8_t *p, uint32_t n) {
     ZWZ_DYN_SMEM(inf_raw);
-    uint32_t *tab = ((InflateWarpSmem *) inf_raw)[warp_id()].lit;
+    uint32_t *tab = ((InflateWarpSmem *) inf_raw)[warp_id()].crc;
     __syncwarp();
     crc32_load_table(tab, lane_id(), 32u);
     __syncwarp();
@@ -452,7 +502,7 @@ ZWZ_DEV void inflate_stream(InflateWarpSmem &S, const uint8_t *__restrict__ comp
                     status = ZWZ_STREAM_BAD;
                     goto done;
                 }
-                uint32_t sym = e >> 16;
+                uint32_t sym = e >> 4;
                 uint32_t eb = sym < 16u ? 0u : (sym == 16u ? 2u : (sym == 17u ? 3u : 7u));
                 if (!INF_NEED(nb + eb)) {
                     status = ZWZ_STREAM_TRUNCATED;
@@ -537,7 +587,7 @@ ZWZ_DEV void inflate_stream(InflateWarpSmem &S, const uint8_t *__restrict__ comp
                 // run is dropped from the bit buffer at once. The chain ends at the first non-literal (handled below) or
                 // past offset 31.
                 const uint32_t el = S.lit[(uint32_t) (B.hold >> lane) & ((1u << ZWZ_INF_LBITS) - 1u)];
-                const bool ok = (lane + 15u <= B.cnt) && ((el >> 8) & 3u) == INF_KIND_LIT;
+                const bool ok = (lane + 15u <= B.cnt) && ZWZ_LL_IS_LIT(el);
                 const unsigned litmask = __ballot_sync(ZWZ_FULL, ok);
                 if (litmask & 1u) {
                     uint32_t J = lane + (el & 15u);
@@ -571,7 +621,7 @@ ZWZ_DEV void inflate_stream(InflateWarpSmem &S, const uint8_t *__restrict__ comp
                     if (pend_lo != pos) INF_FLUSH_LITS(); // only after a step of the scalar path
                     if ((R0 >> lane) & 1u) {
                         const uint32_t q = pos + (uint32_t) __popc(R0 & ((1u << lane) - 1u));
-                        if (q < cap) out[q] = (uint8_t) (el >> 16);
+                        if (q < cap) out[q] = (uint8_t) (el >> 7);
                     }
                     if (pos + nlit > cap) overflow = true;
                     pos += nlit;
@@ -583,37 +633,33 @@ ZWZ_DEV void inflate_stream(InflateWarpSmem &S, const uint8_t *__restrict__ comp
             } else {
                 e = S.lit[(uint32_t) B.hold & ((1u << ZWZ_INF_LBITS) - 1u)];
             }
-            uint32_t kind = (e >> 8) & 3u;
             uint32_t nb = e & 15u;
-            if (kind == INF_KIND_SPECIAL) {
-                if ((e >> 4) & 15u) { // code longer than the table index: canonical walk (complete sets only get here)
-                    uint32_t len = 0;
-                    uint32_t sym = inf_canon_walk((uint32_t) B.hold, S.cnt_ll, S.sorted_ll, max_ll, len);
-                    e = sym == 0xffffffffu ? ZWZ_INF_INVALID(max_ll) : inf_litlen_entry(sym, len);
-                    kind = (e >> 8) & 3u;
-                    nb = e & 15u;
-                }
-                if (kind == INF_KIND_SPECIAL) { // zlib's invalid-code entry: it still has to see the code's bits first
-                    status = INF_NEED(nb) ? ZWZ_STREAM_BAD : ZWZ_STREAM_TRUNCATED;
-                    goto done;
-                }
+            if (ZWZ_LL_IS_LONG(e)) { // code longer than the table index: canonical walk (complete sets only get here)
+                uint32_t len = 0;
+                uint32_t sym = inf_canon_walk((uint32_t) B.hold, S.cnt_ll, S.sorted_ll, max_ll, len);
+                e = sym == 0xffffffffu ? ZWZ_LL_INVALID(max_ll) : inf_litlen_entry(sym, len);
+                nb = e & 15u;
+            }
+            if (ZWZ_LL_IS_INVALID(e)) { // zlib's invalid-code entry: it still has to see the code's bits first
+                status = INF_NEED(nb) ? ZWZ_STREAM_BAD : ZWZ_STREAM_TRUNCATED;
+                goto done;
             }
             if (!INF_NEED(nb)) {
                 status = ZWZ_STREAM_TRUNCATED;
                 goto done;
             }
             infb_drop(B, nb);
-            if (kind == INF_KIND_LIT) {
-                if (lane == (pos & 31u)) mybyte = e >> 16;
+            if (ZWZ_LL_IS_LIT(e)) {
+                if (lane == (pos & 31u)) mybyte = e >> 7;
                 pos++;
                 if ((pos & 31u) == 0u) INF_FLUSH_LITS();
                 continue;
             }
-            if (kind == INF_KIND_EOB) break;
+            if (ZWZ_LL_IS_EOB(e)) break;
             // length (the code may have been the second one since the last refill: top up before the extra bits)
             infb_refill(B);
-            uint32_t eb = (e >> 4) & 15u;
-            uint32_t mlen = (e >> 16) + ((uint32_t) B.hold & ((1u << eb) - 1u));
+            uint32_t eb = (e >> 4) & 7u;
+            uint32_t mlen = (e >> 7) - 253u + ((uint32_t) B.hold & ((1u << eb) - 1u));
             if (!INF_NEED(eb)) {
                 status = ZWZ_STREAM_TRUNCATED;
                 goto done;
@@ -621,27 +667,23 @@ ZWZ_DEV void inflate_stream(InflateWarpSmem &S, const uint8_t *__restrict__ comp
             infb_drop(B, eb);
             infb_refill(B);
             uint32_t d = S.dst[(uint32_t) B.hold & ((1u << ZWZ_INF_DBITS) - 1u)];
-            uint32_t dnb = d & 15u;
-            if (((d >> 8) & 3u) == INF_KIND_SPECIAL) {
-                if ((d >> 4) & 15u) {
-                    uint32_t len = 0;
-                    uint32_t sym = inf_canon_walk((uint32_t) B.hold, S.cnt_d, S.sorted_d, max_d, len);
-                    d = sym == 0xffffffffu ? ZWZ_INF_INVALID(max_d) : inf_dist_entry(sym, len);
-                    dnb = d & 15u;
-                }
-                if (((d >> 8) & 3u) == INF_KIND_SPECIAL) {
-                    status = INF_NEED(dnb) ? ZWZ_STREAM_BAD : ZWZ_STREAM_TRUNCATED;
-                    goto done;
-                }
+            if (ZWZ_D_IS_LONG(d)) {
+                uint32_t len = 0;
+                uint32_t sym = inf_canon_walk((uint32_t) B.hold, S.cnt_d, S.sorted_d, max_d, len);
+                d = sym == 0xffffffffu ? ZWZ_D_INVALID(max_d) : inf_dist_entry(sym, len);
+            }
+            const uint32_t dnb = d & 15u;
+            if (ZWZ_D_IS_SPECIAL(d)) {
+                status = INF_NEED(dnb) ? ZWZ_STREAM_BAD : ZWZ_STREAM_TRUNCATED;
+                goto done;
             }
             uint32_t deb = (d >> 4) & 15u;
             if (!INF_NEED(dnb + deb)) {
                 status = ZWZ_STREAM_TRUNCATED;
                 goto done;
             }
-            infb_drop(B, dnb);
-            uint32_t dist = (d >> 16) + ((uint32_t) B.hold & ((1u << deb) - 1u));
-            infb_drop(B, deb);
+            uint32_t dist = ZWZ_D_DM1(d, (uint32_t) B.hold) + 1u;
+            infb_drop(B, dnb + deb);
             if (dist > pos) { // "invalid distance too far back"
                 status = ZWZ_STREAM_BAD;
                 goto done;
@@ -698,7 +740,7 @@ done:
 
 // Persistent warps: every warp pulls the next stream from a global counter, so a CTA is never kept alive by one long stream
 // while its other warps idle (streams of one batch differ in length by 100x in config C2).
-ZWZ_KERNEL __launch_bounds__(ZWZ_INF_WARPS * 32) inflate_kernel(const uint8_t *__restrict__ comp, const uint64_t *__restrict__ off,
+ZWZ_KERNEL __launch_bounds__(ZWZ_INF_WARPS * 32, ZWZ_INF_MIN_CTAS) inflate_kernel(const uint8_t *__restrict__ comp, const uint64_t *__restrict__ off,
                                                               const uint32_t *__restrict__ len, uint8_t *raw_out,
                                                               const uint64_t *__restrict__ raw_off, uint32_t *raw_len, uint32_t *status,
                                                               uint32_t n, uint32_t flags, uint32_t *work_counter) {

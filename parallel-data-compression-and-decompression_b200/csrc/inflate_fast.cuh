@@ -3,8 +3,8 @@
 // The careful decoder in inflate.cuh computes every symbol redundantly in all 32 lanes (~22 warp-instructions per output
 // byte, profiles/round1/ncu_inflate.txt). This path spends the lanes on DIFFERENT symbols of the same block:
 //
-//   window   the next 32 x 480 bits of the block are staged into shared memory (16 coalesced loads);
-//   decode   lane i decodes the tokens that start in ITS 480 bits, from a speculative start (the first bit of its range),
+//   window   the next 32 x 416 bits of the block are staged into shared memory (14 coalesced loads);
+//   decode   lane i decodes the tokens that start in ITS 416 bits, from a speculative start (the first bit of its range),
 //            into its own token region in shared memory. Lane 0 starts at a known token boundary, so its result — and the
 //            position where it crosses into lane 1's range — is exact. Lanes whose start disagrees with where their
 //            predecessor ended decode again from there; every round proves at least one more lane, and since Huffman
@@ -22,16 +22,14 @@
 
 namespace zwz {
 
-#define ZWZ_IF_SW 15u                          // words of compressed data per lane and window
-#define ZWZ_IF_SBITS (ZWZ_IF_SW * 32u)         // 480 bits: longer than any token (48 bits), 15 is odd -> conflict-free strides
-#define ZWZ_IF_CW (32u * ZWZ_IF_SW + 8u)       // staged words: 32 ranges + the overshoot of the last token
-#define ZWZ_IF_R 96u                           // token entries (u16) a lane may emit per window
-#define ZWZ_IF_RS 98u                          // region stride in u16: 49 words (odd), so equal offsets in 32 regions hit 32 banks
+// ZWZ_IF_SW (words of compressed data per lane and window), ZWZ_IF_CW (staged words) and ZWZ_IF_R / ZWZ_IF_RS (token
+// region size and stride) are defined with the shared-memory layout in inflate.cuh
+#define ZWZ_IF_SBITS (ZWZ_IF_SW * 32u)         // bits per lane and window: longer than any token (48 bits)
 #define ZWZ_IF_MAXIT 6                         // rounds per window; then the proven prefix is committed and a new window starts
 #ifndef ZWZ_IF_MLP
 #define ZWZ_IF_MLP 4u                           // 32-byte rows of a resolve step whose back-reference loads are in flight together
 #endif
-#define ZWZ_IF_STG 1536u                       // output bytes assembled per resolve step (lives in the staged-window area)
+#define ZWZ_IF_STG (ZWZ_IF_CW * 4u > 1536u ? 1536u : ZWZ_IF_CW * 4u) // output bytes assembled per resolve step (lives in the staged-window area)
 
 #ifdef ZWZ_EMU
 // test-only counters of the emulator build: [0] windows, [1] decode rounds, [2] committed lanes, [3] token entries,
@@ -121,38 +119,38 @@ ZWZ_DEV int inf_fast_block(SMEM &S, const BITS &B, uint64_t &bitpos, uint32_t ma
                 if (run) {
                     const uint32_t bits = iff_fetch(S.cw, p);
                     uint32_t en = S.lit[bits & ((1u << ZWZ_INF_LBITS) - 1u)];
-                    if (((en >> 8) & 3u) == INF_KIND_SPECIAL && ((en >> 4) & 15u)) { // code longer than the table index (rare)
+                    if (ZWZ_LL_IS_LONG(en)) { // code longer than the table index (rare)
                         uint32_t len = 0;
                         const uint32_t sym = inf_canon_walk(bits, S.cnt_ll, S.sorted_ll, max_ll, len);
-                        en = sym == 0xffffffffu ? ZWZ_INF_INVALID(max_ll) : inf_litlen_entry(sym, len);
+                        en = sym == 0xffffffffu ? ZWZ_LL_INVALID(max_ll) : inf_litlen_entry(sym, len);
                     }
-                    const uint32_t kind = (en >> 8) & 3u;
-                    const uint32_t nb = en & 15u, eb = (en >> 4) & 15u;
-                    const uint32_t val = (en >> 16) + ((bits >> nb) & ((1u << eb) - 1u)); // literal byte, or match length (eb = 0 for literals)
+                    const bool is_len = ZWZ_LL_IS_LEN(en);
+                    const bool special = ((en >> 4) & 7u) == 7u; // end-of-block or invalid code
+                    const uint32_t nb = en & 15u, eb = is_len ? (en >> 4) & 7u : 0u;
+                    const uint32_t val = (en >> 7) + ((bits >> nb) & ((1u << eb) - 1u)); // literal byte, or 253 + match length
                     const uint32_t p2 = p + nb + eb;
                     // the distance code behind a length code; decoded for every lane, used by the lanes that hold a length
                     const uint32_t bits2 = iff_fetch(S.cw, p2);
                     uint32_t d = S.dst[bits2 & ((1u << ZWZ_INF_DBITS) - 1u)];
-                    const bool is_len = kind == INF_KIND_BASE;
-                    if (is_len && ((d >> 8) & 3u) == INF_KIND_SPECIAL && ((d >> 4) & 15u)) {
+                    if (is_len && ZWZ_D_IS_LONG(d)) {
                         uint32_t len = 0;
                         const uint32_t sym = inf_canon_walk(bits2, S.cnt_d, S.sorted_d, max_d, len);
-                        d = sym == 0xffffffffu ? ZWZ_INF_INVALID(max_d) : inf_dist_entry(sym, len);
+                        d = sym == 0xffffffffu ? ZWZ_D_INVALID(max_d) : inf_dist_entry(sym, len);
                     }
                     const uint32_t dnb = d & 15u, deb = (d >> 4) & 15u;
-                    const uint32_t dist = (d >> 16) + ((bits2 >> dnb) & ((1u << deb) - 1u));
+                    const uint32_t dm1 = ZWZ_D_DM1(d, bits2);
                     const uint32_t pn = is_len ? p2 + dnb + deb : p2;
-                    const bool bad = kind == INF_KIND_SPECIAL || (is_len && ((d >> 8) & 3u) == INF_KIND_SPECIAL) || pn > limit;
+                    const bool bad = (special && (en >> 7) != 0u) || (is_len && ZWZ_D_IS_SPECIAL(d)) || pn > limit;
                     if (bad) { // invalid code, or a token that does not lie completely inside the input: the careful decoder's business
                         flag = IFL_STOP;
                         run = false;
-                    } else if (kind == INF_KIND_EOB) {
+                    } else if (special) { // end-of-block
                         p = pn;
                         flag = IFL_EOB;
                         run = false;
                     } else {
-                        my[ntok] = (uint16_t) (is_len ? (0x8000u | val) : val);
-                        if (is_len) my[ntok + 1u] = (uint16_t) (dist - 1u);
+                        my[ntok] = (uint16_t) (is_len ? (0x8000u - 253u) + val : val);
+                        if (is_len) my[ntok + 1u] = (uint16_t) dm1;
                         ntok += is_len ? 2u : 1u;
                         p = pn;
                         if (p >= hi) {

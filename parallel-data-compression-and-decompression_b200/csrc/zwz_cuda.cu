@@ -93,6 +93,7 @@ struct zwz_ctx {
     int device = 0;
     int sm_count = 0, cc_major = 0, cc_minor = 0;
     size_t total_mem = 0, smem_optin = 0;
+    int inf_blocks_per_sm = 1; // resident inflate_kernel CTAs per SM
     zwz_stream_t stream = nullptr;
     zwz_stream_t md5_stream = nullptr; // deferred digests (DigestSlot)
     zwz::DigestSlot slot[2];
@@ -267,6 +268,10 @@ int zwz_init(int device, zwz_ctx **out) {
         zwz_rt::set_max_dyn_smem((const void *) zwz::md5_files_staged_kernel, ZWZ_MD5S_SMEM) ||
         zwz_rt::set_max_dyn_smem((const void *) zwz::inflate_kernel, ZWZ_INF_SMEM) ||
         zwz_rt::set_max_dyn_smem((const void *) zwz::inflate_lanes_kernel, ZWZ_IL_SMEM)) {
+        delete ctx;
+        return ZWZ_E_NODEVICE;
+    }
+    if (zwz_rt::max_blocks_per_sm(&ctx->inf_blocks_per_sm, (const void *) zwz::inflate_kernel, ZWZ_INF_WARPS * 32, ZWZ_INF_SMEM)) {
         delete ctx;
         return ZWZ_E_NODEVICE;
     }
@@ -801,8 +806,7 @@ int zwz_inflate_batch_device(zwz_ctx *ctx, const uint8_t *d_comp, const uint64_t
                        (const uint32_t *) (dm + m_len), d_raw_out, (const uint64_t *) (dm + m_roff), d_rlen, d_stat,
                        (const uint32_t *) (dm + m_order), n, flags, d_counter);
         } else {
-            const uint32_t per_sm = std::min<uint32_t>(32u, std::max<uint32_t>(1u, (uint32_t) ((228u * 1024u) / (ZWZ_INF_SMEM + 1024u))));
-            uint32_t grid = std::min<uint32_t>((n + ZWZ_INF_WARPS - 1) / ZWZ_INF_WARPS, (uint32_t) ctx->sm_count * per_sm);
+            uint32_t grid = std::min<uint32_t>((n + ZWZ_INF_WARPS - 1) / ZWZ_INF_WARPS, (uint32_t) (ctx->sm_count * ctx->inf_blocks_per_sm));
             if (ctx->inflate_mode == 3) flags |= ZWZ_INFLATE_CAREFUL;
             ZWZ_LAUNCH(zwz::inflate_kernel, grid, ZWZ_INF_WARPS * 32, ZWZ_INF_SMEM, st, d_comp, (const uint64_t *) (dm + m_off),
                        (const uint32_t *) (dm + m_len), d_raw_out, (const uint64_t *) (dm + m_roff), d_rlen, d_stat, n, flags, d_counter);

@@ -4,6 +4,7 @@
 // Emulator build (-DZWZ_EMU, tests only): "device" memory is host memory and a launch runs the kernel body through
 // tests/simt/simt_emu.h. The emulator library is never loaded by the product package.
 #pragma once
+#include <algorithm>
 #include <cstddef>
 #include <cstdint>
 #include <cstdlib>
@@ -45,6 +46,11 @@ inline int memcpy_d2h(void *d, const void *s, size_t n, zwz_stream_t) { if (n) m
 inline int memset_device(void *d, int v, size_t n, zwz_stream_t) { if (n) memset(d, v, n); return 0; }
 inline int last_error(std::string &) { return 0; }
 inline int set_max_dyn_smem(const void *, size_t) { return 0; }
+// resident CTAs per SM: what shared memory alone would allow on a B200 (the emulator has no register file)
+inline int max_blocks_per_sm(int *blocks, const void *, int, size_t smem) {
+    *blocks = (int) std::min<size_t>(32u, std::max<size_t>(1u, (228u * 1024u) / (smem + 1024u)));
+    return 0;
+}
 typedef int zwz_sync_event_t; // ordering-only events: the emulator runs everything in call order
 inline int sync_event_create(zwz_sync_event_t *e) { *e = 0; return 0; }
 inline int sync_event_destroy(zwz_sync_event_t) { return 0; }
@@ -105,6 +111,11 @@ inline int keep_pool_memory(int device) { // freed arena memory stays in the poo
 inline int preload_kernel(const void *fn) {
     cudaFuncAttributes a;
     return cudaFuncGetAttributes(&a, fn) == cudaSuccess ? 0 : 1;
+}
+// resident CTAs per SM for a launch of `threads` threads and `smem` bytes of dynamic shared memory (registers, shared
+// memory and the CTA limit all counted by the driver)
+inline int max_blocks_per_sm(int *blocks, const void *fn, int threads, size_t smem) {
+    return cudaOccupancyMaxActiveBlocksPerMultiprocessor(blocks, fn, threads, smem) == cudaSuccess && *blocks > 0 ? 0 : 1;
 }
 inline int malloc_pinned(void **p, size_t n) { return cudaMallocHost(p, n ? n : 1) == cudaSuccess ? 0 : 2; }
 inline int free_pinned(void *p) { return cudaFreeHost(p) == cudaSuccess ? 0 : 1; }
