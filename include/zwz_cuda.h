@@ -192,6 +192,13 @@ int zwz_decompress_records(zwz_ctx *ctx, const uint8_t *comp, const uint64_t *of
  * and its context allocates 0.2 GB of scratch instead of 0.8 GB — device allocation is the larger part of a short job's
  * start-up). */
 #define ZWZ_TUNE_DEFLATE_SUBBATCH_BYTES 1
+/* ZWZ_TUNE_HOST_THREADS: host threads (the calling one included) that stage the descriptors of one call — copies into and out of
+ * page-locked memory, validation, offset sums; the device waits for this work, since every call ends in a synchronise. 0 =
+ * min(8, cores / 2) (default), 1 = the calling thread alone. The threads belong to the context and end in zwz_destroy.
+ * ZWZ_TUNE_HOST_PARALLEL_MIN: calls with fewer chunks, streams or files than this (default 32 768) run on the calling thread
+ * alone, so that many contexts fed by threads of their own with small batches do not oversubscribe the host. */
+#define ZWZ_TUNE_HOST_THREADS 2
+#define ZWZ_TUNE_HOST_PARALLEL_MIN 3
 int zwz_ctx_tune(zwz_ctx *ctx, int what, uint64_t value);
 
 /* ---- asynchronous forms: the digests are DEFERRED ----------------------------------------------------------------------

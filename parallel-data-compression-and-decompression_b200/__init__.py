@@ -202,9 +202,13 @@ class Context:
     PROF_KINDS = ("lz_match", "deflate_encode", "inflate", "md5", "pack", "adler32")
 
     TUNE_DEFLATE_SUBBATCH_BYTES = 1
+    TUNE_HOST_THREADS = 2
+    TUNE_HOST_PARALLEL_MIN = 3
 
     def tune(self, what: int, value: int):
-        """zwz_ctx_tune: e.g. TUNE_DEFLATE_SUBBATCH_BYTES (raw bytes per internal deflate pass; the scratch is 6 bytes per raw byte of one pass)."""
+        """zwz_ctx_tune: e.g. TUNE_DEFLATE_SUBBATCH_BYTES (raw bytes per internal deflate pass; the scratch is 6 bytes per raw byte of one pass),
+        TUNE_HOST_THREADS (host threads that stage a call's descriptors; 0 = min(8, cores / 2), 1 = the calling thread alone) and
+        TUNE_HOST_PARALLEL_MIN (calls with fewer entries stay on the calling thread; default 32 768)."""
         self._check(self.lib.zwz_ctx_tune(self.h, what, value))
 
     def profile_enable(self, on: bool = True):

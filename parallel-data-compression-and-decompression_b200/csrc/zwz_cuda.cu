@@ -14,11 +14,82 @@
 #include "deflate_match.cuh"
 #include "deflate_encode.cuh"
 
+#if defined(__x86_64__)
+#include <immintrin.h>
+#endif
+
 #include <algorithm>
+#include <atomic>
+#include <condition_variable>
+#include <functional>
+#include <memory>
+#include <mutex>
 #include <new>
+#include <thread>
 #include <vector>
 
 namespace zwz {
+
+// Host threads of one context for the O(n) descriptor work of a call (staging copies, validation, prefix sums): while the
+// calling thread prepares a call the device has nothing queued, since every call of the C ABI ends in a stream synchronise.
+// run(nblk, f) calls f(0..nblk-1) on the workers and the calling thread and returns when all are done.
+class HostPool {
+public:
+    explicit HostPool(unsigned workers) {
+        for (unsigned i = 0; i < workers; ++i) th_.emplace_back([this] { loop(); });
+    }
+    ~HostPool() {
+        {
+            std::lock_guard<std::mutex> lk(m_);
+            stop_ = true;
+        }
+        wake_.notify_all();
+        for (auto &t : th_) t.join();
+    }
+    void run(unsigned nblk, const std::function<void(unsigned)> &f) {
+        {
+            std::lock_guard<std::mutex> lk(m_);
+            f_ = &f;
+            nblk_ = nblk;
+            next_.store(0);
+            busy_ = (unsigned) th_.size();
+            ++gen_;
+        }
+        wake_.notify_all();
+        drain(f, nblk);
+        std::unique_lock<std::mutex> lk(m_);
+        idle_.wait(lk, [this] { return busy_ == 0; });
+        f_ = nullptr;
+    }
+
+private:
+    void drain(const std::function<void(unsigned)> &f, unsigned nblk) {
+        for (unsigned b; (b = next_.fetch_add(1)) < nblk;) f(b);
+    }
+    void loop() {
+        uint64_t seen = 0;
+        std::unique_lock<std::mutex> lk(m_);
+        for (;;) {
+            wake_.wait(lk, [&] { return stop_ || gen_ != seen; });
+            if (stop_) return;
+            seen = gen_;
+            const std::function<void(unsigned)> *f = f_;
+            const unsigned nblk = nblk_;
+            lk.unlock();
+            drain(*f, nblk);
+            lk.lock();
+            if (--busy_ == 0) idle_.notify_one();
+        }
+    }
+    std::vector<std::thread> th_;
+    std::mutex m_;
+    std::condition_variable wake_, idle_;
+    const std::function<void(unsigned)> *f_ = nullptr;
+    unsigned nblk_ = 0, busy_ = 0;
+    std::atomic<unsigned> next_{0};
+    uint64_t gen_ = 0;
+    bool stop_ = false;
+};
 
 // warp-per-chunk gather of the variable-length streams out of their slots into one packed buffer
 ZWZ_KERNEL pack_streams_kernel(const uint8_t *__restrict__ slots, const uint64_t *__restrict__ slot_off, const uint32_t *__restrict__ res,
@@ -106,7 +177,15 @@ struct zwz_ctx {
     bool arena_async = true; // ZWZ_ARENA_SYNC=1: plain cudaMalloc/cudaFree arenas (for A/B timing)
     bool trace = false;   // ZWZ_TRACE=1: wall-clock phases of the host-buffer calls on stderr (syncs the stream at every mark)
     size_t batch_raw_bytes = (size_t) 4 << 30; // raw bytes per internal deflate sub-batch (scratch = 6x that; ZWZ_BATCH_RAW_MB overrides)
-    size_t last_res_off = 0, last_slot_off = 0; // where the last deflate call left results / slot offsets inside `meta`
+    // The last deflate call's slot offsets and results: on the device in `keep` (which only deflate writes), and as a
+    // host copy in `pin_keep` that zwz_pack_streams_device compares the caller's arrays with before it uses the device copy.
+    // Layout of both: [slot_off u64 x keep_n], then at keep_res_off(keep_n) [results 16 B x keep_n].
+    zwz::Arena keep, pin_keep;
+    uint32_t keep_n = 0; // 0 = nothing valid in keep / pin_keep
+    // host threads for the descriptor work of large calls (ZWZ_TUNE_HOST_THREADS, ZWZ_TUNE_HOST_PARALLEL_MIN)
+    unsigned host_threads = 0; // threads per call, the calling one included; 0 = min(8, cores / 2)
+    uint64_t host_parallel_min = 32768; // calls with fewer entries run on the calling thread alone
+    std::unique_ptr<zwz::HostPool> pool;
     // optional per-kernel timing
     bool profiling = false;
     struct Span {
@@ -166,6 +245,86 @@ void release(zwz_ctx *ctx, Arena &a) {
 
 inline size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
 
+inline size_t keep_res_off(size_t n) { return align_up(n * 8, 256); }
+
+unsigned host_thread_count(const zwz_ctx *ctx) {
+    return ctx->host_threads ? ctx->host_threads : std::max(1u, std::min(8u, std::thread::hardware_concurrency() / 2));
+}
+
+// Number of blocks an O(n) host pass over n entries is cut into: one per host thread from host_parallel_min entries on, else 1.
+unsigned host_blocks(zwz_ctx *ctx, size_t n) {
+    const unsigned t = host_thread_count(ctx);
+    return t > 1 && n >= ctx->host_parallel_min ? t : 1u;
+}
+
+// f(b, lo, hi) for the nb blocks [lo, hi) of [0, n), block b starting at n * b / nb; on the context's host threads when nb > 1
+template <class F> void host_for(zwz_ctx *ctx, unsigned nb, size_t n, F &&f) {
+    if (nb > 1 && !ctx->pool) {
+        try {
+            ctx->pool.reset(new zwz::HostPool(host_thread_count(ctx) - 1));
+        } catch (...) { // no threads to be had: this call and the next ones run on the calling thread
+            ctx->pool.reset();
+            ctx->host_threads = 1;
+            nb = 1;
+        }
+    }
+    auto blk = [&](unsigned b) { f(b, n * b / nb, n * (b + 1) / nb); };
+    if (nb <= 1) {
+        f(0u, (size_t) 0, n);
+        return;
+    }
+    ctx->pool->run(nb, std::function<void(unsigned)>(blk));
+}
+
+// Stores into page-locked memory that the copy engine reads next, from the host threads: non-temporal, so that the lines are in
+// DRAM and not left dirty in the private caches of several cores, from where the DMA read of a descriptor upload ran at a
+// quarter of its speed on B200 hosts (profiles/step_gaps). The calling thread alone keeps plain stores: its small batches are
+// read from the cache it wrote them to.
+struct Staging {
+    bool nt;
+    explicit Staging(unsigned nb) : nt(nb > 1) {}
+    void put(uint64_t *p, uint64_t v) const {
+#if defined(__x86_64__)
+        if (nt) return _mm_stream_si64((long long *) p, (long long) v);
+#endif
+        *p = v;
+    }
+    void put(uint32_t *p, uint32_t v) const {
+#if defined(__x86_64__)
+        if (nt) return _mm_stream_si32((int *) p, (int) v);
+#endif
+        *p = v;
+    }
+    void copy(void *dst, const void *src, size_t bytes) const {
+#if defined(__x86_64__)
+        if (nt) {
+            uint8_t *d = (uint8_t *) dst;
+            const uint8_t *s = (const uint8_t *) src;
+            const size_t head = std::min(bytes, (size_t) (-(uintptr_t) d & 15u));
+            memcpy(d, s, head);
+            size_t i = head;
+            for (; i + 16 <= bytes; i += 16) _mm_stream_si128((__m128i *) (d + i), _mm_loadu_si128((const __m128i *) (s + i)));
+            memcpy(d + i, s + i, bytes - i);
+            return;
+        }
+#endif
+        memcpy(dst, src, bytes);
+    }
+    // at the end of a block: the non-temporal stores are globally visible before the upload is queued
+    void done() const {
+#if defined(__x86_64__)
+        if (nt) _mm_sfence();
+#endif
+    }
+};
+
+// memcpy of a descriptor array of `entries` entries
+void host_copy(zwz_ctx *ctx, void *dst, const void *src, size_t bytes, size_t entries) {
+    host_for(ctx, host_blocks(ctx, entries), bytes, [&](unsigned, size_t lo, size_t hi) {
+        memcpy((uint8_t *) dst + lo, (const uint8_t *) src + lo, hi - lo);
+    });
+}
+
 // RAII bracket: records an event pair around one kernel launch when profiling is on
 struct ProfSpan {
     zwz_ctx *ctx;
@@ -194,10 +353,12 @@ int check_launch(zwz_ctx *ctx, const char *what) {
     return ZWZ_OK;
 }
 
-// ZWZ_TRACE=1: phase times of a host-buffer call (debugging aid: every mark synchronises the stream)
+// ZWZ_TRACE=1: phase times of a call (debugging aid: every mark synchronises the call's stream, so a phase that queues
+// device work also holds that work's run time)
 struct Trace {
     zwz_ctx *ctx;
     const char *call;
+    zwz_stream_t st;
     double t0;
     std::string line;
     static double now() {
@@ -205,10 +366,10 @@ struct Trace {
         clock_gettime(CLOCK_MONOTONIC, &ts);
         return (double) ts.tv_sec + 1e-9 * (double) ts.tv_nsec;
     }
-    Trace(zwz_ctx *c, const char *name) : ctx(c), call(name), t0(c->trace ? now() : 0.0) {}
+    Trace(zwz_ctx *c, const char *name, zwz_stream_t s = nullptr) : ctx(c), call(name), st(s ? s : c->stream), t0(c->trace ? now() : 0.0) {}
     void mark(const char *what) {
         if (!ctx->trace) return;
-        zwz_rt::stream_sync(ctx->stream);
+        zwz_rt::stream_sync(st);
         double t = now();
         char buf[64];
         snprintf(buf, sizeof buf, " %s %.2f ms,", what, (t - t0) * 1e3);
@@ -323,6 +484,9 @@ void zwz_destroy(zwz_ctx *ctx) {
     release(ctx, ctx->pin_meta);
     release(ctx, ctx->pin_aux);
     release(ctx, ctx->counter);
+    release(ctx, ctx->keep);
+    release(ctx, ctx->pin_keep);
+    ctx->pool.reset(); // joins the host threads
     zwz_rt::stream_sync(ctx->stream);
     zwz_rt::stream_destroy(ctx->stream);
     zwz_rt::stream_destroy(ctx->md5_stream);
@@ -336,6 +500,16 @@ int zwz_ctx_tune(zwz_ctx *ctx, int what, uint64_t value) {
     if (what == ZWZ_TUNE_DEFLATE_SUBBATCH_BYTES) {
         if (value < ((uint64_t) 1 << 20)) return fail(ctx, ZWZ_E_ARG, "sub-batch below 1 MiB");
         ctx->batch_raw_bytes = (size_t) value;
+        return ZWZ_OK;
+    }
+    if (what == ZWZ_TUNE_HOST_THREADS) {
+        if (value > 256) return fail(ctx, ZWZ_E_ARG, "more than 256 host threads");
+        ctx->pool.reset(); // the next call that wants threads starts as many as asked
+        ctx->host_threads = (unsigned) value;
+        return ZWZ_OK;
+    }
+    if (what == ZWZ_TUNE_HOST_PARALLEL_MIN) {
+        ctx->host_parallel_min = value;
         return ZWZ_OK;
     }
     return fail(ctx, ZWZ_E_ARG, "unknown tuning knob");
@@ -431,84 +605,144 @@ int zwz_deflate_batch_device_ex(zwz_ctx *ctx, const uint8_t *d_raw, const uint64
     if (!off || !len || !out_off || !res || !d_out) return fail(ctx, ZWZ_E_ARG, "null argument");
     zwz_rt::set_device(ctx->device);
     zwz_stream_t st = stream_v ? (zwz_stream_t) stream_v : ctx->stream;
-    uint64_t total_raw = 0;
-    for (uint32_t i = 0; i < n; ++i) {
-        if (len[i] > ZWZ_CHUNK_SIZE) return fail(ctx, ZWZ_E_ARG, "chunk longer than 65535 bytes");
-        if (format == ZWZ_FORMAT_GZIP && len[i] > ZWZ_BGZF_BLOCK) return fail(ctx, ZWZ_E_ARG, "gzip chunk longer than ZWZ_BGZF_BLOCK bytes");
-        if (out_off[i] & 3u) return fail(ctx, ZWZ_E_ARG, "out_off must be a multiple of 4");
-        total_raw += len[i];
+    Trace tr(ctx, "deflate_device", st);
+    ctx->keep_n = 0;
+    // uint32 scratch entries of a chunk: best match per position (+ pad so the parser may peek one past the end), then the u16
+    // position lists of lz_match_kernel (deflate_match.cuh: dm_scratch_match_words; zwz_common.cuh: scratch layout)
+    auto scr_words = [](uint32_t l) { return align_up((size_t) l + 2, 32) + align_up(((size_t) l + 1) / 2 + 32, 32) + ZWZ_SCR_FLAG_WORDS; };
+    // validation, raw bytes and scratch words per block: the first bad chunk of the first block that has one names the error
+    struct Part {
+        uint64_t raw = 0, scr = 0;
+        const char *bad = nullptr;
+    };
+    const unsigned nb = host_blocks(ctx, n);
+    std::vector<Part> part(nb);
+    host_for(ctx, nb, n, [&](unsigned k, size_t lo, size_t hi) {
+        Part p;
+        for (size_t i = lo; i < hi && !p.bad; ++i) {
+            if (len[i] > ZWZ_CHUNK_SIZE) p.bad = "chunk longer than 65535 bytes";
+            else if (format == ZWZ_FORMAT_GZIP && len[i] > ZWZ_BGZF_BLOCK) p.bad = "gzip chunk longer than ZWZ_BGZF_BLOCK bytes";
+            else if (out_off[i] & 3u) p.bad = "out_off must be a multiple of 4";
+            p.raw += len[i];
+            p.scr += scr_words(len[i]);
+        }
+        part[k] = p;
+    });
+    uint64_t total_raw = 0, total_scr = 0;
+    for (const Part &p : part) {
+        if (p.bad) return fail(ctx, ZWZ_E_ARG, p.bad);
+        total_raw += p.raw;
+        total_scr += p.scr;
     }
     if (total_raw && !d_raw) return fail(ctx, ZWZ_E_ARG, "null raw buffer");
+    tr.mark("validate");
 
-    // descriptors: [raw_off u64][scr_off u64][out_off u64][raw_len u32][order u32] per chunk, then results + adler on the device
-    const size_t meta_bytes = (size_t) n * (8 + 8 + 8 + 4 + 4);
-    const size_t dev_meta_bytes = align_up(meta_bytes, 256) + (size_t) n * 16 + (size_t) n * 8 + 256;
+    // descriptors: [raw_off u64][scr_off u64][raw_len u32][order u32] per chunk, then Adler-32 + match counts on the device;
+    // slot offsets and results in the keep arenas ([out_off u64][results 16 B] per chunk)
+    const size_t meta_bytes = (size_t) n * (8 + 8 + 4 + 4), keep_bytes = keep_res_off(n) + (size_t) n * 16;
+    const size_t dev_meta_bytes = align_up(meta_bytes, 256) + (size_t) n * 8 + 256;
     int rc;
-    if ((rc = reserve(ctx, ctx->pin_meta, std::max(meta_bytes, (size_t) n * 16), true))) return rc;
+    if ((rc = reserve(ctx, ctx->pin_meta, meta_bytes, true))) return rc;
     if ((rc = reserve(ctx, ctx->meta, dev_meta_bytes, false))) return rc;
+    if ((rc = reserve(ctx, ctx->pin_keep, keep_bytes, true))) return rc;
+    if ((rc = reserve(ctx, ctx->keep, keep_bytes, false))) return rc;
 
     uint64_t *h_raw_off = (uint64_t *) ctx->pin_meta.p;
     uint64_t *h_scr_off = h_raw_off + n;
-    uint64_t *h_out_off = h_scr_off + n;
-    uint32_t *h_len = (uint32_t *) (h_out_off + n);
+    uint32_t *h_len = (uint32_t *) (h_scr_off + n);
     uint32_t *h_order = h_len + n;
+    uint64_t *h_out_off = (uint64_t *) ctx->pin_keep.p;
 
-    // sub-batches bounded by scratch: scratch offsets restart at 0 in every sub-batch
-    std::vector<uint32_t> sub_begin;
-    size_t max_scr = 0;
-    {
-        size_t scr = 0, raw = 0;
-        sub_begin.push_back(0);
+    // sub-batches bounded by scratch: a new one starts at the chunk that would take the current one past batch_raw_bytes
+    std::vector<uint32_t> sub_begin{0};
+    if (total_raw > ctx->batch_raw_bytes) {
+        uint64_t raw = 0;
         for (uint32_t i = 0; i < n; ++i) {
             if (raw + len[i] > ctx->batch_raw_bytes && i > sub_begin.back()) {
-                max_scr = std::max(max_scr, scr);
                 sub_begin.push_back(i);
-                scr = 0;
                 raw = 0;
             }
-            h_raw_off[i] = off[i];
-            h_scr_off[i] = scr;
-            h_out_off[i] = out_off[i];
-            h_len[i] = len[i];
-            // uint32 entries: best match per position (+ pad so the parser may peek one past the end), then the u16 position
-            // lists of lz_match_kernel (deflate_match.cuh: dm_scratch_match_words)
-            scr += align_up((size_t) len[i] + 2, 32) + align_up(((size_t) len[i] + 1) / 2 + 32, 32) + ZWZ_SCR_FLAG_WORDS; // zwz_common.cuh: scratch layout
             raw += len[i];
         }
-        max_scr = std::max(max_scr, scr);
-        sub_begin.push_back(n);
     }
-    if ((rc = reserve(ctx, ctx->scratch, max_scr * 4 + 256, false))) return rc;
-    // size classes (deflate_match.cuh): per sub-batch, chunk indices grouped by class, longest first inside a class so the
-    // persistent CTAs end together
+    sub_begin.push_back(n);
     const size_t nsub = sub_begin.size() - 1;
-    std::vector<uint32_t> cls_begin(nsub * 5);
+    // scratch offsets: a blocked prefix sum over all chunks, then restarted at 0 in every sub-batch
+    const Staging stg(nb);
+    host_for(ctx, nb, n, [&](unsigned k, size_t lo, size_t hi) {
+        uint64_t scr = 0;
+        for (unsigned j = 0; j < k; ++j) scr += part[j].scr;
+        for (size_t i = lo; i < hi; ++i) {
+            stg.put(h_raw_off + i, off[i]);
+            stg.put(h_scr_off + i, scr);
+            stg.put(h_out_off + i, out_off[i]);
+            stg.put(h_len + i, len[i]);
+            scr += scr_words(len[i]);
+        }
+        stg.done();
+    });
+    size_t max_scr = 0;
     for (size_t s = 0; s < nsub; ++s) {
-        uint32_t b = sub_begin[s], e = sub_begin[s + 1];
+        const uint64_t s0 = h_scr_off[sub_begin[s]], s1 = s + 1 < nsub ? h_scr_off[sub_begin[s + 1]] : total_scr;
+        max_scr = std::max<size_t>(max_scr, s1 - s0);
+        if (s)
+            for (uint32_t i = sub_begin[s]; i < sub_begin[s + 1]; ++i) h_scr_off[i] -= s0;
+    }
+    tr.mark("stage");
+    if ((rc = reserve(ctx, ctx->scratch, max_scr * 4 + 256, false))) return rc;
+    // size classes (deflate_match.cuh): per sub-batch, chunk indices grouped by class in index order (one counting pass,
+    // counts per class and block, then a scatter), longest first inside a class so the persistent CTAs end together
+    std::vector<uint32_t> cls_begin(nsub * 5);
+    static const uint32_t kClassHi[3] = {zwz::MatchClass<0>::kCap, zwz::MatchClass<1>::kCap, zwz::MatchClass<2>::kCap};
+    static_assert(zwz::MatchClass<3>::kCap >= ZWZ_CHUNK_SIZE, "every chunk has a size class");
+    auto cls_of = [](uint32_t l) -> unsigned { return l <= kClassHi[0] ? 0u : (l <= kClassHi[1] ? 1u : (l <= kClassHi[2] ? 2u : 3u)); };
+    for (size_t s = 0; s < nsub; ++s) {
+        const uint32_t b = sub_begin[s], e = sub_begin[s + 1];
         uint32_t *o = h_order + b;
+        const unsigned sb = host_blocks(ctx, e - b);
+        std::vector<uint32_t> pos((size_t) sb * 4);
+        host_for(ctx, sb, e - b, [&](unsigned k, size_t lo, size_t hi) {
+            uint32_t c[4] = {0, 0, 0, 0};
+            for (size_t i = lo; i < hi; ++i) c[cls_of(len[b + i])]++;
+            for (int cls = 0; cls < 4; ++cls) pos[(size_t) k * 4 + cls] = c[cls];
+        });
         uint32_t k = 0;
-        static const uint32_t kClassHi[4] = {zwz::MatchClass<0>::kCap, zwz::MatchClass<1>::kCap, zwz::MatchClass<2>::kCap, zwz::MatchClass<3>::kCap};
         for (int cls = 0; cls < 4; ++cls) {
             cls_begin[s * 5 + cls] = k;
-            uint32_t lo_len = cls == 0 ? 0u : kClassHi[cls - 1] + 1u, hi_len = kClassHi[cls];
-            uint32_t k0 = k;
-            for (uint32_t i = b; i < e; ++i)
-                if (len[i] >= lo_len && len[i] <= hi_len) o[k++] = i - b;
-            auto longer = [&](uint32_t x, uint32_t y) { return len[b + x] > len[b + y]; };
-            if (!std::is_sorted(o + k0, o + k, longer)) std::stable_sort(o + k0, o + k, longer); // size-sorted shards (the reference's deal) skip this
+            for (unsigned j = 0; j < sb; ++j) {
+                const uint32_t c = pos[(size_t) j * 4 + cls];
+                pos[(size_t) j * 4 + cls] = k;
+                k += c;
+            }
         }
         cls_begin[s * 5 + 4] = k;
+        const Staging so(sb);
+        host_for(ctx, sb, e - b, [&](unsigned j, size_t lo, size_t hi) {
+            uint32_t *p = &pos[(size_t) j * 4];
+            for (size_t i = lo; i < hi; ++i) so.put(o + p[cls_of(len[b + i])]++, (uint32_t) i);
+            so.done();
+        });
+        // the four classes side by side (size-sorted shards, the reference's deal, skip the sort)
+        host_for(ctx, sb > 1 ? 4u : 1u, 4, [&](unsigned, size_t c0, size_t c1) {
+            auto longer = [&](uint32_t x, uint32_t y) { return len[b + x] > len[b + y]; };
+            for (size_t cls = c0; cls < c1; ++cls) {
+                uint32_t *o0 = o + cls_begin[s * 5 + cls], *o1 = o + cls_begin[s * 5 + cls + 1];
+                if (!std::is_sorted(o0, o1, longer)) std::stable_sort(o0, o1, longer);
+            }
+        });
     }
+    tr.mark("partition");
     if ((rc = reserve(ctx, ctx->counter, nsub * 32 + 256, false))) return rc;
     if (zwz_rt::memset_device(ctx->counter.p, 0, nsub * 32, st)) return fail(ctx, ZWZ_E_CUDA, "memset failed");
 
     uint8_t *dm = (uint8_t *) ctx->meta.p;
-    if (zwz_rt::memcpy_h2d(dm, ctx->pin_meta.p, meta_bytes, st)) return fail(ctx, ZWZ_E_CUDA, "descriptor upload failed");
-    uint32_t *d_res = (uint32_t *) (dm + align_up(meta_bytes, 256));
-    uint32_t *d_adler = d_res + (size_t) n * 4;
+    uint8_t *dk = (uint8_t *) ctx->keep.p;
+    if (zwz_rt::memcpy_h2d(dm, ctx->pin_meta.p, meta_bytes, st) || zwz_rt::memcpy_h2d(dk, h_out_off, (size_t) n * 8, st))
+        return fail(ctx, ZWZ_E_CUDA, "descriptor upload failed");
+    tr.mark("upload");
+    uint32_t *d_res = (uint32_t *) (dk + keep_res_off(n));
+    uint32_t *d_adler = (uint32_t *) (dm + align_up(meta_bytes, 256));
     uint32_t *d_nmatch = d_adler + n;
-    ctx->last_res_off = align_up(meta_bytes, 256);
-    ctx->last_slot_off = 2 * (size_t) n * 8;
 
     const LevelParams lp = level_params(level);
     for (size_t s = 0; s + 1 < sub_begin.size(); ++s) {
@@ -517,8 +751,8 @@ int zwz_deflate_batch_device_ex(zwz_ctx *ctx, const uint8_t *d_raw, const uint64
         job.raw = d_raw;
         job.raw_off = (const uint64_t *) dm + b;
         job.scr_off = (const uint64_t *) dm + n + b;
-        job.out_off = (const uint64_t *) dm + 2 * (size_t) n + b;
-        job.raw_len = (const uint32_t *) ((const uint64_t *) dm + 3 * (size_t) n) + b;
+        job.out_off = (const uint64_t *) dk + b;
+        job.raw_len = (const uint32_t *) ((const uint64_t *) dm + 2 * (size_t) n) + b;
         job.scratch = (uint32_t *) ctx->scratch.p;
         job.adler = d_adler + b;
         job.nmatch = d_nmatch + b;
@@ -529,7 +763,7 @@ int zwz_deflate_batch_device_ex(zwz_ctx *ctx, const uint8_t *d_raw, const uint64
         job.nice = lp.nice;
         job.work_counter = nullptr;
         job.format = (uint32_t) format;
-        const uint32_t *d_order = (const uint32_t *) ((const uint64_t *) dm + 3 * (size_t) n) + n + b;
+        const uint32_t *d_order = (const uint32_t *) ((const uint64_t *) dm + 2 * (size_t) n) + n + b;
         uint32_t *d_counters = (uint32_t *) ctx->counter.p + s * 8; // [0..3] match classes, [4] encoder
         for (int cls = 0; cls < 4; ++cls) {
             uint32_t w0 = cls_begin[s * 5 + cls], w1 = cls_begin[s * 5 + cls + 1];
@@ -567,11 +801,14 @@ int zwz_deflate_batch_device_ex(zwz_ctx *ctx, const uint8_t *d_raw, const uint64
         }
         if ((rc = check_launch(ctx, "deflate_encode_kernel"))) return rc;
     }
-    // results come back through the pinned arena (descriptors are no longer needed once the kernels are queued ... but
-    // the H2D above must have completed before we overwrite it: same stream => ordered)
-    if (zwz_rt::memcpy_d2h(ctx->pin_meta.p, d_res, (size_t) n * 16, st) || zwz_rt::stream_sync(st))
-        return fail(ctx, ZWZ_E_CUDA, "deflate kernels failed");
-    memcpy(res, ctx->pin_meta.p, (size_t) n * 16);
+    tr.mark("kernels");
+    // results come back behind the slot offsets in pin_keep, which then holds what zwz_pack_streams_device compares with
+    uint8_t *h_res = (uint8_t *) ctx->pin_keep.p + keep_res_off(n);
+    if (zwz_rt::memcpy_d2h(h_res, d_res, (size_t) n * 16, st) || zwz_rt::stream_sync(st)) return fail(ctx, ZWZ_E_CUDA, "deflate kernels failed");
+    tr.mark("download");
+    host_copy(ctx, res, h_res, (size_t) n * 16, n);
+    ctx->keep_n = n;
+    tr.mark("copy-out");
     return ZWZ_OK;
 }
 
@@ -642,10 +879,9 @@ static int deflate_host_impl(zwz_ctx *ctx, const uint8_t *raw, const uint64_t *o
     uint8_t *d_poff = (uint8_t *) ctx->packed.p;
     uint8_t *d_packed = d_poff + align_up(pm, 256);
     if (zwz_rt::memcpy_h2d(d_poff, ctx->pin_meta.p, pm, ctx->stream)) return fail(ctx, ZWZ_E_CUDA, "offset upload failed");
-    // slot offsets and results are still in ctx->meta from the call above
-    const uint8_t *dm = (const uint8_t *) ctx->meta.p;
-    const uint64_t *d_slot_off = (const uint64_t *) (dm + ctx->last_slot_off);
-    const uint32_t *d_res = (const uint32_t *) (dm + ctx->last_res_off);
+    // slot offsets and results are still in ctx->keep from the call above
+    const uint64_t *d_slot_off = (const uint64_t *) ctx->keep.p;
+    const uint32_t *d_res = (const uint32_t *) ((const uint8_t *) ctx->keep.p + keep_res_off(n));
     {
         ProfSpan ps(ctx, ZWZ_PROF_PACK, ctx->stream);
         ZWZ_LAUNCH(zwz::pack_streams_kernel, (n + 7) / 8, 256, 0, ctx->stream, (const uint8_t *) ctx->bulk_out.p, d_slot_off, d_res, d_packed,
@@ -670,24 +906,59 @@ int zwz_pack_streams_device(zwz_ctx *ctx, const uint8_t *d_slots, const uint64_t
     if (!slot_off || !res || !d_slots || !d_packed) return fail(ctx, ZWZ_E_ARG, "null argument");
     zwz_rt::set_device(ctx->device);
     zwz_stream_t st = stream_v ? (zwz_stream_t) stream_v : ctx->stream;
-    for (uint32_t i = 0; i < n; ++i) packed_off[i + 1] = packed_off[i] + res[i].len0 + res[i].len1;
+    Trace tr(ctx, "pack_device", st);
     const size_t m_poff = (size_t) n * 8, m_res = m_poff + (size_t) (n + 1) * 8, meta_bytes = m_res + (size_t) n * 16;
     int rc;
     if ((rc = reserve(ctx, ctx->pin_meta, meta_bytes, true))) return rc;
     if ((rc = reserve(ctx, ctx->meta, meta_bytes + 256, false))) return rc;
     uint8_t *hp = (uint8_t *) ctx->pin_meta.p;
-    memcpy(hp, slot_off, (size_t) n * 8);
-    memcpy(hp + m_poff, packed_off, (size_t) (n + 1) * 8);
-    memcpy(hp + m_res, res, (size_t) n * 16);
+    uint64_t *h_poff = (uint64_t *) (hp + m_poff);
+    // packed offsets: a blocked prefix sum. Beside it, the caller's slot offsets and results are compared with what the last
+    // deflate call used and returned: where they are equal, its device copies in ctx->keep are used and not uploaded again
+    const unsigned nb = host_blocks(ctx, n);
+    const bool kept = ctx->keep_n == n;
+    const uint8_t *hk = (const uint8_t *) ctx->pin_keep.p;
+    std::vector<uint64_t> sum(nb);
+    std::vector<char> same(nb, 0);
+    host_for(ctx, nb, n, [&](unsigned k, size_t lo, size_t hi) {
+        uint64_t a = 0;
+        for (size_t i = lo; i < hi; ++i) a += (uint64_t) res[i].len0 + res[i].len1;
+        sum[k] = a;
+        same[k] = kept && !memcmp(hk + lo * 8, slot_off + lo, (hi - lo) * 8) && !memcmp(hk + keep_res_off(n) + lo * 16, res + lo, (hi - lo) * 16);
+    });
+    const bool reuse = kept && std::all_of(same.begin(), same.end(), [](char c) { return c != 0; });
+    tr.mark("prefix+compare");
+    h_poff[0] = 0;
+    const Staging stg(nb);
+    host_for(ctx, nb, n, [&](unsigned k, size_t lo, size_t hi) {
+        uint64_t a = 0;
+        for (unsigned j = 0; j < k; ++j) a += sum[j];
+        for (size_t i = lo; i < hi; ++i) {
+            a += (uint64_t) res[i].len0 + res[i].len1;
+            packed_off[i + 1] = a;
+            stg.put(h_poff + i + 1, a);
+        }
+        if (!reuse) {
+            stg.copy(hp + lo * 8, slot_off + lo, (hi - lo) * 8);
+            stg.copy(hp + m_res + lo * 16, res + lo, (hi - lo) * 16);
+        }
+        stg.done();
+    });
+    tr.mark("stage");
     uint8_t *dm = (uint8_t *) ctx->meta.p;
-    if (zwz_rt::memcpy_h2d(dm, hp, meta_bytes, st)) return fail(ctx, ZWZ_E_CUDA, "descriptor upload failed");
+    const uint8_t *d_slot_off = reuse ? (const uint8_t *) ctx->keep.p : dm;
+    const uint8_t *d_res = reuse ? (const uint8_t *) ctx->keep.p + keep_res_off(n) : dm + m_res;
+    if (reuse ? zwz_rt::memcpy_h2d(dm + m_poff, h_poff, (size_t) (n + 1) * 8, st) : zwz_rt::memcpy_h2d(dm, hp, meta_bytes, st))
+        return fail(ctx, ZWZ_E_CUDA, "descriptor upload failed");
+    tr.mark("upload");
     {
         ProfSpan ps(ctx, ZWZ_PROF_PACK, st);
-        ZWZ_LAUNCH(zwz::pack_streams_kernel, (n + 7) / 8, 256, 0, st, d_slots, (const uint64_t *) dm, (const uint32_t *) (dm + m_res), d_packed,
+        ZWZ_LAUNCH(zwz::pack_streams_kernel, (n + 7) / 8, 256, 0, st, d_slots, (const uint64_t *) d_slot_off, (const uint32_t *) d_res, d_packed,
                    (const uint64_t *) (dm + m_poff), n);
     }
     if ((rc = check_launch(ctx, "pack_streams_kernel"))) return rc;
     if (zwz_rt::stream_sync(st)) return fail(ctx, ZWZ_E_CUDA, "pack kernel failed");
+    tr.mark("kernels");
     return ZWZ_OK;
 }
 
@@ -764,6 +1035,7 @@ int zwz_inflate_batch_device(zwz_ctx *ctx, const uint8_t *d_comp, const uint64_t
     if (format != ZWZ_FORMAT_ZLIB && ctx->inflate_mode == 2) return fail(ctx, ZWZ_E_ARG, "the one-lane-per-stream decoder reads zlib streams only");
     zwz_rt::set_device(ctx->device);
     zwz_stream_t st = stream_v ? (zwz_stream_t) stream_v : ctx->stream;
+    Trace tr(ctx, "inflate_device", st);
     // Mapping: one warp per stream (inflate.cuh) is the product path. One lane per stream (inflate_lanes.cuh,
     // ZWZ_INFLATE_MODE=lanes) needs ~40x fewer warp-instructions per byte but only three warps fit an SM next to its
     // per-lane tables, and at that occupancy it runs latency-bound: 140 ms against 68 ms per C2 step on B200. It stays as a
@@ -778,9 +1050,15 @@ int zwz_inflate_batch_device(zwz_ctx *ctx, const uint8_t *d_comp, const uint64_t
     if ((rc = reserve(ctx, ctx->pin_meta, std::max(meta_bytes, (size_t) n * 8), true))) return rc;
     if ((rc = reserve(ctx, ctx->meta, r_base + (size_t) n * 8 + 512, false))) return rc;
     uint8_t *hp = (uint8_t *) ctx->pin_meta.p;
-    memcpy(hp + m_off, off, (size_t) n * 8);
-    memcpy(hp + m_roff, raw_off, (size_t) (n + 1) * 8);
-    memcpy(hp + m_len, len, (size_t) n * 4);
+    const unsigned nb = host_blocks(ctx, n);
+    const Staging stg(nb);
+    host_for(ctx, nb, n, [&](unsigned, size_t lo, size_t hi) {
+        stg.copy(hp + m_off + lo * 8, off + lo, (hi - lo) * 8);
+        stg.copy(hp + m_roff + lo * 8, raw_off + lo, (hi - lo) * 8);
+        stg.copy(hp + m_len + lo * 4, len + lo, (hi - lo) * 4);
+        stg.done();
+    });
+    ((uint64_t *) (hp + m_roff))[n] = raw_off[n];
     if (lanes) {
         // streams by decreasing compressed size (counting sort on len / 32), so that the 32 lanes of a warp finish together
         // and the longest groups start first
@@ -792,8 +1070,10 @@ int zwz_inflate_batch_device(zwz_ctx *ctx, const uint8_t *d_comp, const uint64_t
         uint32_t *order = (uint32_t *) (hp + m_order);
         for (uint32_t i = 0; i < n; ++i) order[head[bucket(len[i])]++] = i;
     }
+    tr.mark("stage");
     uint8_t *dm = (uint8_t *) ctx->meta.p;
     if (zwz_rt::memcpy_h2d(dm, hp, meta_bytes, st)) return fail(ctx, ZWZ_E_CUDA, "descriptor upload failed");
+    tr.mark("upload");
     uint32_t *d_rlen = (uint32_t *) (dm + r_base);
     uint32_t *d_stat = d_rlen + n;
     uint32_t *d_counter = d_stat + n; // work queue head of the persistent warps
@@ -813,9 +1093,14 @@ int zwz_inflate_batch_device(zwz_ctx *ctx, const uint8_t *d_comp, const uint64_t
         }
     }
     if ((rc = check_launch(ctx, "inflate_kernel"))) return rc;
+    tr.mark("kernels");
     if (zwz_rt::memcpy_d2h(hp, d_rlen, (size_t) n * 8, st) || zwz_rt::stream_sync(st)) return fail(ctx, ZWZ_E_CUDA, "inflate kernel failed");
-    memcpy(raw_len, hp, (size_t) n * 4);
-    memcpy(status, hp + (size_t) n * 4, (size_t) n * 4);
+    tr.mark("download");
+    host_for(ctx, nb, n, [&](unsigned, size_t lo, size_t hi) {
+        memcpy(raw_len + lo, hp + lo * 4, (hi - lo) * 4);
+        memcpy(status + lo, hp + (size_t) n * 4 + lo * 4, (hi - lo) * 4);
+    });
+    tr.mark("copy-out");
     return ZWZ_OK;
 }
 
@@ -1161,24 +1446,38 @@ int zwz_gunzip_files(zwz_ctx *ctx, const uint8_t *gz, const uint64_t *gz_off, ui
 // Queues the MD5 kernel over n files on `st`: descriptors go up from `pin`, digests (and chained states) come back into `pin`
 // at *digest_off (resp. m_state). Nothing is waited for.
 static int md5_enqueue(zwz_ctx *ctx, zwz_stream_t st, Arena &dev_meta, Arena &pin, uint32_t *state, const uint8_t *d_data, const uint64_t *off,
-                       const uint64_t *len, const uint64_t *total_len, uint32_t n, int finalize, size_t *digest_off) {
+                       const uint64_t *len, const uint64_t *total_len, uint32_t n, int finalize, size_t *digest_off, Trace *tr = nullptr) {
     const size_t m_len = (size_t) n * 8, m_tot = 2 * (size_t) n * 8, m_state = 3 * (size_t) n * 8, meta_bytes = m_state + (size_t) n * 16;
     const size_t r_base = align_up(meta_bytes, 256);
     int rc;
     if ((rc = reserve(ctx, pin, r_base + (size_t) n * 16, true))) return rc;
     if ((rc = reserve(ctx, dev_meta, r_base + (size_t) n * 16 + 256, false))) return rc;
+    // the total length of the files picks the kernel below: summed while the descriptors are staged
     uint8_t *hp = (uint8_t *) pin.p;
-    memcpy(hp, off, (size_t) n * 8);
-    memcpy(hp + m_len, len, (size_t) n * 8);
-    if (total_len) memcpy(hp + m_tot, total_len, (size_t) n * 8);
-    if (state) memcpy(hp + m_state, state, (size_t) n * 16);
+    const unsigned nb = host_blocks(ctx, n);
+    const Staging stg(nb);
+    std::vector<uint64_t> sum(nb);
+    host_for(ctx, nb, n, [&](unsigned k, size_t lo, size_t hi) {
+        stg.copy(hp + lo * 8, off + lo, (hi - lo) * 8);
+        stg.copy(hp + m_len + lo * 8, len + lo, (hi - lo) * 8);
+        if (total_len) stg.copy(hp + m_tot + lo * 8, total_len + lo, (hi - lo) * 8);
+        if (state) stg.copy(hp + m_state + lo * 16, state + lo * 4, (hi - lo) * 16);
+        stg.done();
+        uint64_t a = 0;
+        for (size_t i = lo; i < hi; ++i) a += len[i];
+        sum[k] = a;
+    });
+    if (tr) tr->mark("stage");
+    // only what the kernel reads goes up: the chained states and total lengths only when there are some
+    const size_t up_bytes = state ? meta_bytes : (total_len ? m_state : m_tot);
     uint8_t *dm = (uint8_t *) dev_meta.p;
-    if (zwz_rt::memcpy_h2d(dm, hp, meta_bytes, st)) return fail(ctx, ZWZ_E_CUDA, "descriptor upload failed");
+    if (zwz_rt::memcpy_h2d(dm, hp, up_bytes, st)) return fail(ctx, ZWZ_E_CUDA, "descriptor upload failed");
+    if (tr) tr->mark("upload");
     uint8_t *d_digest = dm + r_base;
     {
         // few long files: the staged kernel (coalesced cp.async into shared memory); many short ones: one lane streams its file
         uint64_t total = 0;
-        for (uint32_t i = 0; i < n; ++i) total += len[i];
+        for (uint64_t a : sum) total += a;
         const bool staged = total / n >= 65536u;
         ProfSpan ps(ctx, ZWZ_PROF_MD5, st);
         if (staged) {
@@ -1205,13 +1504,16 @@ static int md5_launch(zwz_ctx *ctx, uint32_t *state, const uint8_t *d_data, cons
     if (!off || !len || (finalize && !digest)) return fail(ctx, ZWZ_E_ARG, "null argument");
     zwz_rt::set_device(ctx->device);
     zwz_stream_t st = stream_v ? (zwz_stream_t) stream_v : ctx->stream;
+    Trace tr(ctx, "md5_device", st);
     size_t doff = 0;
-    int rc = md5_enqueue(ctx, st, ctx->meta, ctx->pin_meta, state, d_data, off, len, total_len, n, finalize, &doff);
+    int rc = md5_enqueue(ctx, st, ctx->meta, ctx->pin_meta, state, d_data, off, len, total_len, n, finalize, &doff, &tr);
     if (rc) return rc;
     if (zwz_rt::stream_sync(st)) return fail(ctx, ZWZ_E_CUDA, "md5 kernel failed");
+    tr.mark("kernels+download");
     const uint8_t *hp = (const uint8_t *) ctx->pin_meta.p;
-    if (finalize) memcpy(digest, hp + doff, (size_t) n * 16);
+    if (finalize) host_copy(ctx, digest, hp + doff, (size_t) n * 16, n);
     if (state) memcpy(state, hp + 3 * (size_t) n * 8, (size_t) n * 16);
+    tr.mark("copy-out");
     return ZWZ_OK;
 }
 
