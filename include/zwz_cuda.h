@@ -97,7 +97,7 @@ uint64_t zwz_launch_count(const zwz_ctx *ctx);
 #define ZWZ_PROF_INFLATE 2 /* inflate_kernel         */
 #define ZWZ_PROF_MD5 3     /* md5_files_kernel       */
 #define ZWZ_PROF_PACK 4    /* pack_streams_kernel    */
-#define ZWZ_PROF_ADLER 5   /* checksum kernels: adler32_kernel, crc32_kernel */
+#define ZWZ_PROF_ADLER 5   /* checksum kernels: adler32_kernel, crc32_kernel; dict_chain_kernel */
 #define ZWZ_PROF_N 6
 int zwz_profile_enable(zwz_ctx *ctx, int on);
 int zwz_profile_read(zwz_ctx *ctx, double *ms /* [ZWZ_PROF_N] */, uint64_t *launches /* [ZWZ_PROF_N] */, int reset);
@@ -149,6 +149,39 @@ int zwz_inflate_batch_device(zwz_ctx *ctx, const uint8_t *d_comp, const uint64_t
                              uint32_t flags, void *stream);
 int zwz_inflate_batch(zwz_ctx *ctx, const uint8_t *comp, const uint64_t *off, const uint32_t *len, uint32_t n,
                       uint8_t *raw_out, const uint64_t *raw_off, uint32_t *raw_len, uint32_t *status, uint32_t flags);
+
+/* ---- preset dictionaries (zlib's deflateSetDictionary / inflateSetDictionary, Python's zdict=) ----------------------------
+ * A table of dictionaries, and for every chunk / stream the one it uses. Dictionary k is data[off[k] .. off[k+1]) (at most
+ * 2^30 bytes); only its last min(len, 32 768) bytes are the window a stream may refer into, as if they came just before the
+ * stream's first byte. An empty dictionary is no dictionary. `dicts == NULL` is exactly the call without _dict.
+ *   deflate ZLIB : a chunk with a dictionary is written as 78 BB + DICTID (big-endian Adler-32 of the WHOLE dictionary, as
+ *                  deflateSetDictionary), body, Adler-32 of the chunk; it never splits (len1 == 0).
+ *   deflate RAW  : the body may refer into the dictionary; nothing in the stream names it.
+ *   deflate GZIP : a dictionary on any chunk is ZWZ_E_ARG (zlib refuses gzip dictionaries too).
+ *   inflate ZLIB : FDICT with a dictionary: the DICTID must be the dictionary's Adler-32 (also with ZWZ_INFLATE_NO_ADLER), else
+ *                  ZWZ_STREAM_BAD with 0 bytes; FDICT without one: ZWZ_STREAM_BAD; no FDICT: the dictionary is ignored. A
+ *                  stream that ends inside the DICTID is ZWZ_STREAM_TRUNCATED.
+ *   inflate RAW  : the dictionary is the window before the first byte.
+ *   inflate GZIP : a dictionary is ZWZ_E_ARG; so is any dictionary with ZWZ_INFLATE_MODE=lanes.
+ * Chunks / streams marked ZWZ_NO_DICT in a call with dictionaries come out exactly as in the call without. An idx[i] that is
+ * neither ZWZ_NO_DICT nor < ndict, or a NULL off, is ZWZ_E_ARG. Not available for .zwz records (zwz_compress_files,
+ * zwz_decompress_records): the reference's reader inflates without a dictionary. */
+#define ZWZ_NO_DICT 0xffffffffu
+typedef struct zwz_dicts {
+    const uint8_t *data;  /* dictionary k = data[off[k] .. off[k+1]); DEVICE pointer for *_device calls, host pointer otherwise */
+    const uint64_t *off;  /* host, ndict + 1 entries                                                                        */
+    uint32_t ndict;
+    const uint32_t *idx;  /* host, n entries: the dictionary of chunk / stream i, or ZWZ_NO_DICT; NULL = dictionary 0 for all */
+} zwz_dicts;
+int zwz_deflate_batch_device_dict(zwz_ctx *ctx, const uint8_t *d_raw, const uint64_t *off, const uint32_t *len, uint32_t n, uint8_t *d_out,
+                                  const uint64_t *out_off, zwz_deflate_result *res, int level, int format, const zwz_dicts *dicts, void *stream);
+int zwz_deflate_batch_dict(zwz_ctx *ctx, const uint8_t *raw, const uint64_t *off, const uint32_t *len, uint32_t n, uint8_t *out,
+                           uint64_t out_cap, uint64_t *packed_off, zwz_deflate_result *res, int level, int format, const zwz_dicts *dicts);
+int zwz_inflate_batch_device_dict(zwz_ctx *ctx, const uint8_t *d_comp, const uint64_t *off, const uint32_t *len, uint32_t n,
+                                  uint8_t *d_raw_out, const uint64_t *raw_off, uint32_t *raw_len, uint32_t *status, uint32_t flags,
+                                  const zwz_dicts *dicts, void *stream);
+int zwz_inflate_batch_dict(zwz_ctx *ctx, const uint8_t *comp, const uint64_t *off, const uint32_t *len, uint32_t n, uint8_t *raw_out,
+                           const uint64_t *raw_off, uint32_t *raw_len, uint32_t *status, uint32_t flags, const zwz_dicts *dicts);
 
 /* ---- MD5: verification.cpp:13-27 --------------------------------------------------------------------------------- */
 /* File i is data[off[i] .. off[i]+len[i]) (any length, 0 included). digest = 16 raw bytes per file. */

@@ -24,7 +24,7 @@ import numpy as np
 
 __all__ = ["Context", "ZwzError", "load_library", "library_path", "CHUNK_SIZE", "deflate_bound", "chunk_table",
            "STREAM_END", "STREAM_TRUNCATED", "STREAM_BAD", "STREAM_OUTPUT_FULL", "RESULT_DTYPE",
-           "FORMAT_ZLIB", "FORMAT_GZIP", "FORMAT_RAW", "BGZF_BLOCK"]
+           "FORMAT_ZLIB", "FORMAT_GZIP", "FORMAT_RAW", "BGZF_BLOCK", "NO_DICT"]
 
 CHUNK_SIZE = 65535  # process.hpp:12
 STREAM_END, STREAM_TRUNCATED, STREAM_BAD, STREAM_OUTPUT_FULL = 0, 1, 2, 3
@@ -39,6 +39,46 @@ def _format(name: str) -> int:
     if name not in _FORMATS:
         raise ValueError(f"format must be one of {sorted(_FORMATS)}, not {name!r}")
     return _FORMATS[name]
+
+# zdict_index entry of a chunk / stream without a preset dictionary (ZWZ_NO_DICT)
+NO_DICT = 0xFFFFFFFF
+
+
+class _Dicts(C.Structure):  # zwz_dicts
+    _fields_ = [("data", C.c_void_p), ("off", C.c_void_p), ("ndict", C.c_uint32), ("idx", C.c_void_p)]
+
+
+def _dicts(zdict, zdict_index, n: int, device: bool):
+    """The zwz_dicts of a call -> (pointer argument or None, arrays to keep alive during the call). zdict: host forms take bytes
+    (one dictionary for all) or a list of bytes; device forms take (device pointer, offsets[ndict+1]). zdict_index: the
+    dictionary of every chunk / stream (NO_DICT for none); None = dictionary 0 for all."""
+    if zdict is None:
+        if zdict_index is not None:
+            raise ValueError("zdict_index without zdict")
+        return None, ()
+    if device:
+        data, off = zdict
+        off = np.ascontiguousarray(off, dtype=np.uint64)
+        keep = [off]
+        dptr = int(data)
+    else:
+        parts = [zdict] if isinstance(zdict, (bytes, bytearray, memoryview)) else list(zdict)
+        parts = [bytes(p) for p in parts]
+        off = np.zeros(len(parts) + 1, dtype=np.uint64)
+        np.cumsum([len(p) for p in parts], out=off[1:])
+        data = np.frombuffer(b"".join(parts) + b"\0", dtype=np.uint8)
+        keep = [off, data]
+        dptr = data.ctypes.data
+    idx = None
+    if zdict_index is not None:
+        idx = np.ascontiguousarray(zdict_index, dtype=np.uint32)
+        if len(idx) != n:
+            raise ValueError(f"zdict_index has {len(idx)} entries for {n} chunks / streams")
+        keep.append(idx)
+    s = _Dicts(dptr, off.ctypes.data, len(off) - 1, _ptr(idx) if idx is not None and idx.size else None)
+    keep.append(s)
+    return C.byref(s), keep
+
 
 RESULT_DTYPE = np.dtype([("len0", "<u4"), ("len1", "<u4"), ("raw0", "<u4"), ("btype", "<u4")])
 
@@ -108,6 +148,11 @@ def _declare(L):
     L.zwz_wait.argtypes = [vp, u64]
     L.zwz_profile_enable.argtypes = [vp, i32]
     L.zwz_profile_read.argtypes = [vp, vp, vp, i32]
+    dp = C.POINTER(_Dicts)
+    L.zwz_deflate_batch_device_dict.argtypes = [vp, vp, vp, vp, u32, vp, vp, vp, i32, i32, dp, vp]
+    L.zwz_deflate_batch_dict.argtypes = [vp, vp, vp, vp, u32, vp, u64, vp, vp, i32, i32, dp]
+    L.zwz_inflate_batch_device_dict.argtypes = [vp, vp, vp, vp, u32, vp, vp, vp, vp, u32, dp, vp]
+    L.zwz_inflate_batch_dict.argtypes = [vp, vp, vp, vp, u32, vp, vp, vp, vp, u32, dp]
     return L
 
 
@@ -245,9 +290,10 @@ class Context:
         self._check(self.lib.zwz_sync(self.h))
 
     # ---- deflate: compression.cpp:119-134 ----
-    def deflate_batch(self, raw, off, length, level: int = 0, format: str = "zlib"):
+    def deflate_batch(self, raw, off, length, level: int = 0, format: str = "zlib", zdict=None, zdict_index=None):
         """Host buffers. Returns (packed uint8 array, packed_off[n+1] u64, results[n] RESULT_DTYPE). format: "zlib", "gzip" (one
-        BGZF member per chunk, chunks <= BGZF_BLOCK) or "raw"."""
+        BGZF member per chunk, chunks <= BGZF_BLOCK) or "raw". zdict: a preset dictionary as in Python's zlib (bytes, one for all
+        chunks), or a list of them with zdict_index (the dictionary of every chunk, NO_DICT for none); not in gzip format."""
         raw = _u8(raw)
         off = np.ascontiguousarray(off, dtype=np.uint64)
         length = np.ascontiguousarray(length, dtype=np.uint32)
@@ -256,18 +302,22 @@ class Context:
         out = np.empty(max(cap, 1), dtype=np.uint8)
         poff = np.zeros(n + 1, dtype=np.uint64)
         res = np.zeros(n, dtype=RESULT_DTYPE)
-        self._check(self.lib.zwz_deflate_batch_ex(self.h, _ptr(raw), _ptr(off), _ptr(length), n, _ptr(out), cap, poff.ctypes.data,
-                                                  _ptr(res), level, _format(format)))
+        dicts, _keep = _dicts(zdict, zdict_index, n, device=False)
+        self._check(self.lib.zwz_deflate_batch_dict(self.h, _ptr(raw), _ptr(off), _ptr(length), n, _ptr(out), cap, poff.ctypes.data,
+                                                    _ptr(res), level, _format(format), dicts))
         return out[:int(poff[n])], poff, res
 
-    def deflate_batch_device(self, d_raw: int, off, length, d_out: int, out_off, level: int = 0, stream: int = 0, format: str = "zlib"):
+    def deflate_batch_device(self, d_raw: int, off, length, d_out: int, out_off, level: int = 0, stream: int = 0, format: str = "zlib",
+                             zdict=None, zdict_index=None):
+        """Device buffers. zdict: (device pointer, offsets[ndict+1]) of the preset dictionaries, with zdict_index as in deflate_batch."""
         off = np.ascontiguousarray(off, dtype=np.uint64)
         length = np.ascontiguousarray(length, dtype=np.uint32)
         out_off = np.ascontiguousarray(out_off, dtype=np.uint64)
         n = len(off)
         res = np.zeros(n, dtype=RESULT_DTYPE)
-        self._check(self.lib.zwz_deflate_batch_device_ex(self.h, d_raw, _ptr(off), _ptr(length), n, d_out, _ptr(out_off), _ptr(res), level,
-                                                         _format(format), stream or None))
+        dicts, _keep = _dicts(zdict, zdict_index, n, device=True)
+        self._check(self.lib.zwz_deflate_batch_device_dict(self.h, d_raw, _ptr(off), _ptr(length), n, d_out, _ptr(out_off), _ptr(res), level,
+                                                           _format(format), dicts, stream or None))
         return res
 
     def pack_streams_device(self, d_slots: int, slot_off, res, d_packed: int, stream: int = 0) -> np.ndarray:
@@ -280,9 +330,10 @@ class Context:
         return poff
 
     # ---- inflate: decompression.cpp:11-37 ----
-    def inflate_batch(self, comp, off, length, raw_off, flags: int = 0, format: str = "zlib"):
+    def inflate_batch(self, comp, off, length, raw_off, flags: int = 0, format: str = "zlib", zdict=None, zdict_index=None):
         """Host buffers. raw_off[n+1] gives every stream's output window. Returns (raw_out, raw_len[n], status[n]).
-        format: "zlib", "gzip" (one member per stream, as zlib with windowBits 31) or "raw"."""
+        format: "zlib", "gzip" (one member per stream, as zlib with windowBits 31) or "raw". zdict / zdict_index: preset
+        dictionaries as in deflate_batch (what zlib.decompressobj(wbits, zdict=) is given); not in gzip format."""
         comp = _u8(comp)
         off = np.ascontiguousarray(off, dtype=np.uint64)
         length = np.ascontiguousarray(length, dtype=np.uint32)
@@ -291,19 +342,23 @@ class Context:
         out = np.zeros(max(int(raw_off[n]) if n else 0, 1), dtype=np.uint8)
         rl = np.zeros(n, dtype=np.uint32)
         st = np.zeros(n, dtype=np.uint32)
-        self._check(self.lib.zwz_inflate_batch(self.h, _ptr(comp), _ptr(off), _ptr(length), n, _ptr(out), _ptr(raw_off), _ptr(rl), _ptr(st),
-                                               flags | (_format(format) << 8)))
+        dicts, _keep = _dicts(zdict, zdict_index, n, device=False)
+        self._check(self.lib.zwz_inflate_batch_dict(self.h, _ptr(comp), _ptr(off), _ptr(length), n, _ptr(out), _ptr(raw_off), _ptr(rl), _ptr(st),
+                                                    flags | (_format(format) << 8), dicts))
         return out, rl, st
 
-    def inflate_batch_device(self, d_comp: int, off, length, d_raw_out: int, raw_off, flags: int = 0, stream: int = 0, format: str = "zlib"):
+    def inflate_batch_device(self, d_comp: int, off, length, d_raw_out: int, raw_off, flags: int = 0, stream: int = 0, format: str = "zlib",
+                             zdict=None, zdict_index=None):
+        """Device buffers. zdict: (device pointer, offsets[ndict+1]) of the preset dictionaries, with zdict_index as in deflate_batch."""
         off = np.ascontiguousarray(off, dtype=np.uint64)
         length = np.ascontiguousarray(length, dtype=np.uint32)
         raw_off = np.ascontiguousarray(raw_off, dtype=np.uint64)
         n = len(off)
         rl = np.zeros(n, dtype=np.uint32)
         st = np.zeros(n, dtype=np.uint32)
-        self._check(self.lib.zwz_inflate_batch_device(self.h, d_comp, _ptr(off), _ptr(length), n, d_raw_out, _ptr(raw_off), _ptr(rl), _ptr(st),
-                                                      flags | (_format(format) << 8), stream or None))
+        dicts, _keep = _dicts(zdict, zdict_index, n, device=True)
+        self._check(self.lib.zwz_inflate_batch_device_dict(self.h, d_comp, _ptr(off), _ptr(length), n, d_raw_out, _ptr(raw_off), _ptr(rl), _ptr(st),
+                                                           flags | (_format(format) << 8), dicts, stream or None))
         return rl, st
 
     def decompress_records(self, comp, off, length, rec_cap, rec_file, nf: int, out_cap: int, want_md5: bool = True, flags: int = 0):

@@ -299,8 +299,13 @@ ZWZ_DEV_NOINLINE uint32_t enc_adler_global(const uint8_t *p, uint32_t n) {
 }
 
 // wrapper bytes in front of the DEFLATE body, and in front plus behind it
-ZWZ_DEV uint32_t enc_head_bytes(uint32_t format) { return format == ZWZ_FORMAT_GZIP ? 18u : (format == ZWZ_FORMAT_ZLIB ? 2u : 0u); }
-ZWZ_DEV uint32_t enc_wrap_bytes(uint32_t format) { return format == ZWZ_FORMAT_GZIP ? 26u : (format == ZWZ_FORMAT_ZLIB ? 6u : 0u); }
+// ZWZ_WRAP_ZLIB_DICT: the wrapper of a zlib chunk with a preset dictionary, 78 BB (FDICT set) + DICTID in front. It has no split
+// rule and no 65 535-byte limit (neither has GZIP or RAW): the split rule serves .zwz records, which never have a dictionary.
+#define ZWZ_WRAP_ZLIB_DICT 3u
+ZWZ_DEV uint32_t enc_head_bytes(uint32_t format) {
+    return format == ZWZ_FORMAT_GZIP ? 18u : (format == ZWZ_FORMAT_ZLIB ? 2u : (format == ZWZ_WRAP_ZLIB_DICT ? 6u : 0u));
+}
+ZWZ_DEV uint32_t enc_wrap_bytes(uint32_t format) { return enc_head_bytes(format) + (format == ZWZ_FORMAT_GZIP ? 8u : (format == ZWZ_FORMAT_RAW ? 0u : 4u)); }
 
 // BSIZE of a BGZF member header (bytes 16-17): the member's length minus 1
 ZWZ_DEV void enc_bgzf_bsize(uint8_t *out, uint32_t member_bytes) {
@@ -309,13 +314,17 @@ ZWZ_DEV void enc_bgzf_bsize(uint8_t *out, uint32_t member_bytes) {
 }
 
 // one complete stream in `format` with a single stored block (check = Adler-32 for zlib, CRC-32 for gzip); returns its size
-ZWZ_DEV_NOINLINE uint32_t enc_stored_stream(uint8_t *out, const uint8_t *src, uint32_t n, uint32_t check, uint32_t format) {
+ZWZ_DEV_NOINLINE uint32_t enc_stored_stream(uint8_t *out, const uint8_t *src, uint32_t n, uint32_t check, uint32_t format, uint32_t dictid) {
     const unsigned lane = lane_id();
     const uint32_t h = enc_head_bytes(format);
     if (lane == 0) {
         if (format == ZWZ_FORMAT_ZLIB) {
             out[0] = 0x78;
             out[1] = 0x9c;
+        } else if (format == ZWZ_WRAP_ZLIB_DICT) {
+            out[0] = 0x78;
+            out[1] = 0xbb;
+            for (int i = 0; i < 4; ++i) out[2 + i] = (uint8_t) (dictid >> (24 - 8 * i));
         } else if (format == ZWZ_FORMAT_GZIP) {
             uint32_t *w = (uint32_t *) out; // the slot start: 4-byte aligned
             w[0] = 0x04088b1fu;             // 1f 8b 08 04 | MTIME 0 | XFL 0, OS ff | XLEN 6 | 'B' 'C' 2 0
@@ -330,7 +339,7 @@ ZWZ_DEV_NOINLINE uint32_t enc_stored_stream(uint8_t *out, const uint8_t *src, ui
         out[h + 3u] = (uint8_t) ~n;
         out[h + 4u] = (uint8_t) (~n >> 8);
         uint8_t *t = out + h + 5u + n;
-        if (format == ZWZ_FORMAT_ZLIB) {
+        if (format == ZWZ_FORMAT_ZLIB || format == ZWZ_WRAP_ZLIB_DICT) {
             t[0] = (uint8_t) (check >> 24);
             t[1] = (uint8_t) (check >> 16);
             t[2] = (uint8_t) (check >> 8);
@@ -588,13 +597,17 @@ ZWZ_DEV_NOINLINE void enc_emit_block(BitSink *kp, const uint32_t *m, uint32_t t0
 }
 
 // The wrapper around the Huffman-coded body (out of line: the format costs the encoder's main loop no registers).
-// Header: zlib 78 9C; gzip the 18-byte BGZF header with BSIZE left 0 (set by enc_wrap_tail); raw none.
-ZWZ_DEV_NOINLINE void enc_wrap_head(BitSink *kp, uint32_t format) {
+// Header: zlib 78 9C (78 BB + DICTID big-endian with a preset dictionary); gzip the 18-byte BGZF header with BSIZE left 0 (set by
+// enc_wrap_tail); raw none.
+ZWZ_DEV_NOINLINE void enc_wrap_head(BitSink *kp, uint32_t format, uint32_t dictid) {
     EncWarpSmem &S = enc_smem();
     const unsigned lane = lane_id();
     BitSink k = *kp;
     if (format == ZWZ_FORMAT_ZLIB) {
         sink_put(S, k, lane == 0 ? 0x9c78ull : 0ull, lane == 0 ? 16u : 0u); // RFC 1950 header 78 9C
+    } else if (format == ZWZ_WRAP_ZLIB_DICT) {
+        const uint32_t be = ((dictid & 0xffu) << 24) | ((dictid & 0xff00u) << 8) | ((dictid >> 8) & 0xff00u) | (dictid >> 24);
+        sink_put(S, k, lane == 0 ? 0xbb78ull : (lane == 1u ? (uint64_t) be : 0ull), lane == 0 ? 16u : (lane == 1u ? 32u : 0u));
     } else if (format == ZWZ_FORMAT_GZIP) {
         // 1f 8b 08 04 | MTIME 0 | XFL 0, OS ff | XLEN 6 | 'B' 'C' 2 0 | BSIZE
         const uint32_t w = lane == 0 ? 0x04088b1fu : (lane == 2u ? 0x0006ff00u : (lane == 3u ? 0x00024342u : 0u));
@@ -613,7 +626,7 @@ ZWZ_DEV_NOINLINE void enc_wrap_tail(BitSink *kp, uint32_t format, uint32_t check
     uint64_t v = 0;
     uint32_t nb = lane == 0 ? padbits : 0u;
     if (lane == 1u && format != ZWZ_FORMAT_RAW) {
-        v = format == ZWZ_FORMAT_ZLIB ? be : check;
+        v = format == ZWZ_FORMAT_GZIP ? check : be;
         nb = 32u;
     } else if (lane == 2u && format == ZWZ_FORMAT_GZIP) {
         v = n;
@@ -774,9 +787,18 @@ ZWZ_DEV_NOINLINE void enc_emit_range(BitSink *kp, const uint32_t *m, uint32_t t0
     enc_emit_block(kp, m, t0, t1, xb, last);
 }
 
-ZWZ_DEV void enc_chunk(EncWarpSmem &S, const DeflateJob &job, uint32_t c) {
+template <bool DICT> ZWZ_DEV void enc_chunk(EncWarpSmem &S, const DeflateJob &job, uint32_t c) {
     const unsigned lane = lane_id();
     const uint32_t n = job.raw_len[c];
+    // the wrapper of this chunk: a zlib chunk with a preset dictionary names it in its header (RAW streams do not)
+    uint32_t fmt = job.format, dictid = 0;
+    if (DICT) {
+        const uint32_t di = job.dict.idx[c];
+        if (di != ZWZ_NO_DICT && fmt == ZWZ_FORMAT_ZLIB) {
+            fmt = ZWZ_WRAP_ZLIB_DICT;
+            dictid = job.dict.id[di];
+        }
+    }
     const uint8_t *src = job.raw + job.raw_off[c];
     uint32_t *m = job.scratch + job.scr_off[c];
     uint8_t *out = job.out + job.out_off[c];
@@ -796,8 +818,8 @@ ZWZ_DEV void enc_chunk(EncWarpSmem &S, const DeflateJob &job, uint32_t c) {
         uint32_t nu;
         const float hb = enc_entropy_bits(0u, &nu);
         const float bound_bytes = hb * 0.125f + 7.f + (float) (nu >> 2);
-        if (bound_bytes * 0.9995f >= (float) (n + 11u) - (float) (n >> 8) && (job.format != ZWZ_FORMAT_ZLIB || n + 11u <= ZWZ_CHUNK)) {
-            uint32_t l0 = enc_stored_stream(out, src, n, job.adler[c], job.format);
+        if (bound_bytes * 0.9995f >= (float) (n + 11u) - (float) (n >> 8) && (fmt != ZWZ_FORMAT_ZLIB || n + 11u <= ZWZ_CHUNK)) {
+            uint32_t l0 = enc_stored_stream(out, src, n, job.adler[c], fmt, dictid);
             if (lane == 0) {
                 job.res[4u * c + 0u] = l0;
                 job.res[4u * c + 1u] = 0u;
@@ -920,7 +942,7 @@ ZWZ_DEV void enc_chunk(EncWarpSmem &S, const DeflateJob &job, uint32_t c) {
     // n/256 bytes the three Huffman constructions below are skipped altogether.
     // The estimates are compared with the zlib-wrapped stored size in every format, so that the choice (and the body) does not
     // depend on the wrapper; the 65 535-byte record limit applies to zlib streams only.
-    const uint32_t sto_bytes = n + 5u + enc_wrap_bytes(job.format);
+    const uint32_t sto_bytes = n + 5u + enc_wrap_bytes(fmt);
     const uint32_t zsto_bytes = n + 11u;
     const uint32_t sto_slack = n >> 8;
     bool force_stored = false;
@@ -947,11 +969,11 @@ ZWZ_DEV void enc_chunk(EncWarpSmem &S, const DeflateJob &job, uint32_t c) {
         // + zlib wrapper and block header, + ~2 bits per used symbol for a dynamic header (a small random sample sits ~23
         // bytes under 8 bits/byte of empirical entropy; its code-length header costs several times that)
         float bound_bytes = (hl_bits + (float) extra_bits) * 0.125f + 7.f + (float) (nused >> 2);
-        force_stored = bound_bytes * 0.9995f >= (float) zsto_bytes - (float) sto_slack && (job.format != ZWZ_FORMAT_ZLIB || zsto_bytes <= ZWZ_CHUNK) &&
+        force_stored = bound_bytes * 0.9995f >= (float) zsto_bytes - (float) sto_slack && (fmt != ZWZ_FORMAT_ZLIB || zsto_bytes <= ZWZ_CHUNK) &&
                        n >= 512u;
     }
     if (force_stored) {
-        uint32_t l0 = enc_stored_stream(out, src, n, job.adler[c], job.format);
+        uint32_t l0 = enc_stored_stream(out, src, n, job.adler[c], fmt, dictid);
         if (lane == 0) {
             job.res[4u * c + 0u] = l0;
             job.res[4u * c + 1u] = 0u;
@@ -973,7 +995,7 @@ ZWZ_DEV void enc_chunk(EncWarpSmem &S, const DeflateJob &job, uint32_t c) {
     const uint32_t cap_words = ((n + ZWZ_DEFLATE_MARGIN + 15u) & ~15u) >> 2; // zwz_deflate_bound(n) / 4
     BitSink k;
     sink_init(S, k, (uint32_t *) out, cap_words);
-    enc_wrap_head(&k, job.format);
+    enc_wrap_head(&k, fmt, dictid);
     __syncwarp();
     const uint32_t nreg = enc_find_stored_regions(m, n, ntok);
     if (nreg == 0u) {
@@ -989,22 +1011,22 @@ ZWZ_DEV void enc_chunk(EncWarpSmem &S, const DeflateJob &job, uint32_t c) {
         if (t < ntok) enc_emit_range(&k, m, t, ntok, 0, true, false);
     }
     const uint32_t adler = job.adler[c];
-    enc_wrap_tail(&k, job.format, adler, n);
+    enc_wrap_tail(&k, fmt, adler, n);
     const uint32_t huff_bytes = sink_finish(S, k);
     __syncwarp();
 
     uint32_t len0 = huff_bytes, len1 = 0, raw0 = n, btype = 2u;
-    if (sto_bytes <= huff_bytes + sto_slack || (job.format == ZWZ_FORMAT_ZLIB && huff_bytes > ZWZ_CHUNK) || huff_bytes > cap_words * 4u) { // see the policy above
+    if (sto_bytes <= huff_bytes + sto_slack || (fmt == ZWZ_FORMAT_ZLIB && huff_bytes > ZWZ_CHUNK) || huff_bytes > cap_words * 4u) { // see the policy above
         btype = 0u;
-        if (job.format == ZWZ_FORMAT_ZLIB && sto_bytes > ZWZ_CHUNK) {
+        if (fmt == ZWZ_FORMAT_ZLIB && sto_bytes > ZWZ_CHUNK) {
             // split rule: two stored streams over the halves (each needs its own Adler-32)
             raw0 = 32768u;
             uint32_t a0 = enc_adler_global(src, raw0);
             uint32_t a1 = enc_adler_global(src + raw0, n - raw0);
-            len0 = enc_stored_stream(out, src, raw0, a0, ZWZ_FORMAT_ZLIB);
-            len1 = enc_stored_stream(out + len0, src + raw0, n - raw0, a1, ZWZ_FORMAT_ZLIB);
+            len0 = enc_stored_stream(out, src, raw0, a0, ZWZ_FORMAT_ZLIB, 0u);
+            len1 = enc_stored_stream(out + len0, src + raw0, n - raw0, a1, ZWZ_FORMAT_ZLIB, 0u);
         } else {
-            len0 = enc_stored_stream(out, src, n, adler, job.format);
+            len0 = enc_stored_stream(out, src, n, adler, fmt, dictid);
         }
     }
     if (lane == 0) {
@@ -1016,13 +1038,15 @@ ZWZ_DEV void enc_chunk(EncWarpSmem &S, const DeflateJob &job, uint32_t c) {
 }
 
 // Persistent warps pulling chunks from a global counter (same reason as inflate_kernel: no idle warps behind a long chunk).
+// DICT: some chunks have a preset dictionary (job.dict): their zlib header names it. DICT = false is the kernel of the calls without.
+template <bool DICT = false>
 ZWZ_KERNEL __launch_bounds__(ZWZ_DE_WARPS * 32) deflate_encode_kernel(DeflateJob job, uint32_t *work_counter) {
     for (;;) {
         uint32_t c = 0;
         if (lane_id() == 0) c = atomicAdd(work_counter, 1u);
         c = __shfl_sync(ZWZ_FULL, c, 0);
         if (c >= job.n) break;
-        enc_chunk(enc_smem(), job, c);
+        enc_chunk<DICT>(enc_smem(), job, c);
         __syncwarp();
     }
 }

@@ -132,7 +132,9 @@ ZWZ_DEV void dm_mbar_wait(unsigned long long *bar, uint32_t parity) {
 
 ZWZ_DEV uint32_t sD_of(const unsigned char *smem, uint32_t skew) { return smem_addr(smem) + skew; }
 
-template <int CLS>
+// DICT: chunks with a preset dictionary (job.dict) go on searching in the dictionary's chains once their own chain is exhausted
+// (step 6). DICT = false is the kernel of the calls without dictionaries.
+template <int CLS, bool DICT = false>
 ZWZ_KERNEL __launch_bounds__(MatchClass<CLS>::kThreads, MatchClass<CLS>::kCtasPerSm) lz_match_kernel(DeflateJob job, const uint32_t *__restrict__ order, uint32_t n_work,
                                                                          uint32_t *work_counter) {
     constexpr uint32_t T = MatchClass<CLS>::kThreads, HB = MatchClass<CLS>::kHBits, DATA = MatchClass<CLS>::kData;
@@ -164,6 +166,16 @@ ZWZ_KERNEL __launch_bounds__(MatchClass<CLS>::kThreads, MatchClass<CLS>::kCtasPe
         const uint8_t *src = job.raw + job.raw_off[c];
         const uint32_t skew = (uint32_t) ((uintptr_t) src & 15u);
         const uint32_t stage_bytes = (skew + n + 15u) & ~15u;
+        // the chunk's preset dictionary (CTA-uniform): its record in the dictionary arena and its window length, 0 = none
+        const uint8_t *drec = nullptr;
+        uint32_t dwl = 0;
+        if (DICT) {
+            const uint32_t di = job.dict.idx[c];
+            if (di != ZWZ_NO_DICT) {
+                drec = job.dict.arena + (size_t) di * ZWZ_DICT_STRIDE;
+                dwl = job.dict.wlen[di];
+            }
+        }
 
         // ---- 1. stage the chunk ----
 #ifndef ZWZ_EMU
@@ -201,7 +213,8 @@ ZWZ_KERNEL __launch_bounds__(MatchClass<CLS>::kThreads, MatchClass<CLS>::kCtasPe
         //       n_c positions in m bits collides n_c^2 / 2m times (+- its square root); n_c / 64 + 48 more than that and NO
         //       stretch is left out. The candidates' windows are also looked up among the windows of all other positions (below).
         // What this gives up: repeats that cover less than ~2 % of the noise (zlib would find them). The encoder emits these
-        // stretches as stored blocks (deflate_encode.cuh: quiet stretches).
+        // stretches as stored blocks (deflate_encode.cuh: quiet stretches). With a preset dictionary such a stretch is not
+        // searched against the dictionary either: a copy of dictionary bytes inside noise goes out as literals.
         {
             uint32_t *hist = (uint32_t *) head + wid * 256u;
             const uint32_t nfull = n >> 10; // the partial last stretch is always searched
@@ -466,13 +479,14 @@ ZWZ_KERNEL __launch_bounds__(MatchClass<CLS>::kThreads, MatchClass<CLS>::kCtasPe
                 const uint32_t limit = p > ZWZ_MAX_DIST ? p - ZWZ_MAX_DIST : 0u;
                 const uint32_t span = p - limit;            // a candidate is usable iff 0 <= cand - limit < span (NIL fails)
                 uint32_t cand = lds16(sP + 2u * p);
-                if ((cand - limit) < span) {
+                if ((cand - limit) < span || (DICT && dwl != 0u && p < ZWZ_MAX_DIST)) {
                     const uint32_t ap = sD + p;             // shared address of the scan position
                     const uint32_t ka = ap & ~3u, sa = (ap & 3u) * 8u;
                     const uint32_t a0 = lds32(ka), a1 = lds32(ka + 4u), a2 = lds32(ka + 8u), a3 = lds32(ka + 12u);
                     const uint32_t S0 = __funnelshift_r(a0, a1, sa), S1 = __funnelshift_r(a1, a2, sa), S2 = __funnelshift_r(a2, a3, sa); // bytes [0, 12)
                     uint32_t scan_end = (S0 >> 16) & 0xffu, scan_end1 = (S0 >> 8) & 0xffu; // bytes at best_len and best_len - 1
-                    for (uint32_t budget = job.depth; budget != 0u && (cand - limit) < span; --budget) {
+                    uint32_t budget = job.depth;
+                    for (; budget != 0u && (cand - limit) < span; --budget) {
                         const uint32_t ac = sD + cand;
                         const uint32_t nxt = lds16(sP + 2u * cand); // next link is fetched while this candidate is examined
                         if (lds8(ac + best_len) == scan_end && lds8(ac + best_len - 1u) == scan_end1) {
@@ -508,6 +522,43 @@ ZWZ_KERNEL __launch_bounds__(MatchClass<CLS>::kThreads, MatchClass<CLS>::kCtasPe
                             }
                         }
                         cand = nxt;
+                    }
+                    // The chunk's own chain is exhausted with budget left and no match of `nice` bytes: the walk goes on in the
+                    // dictionary's chain, most recent position first as in zlib (whose window holds the dictionary right before
+                    // the chunk), within the same budget. Window position q is at distance p + dwl - q. The 14-bit hash of the
+                    // scan position holds this class's hash in its top bits, so no candidate of a true match is lost. The
+                    // window is read from global memory (the record is L2-resident, read by every chunk of the call); a match
+                    // that starts in the window ends at its end — DEFLATE would let it run on into the chunk, zlib does.
+                    if (DICT && budget != 0u && best_len < job.nice && best_len < maxlen && dwl != 0u && p < ZWZ_MAX_DIST) {
+                        const uint16_t *dhead = (const uint16_t *) (drec + ZWZ_DICT_HEAD), *dprev = (const uint16_t *) (drec + ZWZ_DICT_PREV);
+                        const uint8_t *dwin = drec + ZWZ_DICT_WIN;
+                        const uint32_t dlim = p + dwl > ZWZ_MAX_DIST ? p + dwl - ZWZ_MAX_DIST : 0u; // oldest usable window position
+                        const uint32_t dspan = dwl - dlim;                                         // NIL fails (q - dlim) < dspan
+                        uint32_t q = __ldg(dhead + dm_hash3<ZWZ_DICT_HBITS>(S0 & 0xffu, (S0 >> 8) & 0xffu, (S0 >> 16) & 0xffu));
+                        for (; budget != 0u && (q - dlim) < dspan; --budget) {
+                            const uint32_t nxt = __ldg(dprev + q);
+                            const uint32_t dmax = dwl - q < maxlen ? dwl - q : maxlen;
+                            if (best_len < dmax && __ldg(dwin + q + best_len) == scan_end && __ldg(dwin + q + best_len - 1u) == scan_end1) {
+                                uint32_t len = 0;
+                                while (len < dmax) {
+                                    const uint32_t y = ld32u((const uint32_t *) dwin, q + len) ^ lds32u(ap + len);
+                                    if (y) {
+                                        len += ((uint32_t) __ffs((int) y) - 1u) >> 3;
+                                        break;
+                                    }
+                                    len += 4u;
+                                }
+                                if (len > dmax) len = dmax;
+                                if (len > best_len) {
+                                    best_len = len;
+                                    best_dist = p + dwl - q;
+                                    if (len >= job.nice || len >= maxlen) break;
+                                    scan_end = lds8(ap + len);
+                                    scan_end1 = lds8(ap + len - 1u);
+                                }
+                            }
+                            q = nxt;
+                        }
                     }
                 }
             }
@@ -599,6 +650,64 @@ ZWZ_KERNEL __launch_bounds__(MatchClass<CLS>::kThreads, MatchClass<CLS>::kCtasPe
         }
         __syncthreads(); // smem is reused by the next chunk
     }
+}
+
+// One CTA per preset dictionary of a call: its record in the dictionary arena (zwz_common.cuh, ZWZ_DICT_*), read by every chunk
+// that uses the dictionary. Window k is data[win_off[k] .. + wlen[k]). The chains are built as in step 5 of lz_match_kernel (all
+// positions hashed in parallel, then 32 positions per step with the same collision repair), by one warp over the whole window:
+// exact zlib-order chains in ~1 000 steps, once per dictionary and call.
+#define ZWZ_DICT_SMEM (2u * 32768u + (2u << ZWZ_DICT_HBITS))
+ZWZ_KERNEL __launch_bounds__(1024) dict_chain_kernel(const uint8_t *__restrict__ data, const uint64_t *__restrict__ win_off,
+                                                     const uint32_t *__restrict__ wlen, uint8_t *arena) {
+    ZWZ_DYN_SMEM(smem);
+    uint16_t *prev = (uint16_t *) smem;                // hash of position q until the builder replaces it by the link
+    uint16_t *head = (uint16_t *) (smem + 2u * 32768u);
+    const unsigned tid = threadIdx.x, lane = lane_id(), T = blockDim.x;
+    const unsigned lt = (1u << lane) - 1u;
+    const uint32_t k = blockIdx.x, W = wlen[k];
+    const uint8_t *src = data + win_off[k];
+    uint8_t *rec = arena + (size_t) k * ZWZ_DICT_STRIDE;
+    const uint32_t nh = W >= 3u ? W - 2u : 0u; // positions that own a 3-byte hash inside the window
+    for (uint32_t i = tid; i < W + 64u; i += T) rec[ZWZ_DICT_WIN + i] = i < W ? src[i] : (uint8_t) 0;
+    for (uint32_t i = tid; i < (1u << ZWZ_DICT_HBITS); i += T) head[i] = (uint16_t) ZWZ_DM_NIL;
+    for (uint32_t q = tid; q < nh; q += T) prev[q] = (uint16_t) dm_hash3<ZWZ_DICT_HBITS>(src[q], src[q + 1u], src[q + 2u]);
+    __syncthreads();
+    if (tid < 32u) {
+        for (uint32_t i0 = 0; i0 < nh; i0 += 32u) {
+            const uint32_t q = i0 + lane;
+            const bool valid = q < nh;
+            const uint32_t h = valid ? prev[q] : 0u;
+            const uint32_t old = valid ? head[h] : (uint32_t) ZWZ_DM_NIL;
+            __syncwarp(); // all reads of head[] precede the writes of this step
+            if (valid) {
+                prev[q] = (uint16_t) old;
+                head[h] = (uint16_t) q;
+            }
+            __syncwarp();
+            const uint32_t rb = valid ? head[h] : q;
+            unsigned rem = __ballot_sync(ZWZ_FULL, rb != q); // lanes that lost a store race
+            while (rem) {
+                const int leader = __ffs((int) rem) - 1;
+                const uint32_t hl = __shfl_sync(ZWZ_FULL, h, leader);
+                const bool mine = valid && h == hl;
+                const unsigned same = __ballot_sync(ZWZ_FULL, mine);
+                const unsigned lower = same & lt;
+                const int from = (mine && lower) ? 31 - __clz((int) lower) : (int) lane;
+                const uint32_t qlow = __shfl_sync(ZWZ_FULL, q, from);
+                if (mine) {
+                    if (lower) prev[q] = (uint16_t) qlow;
+                    if ((same >> lane) == 1u) head[h] = (uint16_t) q;
+                }
+                __syncwarp();
+                rem &= ~same;
+            }
+            __syncwarp();
+        }
+    }
+    __syncthreads();
+    uint16_t *ghead = (uint16_t *) (rec + ZWZ_DICT_HEAD), *gprev = (uint16_t *) (rec + ZWZ_DICT_PREV);
+    for (uint32_t i = tid; i < (1u << ZWZ_DICT_HBITS); i += T) ghead[i] = head[i];
+    for (uint32_t q = tid; q < nh; q += T) gprev[q] = prev[q];
 }
 
 } // namespace zwz

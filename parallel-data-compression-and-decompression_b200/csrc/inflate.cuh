@@ -351,9 +351,11 @@ ZWZ_DEV_NOINLINE uint32_t inf_gzip_header(const uint8_t *comp, uint32_t comp_len
     return (p << 2) | ZWZ_STREAM_END;
 }
 
-// One warp decodes stream `sid`.
+// One warp decodes stream `sid`. DICT: the stream may have a preset dictionary, whose window (dwl bytes at dwin, 0 = none) comes
+// before output position 0; a zlib stream asks for it with FDICT and names it by its DICTID (did), a raw stream just uses it.
+template <bool DICT>
 ZWZ_DEV void inflate_stream(InflateWarpSmem &S, const uint8_t *__restrict__ comp, uint32_t comp_len, uint8_t *out, uint32_t cap,
-                            uint32_t flags, uint32_t &raw_len_out, uint32_t &status_out) {
+                            uint32_t flags, uint32_t &raw_len_out, uint32_t &status_out, const uint8_t *dwin, uint32_t dwl, uint32_t did) {
     const unsigned lane = lane_id();
     const uint64_t total_bits = (uint64_t) comp_len * 8u;
     InfBits B;
@@ -395,11 +397,28 @@ ZWZ_DEV void inflate_stream(InflateWarpSmem &S, const uint8_t *__restrict__ comp
             goto done;
         }
         uint32_t cmf = (uint32_t) B.hold & 0xffu, flg = ((uint32_t) B.hold >> 8) & 0xffu;
-        if (((cmf << 8) + flg) % 31u != 0u || (cmf & 15u) != 8u || (cmf >> 4) + 8u > 15u || (flg & 0x20u)) {
-            status = ZWZ_STREAM_BAD;
+        if (((cmf << 8) + flg) % 31u != 0u || (cmf & 15u) != 8u || (cmf >> 4) + 8u > 15u || ((flg & 0x20u) && (!DICT || dwl == 0u))) {
+            status = ZWZ_STREAM_BAD; // FDICT without a dictionary is zlib's Z_NEED_DICT: nothing can be decoded
             goto done;
         }
         infb_drop(B, 16);
+        if (DICT) {
+            if (flg & 0x20u) { // DICTID (inflate.c DICTID): it must name the dictionary given, else inflateSetDictionary's Z_DATA_ERROR
+                infb_refill(B);
+                if (!INF_NEED(32)) {
+                    status = ZWZ_STREAM_TRUNCATED;
+                    goto done;
+                }
+                const uint32_t v = (uint32_t) B.hold;
+                if ((((v & 0xffu) << 24) | ((v & 0xff00u) << 8) | ((v >> 8) & 0xff00u) | (v >> 24)) != did) {
+                    status = ZWZ_STREAM_BAD;
+                    goto done;
+                }
+                infb_drop(B, 32);
+            } else {
+                dwl = 0; // a zlib stream without FDICT ignores the dictionary (as CPython's decompressobj(zdict=) does)
+            }
+        }
     }
 
     for (;;) {
@@ -563,7 +582,7 @@ ZWZ_DEV void inflate_stream(InflateWarpSmem &S, const uint8_t *__restrict__ comp
             INF_FLUSH_LITS();
             __syncwarp();
             uint64_t bp = infb_used(B);
-            const int fr = inf_fast_block(S, B, bp, max_ll, max_d, out, cap, pos, overflow);
+            const int fr = inf_fast_block<DICT>(S, B, bp, max_ll, max_d, out, cap, pos, overflow, dwin, dwl);
             pend_lo = pos;
             if (fr == IFR_BAD) {
                 status = ZWZ_STREAM_BAD;
@@ -684,7 +703,7 @@ ZWZ_DEV void inflate_stream(InflateWarpSmem &S, const uint8_t *__restrict__ comp
             }
             uint32_t dist = ZWZ_D_DM1(d, (uint32_t) B.hold) + 1u;
             infb_drop(B, dnb + deb);
-            if (dist > pos) { // "invalid distance too far back"
+            if (dist > pos + dwl) { // "invalid distance too far back" (a preset dictionary's window counts as written)
                 status = ZWZ_STREAM_BAD;
                 goto done;
             }
@@ -693,7 +712,7 @@ ZWZ_DEV void inflate_stream(InflateWarpSmem &S, const uint8_t *__restrict__ comp
             INF_FLUSH_LITS();
             __syncwarp();
             if (pos + mlen > cap) overflow = true;
-            inf_copy_match(out, pos, mlen, dist, cap);
+            inf_copy_match<DICT>(out, pos, mlen, dist, cap, dwin, dwl);
             pos += mlen;
             pend_lo = pos;
         }
@@ -740,10 +759,12 @@ done:
 
 // Persistent warps: every warp pulls the next stream from a global counter, so a CTA is never kept alive by one long stream
 // while its other warps idle (streams of one batch differ in length by 100x in config C2).
+// DICT: some streams have a preset dictionary (dict, zwz_common.cuh); DICT = false is the kernel of the calls without.
+template <bool DICT = false>
 ZWZ_KERNEL __launch_bounds__(ZWZ_INF_WARPS * 32, ZWZ_INF_MIN_CTAS) inflate_kernel(const uint8_t *__restrict__ comp, const uint64_t *__restrict__ off,
                                                               const uint32_t *__restrict__ len, uint8_t *raw_out,
                                                               const uint64_t *__restrict__ raw_off, uint32_t *raw_len, uint32_t *status,
-                                                              uint32_t n, uint32_t flags, uint32_t *work_counter) {
+                                                              uint32_t n, uint32_t flags, uint32_t *work_counter, DictTable dict) {
     ZWZ_DYN_SMEM(inf_raw);
     InflateWarpSmem *smem = (InflateWarpSmem *) inf_raw;
     for (;;) {
@@ -754,7 +775,17 @@ ZWZ_KERNEL __launch_bounds__(ZWZ_INF_WARPS * 32, ZWZ_INF_MIN_CTAS) inflate_kerne
         uint64_t cap64 = raw_off[sid + 1] - raw_off[sid];
         uint32_t cap = cap64 > 0xfffffff0ull ? 0xfffffff0u : (uint32_t) cap64;
         uint32_t rl = 0, st = 0;
-        inflate_stream(smem[warp_id()], comp + off[sid], len[sid], raw_out + raw_off[sid], cap, flags, rl, st);
+        const uint8_t *dwin = nullptr;
+        uint32_t dwl = 0, did = 0;
+        if (DICT) {
+            const uint32_t di = dict.idx[sid];
+            if (di != ZWZ_NO_DICT) {
+                dwin = dict.arena + (size_t) di * ZWZ_DICT_STRIDE + ZWZ_DICT_WIN;
+                dwl = dict.wlen[di];
+                did = dict.id[di];
+            }
+        }
+        inflate_stream<DICT>(smem[warp_id()], comp + off[sid], len[sid], raw_out + raw_off[sid], cap, flags, rl, st, dwin, dwl, did);
         if (lane_id() == 0) {
             raw_len[sid] = rl;
             status[sid] = st;

@@ -55,23 +55,31 @@ ZWZ_DEV uint32_t iff_fetch(const uint32_t *cw, uint32_t p) {
     return __funnelshift_r(cw[k], cw[k + 1u], p & 31u);
 }
 
-// back-reference copy by the whole warp: bytes [pos, pos + mlen) = bytes [pos - dist, ...), overlapping allowed
-ZWZ_DEV void inf_copy_match(uint8_t *out, uint32_t pos, uint32_t mlen, uint32_t dist, uint32_t cap) {
+// The byte at output position s - d of a stream. DICT: a stream with a preset dictionary (window of dwl bytes at dwin) finds the
+// bytes before its output position 0 in the dictionary's window, as if they had been written right before it.
+template <bool DICT> ZWZ_DEV uint32_t inf_ref(const uint8_t *out, const uint8_t *dwin, uint32_t dwl, uint32_t s, uint32_t d) {
+    if (DICT && s < d) return __ldg(dwin + (dwl + s - d));
+    return __ldcg(out + (s - d));
+}
+
+// back-reference copy by the whole warp: bytes [pos, pos + mlen) = bytes [pos - dist, ...), overlapping allowed (also across
+// the boundary between a preset dictionary's window and the output)
+template <bool DICT = false>
+ZWZ_DEV void inf_copy_match(uint8_t *out, uint32_t pos, uint32_t mlen, uint32_t dist, uint32_t cap, const uint8_t *dwin = nullptr, uint32_t dwl = 0u) {
     const unsigned lane = lane_id();
     if (mlen <= 32u && dist >= mlen) { // the common case: short, non-overlapping — one step, no loop
         const uint32_t q = pos + lane;
-        if (lane < mlen && q < cap) out[q] = __ldcg(out + (q - dist));
+        if (lane < mlen && q < cap) out[q] = inf_ref<DICT>(out, dwin, dwl, q, dist);
     } else if (dist >= 32u || dist >= mlen) {
         for (uint32_t base = 0; base < mlen; base += 32u) { // warp-uniform trip count
             const uint32_t q = pos + base + lane;
-            if (base + lane < mlen && q < cap) out[q] = __ldcg(out + (q - dist));
+            if (base + lane < mlen && q < cap) out[q] = inf_ref<DICT>(out, dwin, dwl, q, dist);
             __syncwarp(); // later steps may read what this step wrote (dist < mlen)
         }
     } else { // overlapping run with a period < 32: every byte comes from the already written period
-        const uint32_t src0 = pos - dist;
         for (uint32_t i = lane; i < mlen; i += 32u) {
             const uint32_t q = pos + i;
-            if (q < cap) out[q] = __ldcg(out + (src0 + (i % dist)));
+            if (q < cap) out[q] = inf_ref<DICT>(out, dwin, dwl, pos + (i % dist), dist);
         }
     }
     __syncwarp();
@@ -80,10 +88,10 @@ ZWZ_DEV void inf_copy_match(uint8_t *out, uint32_t pos, uint32_t mlen, uint32_t 
 // Decodes the Huffman block whose next literal/length code starts at stream bit `bitpos`, as far as the fast path can.
 // Returns IFR_EOB (end-of-block consumed, bitpos behind it), IFR_SLOW (bitpos = first bit of a token the careful decoder
 // must look at) or IFR_BAD (distance too far back: pos = bytes before that match). All arguments and results are
-// warp-uniform.
-template <class SMEM, class BITS>
+// warp-uniform. DICT: the dwl bytes of a preset dictionary's window at dwin come before output position 0.
+template <bool DICT, class SMEM, class BITS>
 ZWZ_DEV int inf_fast_block(SMEM &S, const BITS &B, uint64_t &bitpos, uint32_t max_ll, uint32_t max_d, uint8_t *out, uint32_t cap, uint32_t &pos,
-                           bool &overflow) {
+                           bool &overflow, const uint8_t *dwin, uint32_t dwl) {
     const unsigned lane = lane_id();
     const uint64_t g_end = (uint64_t) B.skew * 8u + (uint64_t) B.nbytes * 8u; // one past the last real bit, relative to wbase
     uint16_t *const my = S.tok + lane * ZWZ_IF_RS;
@@ -234,7 +242,7 @@ ZWZ_DEV int inf_fast_block(SMEM &S, const BITS &B, uint64_t &bitpos, uint32_t ma
                 const uint32_t total = __shfl_sync(ZWZ_FULL, incl, 31);
                 const uint32_t dn = __shfl_down_sync(ZWZ_FULL, t, 1); // distance - 1 of a head lane
                 // invalid distance too far back: zlib stops at the first such match with everything before it written
-                const unsigned far = __ballot_sync(ZWZ_FULL, is_head && lane < take && dn + 1u > pos + excl);
+                const unsigned far = __ballot_sync(ZWZ_FULL, is_head && lane < take && dn + 1u > pos + excl + dwl);
                 // matches that reach into this step's own output (source position + min(len, dist) > step start)
                 const unsigned deps = __ballot_sync(ZWZ_FULL, is_head && lane < take && excl + (olen < dn + 1u ? olen : dn + 1u) > dn + 1u);
                 // ---- every byte of the step by its own lane ----
@@ -266,9 +274,9 @@ ZWZ_DEV int inf_fast_block(SMEM &S, const BITS &B, uint64_t &bitpos, uint32_t ma
                             const uint32_t i = b - ej;                                                // byte i of the match
                             const uint32_t src = ej + (dj >= (tj & 0x1ffu) || i < dj ? i : i % dj);   // its source + dist, relative to the step
                             // before the step iff src < dj. No load for bytes that will not be written: those of a too-far match
-                            // (dj > pos + ej) and those past the capacity of the output window (a sizing pass still counts them)
-                            put[u] = src < dj && dj <= pos + ej && pos + b < cap;
-                            if (put[u]) val[u] = __ldcg(out + (pos + src - dj));
+                            // (dj > pos + ej + dwl) and those past the capacity of the output window (a sizing pass still counts them)
+                            put[u] = src < dj && dj <= pos + ej + dwl && pos + b < cap;
+                            if (put[u]) val[u] = inf_ref<DICT>(out, dwin, dwl, pos + src, dj);
                         }
                     }
 #pragma unroll

@@ -42,6 +42,25 @@ namespace zwz {
 ZWZ_DEV unsigned lane_id() { return threadIdx.x & 31u; }
 ZWZ_DEV unsigned warp_id() { return threadIdx.x >> 5; }
 
+// ---- preset dictionaries (zwz_*_dict calls) ----
+// Every dictionary of a call has one record in the context's dictionary arena, built by dict_chain_kernel (deflate_match.cuh):
+//   [ZWZ_DICT_HEAD, +32 KiB)  head[2^14] u16: latest window position of each 14-bit hash (dm_hash3<14>), NIL = 0xffff
+//   [ZWZ_DICT_PREV, +64 KiB)  prev[32 768] u16: the next older position of the same hash (exact zlib-order chains)
+//   [ZWZ_DICT_WIN, +32 KiB)   the window (the dictionary's last <= 32 768 bytes), 16-byte aligned and zero padded, so that
+//                             both the match search and inflate read it with aligned loads
+// The last two window positions are not chained: their 3-byte hash would need the chunk's first bytes.
+#define ZWZ_DICT_HBITS 14u
+#define ZWZ_DICT_HEAD 0u
+#define ZWZ_DICT_PREV 32768u
+#define ZWZ_DICT_WIN 98304u
+#define ZWZ_DICT_STRIDE (98304u + 32768u + 256u)
+struct DictTable {
+    const uint32_t *idx;   // [n] dictionary of chunk / stream i, or ZWZ_NO_DICT (nullptr: the call has no dictionary)
+    const uint8_t *arena;  // ZWZ_DICT_STRIDE bytes per dictionary
+    const uint32_t *wlen;  // [ndict] window length (1 .. 32 768)
+    const uint32_t *id;    // [ndict] DICTID: Adler-32 of the whole dictionary
+};
+
 // chunk descriptor / result as laid out in device memory (structure of arrays, one entry per chunk)
 struct DeflateJob {
     const uint8_t *raw;        // all chunks' raw bytes
@@ -60,6 +79,7 @@ struct DeflateJob {
     uint32_t nice;             // stop searching at this length
     uint32_t *work_counter;    // persistent-CTA work queue
     uint32_t format;           // ZWZ_FORMAT_*: the wrapper deflate_encode_kernel puts around the body
+    DictTable dict;            // read only by the DICT instantiations of the kernels
 };
 
 // ---- unaligned little-endian loads built from aligned 32-bit words -------------------------------------------------

@@ -165,6 +165,7 @@ struct zwz_ctx {
     int sm_count = 0, cc_major = 0, cc_minor = 0;
     size_t total_mem = 0, smem_optin = 0;
     int inf_blocks_per_sm = 1; // resident inflate_kernel CTAs per SM
+    int inf_dict_blocks_per_sm = 1; // the same for inflate_kernel<true>
     zwz_stream_t stream = nullptr;
     zwz_stream_t md5_stream = nullptr; // deferred digests (DigestSlot)
     zwz::DigestSlot slot[2];
@@ -181,6 +182,10 @@ struct zwz_ctx {
     // host copy in `pin_keep` that zwz_pack_streams_device compares the caller's arrays with before it uses the device copy.
     // Layout of both: [slot_off u64 x keep_n], then at keep_res_off(keep_n) [results 16 B x keep_n].
     zwz::Arena keep, pin_keep;
+    // preset dictionaries of the current call (zwz_*_dict): descriptors (device + page-locked staging), the dictionary records
+    // built by dict_chain_kernel, and the dictionaries' bytes when the caller gave host memory
+    zwz::Arena dict_meta, pin_dict, dict_arena, dict_data;
+    std::vector<uint64_t> dict_host_off;
     uint32_t keep_n = 0; // 0 = nothing valid in keep / pin_keep
     // host threads for the descriptor work of large calls (ZWZ_TUNE_HOST_THREADS, ZWZ_TUNE_HOST_PARALLEL_MIN)
     unsigned host_threads = 0; // threads per call, the calling one included; 0 = min(8, cores / 2)
@@ -396,6 +401,97 @@ LevelParams level_params(int level) {
     return t[level];
 }
 
+// Preset dictionaries of one call (zwz_*_dict). Checks `d` for n chunks / streams and stages the per-entry dictionary index (on
+// the host threads above host_parallel_min; an empty dictionary becomes ZWZ_NO_DICT: it is no dictionary). `refuse`: the format
+// or decoder takes no dictionary, so any entry that names one is ZWZ_E_ARG. When some entry has a dictionary, every dictionary
+// of the table gets its record (dict_chain_kernel) and its DICTID (adler32_kernel) on stream st, and *out points at them;
+// otherwise *out stays empty and the call launches what the call without dictionaries launches.
+int stage_dicts(zwz_ctx *ctx, const zwz_dicts *d, uint32_t n, bool refuse, zwz_stream_t st, zwz::DictTable *out) {
+    *out = zwz::DictTable{};
+    if (!d) return ZWZ_OK;
+    if (!d->off) return fail(ctx, ZWZ_E_ARG, "null dictionary offsets");
+    const uint32_t nd = d->ndict;
+    for (uint32_t k = 0; k < nd; ++k)
+        if (d->off[k + 1] < d->off[k] || d->off[k + 1] - d->off[k] > ((uint64_t) 1 << 30))
+            return fail(ctx, ZWZ_E_ARG, "dictionary offsets must not decrease, dictionaries hold at most 2^30 bytes");
+    if (nd && d->off[nd] > d->off[0] && !d->data) return fail(ctx, ZWZ_E_ARG, "null dictionary data");
+    const size_t m_off = align_up((size_t) n * 4, 256), m_woff = m_off + (size_t) nd * 8, m_len = m_woff + (size_t) nd * 8,
+                 m_wlen = m_len + (size_t) nd * 4, m_id = m_wlen + (size_t) nd * 4;
+    int rc;
+    if ((rc = reserve(ctx, ctx->pin_dict, m_id, true))) return rc;
+    uint8_t *hp = (uint8_t *) ctx->pin_dict.p;
+    uint32_t *h_idx = (uint32_t *) hp;
+    const unsigned nb = host_blocks(ctx, n);
+    std::vector<char> bad(nb, 0), named(nb, 0), used(nb, 0);
+    const Staging stg(nb);
+    host_for(ctx, nb, n, [&](unsigned b, size_t lo, size_t hi) {
+        bool b_bad = false, b_named = false, b_used = false; // per block in registers: the flags of all blocks share a cache line
+        for (size_t i = lo; i < hi; ++i) {
+            const uint32_t k = d->idx ? d->idx[i] : (nd ? 0u : ZWZ_NO_DICT);
+            const bool ok = k < nd && d->off[k + 1] > d->off[k];
+            b_bad |= k != ZWZ_NO_DICT && k >= nd;
+            b_named |= k != ZWZ_NO_DICT;
+            b_used |= ok;
+            stg.put(h_idx + i, ok ? k : ZWZ_NO_DICT);
+        }
+        stg.done();
+        bad[b] = b_bad;
+        named[b] = b_named;
+        used[b] = b_used;
+    });
+    auto any = [](const std::vector<char> &v) { return std::any_of(v.begin(), v.end(), [](char c) { return c != 0; }); };
+    if (any(bad)) return fail(ctx, ZWZ_E_ARG, "dictionary index out of range");
+    if (refuse && any(named)) return fail(ctx, ZWZ_E_ARG, "no preset dictionary in gzip format or with the one-lane-per-stream decoder");
+    if (!any(used)) return ZWZ_OK;
+    for (uint32_t k = 0; k < nd; ++k) {
+        const uint64_t l = d->off[k + 1] - d->off[k], w = std::min<uint64_t>(l, ZWZ_MAX_DIST);
+        ((uint64_t *) (hp + m_off))[k] = d->off[k];
+        ((uint64_t *) (hp + m_woff))[k] = d->off[k] + l - w;
+        ((uint32_t *) (hp + m_len))[k] = (uint32_t) l;
+        ((uint32_t *) (hp + m_wlen))[k] = (uint32_t) w;
+    }
+    if ((rc = reserve(ctx, ctx->dict_meta, m_id + (size_t) nd * 4 + 256, false))) return rc;
+    if ((rc = reserve(ctx, ctx->dict_arena, (size_t) nd * ZWZ_DICT_STRIDE, false))) return rc;
+    uint8_t *dm = (uint8_t *) ctx->dict_meta.p;
+    if (zwz_rt::memcpy_h2d(dm, hp, m_id, st)) return fail(ctx, ZWZ_E_CUDA, "dictionary descriptor upload failed");
+    {
+        ProfSpan ps(ctx, ZWZ_PROF_ADLER, st);
+        ZWZ_LAUNCH(zwz::dict_chain_kernel, nd, 1024, ZWZ_DICT_SMEM, st, d->data, (const uint64_t *) (dm + m_woff), (const uint32_t *) (dm + m_wlen),
+                   (uint8_t *) ctx->dict_arena.p);
+    }
+    if ((rc = check_launch(ctx, "dict_chain_kernel"))) return rc;
+    {
+        ProfSpan ps(ctx, ZWZ_PROF_ADLER, st);
+        ZWZ_LAUNCH(zwz::adler32_kernel, (nd + 7) / 8, 256, 0, st, d->data, (const uint64_t *) (dm + m_off), (const uint32_t *) (dm + m_len),
+                   (uint32_t *) (dm + m_id), nd);
+    }
+    if ((rc = check_launch(ctx, "adler32_kernel"))) return rc;
+    out->idx = (const uint32_t *) dm;
+    out->arena = (const uint8_t *) ctx->dict_arena.p;
+    out->wlen = (const uint32_t *) (dm + m_wlen);
+    out->id = (const uint32_t *) (dm + m_id);
+    return ZWZ_OK;
+}
+
+// The plain (host-buffer) calls: the dictionaries' bytes go to the device once per call. *out is *d with device data and
+// offsets relative to it (kept in the context until the next call).
+int upload_dicts(zwz_ctx *ctx, const zwz_dicts *d, zwz_dicts *out) {
+    if (!d) return ZWZ_OK;
+    *out = *d;
+    if (!d->off || d->ndict == 0) return ZWZ_OK; // stage_dicts names the error
+    const uint64_t lo = d->off[0], hi = d->off[d->ndict];
+    if (hi < lo) return fail(ctx, ZWZ_E_ARG, "dictionary offsets must not decrease");
+    if (hi > lo && !d->data) return fail(ctx, ZWZ_E_ARG, "null dictionary data");
+    ctx->dict_host_off.resize(d->ndict + 1);
+    for (uint32_t k = 0; k <= d->ndict; ++k) ctx->dict_host_off[k] = d->off[k] - lo;
+    int rc;
+    if ((rc = reserve(ctx, ctx->dict_data, (size_t) (hi - lo) + 64, false))) return rc;
+    if (zwz_rt::memcpy_h2d(ctx->dict_data.p, d->data + lo, (size_t) (hi - lo), ctx->stream)) return fail(ctx, ZWZ_E_CUDA, "dictionary upload failed");
+    out->data = (const uint8_t *) ctx->dict_data.p;
+    out->off = ctx->dict_host_off.data();
+    return ZWZ_OK;
+}
+
 } // namespace
 
 extern "C" {
@@ -426,13 +522,20 @@ int zwz_init(int device, zwz_ctx **out) {
         zwz_rt::set_max_dyn_smem((const void *) zwz::lz_match_kernel<1>, zwz::MatchClass<1>::kSmem) ||
         zwz_rt::set_max_dyn_smem((const void *) zwz::lz_match_kernel<2>, zwz::MatchClass<2>::kSmem) ||
         zwz_rt::set_max_dyn_smem((const void *) zwz::lz_match_kernel<3>, zwz::MatchClass<3>::kSmem) ||
+        zwz_rt::set_max_dyn_smem((const void *) zwz::lz_match_kernel<0, true>, zwz::MatchClass<0>::kSmem) ||
+        zwz_rt::set_max_dyn_smem((const void *) zwz::lz_match_kernel<1, true>, zwz::MatchClass<1>::kSmem) ||
+        zwz_rt::set_max_dyn_smem((const void *) zwz::lz_match_kernel<2, true>, zwz::MatchClass<2>::kSmem) ||
+        zwz_rt::set_max_dyn_smem((const void *) zwz::lz_match_kernel<3, true>, zwz::MatchClass<3>::kSmem) ||
+        zwz_rt::set_max_dyn_smem((const void *) zwz::dict_chain_kernel, ZWZ_DICT_SMEM) ||
+        zwz_rt::set_max_dyn_smem((const void *) zwz::inflate_kernel<true>, ZWZ_INF_SMEM) ||
         zwz_rt::set_max_dyn_smem((const void *) zwz::md5_files_staged_kernel, ZWZ_MD5S_SMEM) ||
-        zwz_rt::set_max_dyn_smem((const void *) zwz::inflate_kernel, ZWZ_INF_SMEM) ||
+        zwz_rt::set_max_dyn_smem((const void *) zwz::inflate_kernel<false>, ZWZ_INF_SMEM) ||
         zwz_rt::set_max_dyn_smem((const void *) zwz::inflate_lanes_kernel, ZWZ_IL_SMEM)) {
         delete ctx;
         return ZWZ_E_NODEVICE;
     }
-    if (zwz_rt::max_blocks_per_sm(&ctx->inf_blocks_per_sm, (const void *) zwz::inflate_kernel, ZWZ_INF_WARPS * 32, ZWZ_INF_SMEM)) {
+    if (zwz_rt::max_blocks_per_sm(&ctx->inf_blocks_per_sm, (const void *) zwz::inflate_kernel<false>, ZWZ_INF_WARPS * 32, ZWZ_INF_SMEM) ||
+        zwz_rt::max_blocks_per_sm(&ctx->inf_dict_blocks_per_sm, (const void *) zwz::inflate_kernel<true>, ZWZ_INF_WARPS * 32, ZWZ_INF_SMEM)) {
         delete ctx;
         return ZWZ_E_NODEVICE;
     }
@@ -446,8 +549,8 @@ int zwz_init(int device, zwz_ctx **out) {
             return ZWZ_E_NODEVICE;
         }
     zwz_rt::keep_pool_memory(device);
-    zwz_rt::preload_kernel((const void *) zwz::deflate_encode_kernel);
-    zwz_rt::preload_kernel((const void *) zwz::inflate_kernel);
+    zwz_rt::preload_kernel((const void *) zwz::deflate_encode_kernel<false>);
+    zwz_rt::preload_kernel((const void *) zwz::inflate_kernel<false>);
     zwz_rt::preload_kernel((const void *) zwz::md5_files_kernel);
     zwz_rt::preload_kernel((const void *) zwz::pack_streams_kernel);
     zwz_rt::preload_kernel((const void *) zwz::gather_records_kernel);
@@ -486,6 +589,10 @@ void zwz_destroy(zwz_ctx *ctx) {
     release(ctx, ctx->counter);
     release(ctx, ctx->keep);
     release(ctx, ctx->pin_keep);
+    release(ctx, ctx->dict_meta);
+    release(ctx, ctx->pin_dict);
+    release(ctx, ctx->dict_arena);
+    release(ctx, ctx->dict_data);
     ctx->pool.reset(); // joins the host threads
     zwz_rt::stream_sync(ctx->stream);
     zwz_rt::stream_destroy(ctx->stream);
@@ -599,6 +706,11 @@ int zwz_deflate_batch_device(zwz_ctx *ctx, const uint8_t *d_raw, const uint64_t 
 
 int zwz_deflate_batch_device_ex(zwz_ctx *ctx, const uint8_t *d_raw, const uint64_t *off, const uint32_t *len, uint32_t n, uint8_t *d_out,
                                 const uint64_t *out_off, zwz_deflate_result *res, int level, int format, void *stream_v) {
+    return zwz_deflate_batch_device_dict(ctx, d_raw, off, len, n, d_out, out_off, res, level, format, nullptr, stream_v);
+}
+
+int zwz_deflate_batch_device_dict(zwz_ctx *ctx, const uint8_t *d_raw, const uint64_t *off, const uint32_t *len, uint32_t n, uint8_t *d_out,
+                                  const uint64_t *out_off, zwz_deflate_result *res, int level, int format, const zwz_dicts *dicts, void *stream_v) {
     if (!ctx) return ZWZ_E_ARG;
     if (format < ZWZ_FORMAT_ZLIB || format > ZWZ_FORMAT_RAW) return fail(ctx, ZWZ_E_ARG, "unknown stream format");
     if (n == 0) return ZWZ_OK;
@@ -635,13 +747,15 @@ int zwz_deflate_batch_device_ex(zwz_ctx *ctx, const uint8_t *d_raw, const uint64
         total_scr += p.scr;
     }
     if (total_raw && !d_raw) return fail(ctx, ZWZ_E_ARG, "null raw buffer");
+    zwz::DictTable dict{};
+    int rc;
+    if ((rc = stage_dicts(ctx, dicts, n, format == ZWZ_FORMAT_GZIP, st, &dict))) return rc;
     tr.mark("validate");
 
     // descriptors: [raw_off u64][scr_off u64][raw_len u32][order u32] per chunk, then Adler-32 + match counts on the device;
     // slot offsets and results in the keep arenas ([out_off u64][results 16 B] per chunk)
     const size_t meta_bytes = (size_t) n * (8 + 8 + 4 + 4), keep_bytes = keep_res_off(n) + (size_t) n * 16;
     const size_t dev_meta_bytes = align_up(meta_bytes, 256) + (size_t) n * 8 + 256;
-    int rc;
     if ((rc = reserve(ctx, ctx->pin_meta, meta_bytes, true))) return rc;
     if ((rc = reserve(ctx, ctx->meta, dev_meta_bytes, false))) return rc;
     if ((rc = reserve(ctx, ctx->pin_keep, keep_bytes, true))) return rc;
@@ -763,6 +877,8 @@ int zwz_deflate_batch_device_ex(zwz_ctx *ctx, const uint8_t *d_raw, const uint64
         job.nice = lp.nice;
         job.work_counter = nullptr;
         job.format = (uint32_t) format;
+        job.dict = dict;
+        if (dict.idx) job.dict.idx = dict.idx + b;
         const uint32_t *d_order = (const uint32_t *) ((const uint64_t *) dm + 2 * (size_t) n) + n + b;
         uint32_t *d_counters = (uint32_t *) ctx->counter.p + s * 8; // [0..3] match classes, [4] encoder
         for (int cls = 0; cls < 4; ++cls) {
@@ -770,7 +886,14 @@ int zwz_deflate_batch_device_ex(zwz_ctx *ctx, const uint8_t *d_raw, const uint64
             if (w1 == w0) continue;
             ProfSpan ps(ctx, ZWZ_PROF_MATCH, st);
             const uint32_t nwork = w1 - w0, sms = (uint32_t) ctx->sm_count;
-            if (cls == 0) {
+            if (dict.idx) { // the DICT instantiations only when some chunk of the call has a dictionary
+                auto *k0 = zwz::lz_match_kernel<0, true>, *k1 = zwz::lz_match_kernel<1, true>, *k2 = zwz::lz_match_kernel<2, true>,
+                     *k3 = zwz::lz_match_kernel<3, true>;
+                if (cls == 0) ZWZ_LAUNCH(k0, std::min(nwork, sms * 6u), zwz::MatchClass<0>::kThreads, zwz::MatchClass<0>::kSmem, st, job, d_order + w0, nwork, d_counters + cls);
+                else if (cls == 1) ZWZ_LAUNCH(k1, std::min(nwork, sms * 3u), zwz::MatchClass<1>::kThreads, zwz::MatchClass<1>::kSmem, st, job, d_order + w0, nwork, d_counters + cls);
+                else if (cls == 2) ZWZ_LAUNCH(k2, std::min(nwork, sms * 2u), zwz::MatchClass<2>::kThreads, zwz::MatchClass<2>::kSmem, st, job, d_order + w0, nwork, d_counters + cls);
+                else ZWZ_LAUNCH(k3, std::min(nwork, sms), zwz::MatchClass<3>::kThreads, zwz::MatchClass<3>::kSmem, st, job, d_order + w0, nwork, d_counters + cls);
+            } else if (cls == 0) {
                 ZWZ_LAUNCH(zwz::lz_match_kernel<0>, std::min(nwork, sms * 6u), zwz::MatchClass<0>::kThreads, zwz::MatchClass<0>::kSmem, st, job,
                            d_order + w0, nwork, d_counters + cls);
             } else if (cls == 1) {
@@ -797,7 +920,12 @@ int zwz_deflate_batch_device_ex(zwz_ctx *ctx, const uint8_t *d_raw, const uint64
         uint32_t grid2 = std::min<uint32_t>((job.n + ZWZ_DE_WARPS - 1) / ZWZ_DE_WARPS, (uint32_t) ctx->sm_count * 8u);
         {
             ProfSpan ps(ctx, ZWZ_PROF_ENCODE, st);
-            ZWZ_LAUNCH(zwz::deflate_encode_kernel, grid2, ZWZ_DE_WARPS * 32, ZWZ_DE_SMEM, st, job, d_counters + 4);
+            if (dict.idx) {
+                auto *ke = zwz::deflate_encode_kernel<true>;
+                ZWZ_LAUNCH(ke, grid2, ZWZ_DE_WARPS * 32, ZWZ_DE_SMEM, st, job, d_counters + 4);
+            } else {
+                ZWZ_LAUNCH(zwz::deflate_encode_kernel<false>, grid2, ZWZ_DE_WARPS * 32, ZWZ_DE_SMEM, st, job, d_counters + 4);
+            }
         }
         if ((rc = check_launch(ctx, "deflate_encode_kernel"))) return rc;
     }
@@ -820,7 +948,7 @@ static int slot_queue_md5(zwz_ctx *ctx, zwz::DigestSlot &sl, const uint64_t *off
 
 static int deflate_host_impl(zwz_ctx *ctx, const uint8_t *raw, const uint64_t *off, const uint32_t *len, uint32_t n, uint8_t *out, uint64_t out_cap,
                              uint64_t *packed_off, zwz_deflate_result *res, int level, int format, const uint64_t *md5_off, const uint64_t *md5_len,
-                             uint32_t md5_n, uint8_t *digest, uint64_t *ticket) {
+                             uint32_t md5_n, uint8_t *digest, uint64_t *ticket, const zwz_dicts *dicts = nullptr) {
     if (!ctx) return ZWZ_E_ARG;
     if (ticket) *ticket = 0;
     if (!packed_off) return fail(ctx, ZWZ_E_ARG, "null argument");
@@ -864,8 +992,10 @@ static int deflate_host_impl(zwz_ctx *ctx, const uint8_t *raw, const uint64_t *o
             if (!ok) s->digest_dst = nullptr;
         }
     } disarm{sl};
-    if ((rc = zwz_deflate_batch_device_ex(ctx, (const uint8_t *) sl->data.p, roff.data(), len, n, (uint8_t *) ctx->bulk_out.p, slot.data(), res,
-                                          level, format, nullptr)))
+    zwz_dicts ddev;
+    if ((rc = upload_dicts(ctx, dicts, &ddev))) return rc;
+    if ((rc = zwz_deflate_batch_device_dict(ctx, (const uint8_t *) sl->data.p, roff.data(), len, n, (uint8_t *) ctx->bulk_out.p, slot.data(), res,
+                                            level, format, dicts ? &ddev : nullptr, nullptr)))
         return rc;
     tr.mark("md5+deflate");
     for (uint32_t i = 0; i < n; ++i) packed_off[i + 1] = packed_off[i] + res[i].len0 + res[i].len1;
@@ -972,6 +1102,11 @@ int zwz_deflate_batch_ex(zwz_ctx *ctx, const uint8_t *raw, const uint64_t *off, 
     return deflate_host_impl(ctx, raw, off, len, n, out, out_cap, packed_off, res, level, format, nullptr, nullptr, 0, nullptr, nullptr);
 }
 
+int zwz_deflate_batch_dict(zwz_ctx *ctx, const uint8_t *raw, const uint64_t *off, const uint32_t *len, uint32_t n, uint8_t *out, uint64_t out_cap,
+                           uint64_t *packed_off, zwz_deflate_result *res, int level, int format, const zwz_dicts *dicts) {
+    return deflate_host_impl(ctx, raw, off, len, n, out, out_cap, packed_off, res, level, format, nullptr, nullptr, 0, nullptr, nullptr, dicts);
+}
+
 uint64_t zwz_count_chunks(const uint64_t *file_off, uint32_t nf) {
     uint64_t c = 0;
     for (uint32_t i = 0; i < nf; ++i) c += (file_off[i + 1] - file_off[i]) / ZWZ_CHUNK_SIZE + 1;
@@ -1027,6 +1162,12 @@ int zwz_wait(zwz_ctx *ctx, uint64_t ticket) {
 // ======================================================================================================================
 int zwz_inflate_batch_device(zwz_ctx *ctx, const uint8_t *d_comp, const uint64_t *off, const uint32_t *len, uint32_t n, uint8_t *d_raw_out,
                              const uint64_t *raw_off, uint32_t *raw_len, uint32_t *status, uint32_t flags, void *stream_v) {
+    return zwz_inflate_batch_device_dict(ctx, d_comp, off, len, n, d_raw_out, raw_off, raw_len, status, flags, nullptr, stream_v);
+}
+
+int zwz_inflate_batch_device_dict(zwz_ctx *ctx, const uint8_t *d_comp, const uint64_t *off, const uint32_t *len, uint32_t n, uint8_t *d_raw_out,
+                                  const uint64_t *raw_off, uint32_t *raw_len, uint32_t *status, uint32_t flags, const zwz_dicts *dicts,
+                                  void *stream_v) {
     if (!ctx) return ZWZ_E_ARG;
     if (n == 0) return ZWZ_OK;
     if (!off || !len || !raw_off || !raw_len || !status) return fail(ctx, ZWZ_E_ARG, "null argument");
@@ -1036,6 +1177,9 @@ int zwz_inflate_batch_device(zwz_ctx *ctx, const uint8_t *d_comp, const uint64_t
     zwz_rt::set_device(ctx->device);
     zwz_stream_t st = stream_v ? (zwz_stream_t) stream_v : ctx->stream;
     Trace tr(ctx, "inflate_device", st);
+    zwz::DictTable dict{};
+    int rc;
+    if ((rc = stage_dicts(ctx, dicts, n, format == ZWZ_FORMAT_GZIP || ctx->inflate_mode == 2, st, &dict))) return rc;
     // Mapping: one warp per stream (inflate.cuh) is the product path. One lane per stream (inflate_lanes.cuh,
     // ZWZ_INFLATE_MODE=lanes) needs ~40x fewer warp-instructions per byte but only three warps fit an SM next to its
     // per-lane tables, and at that occupancy it runs latency-bound: 140 ms against 68 ms per C2 step on B200. It stays as a
@@ -1046,7 +1190,6 @@ int zwz_inflate_batch_device(zwz_ctx *ctx, const uint8_t *d_comp, const uint64_t
     const size_t m_off = 0, m_roff = (size_t) n * 8, m_len = m_roff + (size_t) (n + 1) * 8, m_order = m_len + (size_t) n * 4,
                  meta_bytes = m_order + (lanes ? (size_t) n * 4 : 0);
     const size_t r_base = align_up(meta_bytes, 256);
-    int rc;
     if ((rc = reserve(ctx, ctx->pin_meta, std::max(meta_bytes, (size_t) n * 8), true))) return rc;
     if ((rc = reserve(ctx, ctx->meta, r_base + (size_t) n * 8 + 512, false))) return rc;
     uint8_t *hp = (uint8_t *) ctx->pin_meta.p;
@@ -1088,8 +1231,15 @@ int zwz_inflate_batch_device(zwz_ctx *ctx, const uint8_t *d_comp, const uint64_t
         } else {
             uint32_t grid = std::min<uint32_t>((n + ZWZ_INF_WARPS - 1) / ZWZ_INF_WARPS, (uint32_t) (ctx->sm_count * ctx->inf_blocks_per_sm));
             if (ctx->inflate_mode == 3) flags |= ZWZ_INFLATE_CAREFUL;
-            ZWZ_LAUNCH(zwz::inflate_kernel, grid, ZWZ_INF_WARPS * 32, ZWZ_INF_SMEM, st, d_comp, (const uint64_t *) (dm + m_off),
-                       (const uint32_t *) (dm + m_len), d_raw_out, (const uint64_t *) (dm + m_roff), d_rlen, d_stat, n, flags, d_counter);
+            if (dict.idx) { // the DICT instantiation only when some stream of the call has a dictionary
+                grid = std::min<uint32_t>((n + ZWZ_INF_WARPS - 1) / ZWZ_INF_WARPS, (uint32_t) (ctx->sm_count * ctx->inf_dict_blocks_per_sm));
+                auto *ki = zwz::inflate_kernel<true>;
+                ZWZ_LAUNCH(ki, grid, ZWZ_INF_WARPS * 32, ZWZ_INF_SMEM, st, d_comp, (const uint64_t *) (dm + m_off), (const uint32_t *) (dm + m_len),
+                           d_raw_out, (const uint64_t *) (dm + m_roff), d_rlen, d_stat, n, flags, d_counter, dict);
+            } else {
+                ZWZ_LAUNCH(zwz::inflate_kernel<false>, grid, ZWZ_INF_WARPS * 32, ZWZ_INF_SMEM, st, d_comp, (const uint64_t *) (dm + m_off),
+                           (const uint32_t *) (dm + m_len), d_raw_out, (const uint64_t *) (dm + m_roff), d_rlen, d_stat, n, flags, d_counter, dict);
+            }
         }
     }
     if ((rc = check_launch(ctx, "inflate_kernel"))) return rc;
@@ -1106,6 +1256,11 @@ int zwz_inflate_batch_device(zwz_ctx *ctx, const uint8_t *d_comp, const uint64_t
 
 int zwz_inflate_batch(zwz_ctx *ctx, const uint8_t *comp, const uint64_t *off, const uint32_t *len, uint32_t n, uint8_t *raw_out,
                       const uint64_t *raw_off, uint32_t *raw_len, uint32_t *status, uint32_t flags) {
+    return zwz_inflate_batch_dict(ctx, comp, off, len, n, raw_out, raw_off, raw_len, status, flags, nullptr);
+}
+
+int zwz_inflate_batch_dict(zwz_ctx *ctx, const uint8_t *comp, const uint64_t *off, const uint32_t *len, uint32_t n, uint8_t *raw_out,
+                           const uint64_t *raw_off, uint32_t *raw_len, uint32_t *status, uint32_t flags, const zwz_dicts *dicts) {
     if (!ctx) return ZWZ_E_ARG;
     if (n == 0) return ZWZ_OK;
     if (!off || !len || !raw_off || !raw_len || !status) return fail(ctx, ZWZ_E_ARG, "null argument");
@@ -1123,8 +1278,10 @@ int zwz_inflate_batch(zwz_ctx *ctx, const uint8_t *comp, const uint64_t *off, co
     if ((rc = reserve(ctx, ctx->bulk_in, (size_t) (hi - lo) + 64, false))) return rc;
     if ((rc = reserve(ctx, ctx->bulk_out, (size_t) roff[n] + 64, false))) return rc;
     if (zwz_rt::memcpy_h2d(ctx->bulk_in.p, comp + lo, (size_t) (hi - lo), ctx->stream)) return fail(ctx, ZWZ_E_CUDA, "compressed upload failed");
-    if ((rc = zwz_inflate_batch_device(ctx, (const uint8_t *) ctx->bulk_in.p, coff.data(), len, n, (uint8_t *) ctx->bulk_out.p, roff.data(), raw_len,
-                                       status, flags, nullptr)))
+    zwz_dicts ddev;
+    if ((rc = upload_dicts(ctx, dicts, &ddev))) return rc;
+    if ((rc = zwz_inflate_batch_device_dict(ctx, (const uint8_t *) ctx->bulk_in.p, coff.data(), len, n, (uint8_t *) ctx->bulk_out.p, roff.data(),
+                                            raw_len, status, flags, dicts ? &ddev : nullptr, nullptr)))
         return rc;
     if (zwz_rt::memcpy_d2h(raw_out + raw_off[0], ctx->bulk_out.p, (size_t) roff[n], ctx->stream) || zwz_rt::stream_sync(ctx->stream))
         return fail(ctx, ZWZ_E_CUDA, "raw download failed");
