@@ -94,9 +94,9 @@ uint64_t zwz_launch_count(const zwz_ctx *ctx);
  * launch counts per kernel kind since the last reset. */
 #define ZWZ_PROF_MATCH 0   /* lz_match_kernel        */
 #define ZWZ_PROF_ENCODE 1  /* deflate_encode_kernel  */
-#define ZWZ_PROF_INFLATE 2 /* inflate_kernel         */
+#define ZWZ_PROF_INFLATE 2 /* inflate_kernel; block_find_kernel, inflate_span_kernel */
 #define ZWZ_PROF_MD5 3     /* md5_files_kernel       */
-#define ZWZ_PROF_PACK 4    /* pack_streams_kernel    */
+#define ZWZ_PROF_PACK 4    /* pack_streams_kernel; win_map_kernel, win_scan_kernel, stream_gather_kernel */
 #define ZWZ_PROF_ADLER 5   /* checksum kernels: adler32_kernel, crc32_kernel; dict_chain_kernel */
 #define ZWZ_PROF_N 6
 int zwz_profile_enable(zwz_ctx *ctx, int on);
@@ -149,6 +149,34 @@ int zwz_inflate_batch_device(zwz_ctx *ctx, const uint8_t *d_comp, const uint64_t
                              uint32_t flags, void *stream);
 int zwz_inflate_batch(zwz_ctx *ctx, const uint8_t *comp, const uint64_t *off, const uint32_t *len, uint32_t n,
                       uint8_t *raw_out, const uint64_t *raw_off, uint32_t *raw_len, uint32_t *status, uint32_t flags);
+
+/* ---- one long stream on the whole GPU ----------------------------------------------------------------------------------
+ * The batch calls give every stream one warp. A .gz file written by gzip, pigz, zlib or tar is one long stream (or a few
+ * concatenated members), so these calls cut it into spans of compressed bytes instead: the spans start at block headers found by
+ * searching (dynamic and stored blocks; a stream made of fixed blocks only decodes as one span), are decoded in parallel with
+ * their 32 KiB window still unknown, confirmed against each other (a false start is decoded again), and the windows are then
+ * resolved by a log-depth scan (DESIGN.md §4.8).
+ *   comp[0 .. comp_len) is ONE stream, comp_len < 4 GiB; the output may be larger than 4 GiB. flags are the inflate flags with
+ *   the format in bits 8..15, whatever ZWZ_INFLATE_MODE says:
+ *     GZIP : every member, as gzip -d: a member follows where the previous trailer ends when the next two bytes are 1f 8b; any
+ *            other bytes behind a trailer are ignored. The result is that of zlib 1.3 (windowBits 31) decoding the members one
+ *            after another and stopping at the first that does not end cleanly; a CRC-32 or ISIZE mismatch is ZWZ_STREAM_BAD
+ *            behind all of that member's bytes. A BGZF file is one case of this.
+ *     ZLIB : one stream (windowBits 15). FDICT is ZWZ_STREAM_BAD with 0 bytes: this call takes no dictionary.
+ *     RAW  : one stream (windowBits -15).
+ *   Bytes and status are zlib's otherwise (ZWZ_STREAM_END / TRUNCATED / BAD, bytes before an error included); NO_ADLER skips
+ *   CRC-32 / Adler-32 (ISIZE is still checked). Bytes of out past *raw_len may have been written.
+ *   ZWZ_STREAM_OUTPUT_FULL: out_cap is smaller than what the stream decodes to (up to its end or first decoding error, check
+ *   values aside); *raw_len is that size. Nothing is written when the stream fits one scratch wave (below); otherwise the waves
+ *   before the one that would pass out_cap have been written. (The batch calls instead fill up to the capacity.)
+ *   NULL pointers and an unknown format are ZWZ_E_ARG.
+ * Device scratch: u16 span slots (2 bytes per output byte) of one wave at a time, about ZWZ_TUNE_STREAM_SCRATCH_BYTES, plus 128 KiB
+ * of window maps per span of the wave; allocated for the call and freed after it.
+ * Adversarial input with a false block start in every span costs one confirmation round per span; it still decodes exactly. */
+int zwz_inflate_stream_device(zwz_ctx *ctx, const uint8_t *d_comp, uint64_t comp_len, uint8_t *d_out, uint64_t out_cap,
+                              uint64_t *raw_len, uint32_t *status, uint32_t flags, void *stream);
+int zwz_inflate_stream(zwz_ctx *ctx, const uint8_t *comp, uint64_t comp_len, uint8_t *out, uint64_t out_cap,
+                       uint64_t *raw_len, uint32_t *status, uint32_t flags);
 
 /* ---- preset dictionaries (zlib's deflateSetDictionary / inflateSetDictionary, Python's zdict=) ----------------------------
  * A table of dictionaries, and for every chunk / stream the one it uses. Dictionary k is data[off[k] .. off[k+1]) (at most
@@ -232,6 +260,13 @@ int zwz_decompress_records(zwz_ctx *ctx, const uint8_t *comp, const uint64_t *of
  * alone, so that many contexts fed by threads of their own with small batches do not oversubscribe the host. */
 #define ZWZ_TUNE_HOST_THREADS 2
 #define ZWZ_TUNE_HOST_PARALLEL_MIN 3
+/* ZWZ_TUNE_STREAM_SPAN_BYTES: compressed bytes per span of zwz_inflate_stream* (>= 1024; 0 = default: max(64 KiB, enough for two
+ * spans per resident decoder warp)). */
+#define ZWZ_TUNE_STREAM_SPAN_BYTES 4
+/* ZWZ_TUNE_STREAM_SCRATCH_BYTES: u16 span slots of one wave of zwz_inflate_stream* (0 = default, 4 GiB). Larger streams are decoded
+ * in waves of consecutive spans that hand on the resolved window and the running check value; a single span larger than the budget
+ * still forms a wave of its own. */
+#define ZWZ_TUNE_STREAM_SCRATCH_BYTES 5
 int zwz_ctx_tune(zwz_ctx *ctx, int what, uint64_t value);
 
 /* ---- asynchronous forms: the digests are DEFERRED ----------------------------------------------------------------------

@@ -153,6 +153,8 @@ def _declare(L):
     L.zwz_deflate_batch_dict.argtypes = [vp, vp, vp, vp, u32, vp, u64, vp, vp, i32, i32, dp]
     L.zwz_inflate_batch_device_dict.argtypes = [vp, vp, vp, vp, u32, vp, vp, vp, vp, u32, dp, vp]
     L.zwz_inflate_batch_dict.argtypes = [vp, vp, vp, vp, u32, vp, vp, vp, vp, u32, dp]
+    L.zwz_inflate_stream_device.argtypes = [vp, vp, u64, vp, u64, vp, vp, u32, vp]
+    L.zwz_inflate_stream.argtypes = [vp, vp, u64, vp, u64, vp, vp, u32]
     return L
 
 
@@ -249,6 +251,8 @@ class Context:
     TUNE_DEFLATE_SUBBATCH_BYTES = 1
     TUNE_HOST_THREADS = 2
     TUNE_HOST_PARALLEL_MIN = 3
+    TUNE_STREAM_SPAN_BYTES = 4
+    TUNE_STREAM_SCRATCH_BYTES = 5
 
     def tune(self, what: int, value: int):
         """zwz_ctx_tune: e.g. TUNE_DEFLATE_SUBBATCH_BYTES (raw bytes per internal deflate pass; the scratch is 6 bytes per raw byte of one pass),
@@ -360,6 +364,45 @@ class Context:
         self._check(self.lib.zwz_inflate_batch_device_dict(self.h, d_comp, _ptr(off), _ptr(length), n, d_raw_out, _ptr(raw_off), _ptr(rl), _ptr(st),
                                                            flags | (_format(format) << 8), dicts, stream or None))
         return rl, st
+
+    # ---- one long stream on the whole GPU ----
+    def inflate_stream(self, comp, format: str = "gzip", out_cap: Optional[int] = None, flags: int = 0):
+        """Host buffer holding ONE stream: a .gz file (every member, as gzip -d), a zlib stream or raw DEFLATE, inflated by all SMs.
+        Returns (out uint8 array, status). Without out_cap the output buffer starts at the last gzip ISIZE (exact for one member
+        under 4 GiB), at most 1032 times the input (DEFLATE's largest ratio), and the call is repeated once with the size it reports
+        as needed. With STREAM_OUTPUT_FULL (only with out_cap given) out is empty and self.last_needed is the size the stream needs."""
+        comp = _u8(comp)
+        f = _format(format)
+        if out_cap is None:
+            cap = 4 * len(comp) + 1024
+            if f == FORMAT_GZIP and len(comp) >= 4:
+                cap = min(int.from_bytes(comp[-4:].tobytes(), "little"), 1032 * len(comp) + 1024)
+            out, st, need = self._inflate_stream(comp, f, cap, flags)
+            if st != STREAM_OUTPUT_FULL:
+                return out, st
+            return self._inflate_stream(comp, f, need, flags)[:2]
+        out, st, need = self._inflate_stream(comp, f, out_cap, flags)
+        self.last_needed = need
+        return out, st
+
+    def _inflate_stream(self, comp, f: int, cap: int, flags: int):
+        out = np.empty(max(cap, 1), dtype=np.uint8)
+        rl = np.zeros(1, dtype=np.uint64)
+        st = np.zeros(1, dtype=np.uint32)
+        self._check(self.lib.zwz_inflate_stream(self.h, comp.ctypes.data if comp.size else _ptr(out), comp.size, out.ctypes.data, cap, rl.ctypes.data,
+                                                st.ctypes.data, flags | (f << 8)))
+        if int(st[0]) == STREAM_OUTPUT_FULL:
+            return np.empty(0, dtype=np.uint8), STREAM_OUTPUT_FULL, int(rl[0])
+        return out[:int(rl[0])], int(st[0]), int(rl[0])
+
+    def inflate_stream_device(self, d_comp: int, comp_len: int, d_out: int, out_cap: int, format: str = "gzip", flags: int = 0, stream: int = 0):
+        """Device buffers: d_comp[0 .. comp_len) is one stream, d_out has out_cap bytes. Returns (raw_len, status); with
+        STREAM_OUTPUT_FULL raw_len is the size needed and nothing was written."""
+        rl = np.zeros(1, dtype=np.uint64)
+        st = np.zeros(1, dtype=np.uint32)
+        self._check(self.lib.zwz_inflate_stream_device(self.h, d_comp, comp_len, d_out, out_cap, rl.ctypes.data, st.ctypes.data,
+                                                       flags | (_format(format) << 8), stream or None))
+        return int(rl[0]), int(st[0])
 
     def decompress_records(self, comp, off, length, rec_cap, rec_file, nf: int, out_cap: int, want_md5: bool = True, flags: int = 0):
         """Worker side of decompression.cpp:100-151 for a group of records (host buffers): inflate every record, concatenate the

@@ -11,6 +11,7 @@
 #include "crc32.cuh"
 #include "inflate.cuh"
 #include "inflate_lanes.cuh"
+#include "inflate_stream.cuh"
 #include "deflate_match.cuh"
 #include "deflate_encode.cuh"
 
@@ -21,6 +22,7 @@
 #include <algorithm>
 #include <atomic>
 #include <condition_variable>
+#include <deque>
 #include <functional>
 #include <memory>
 #include <mutex>
@@ -166,6 +168,9 @@ struct zwz_ctx {
     size_t total_mem = 0, smem_optin = 0;
     int inf_blocks_per_sm = 1; // resident inflate_kernel CTAs per SM
     int inf_dict_blocks_per_sm = 1; // the same for inflate_kernel<true>
+    int span_blocks_per_sm = 1; // the same for inflate_span_kernel
+    uint64_t stream_span_bytes = 0; // ZWZ_TUNE_STREAM_SPAN_BYTES (0 = default)
+    uint64_t stream_scratch_bytes = 0; // ZWZ_TUNE_STREAM_SCRATCH_BYTES (0 = default)
     zwz_stream_t stream = nullptr;
     zwz_stream_t md5_stream = nullptr; // deferred digests (DigestSlot)
     zwz::DigestSlot slot[2];
@@ -530,12 +535,15 @@ int zwz_init(int device, zwz_ctx **out) {
         zwz_rt::set_max_dyn_smem((const void *) zwz::inflate_kernel<true>, ZWZ_INF_SMEM) ||
         zwz_rt::set_max_dyn_smem((const void *) zwz::md5_files_staged_kernel, ZWZ_MD5S_SMEM) ||
         zwz_rt::set_max_dyn_smem((const void *) zwz::inflate_kernel<false>, ZWZ_INF_SMEM) ||
-        zwz_rt::set_max_dyn_smem((const void *) zwz::inflate_lanes_kernel, ZWZ_IL_SMEM)) {
+        zwz_rt::set_max_dyn_smem((const void *) zwz::inflate_lanes_kernel, ZWZ_IL_SMEM) ||
+        zwz_rt::set_max_dyn_smem((const void *) zwz::inflate_span_kernel, ZWZ_INF_SMEM) ||
+        zwz_rt::set_max_dyn_smem((const void *) zwz::block_find_kernel, ZWZ_INF_SMEM)) {
         delete ctx;
         return ZWZ_E_NODEVICE;
     }
     if (zwz_rt::max_blocks_per_sm(&ctx->inf_blocks_per_sm, (const void *) zwz::inflate_kernel<false>, ZWZ_INF_WARPS * 32, ZWZ_INF_SMEM) ||
-        zwz_rt::max_blocks_per_sm(&ctx->inf_dict_blocks_per_sm, (const void *) zwz::inflate_kernel<true>, ZWZ_INF_WARPS * 32, ZWZ_INF_SMEM)) {
+        zwz_rt::max_blocks_per_sm(&ctx->inf_dict_blocks_per_sm, (const void *) zwz::inflate_kernel<true>, ZWZ_INF_WARPS * 32, ZWZ_INF_SMEM) ||
+        zwz_rt::max_blocks_per_sm(&ctx->span_blocks_per_sm, (const void *) zwz::inflate_span_kernel, ZWZ_INF_WARPS * 32, ZWZ_INF_SMEM)) {
         delete ctx;
         return ZWZ_E_NODEVICE;
     }
@@ -617,6 +625,15 @@ int zwz_ctx_tune(zwz_ctx *ctx, int what, uint64_t value) {
     }
     if (what == ZWZ_TUNE_HOST_PARALLEL_MIN) {
         ctx->host_parallel_min = value;
+        return ZWZ_OK;
+    }
+    if (what == ZWZ_TUNE_STREAM_SPAN_BYTES) {
+        if (value != 0 && value < 1024) return fail(ctx, ZWZ_E_ARG, "span below 1 KiB");
+        ctx->stream_span_bytes = value;
+        return ZWZ_OK;
+    }
+    if (what == ZWZ_TUNE_STREAM_SCRATCH_BYTES) {
+        ctx->stream_scratch_bytes = value;
         return ZWZ_OK;
     }
     return fail(ctx, ZWZ_E_ARG, "unknown tuning knob");
@@ -1810,6 +1827,464 @@ int zwz_crc32_batch_device(zwz_ctx *ctx, const uint8_t *d_data, const uint64_t *
     if (zwz_rt::memcpy_d2h(hp, dm + r_base, (size_t) n * 4, st) || zwz_rt::stream_sync(st)) return fail(ctx, ZWZ_E_CUDA, "crc32 kernel failed");
     memcpy(crc, hp, (size_t) n * 4);
     return ZWZ_OK;
+}
+
+// ======================================================================================================================
+// one long stream on the whole GPU (inflate_stream.cuh)
+// ======================================================================================================================
+#ifdef ZWZ_EMU
+// test-only counters of the emulator build: [0] spans decoded (reruns included), [1] repair rounds, [2] spans decoded again from
+// their predecessor's stop (false or missed candidates), [3] slot overflows decoded again, [4] candidates found, [5] waves
+static uint64_t g_stream_stats[8];
+extern "C" void zwz_emu_stream_stats(uint64_t *out, int reset) {
+    for (int i = 0; i < 8; ++i) {
+        out[i] = g_stream_stats[i];
+        if (reset) g_stream_stats[i] = 0;
+    }
+}
+#define ZWZ_STREAM_STAT(i, v) (g_stream_stats[i] += (v))
+// test-only: the log-depth window scan (win_scan_kernel, launched as inflate_stream_impl launches it) over m maps of 32 768 entries,
+// in place; map 0 must hold no window references
+extern "C" void zwz_emu_win_scan(uint16_t *maps, uint32_t m) {
+    std::vector<uint16_t> tmp((size_t) m * ZWZ_SPAN_WIN);
+    uint16_t *w0 = maps, *w1 = tmp.data();
+    const uint32_t grid = m * (ZWZ_SPAN_WIN / 256u);
+    for (uint32_t d = 1; d < m; d <<= 1) {
+        ZWZ_LAUNCH(zwz::win_scan_kernel, grid, 256, 0, nullptr, (const uint16_t *) w0, w1, m, d);
+        std::swap(w0, w1);
+    }
+    if (w0 != maps) memcpy(maps, w0, tmp.size() * 2);
+}
+#else
+#define ZWZ_STREAM_STAT(i, v) ((void) 0)
+#endif
+
+static uint32_t crc32_combine_host(uint32_t c1, uint32_t c2, uint64_t len2) {
+    static const zwz::Crc32Tables T = zwz::crc32_make_tables();
+    uint32_t p = 0x80000000u; // x^(8 len2) mod P, as crc32_x8n
+    for (uint32_t k = 3; len2; len2 >>= 1, ++k)
+        if (len2 & 1u) p = zwz::crc32_multmodp_c(T.x2n[k & 31u], p);
+    return zwz::crc32_multmodp_c(p, c1) ^ c2;
+}
+static uint32_t adler32_combine_host(uint32_t a1, uint32_t a2, uint64_t len2) { // zlib's adler32_combine
+    const uint32_t BASE = 65521u, rem = (uint32_t) (len2 % BASE);
+    uint32_t sum1 = a1 & 0xffffu;
+    uint32_t sum2 = (uint32_t) (((uint64_t) rem * sum1) % BASE);
+    sum1 += (a2 & 0xffffu) + BASE - 1u;
+    sum2 += ((a1 >> 16) & 0xffffu) + ((a2 >> 16) & 0xffffu) + BASE - rem;
+    if (sum1 >= BASE) sum1 -= BASE;
+    if (sum1 >= BASE) sum1 -= BASE;
+    if (sum2 >= (BASE << 1)) sum2 -= (BASE << 1);
+    if (sum2 >= BASE) sum2 -= BASE;
+    return sum1 | (sum2 << 16);
+}
+
+// device buffers of one zwz_inflate_stream call, freed (stream-ordered) when it returns
+struct StreamBufs {
+    zwz_stream_t st;
+    std::vector<void *> p;
+    explicit StreamBufs(zwz_stream_t s) : st(s) {}
+    ~StreamBufs() {
+        if (p.empty()) return;
+        zwz_rt::stream_sync(st);
+        for (void *q : p) zwz_rt::free_arena(q, st);
+    }
+    void *get(size_t bytes) {
+        void *q = nullptr;
+        if (zwz_rt::malloc_arena(&q, bytes ? bytes : 1, st)) return nullptr;
+        p.push_back(q);
+        return q;
+    }
+};
+
+struct SpanEnt {
+    uint64_t start;     // SpanJob::start
+    uint32_t mode;
+    bool decoded = false;
+    zwz::SpanRes r{};
+    std::vector<zwz::SpanMember> mem;
+    uint16_t *slot = nullptr;
+    uint64_t cap = 0;
+};
+static bool span_terminal(const SpanEnt &e) {
+    return e.r.status != zwz::SPAN_STOPPED && e.r.status != zwz::SPAN_STOP_MEMBER && e.r.status != zwz::SPAN_STOPPED_STORED;
+}
+// the mode a span starting where e stopped decodes in
+static uint32_t span_stop_mode(const SpanEnt &e) {
+    return e.r.status == zwz::SPAN_STOP_MEMBER ? zwz::SPAN_MODE_MEMBER : (e.r.status == zwz::SPAN_STOPPED_STORED ? zwz::SPAN_MODE_STORED : zwz::SPAN_MODE_BLOCK);
+}
+// slot elements a span gets at first: about 4x its compressed bytes (enough for text); a span that needs more is decoded again
+// with its exact size
+static uint64_t span_estimate(uint64_t start, uint64_t target, uint64_t comp_len) {
+    const uint64_t b0 = (start >> 1) >> 3, b1 = target == ~(uint64_t) 0 ? comp_len : std::min<uint64_t>(comp_len, (target >> 1) >> 3);
+    return (b1 > b0 ? b1 - b0 : 0) * 4u + 4096u;
+}
+
+// Decode the entries `todo` of L in one launch, each up to the start of its successor (the last one of L up to `tail`); `exact`:
+// slots of exactly the size the previous decode of the entry reported.
+static int span_decode_round(zwz_ctx *ctx, zwz_stream_t st, StreamBufs &bufs, const uint8_t *d_comp, uint64_t comp_len, uint32_t flags,
+                             std::vector<SpanEnt> &L, uint64_t tail, const std::vector<size_t> &todo, bool exact) {
+    const size_t n = todo.size();
+    if (!n) return ZWZ_OK;
+    std::vector<zwz::SpanJob> jobs(n);
+    size_t elems = 0;
+    for (size_t k = 0; k < n; ++k) {
+        SpanEnt &e = L[todo[k]];
+        const uint64_t target = todo[k] + 1 < L.size() ? L[todo[k] + 1].start : tail;
+        const uint64_t cap = exact ? e.r.nout : span_estimate(e.start, target, comp_len);
+        jobs[k].start = e.start;
+        jobs[k].target = target;
+        jobs[k].cap = cap;
+        jobs[k].mode = e.mode;
+        jobs[k].pad = 0;
+        elems += align_up(cap, 64);
+    }
+    uint16_t *slab = (uint16_t *) bufs.get(elems * 2);
+    uint8_t *dj = (uint8_t *) bufs.get(n * (sizeof(zwz::SpanJob) + sizeof(zwz::SpanRes) + ZWZ_SPAN_MAXM * sizeof(zwz::SpanMember)) + 256);
+    if (!slab || !dj) return fail(ctx, ZWZ_E_NOMEM, "stream scratch allocation failed");
+    for (size_t k = 0, o = 0; k < n; ++k) {
+        jobs[k].slot = slab + o;
+        o += align_up(jobs[k].cap, 64);
+    }
+    zwz::SpanJob *d_jobs = (zwz::SpanJob *) dj;
+    zwz::SpanRes *d_res = (zwz::SpanRes *) (dj + n * sizeof(zwz::SpanJob));
+    zwz::SpanMember *d_mem = (zwz::SpanMember *) (dj + n * (sizeof(zwz::SpanJob) + sizeof(zwz::SpanRes)));
+    uint32_t *d_counter = (uint32_t *) (dj + n * (sizeof(zwz::SpanJob) + sizeof(zwz::SpanRes) + ZWZ_SPAN_MAXM * sizeof(zwz::SpanMember)));
+    if (zwz_rt::memcpy_h2d(d_jobs, jobs.data(), n * sizeof(zwz::SpanJob), st) || zwz_rt::memset_device(d_counter, 0, 4, st))
+        return fail(ctx, ZWZ_E_CUDA, "span upload failed");
+    {
+        ProfSpan ps(ctx, ZWZ_PROF_INFLATE, st);
+        const uint32_t grid = (uint32_t) std::min<size_t>(n, (size_t) ctx->sm_count * ctx->span_blocks_per_sm);
+        ZWZ_LAUNCH(zwz::inflate_span_kernel, grid, ZWZ_INF_WARPS * 32, ZWZ_INF_SMEM, st, d_comp, comp_len, (const zwz::SpanJob *) d_jobs, d_res, d_mem,
+                   (uint32_t) n, flags, d_counter);
+    }
+    int rc;
+    if ((rc = check_launch(ctx, "inflate_span_kernel"))) return rc;
+    std::vector<zwz::SpanRes> res(n);
+    std::vector<zwz::SpanMember> mem(n * ZWZ_SPAN_MAXM);
+    if (zwz_rt::memcpy_d2h(res.data(), d_res, n * sizeof(zwz::SpanRes), st) ||
+        zwz_rt::memcpy_d2h(mem.data(), d_mem, n * ZWZ_SPAN_MAXM * sizeof(zwz::SpanMember), st) || zwz_rt::stream_sync(st))
+        return fail(ctx, ZWZ_E_CUDA, "inflate_span_kernel failed");
+    ZWZ_STREAM_STAT(0, n);
+    for (size_t k = 0; k < n; ++k) {
+        SpanEnt &e = L[todo[k]];
+        e.decoded = true;
+        e.r = res[k];
+        e.mem.assign(mem.begin() + k * ZWZ_SPAN_MAXM, mem.begin() + k * ZWZ_SPAN_MAXM + res[k].nmem);
+        e.slot = jobs[k].slot;
+        e.cap = jobs[k].cap;
+    }
+    return ZWZ_OK;
+}
+
+// the slots that overflowed, decoded again with their exact size
+static int span_decode_exact(zwz_ctx *ctx, zwz_stream_t st, StreamBufs &bufs, const uint8_t *d_comp, uint64_t comp_len, uint32_t flags,
+                             std::vector<SpanEnt> &L, uint64_t tail, const std::vector<size_t> &todo) {
+    std::vector<size_t> over;
+    for (size_t i : todo)
+        if (L[i].r.nout > L[i].cap) over.push_back(i);
+    ZWZ_STREAM_STAT(3, over.size());
+    return span_decode_round(ctx, st, bufs, d_comp, comp_len, flags, L, tail, over, true);
+}
+
+// Waves: the spans are decoded, confirmed, resolved and gathered in order, a wave at a time, so that the u16 slots of one wave stay
+// near the scratch budget (ZWZ_TUNE_STREAM_SCRATCH_BYTES). A wave hands the next one the resolved window behind its last span, the
+// position where that span stopped and the running check value of the member still open. d_out == NULL (the host-buffer form):
+// every wave is gathered into grow_out and downloaded to h_out.
+static int inflate_stream_impl(zwz_ctx *ctx, const uint8_t *d_comp, uint64_t comp_len, uint8_t *d_out, uint8_t *h_out, uint64_t out_cap,
+                               Arena *grow_out, uint64_t *raw_len, uint32_t *status, uint32_t flags, zwz_stream_t st) {
+    const uint32_t format = (flags >> 8) & 0xffu;
+    Trace tr(ctx, "inflate_stream", st);
+    int rc;
+    // ---- spans and their candidate starts ----
+    const uint64_t warps = (uint64_t) ctx->sm_count * ctx->span_blocks_per_sm * ZWZ_INF_WARPS;
+    const uint64_t S = ctx->stream_span_bytes ? ctx->stream_span_bytes : std::max<uint64_t>(65536u, (comp_len + 2 * warps - 1) / (2 * warps));
+    const uint64_t nspan = std::max<uint64_t>(1u, (comp_len + S - 1) / S);
+    const uint64_t budget = ctx->stream_scratch_bytes ? ctx->stream_scratch_bytes : ((uint64_t) 4 << 30);
+    std::deque<SpanEnt> Q; // candidate starts not decoded yet, in stream order
+    if (nspan > 1) {
+        StreamBufs fb(st);
+        uint64_t *d_cand = (uint64_t *) fb.get((nspan - 1) * 8);
+        if (!d_cand) return fail(ctx, ZWZ_E_NOMEM, "stream scratch allocation failed");
+        {
+            ProfSpan ps(ctx, ZWZ_PROF_INFLATE, st);
+            ZWZ_LAUNCH(zwz::block_find_kernel, (uint32_t) (nspan - 1), 32, ZWZ_INF_SMEM, st, d_comp, comp_len, S, d_cand, (uint32_t) (nspan - 1));
+        }
+        if ((rc = check_launch(ctx, "block_find_kernel"))) return rc;
+        std::vector<uint64_t> cand(nspan - 1);
+        if (zwz_rt::memcpy_d2h(cand.data(), d_cand, cand.size() * 8, st) || zwz_rt::stream_sync(st)) return fail(ctx, ZWZ_E_CUDA, "block_find_kernel failed");
+        for (uint64_t c : cand)
+            if (c != ~(uint64_t) 0)
+                Q.push_back(SpanEnt{c & ~ZWZ_SPAN_CAND_STORED, (c & ZWZ_SPAN_CAND_STORED) ? (uint32_t) zwz::SPAN_MODE_STORED : (uint32_t) zwz::SPAN_MODE_BLOCK});
+        ZWZ_STREAM_STAT(4, Q.size());
+    }
+    tr.mark("find");
+    SpanEnt cur{0, zwz::SPAN_MODE_FIRST};
+    std::unique_ptr<StreamBufs> prevb; // keeps the window handed on by the previous wave alive
+    const uint16_t *win_in = nullptr;
+    const bool sums = format != ZWZ_FORMAT_RAW && !(flags & ZWZ_INFLATE_NO_ADLER);
+    const uint32_t init = format == ZWZ_FORMAT_GZIP ? 0u : 1u;
+    uint32_t open_val = init;     // check value of the open member so far
+    uint64_t open_start = 0;      // where it started
+    uint64_t base = 0, len = 0;   // output position of the wave; bytes valid in the end
+    uint32_t stat = ZWZ_STREAM_END;
+    bool full = false;
+    size_t rounds = 0, reruns = 0, nspans = 0, waves = 0;
+    for (bool finished = false; !finished;) {
+        waves++;
+        std::unique_ptr<StreamBufs> wb(new StreamBufs(st));
+        // ---- the wave: the spans from `cur` on whose estimated slots fit the budget (one at least) ----
+        while (!Q.empty() && (Q.front().start >> 1) <= (cur.start >> 1)) Q.pop_front();
+        std::vector<SpanEnt> W;
+        W.push_back(std::move(cur));
+        auto tail = [&]() { return Q.empty() ? ~(uint64_t) 0 : Q.front().start; };
+        {
+            uint64_t est = 2 * span_estimate(W[0].start, tail(), comp_len);
+            while (!Q.empty()) {
+                const uint64_t nxt = Q.size() > 1 ? Q[1].start : ~(uint64_t) 0;
+                const uint64_t e = 2 * span_estimate(Q.front().start, nxt, comp_len);
+                if (est + e > budget) break;
+                est += e;
+                W.push_back(std::move(Q.front()));
+                Q.pop_front();
+            }
+        }
+        std::vector<size_t> all(W.size());
+        for (size_t i = 0; i < all.size(); ++i) all[i] = i;
+        if ((rc = span_decode_round(ctx, st, *wb, d_comp, comp_len, flags, W, tail(), all, false))) return rc;
+        // the slots they really need: spans past the budget go back to the queue (one span stays, whatever it needs)
+        {
+            size_t keep = 1;
+            uint64_t acc = 2 * W[0].r.nout;
+            while (keep < W.size() && acc + 2 * W[keep].r.nout <= budget) acc += 2 * W[keep++].r.nout;
+            for (size_t i = W.size(); i-- > keep;) Q.push_front(SpanEnt{W[i].start, W[i].mode});
+            W.resize(keep);
+            all.resize(keep);
+        }
+        if ((rc = span_decode_exact(ctx, st, *wb, d_comp, comp_len, flags, W, tail(), all))) return rc;
+        // ---- confirmation: W[0] is real; W[i + 1] is when W[i] (real) stopped exactly at its start. Every round decodes again each
+        // span whose decoded predecessor stopped elsewhere, from that stop; the confirmed prefix grows by one span at least. The
+        // last span's stop is where the next wave starts ----
+        size_t f = 0;
+        for (;;) {
+            bool settled = false;
+            for (;;) {
+                const SpanEnt &e = W[f];
+                if (span_terminal(e)) {
+                    W.resize(f + 1);
+                    finished = settled = true;
+                    break;
+                }
+                if (f + 1 == W.size()) {
+                    settled = true;
+                    break;
+                }
+                if (W[f + 1].decoded && W[f + 1].start == e.r.stop && W[f + 1].mode == span_stop_mode(e)) {
+                    f++;
+                    continue;
+                }
+                break;
+            }
+            if (settled) break;
+            std::vector<SpanEnt> nl(W.begin(), W.begin() + (ptrdiff_t) f + 1);
+            for (size_t j = f + 1; j < W.size(); ++j) {
+                const SpanEnt &p = nl.back();
+                if (p.decoded && !span_terminal(p)) {
+                    const uint64_t b = p.r.stop;
+                    const uint32_t m = span_stop_mode(p);
+                    if ((W[j].start >> 1) < (b >> 1)) continue; // overrun by its predecessor
+                    if (W[j].start != b || W[j].mode != m) {
+                        nl.push_back(SpanEnt{b, m}); // decode from where the predecessor stopped
+                        reruns++;
+                        if ((W[j].start >> 1) == (b >> 1)) continue; // same position, other BFINAL / mode: replaced
+                    }
+                }
+                nl.push_back(std::move(W[j]));
+            }
+            W.swap(nl);
+            std::vector<size_t> todo;
+            for (size_t i = f; i < W.size(); ++i)
+                if (!W[i].decoded) todo.push_back(i);
+            rounds++;
+            if ((rc = span_decode_round(ctx, st, *wb, d_comp, comp_len, flags, W, tail(), todo, false)) ||
+                (rc = span_decode_exact(ctx, st, *wb, d_comp, comp_len, flags, W, tail(), todo)))
+                return rc;
+        }
+        nspans += W.size();
+        if (!finished) cur = SpanEnt{W.back().r.stop, span_stop_mode(W.back())};
+        // ---- lengths and members of the wave ----
+        const size_t ns = W.size();
+        std::vector<zwz::SpanWin> sw(ns);
+        struct Member {
+            uint64_t end; // in the wave
+            zwz::SpanMember t;
+        };
+        std::vector<Member> members;
+        uint64_t total = 0;
+        for (size_t i = 0; i < ns; ++i) {
+            sw[i].slot = W[i].slot;
+            sw[i].nout = W[i].r.nout;
+            sw[i].reset = W[i].r.reset;
+            sw[i].base = total;
+            for (const zwz::SpanMember &m : W[i].mem) members.push_back(Member{total + m.end, m});
+            total += W[i].r.nout;
+        }
+        if (!full && base + total > out_cap) full = true;
+        if (full) { // only the size needed from here on
+            base += total;
+            continue;
+        }
+        uint8_t *wdst = d_out ? d_out + base : nullptr;
+        if (!wdst) {
+            if ((rc = reserve(ctx, *grow_out, total + 64, false))) return rc;
+            wdst = (uint8_t *) grow_out->p;
+        }
+        // ---- windows: map per span, inclusive scan of the compositions, then the gather ----
+        unsigned long long first_bad = ~0ull;
+        const uint32_t m = (uint32_t) (finished ? ns - 1 : ns); // spans whose outgoing window someone reads
+        uint16_t *w0 = nullptr, *w1 = nullptr;
+        if (m) {
+            w0 = (uint16_t *) wb->get((size_t) m * ZWZ_SPAN_WIN * 2);
+            w1 = (uint16_t *) wb->get((size_t) m * ZWZ_SPAN_WIN * 2);
+        }
+        if (total) {
+            std::vector<uint64_t> tiles;
+            for (size_t i = 0; i < ns; ++i)
+                for (uint64_t e = 0; e < sw[i].nout; e += ZWZ_GATHER_TILE) tiles.push_back(((uint64_t) i << 40) | e);
+            uint8_t *dm = (uint8_t *) wb->get(ns * sizeof(zwz::SpanWin) + tiles.size() * 8 + 64);
+            if ((m && (!w0 || !w1)) || !dm) return fail(ctx, ZWZ_E_NOMEM, "stream scratch allocation failed");
+            zwz::SpanWin *d_sw = (zwz::SpanWin *) dm;
+            uint64_t *d_tiles = (uint64_t *) (dm + ns * sizeof(zwz::SpanWin));
+            unsigned long long *d_bad = (unsigned long long *) (dm + ns * sizeof(zwz::SpanWin) + tiles.size() * 8);
+            if (zwz_rt::memcpy_h2d(d_sw, sw.data(), ns * sizeof(zwz::SpanWin), st) || zwz_rt::memcpy_h2d(d_tiles, tiles.data(), tiles.size() * 8, st) ||
+                zwz_rt::memcpy_h2d(d_bad, &first_bad, 8, st))
+                return fail(ctx, ZWZ_E_CUDA, "window upload failed");
+            {
+                ProfSpan ps(ctx, ZWZ_PROF_PACK, st);
+                if (m) {
+                    const uint32_t grid = m * (ZWZ_SPAN_WIN / 256u);
+                    ZWZ_LAUNCH(zwz::win_map_kernel, grid, 256, 0, st, (const zwz::SpanWin *) d_sw, win_in, w0, m);
+                    for (uint32_t d = 1; d < m; d <<= 1) {
+                        ZWZ_LAUNCH(zwz::win_scan_kernel, grid, 256, 0, st, (const uint16_t *) w0, w1, m, d);
+                        std::swap(w0, w1);
+                    }
+                }
+                ZWZ_LAUNCH(zwz::stream_gather_kernel, (uint32_t) tiles.size(), 256, 0, st, (const zwz::SpanWin *) d_sw, (const uint64_t *) d_tiles,
+                           (const uint16_t *) w0, win_in, wdst, d_bad);
+            }
+            if ((rc = check_launch(ctx, "stream_gather_kernel"))) return rc;
+            if (zwz_rt::memcpy_d2h(&first_bad, d_bad, 8, st) || zwz_rt::stream_sync(st)) return fail(ctx, ZWZ_E_CUDA, "stream_gather_kernel failed");
+        }
+        uint64_t wlen = total; // valid bytes of the wave
+        if (first_bad < total) {
+            wlen = first_bad;
+            stat = ZWZ_STREAM_BAD;
+            finished = true;
+        } else if (finished) {
+            stat = W.back().r.status;
+        }
+        // ---- check values: the members that ended in the wave (before an error), and the open member's running value; pieces of
+        // <= 1 MiB, combined in order ----
+        size_t nm = 0;
+        while (nm < members.size() && members[nm].end <= wlen) nm++;
+        if (format != ZWZ_FORMAT_RAW) {
+            std::vector<uint64_t> poff;
+            std::vector<uint32_t> plen, pseg;
+            uint64_t s0 = open_start > base ? open_start - base : 0;
+            for (size_t k = 0; k <= nm && sums; ++k) {
+                const uint64_t e = k < nm ? members[k].end : (finished ? s0 : wlen); // k == nm: the open member
+                for (uint64_t a = s0; a < e; a += (1u << 20)) {
+                    poff.push_back(a);
+                    plen.push_back((uint32_t) std::min<uint64_t>(1u << 20, e - a));
+                    pseg.push_back((uint32_t) k);
+                }
+                if (k < nm) s0 = members[k].end;
+            }
+            std::vector<uint32_t> pv(poff.size());
+            if (!poff.empty()) {
+                const size_t np = poff.size();
+                uint8_t *dm = (uint8_t *) wb->get(np * 16 + 64);
+                if (!dm) return fail(ctx, ZWZ_E_NOMEM, "stream scratch allocation failed");
+                if (zwz_rt::memcpy_h2d(dm, poff.data(), np * 8, st) || zwz_rt::memcpy_h2d(dm + np * 8, plen.data(), np * 4, st))
+                    return fail(ctx, ZWZ_E_CUDA, "check upload failed");
+                {
+                    ProfSpan ps(ctx, ZWZ_PROF_ADLER, st);
+                    if (format == ZWZ_FORMAT_GZIP)
+                        ZWZ_LAUNCH(zwz::crc32_kernel, (uint32_t) ((np + 7) / 8), 256, 0, st, wdst, (const uint64_t *) dm, (const uint32_t *) (dm + np * 8),
+                                   (uint32_t *) (dm + np * 12), (uint32_t) np);
+                    else
+                        ZWZ_LAUNCH(zwz::adler32_kernel, (uint32_t) ((np + 7) / 8), 256, 0, st, wdst, (const uint64_t *) dm, (const uint32_t *) (dm + np * 8),
+                                   (uint32_t *) (dm + np * 12), (uint32_t) np);
+                }
+                if ((rc = check_launch(ctx, "stream check kernel"))) return rc;
+                if (zwz_rt::memcpy_d2h(pv.data(), dm + np * 12, np * 4, st) || zwz_rt::stream_sync(st)) return fail(ctx, ZWZ_E_CUDA, "check kernel failed");
+            }
+            size_t q = 0;
+            for (size_t k = 0; k <= nm; ++k) {
+                for (; q < pseg.size() && pseg[q] == k; ++q)
+                    open_val = format == ZWZ_FORMAT_GZIP ? crc32_combine_host(open_val, pv[q], plen[q]) : adler32_combine_host(open_val, pv[q], plen[q]);
+                if (k == nm) break;
+                const Member &mb = members[k];
+                bool bad = sums && (mb.t.have & 1u) && open_val != mb.t.check;
+                if (!bad && (mb.t.have & 2u)) bad = (uint32_t) (base + mb.end - open_start) != mb.t.isize;
+                open_val = init;
+                open_start = base + mb.end;
+                if (bad) {
+                    wlen = mb.end;
+                    stat = ZWZ_STREAM_BAD;
+                    finished = true;
+                    break;
+                }
+            }
+        }
+        if (h_out && wlen && (zwz_rt::memcpy_d2h(h_out + base, wdst, (size_t) wlen, st) || zwz_rt::stream_sync(st)))
+            return fail(ctx, ZWZ_E_CUDA, "raw download failed");
+        len = base + wlen;
+        base += total;
+        win_in = m && !finished ? w0 + (size_t) (ns - 1) * ZWZ_SPAN_WIN : nullptr;
+        prevb = std::move(wb); // the previous wave's buffers go; this wave's window stays for the next
+    }
+    ZWZ_STREAM_STAT(1, rounds);
+    ZWZ_STREAM_STAT(2, reruns);
+    ZWZ_STREAM_STAT(5, waves);
+    if (ctx->trace) {
+        char buf[128];
+        snprintf(buf, sizeof buf, " spans %zu rounds %zu reruns %zu waves %zu,", nspans, rounds, reruns, waves);
+        tr.line += buf;
+    }
+    tr.mark("waves");
+    if (full) {
+        *raw_len = base;
+        *status = ZWZ_STREAM_OUTPUT_FULL;
+    } else {
+        *raw_len = len;
+        *status = stat;
+    }
+    return ZWZ_OK;
+}
+
+int zwz_inflate_stream_device(zwz_ctx *ctx, const uint8_t *d_comp, uint64_t comp_len, uint8_t *d_out, uint64_t out_cap, uint64_t *raw_len,
+                              uint32_t *status, uint32_t flags, void *stream_v) {
+    if (!ctx) return ZWZ_E_ARG;
+    if (!d_comp || !d_out || !raw_len || !status) return fail(ctx, ZWZ_E_ARG, "null argument");
+    if (((flags >> 8) & 0xffu) > ZWZ_FORMAT_RAW) return fail(ctx, ZWZ_E_ARG, "unknown stream format");
+    if (comp_len > 0xffffff00ull) return fail(ctx, ZWZ_E_ARG, "compressed stream of 4 GiB or more");
+    zwz_rt::set_device(ctx->device);
+    return inflate_stream_impl(ctx, d_comp, comp_len, d_out, nullptr, out_cap, nullptr, raw_len, status, flags,
+                               stream_v ? (zwz_stream_t) stream_v : ctx->stream);
+}
+
+int zwz_inflate_stream(zwz_ctx *ctx, const uint8_t *comp, uint64_t comp_len, uint8_t *out, uint64_t out_cap, uint64_t *raw_len, uint32_t *status,
+                       uint32_t flags) {
+    if (!ctx) return ZWZ_E_ARG;
+    if (!comp || !out || !raw_len || !status) return fail(ctx, ZWZ_E_ARG, "null argument");
+    if (((flags >> 8) & 0xffu) > ZWZ_FORMAT_RAW) return fail(ctx, ZWZ_E_ARG, "unknown stream format");
+    if (comp_len > 0xffffff00ull) return fail(ctx, ZWZ_E_ARG, "compressed stream of 4 GiB or more");
+    zwz_rt::set_device(ctx->device);
+    int rc;
+    if ((rc = reserve(ctx, ctx->bulk_in, (size_t) comp_len + 64, false))) return rc;
+    if (zwz_rt::memcpy_h2d(ctx->bulk_in.p, comp, (size_t) comp_len, ctx->stream)) return fail(ctx, ZWZ_E_CUDA, "compressed upload failed");
+    return inflate_stream_impl(ctx, (const uint8_t *) ctx->bulk_in.p, comp_len, nullptr, out, out_cap, &ctx->bulk_out, raw_len, status, flags, ctx->stream);
 }
 
 } // extern "C"
