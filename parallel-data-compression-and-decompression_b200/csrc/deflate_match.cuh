@@ -52,8 +52,34 @@ extern "C" void zwz_emu_match_stats(uint64_t *out, int reset) {
     }
 }
 #define ZWZ_DM_STAT(i, v) do { g_dm_stats[i] += (v); } while (0)
+// the final skip mask of each chunk of the last call (chunk index < 65 536), for the tests that restate the noise test
+static uint64_t g_dm_skip[1u << 16];
+extern "C" void zwz_emu_match_skipmasks(uint64_t *out, uint32_t n) {
+    for (uint32_t i = 0; i < n && i < (1u << 16); ++i) out[i] = g_dm_skip[i];
+}
+#define ZWZ_DM_SKIP(c, m) do { if ((c) < (1u << 16)) g_dm_skip[c] = (m); } while (0)
 #else
 #define ZWZ_DM_STAT(i, v) do { } while (0)
+#define ZWZ_DM_SKIP(c, m) do { } while (0)
+#endif
+
+// Phase clocks (nvcc build with -DZWZ_DM_PHASE_CLOCKS only, tools/match_phases.py): thread 0 of every CTA adds the clock64()
+// cycles between the CTA barriers that close the phases of a chunk, per size class; [cls][ZWZ_DM_NPHASE] counts the chunks.
+#define ZWZ_DM_NPHASE 10
+#if defined(ZWZ_DM_PHASE_CLOCKS) && !defined(ZWZ_EMU)
+__device__ unsigned long long g_dm_phase_clk[4][ZWZ_DM_NPHASE + 1];
+extern "C" int zwz_dm_phase_clocks(unsigned long long *out, int reset) {
+    if (cudaDeviceSynchronize() != cudaSuccess || cudaMemcpyFromSymbol(out, g_dm_phase_clk, sizeof(g_dm_phase_clk)) != cudaSuccess) return 1;
+    static const unsigned long long zero[4][ZWZ_DM_NPHASE + 1] = {};
+    return reset && cudaMemcpyToSymbol(g_dm_phase_clk, zero, sizeof(zero)) != cudaSuccess ? 1 : 0;
+}
+#define ZWZ_DM_CLK_DECL uint32_t dm_clk[ZWZ_DM_NPHASE + 1] = {}; long long dm_t0 = clock64();
+#define ZWZ_DM_CLK(k) do { if (tid == 0) { const long long t = clock64(); dm_clk[k] += (uint32_t) (t - dm_t0); dm_clk[ZWZ_DM_NPHASE] += (k == 0); dm_t0 = t; } } while (0)
+#define ZWZ_DM_CLK_FLUSH() do { if (tid == 0) for (int k = 0; k <= ZWZ_DM_NPHASE; ++k) atomicAdd(&g_dm_phase_clk[CLS][k], (unsigned long long) dm_clk[k]); } while (0)
+#else
+#define ZWZ_DM_CLK_DECL
+#define ZWZ_DM_CLK(k) do { } while (0)
+#define ZWZ_DM_CLK_FLUSH() do { } while (0)
 #endif
 
 template <int CLS> struct MatchClass;
@@ -78,14 +104,15 @@ template <> struct MatchClass<3> {
 // control block (after the tables); cnt[NW][NW] u16 follows it
 struct MatchCtl {
     unsigned long long mbar;   // mbarrier for the bulk copy
-    uint32_t next_tile;
     uint32_t cur_work;
+    uint32_t next_tile;        // search: the next of the searched tiles to hand out
     uint32_t nmatch;           // positions of this chunk that found a match
     uint32_t skip[2];          // bit k: the 1 024-byte stretch k looks like noise and is left out of the search
     uint32_t coll;             // repeated 4-byte windows among the noise candidates
     uint32_t coll2;            // candidate windows that also occur (by hash) among the other positions
     uint32_t set2;             // bits set in the other positions' bit set
     uint32_t base[33];         // list k = entries [base[k], base[k+1]) of the position list
+    uint8_t slist[64];         // the stretches that are searched, in order
     uint32_t adler_a[32], adler_b[32], adler_len[32];
 };
 static_assert(sizeof(MatchCtl) <= 640, "MatchCtl must fit its slot");
@@ -155,12 +182,16 @@ ZWZ_KERNEL __launch_bounds__(MatchClass<CLS>::kThreads, MatchClass<CLS>::kCtasPe
     if (tid == 0) dm_mbar_init(&ctl->mbar);
 #endif
     __syncthreads();
+    ZWZ_DM_CLK_DECL
 
     for (;;) {
         if (tid == 0) ctl->cur_work = atomicAdd(work_counter, 1u);
         __syncthreads();
         const uint32_t w = ctl->cur_work;
-        if (w >= n_work) break;
+        if (w >= n_work) {
+            ZWZ_DM_CLK_FLUSH();
+            break;
+        }
         const uint32_t c = order[w];
         const uint32_t n = job.raw_len[c];
         const uint8_t *src = job.raw + job.raw_off[c];
@@ -183,7 +214,6 @@ ZWZ_KERNEL __launch_bounds__(MatchClass<CLS>::kThreads, MatchClass<CLS>::kCtasPe
 #else
         for (uint32_t i = tid; i < skew + n; i += T) smem[i] = i < skew ? 0 : src[i - skew];
 #endif
-        for (uint32_t i = tid; i < NW * NW / 2u; i += T) ((uint32_t *) cnt)[i] = 0u;
         if (tid == 0) {
             ctl->next_tile = 0;
             ctl->nmatch = 0;
@@ -195,6 +225,7 @@ ZWZ_KERNEL __launch_bounds__(MatchClass<CLS>::kThreads, MatchClass<CLS>::kCtasPe
         parity ^= (stage_bytes != 0u);
 #endif
         __syncthreads();
+        ZWZ_DM_CLK(0);
         // bytes past the end take part in 4-byte compares: make them deterministic (the final clamp to `maxlen` makes
         // their value irrelevant for the result)
         if (tid < 32u) smem[skew + n + tid] = 0;
@@ -215,6 +246,7 @@ ZWZ_KERNEL __launch_bounds__(MatchClass<CLS>::kThreads, MatchClass<CLS>::kCtasPe
         // What this gives up: repeats that cover less than ~2 % of the noise (zlib would find them). The encoder emits these
         // stretches as stored blocks (deflate_encode.cuh: quiet stretches). With a preset dictionary such a stretch is not
         // searched against the dictionary either: a copy of dictionary bytes inside noise goes out as literals.
+        uint64_t cand, skipmask; // bit k: stretch k passed the histogram test / is left out
         {
             uint32_t *hist = (uint32_t *) head + wid * 256u;
             const uint32_t nfull = n >> 10; // the partial last stretch is always searched
@@ -252,11 +284,14 @@ ZWZ_KERNEL __launch_bounds__(MatchClass<CLS>::kThreads, MatchClass<CLS>::kCtasPe
                 __syncwarp();
             }
             __syncthreads();
-            const uint64_t cand = (uint64_t) ctl->skip[0] | ((uint64_t) ctl->skip[1] << 32);
+            ZWZ_DM_CLK(1);
+            cand = (uint64_t) ctl->skip[0] | ((uint64_t) ctl->skip[1] << 32);
+            skipmask = cand;
             if (cand) { // CTA-uniform
+                // (2) runs stretch by stretch: its three counts do not depend on the order of the windows, so neither does
+                // the verdict. The histograms are done with (barrier above): both bit sets are cleared at once.
                 constexpr uint32_t BB = HB + 4u; // head[] is 2 << HB bytes = 1 << BB bits
                 uint32_t *bits = (uint32_t *) head;
-                __syncthreads(); // the histograms are done with
                 uint32_t *bits2 = (uint32_t *) prev; // >= as large as head[] in every class
                 for (uint32_t i = tid; i < (1u << BB) / 32u; i += T) {
                     bits[i] = 0u;
@@ -268,132 +303,161 @@ ZWZ_KERNEL __launch_bounds__(MatchClass<CLS>::kThreads, MatchClass<CLS>::kCtasPe
                     ctl->set2 = 0;
                 }
                 __syncthreads();
+                const uint32_t sD0 = sD_of(smem, skew);
                 uint32_t mine = 0;
-                for (uint32_t st = wid; st < nfull * 32u; st += NW) {
-                    if (!((cand >> (st >> 5)) & 1ull)) continue;
-                    const uint32_t h = (lds32u(sD_of(smem, skew) + st * 32u + lane) * 0x9E3779B1u) >> (32u - BB);
-                    const uint32_t old = atomicOr(&bits[h >> 5], 1u << (h & 31u));
-                    mine += (uint32_t) __popc(__ballot_sync(ZWZ_FULL, (old >> (h & 31u)) & 1u));
+                for (uint64_t cm = cand; cm; cm &= cm - 1ull) {
+                    const uint32_t q0 = (uint32_t) (__ffsll((long long) cm) - 1) << 10;
+                    for (uint32_t j = wid; j < 32u; j += NW) {
+                        const uint32_t h = (lds32u(sD0 + q0 + j * 32u + lane) * 0x9E3779B1u) >> (32u - BB);
+                        const uint32_t old = atomicOr(&bits[h >> 5], 1u << (h & 31u));
+                        mine += (uint32_t) __popc(__ballot_sync(ZWZ_FULL, (old >> (h & 31u)) & 1u));
+                    }
                 }
                 if (lane == 0 && mine) atomicAdd(&ctl->coll, mine);
-                __syncthreads();
                 // ... and against the OTHER positions: the copy of PART of a noise stretch need not be a candidate itself (its
                 // histogram is narrower), and bytes that are not inserted cannot be found by anyone. The other positions' windows
                 // set a second bit set (in the prev[] area, unused so far), the candidates' windows are looked up in it: noise
                 // windows are all different, so the hits are independent — n_c * (bits set) / m of them by chance (the
                 // other way round, text windows looked up in the noise set, one unlucky window repeats its hit a hundred times).
+                // This set is built in the same phase as the first: the two sets are disjoint.
                 const uint32_t nh = n >= 3u ? n - 2u : 0u;
                 uint32_t fresh = 0; // bits this warp was the first to set: the set's load decides what chance looks like
-                for (uint32_t st = wid; st * 32u < nh; st += NW) {
-                    if (st < nfull * 32u && ((cand >> (st >> 5)) & 1ull)) continue;
-                    const uint32_t q = st * 32u + lane;
-                    const uint32_t h = (lds32u(sD_of(smem, skew) + q) * 0x9E3779B1u) >> (32u - BB);
-                    const uint32_t old2 = q < nh ? atomicOr(&bits2[h >> 5], 1u << (h & 31u)) : 0xffffffffu;
-                    fresh += (uint32_t) __popc(__ballot_sync(ZWZ_FULL, !((old2 >> (h & 31u)) & 1u)));
+                for (uint32_t q0 = 0; q0 < nh; q0 += 1024u) {
+                    if ((cand >> (q0 >> 10)) & 1ull) continue;
+                    for (uint32_t j = wid; j < 32u && q0 + j * 32u < nh; j += NW) {
+                        const uint32_t q = q0 + j * 32u + lane;
+                        const uint32_t h = (lds32u(sD0 + q) * 0x9E3779B1u) >> (32u - BB);
+                        const uint32_t old2 = q < nh ? atomicOr(&bits2[h >> 5], 1u << (h & 31u)) : 0xffffffffu;
+                        fresh += (uint32_t) __popc(__ballot_sync(ZWZ_FULL, !((old2 >> (h & 31u)) & 1u)));
+                    }
                 }
                 if (lane == 0 && fresh) atomicAdd(&ctl->set2, fresh);
                 __syncthreads();
                 uint32_t hits = 0;
-                for (uint32_t st = wid; st < nfull * 32u; st += NW) {
-                    if (!((cand >> (st >> 5)) & 1ull)) continue;
-                    const uint32_t h = (lds32u(sD_of(smem, skew) + st * 32u + lane) * 0x9E3779B1u) >> (32u - BB);
-                    hits += (uint32_t) __popc(__ballot_sync(ZWZ_FULL, (bits2[h >> 5] >> (h & 31u)) & 1u));
+                for (uint64_t cm = cand; cm; cm &= cm - 1ull) {
+                    const uint32_t q0 = (uint32_t) (__ffsll((long long) cm) - 1) << 10;
+                    for (uint32_t j = wid; j < 32u; j += NW) {
+                        const uint32_t h = (lds32u(sD0 + q0 + j * 32u + lane) * 0x9E3779B1u) >> (32u - BB);
+                        hits += (uint32_t) __popc(__ballot_sync(ZWZ_FULL, (bits2[h >> 5] >> (h & 31u)) & 1u));
+                    }
                 }
                 if (lane == 0 && hits) atomicAdd(&ctl->coll2, hits);
                 __syncthreads();
+                // every thread reaches the same verdict from the same counts; bits[] (in head[]) is no longer read
                 const uint32_t nc = (uint32_t) __popcll((long long) cand) << 10;
                 const uint32_t allowed = (uint32_t) (((uint64_t) nc * nc) >> (BB + 1u)) + (nc >> 6) + 48u;
                 const uint32_t allowed2 = (uint32_t) (((uint64_t) ctl->set2 * nc) >> BB) + (nc >> 6) + 48u; // chance: n_c * (bits set) / m
-                if (tid == 0 && (ctl->coll > allowed || ctl->coll2 > allowed2)) {
-                    ctl->skip[0] = 0;
-                    ctl->skip[1] = 0;
-                    ZWZ_DM_STAT(1, 1);
+                if (ctl->coll > allowed || ctl->coll2 > allowed2) {
+                    skipmask = 0;
+                    if (tid == 0) ZWZ_DM_STAT(1, 1);
                 }
             }
         }
-        __syncthreads();
+        ZWZ_DM_CLK(2);
         for (uint32_t i = tid; i < (1u << HB) / 2u; i += T) ((uint32_t *) head)[i] = 0xffffffffu;
-        const uint64_t skipmask = (uint64_t) ctl->skip[0] | ((uint64_t) ctl->skip[1] << 32);
+        // the stretches that are searched, in order: step / tile i of the searched ones is (slist[i >> 5] << 5) | (i & 31)
+        const uint32_t nstr = (n + 1023u) >> 10;
+        if (wid == 0) {
+#pragma unroll
+            for (uint32_t k = 0; k < 2u; ++k) {
+                const uint32_t sidx = 32u * k + lane;
+                const bool keep = sidx < nstr && !((skipmask >> sidx) & 1ull);
+                const unsigned km = __ballot_sync(ZWZ_FULL, keep);
+                if (keep) ctl->slist[(k ? (uint32_t) __popc((unsigned) ~skipmask) : 0u) + (uint32_t) __popc(km & lt)] = (uint8_t) sidx;
+            }
+        }
         if (tid == 0) {
             ZWZ_DM_STAT(0, (uint64_t) __popcll((long long) skipmask));
             ZWZ_DM_STAT(2, 1);
+            ZWZ_DM_SKIP(c, skipmask);
         }
         __syncthreads();
+        ZWZ_DM_CLK(3);
 
         uint32_t *mout = job.scratch + job.scr_off[c];
         uint16_t *list = (uint16_t *) (mout + dm_scratch_match_words(n));
         const uint32_t nhash = n >= 3u ? n - 2u : 0u; // positions that own a 3-byte hash
-        const uint32_t ntiles = (n + 31u) >> 5;
-        const uint32_t nsteps = (nhash + 31u) >> 5;
-        const uint32_t spw = (nsteps + NW - 1u) / NW;  // steps per warp: warp w owns positions [w*spw*32, (w+1)*spw*32)
+        const uint32_t nskip = 32u * (uint32_t) __popcll((long long) skipmask);
+        const uint32_t ntiles = ((n + 31u) >> 5) - nskip;  // searched tiles
+        const uint32_t nsteps = ((nhash + 31u) >> 5) - nskip; // searched hash steps (noise stretches are whole steps < nhash)
+        const uint32_t spw = (nsteps + NW - 1u) / NW;  // searched steps per warp: warp w owns [w*spw, (w+1)*spw)
+        const uint32_t s_lo = wid * spw, s_hi = min(s_lo + spw, nsteps);
 
         const uint32_t sD = smem_addr(smem) + skew; // shared address of chunk byte 0
         const uint32_t sP = smem_addr(prev);        // prev[0]
         const uint32_t sH = smem_addr(head);        // head[0]
-        const uint32_t sC = smem_addr(cnt);         // cnt[0]
-        const uint32_t sB = smem_addr(&ctl->base[0]);
+        const uint8_t *slist = ctl->slist;
         // ---- 2. hash every position; count, per warp, how many of its positions fall in each of the NW hash ranges ----
-        // Same-range lanes of a step are found with LB ballots (a 5-bit match_any), so ranks inside a step follow lane
-        // (= position) order and the lists come out sorted by position.
-        for (uint32_t st = wid * spw; st < (wid + 1u) * spw && st < nsteps; ++st) {
-            if ((skipmask >> (st >> 5)) & 1ull) continue; // noise: not inserted
-            const uint32_t p = st * 32u + lane;
-            const bool valid = p < nhash;
-            uint32_t h = 0;
-            if (valid) {
-                uint32_t v = lds32u(sD + p);
-                h = dm_hash3<HB>(v & 0xffu, (v >> 8) & 0xffu, (v >> 16) & 0xffu);
-                sts16(sP + 2u * p, h); // prev[p] holds hash(p) until the builder replaces it by the link
-            }
-            const uint32_t b = h >> (HB - LB);
-            unsigned m = __ballot_sync(ZWZ_FULL, valid);
+        // The counts stay in registers: from the LB ballots of the range bits, lane b picks out the positions of the step that
+        // fall in list b. The scatter below uses the same ballots for the rank of each position inside its list, so ranks follow
+        // lane (= position) order and the lists come out sorted by position.
+        {
+            uint32_t my = 0;
+            for (uint32_t i = s_lo; i < s_hi; ++i) {
+                const uint32_t p = (((uint32_t) slist[i >> 5] << 5) | (i & 31u)) * 32u + lane;
+                const bool valid = p < nhash;
+                uint32_t h = 0;
+                if (valid) {
+                    uint32_t v = lds32u(sD + p);
+                    h = dm_hash3<HB>(v & 0xffu, (v >> 8) & 0xffu, (v >> 16) & 0xffu);
+                    sts16(sP + 2u * p, h); // prev[p] holds hash(p) until the builder replaces it by the link
+                }
+                const uint32_t b = h >> (HB - LB);
+                unsigned ml = __ballot_sync(ZWZ_FULL, valid);
 #pragma unroll
-            for (uint32_t k = 0; k < LB; ++k) {
-                unsigned v = __ballot_sync(ZWZ_FULL, (b >> k) & 1u);
-                m &= ((b >> k) & 1u) ? v : ~v;
+                for (uint32_t k = 0; k < LB; ++k) {
+                    const unsigned v = __ballot_sync(ZWZ_FULL, (b >> k) & 1u);
+                    ml &= ((lane >> k) & 1u) ? v : ~v;
+                }
+                my += (uint32_t) __popc(ml);
             }
-            if (valid && (m >> lane) == 1u) sts16(sC + 2u * (wid * NW + b), lds16(sC + 2u * (wid * NW + b)) + (uint32_t) __popc(m)); // entry owned by this warp
-            __syncwarp();
+            if (lane < NW) cnt[wid * NW + lane] = (uint16_t) my;
         }
         __syncthreads();
+        ZWZ_DM_CLK(4);
         // ---- 3. offsets: list b = [base[b], base[b+1]), inside it warp 0's positions first, then warp 1's, ... ----
-        if (wid == 0) {
-            uint32_t run = 0;
+        // Every warp scans the NW x NW counts itself: lane b ends up with where this warp's next position of list b goes.
+        uint32_t off;
+        {
+            uint32_t before = 0, total = 0;
             if (lane < NW) {
                 for (uint32_t ww = 0; ww < NW; ++ww) {
-                    uint32_t t = cnt[ww * NW + lane];
-                    cnt[ww * NW + lane] = (uint16_t) run;
-                    run += t;
+                    const uint32_t t = cnt[ww * NW + lane];
+                    before += ww < wid ? t : 0u;
+                    total += t;
                 }
             }
-            uint32_t incl = warp_incl_scan(run);
-            if (lane < NW) ctl->base[lane] = incl - run;
-            if (lane == NW - 1u) ctl->base[NW] = incl;
+            const uint32_t incl = warp_incl_scan(total);
+            off = incl - total + before;
+            if (wid == 0) {
+                if (lane < NW) ctl->base[lane] = incl - total;
+                if (lane == NW - 1u) ctl->base[NW] = incl;
+            }
         }
-        __syncthreads();
+        ZWZ_DM_CLK(5);
         // ---- 4. scatter positions into the lists (stable) ----
-        for (uint32_t st = wid * spw; st < (wid + 1u) * spw && st < nsteps; ++st) {
-            if ((skipmask >> (st >> 5)) & 1ull) continue;
-            const uint32_t p = st * 32u + lane;
+        for (uint32_t i = s_lo; i < s_hi; ++i) {
+            const uint32_t p = (((uint32_t) slist[i >> 5] << 5) | (i & 31u)) * 32u + lane;
             const bool valid = p < nhash;
             const uint32_t h = valid ? lds16(sP + 2u * p) : 0u;
             const uint32_t b = h >> (HB - LB);
-            unsigned m = __ballot_sync(ZWZ_FULL, valid);
+            unsigned m = __ballot_sync(ZWZ_FULL, valid), ml = m;
 #pragma unroll
             for (uint32_t k = 0; k < LB; ++k) {
-                unsigned v = __ballot_sync(ZWZ_FULL, (b >> k) & 1u);
+                const unsigned v = __ballot_sync(ZWZ_FULL, (b >> k) & 1u);
                 m &= ((b >> k) & 1u) ? v : ~v;
+                ml &= ((lane >> k) & 1u) ? v : ~v;
             }
-            if (valid) {
-                uint32_t slot = lds32(sB + 4u * b) + lds16(sC + 2u * (wid * NW + b)) + (uint32_t) __popc(m & lt);
-                list[slot] = (uint16_t) p;
-            }
-            __syncwarp();
-            if (valid && (m >> lane) == 1u) sts16(sC + 2u * (wid * NW + b), lds16(sC + 2u * (wid * NW + b)) + (uint32_t) __popc(m));
-            __syncwarp();
+            const uint32_t o = __shfl_sync(ZWZ_FULL, off, b);
+            if (valid) list[o + (uint32_t) __popc(m & lt)] = (uint16_t) p;
+            off += (uint32_t) __popc(ml);
         }
         __threadfence_block();
         __syncthreads();
+        ZWZ_DM_CLK(6);
+        // tile flags of this chunk, collected in the cnt area (free since the offsets): bit t = tile t holds a match
+        uint32_t *tflags = (uint32_t *) cnt;
+        for (uint32_t i = tid; i < ZWZ_SCR_FLAG_WORDS && i < NW * NW / 2u; i += T) tflags[i] = 0u;
 
         // ---- 5. EXACT hash chains, one warp per list, 32 positions per step ----
         // Lists hold disjoint hash ranges, so the NW builders never touch the same head[] entry. Common case (all 32 hashes
@@ -438,16 +502,7 @@ ZWZ_KERNEL __launch_bounds__(MatchClass<CLS>::kThreads, MatchClass<CLS>::kCtasPe
             }
         }
         __syncthreads();
-        // The lists are dead now. They were written and read back through L2 by this CTA alone: tell L2 to drop the lines instead
-        // of writing 2 bytes per input byte back to DRAM (profiles/round1: lz_match moved 6.9x its algorithmic bytes).
-        {
-            const uint32_t list_lines = (nhash * 2u + 127u) >> 7;
-            for (uint32_t i = tid; i < list_lines; i += T) discard_l2_line((const unsigned char *) list + 128u * i);
-        }
-        // tile flags of this chunk, collected in the (now free) cnt area: bit t = tile t holds a match
-        uint32_t *tflags = (uint32_t *) cnt;
-        for (uint32_t i = tid; i < ZWZ_SCR_FLAG_WORDS && i < NW * NW / 2u; i += T) tflags[i] = 0u;
-        __syncthreads();
+        ZWZ_DM_CLK(7);
 
         // ---- 6. search: one lane per position, 32-position tiles ----
         // Every lane walks the chain of its position: the cheap test (the two bytes that would extend its best match — zlib's
@@ -457,152 +512,147 @@ ZWZ_KERNEL __launch_bounds__(MatchClass<CLS>::kThreads, MatchClass<CLS>::kCtasPe
         // at position j is a match (L - k, d) at j + k, so a prefix maximum of L_j + j over the tile (5 shuffle steps) hands
         // every lane the best such match of its left neighbours where its own walk found less (the depth limit cuts walks
         // short; in text the best match of p + 1 is usually the tail of the one at p).
+        // Only the searched tiles are handed out (noise tiles are neither searched nor written: the encoder reads the raw bytes).
+        // Measured and dropped: a static schedule (warp w takes the searched tiles w, w + NW, ...) saves the shared atomic per
+        // tile but leaves warps idle behind the slowest one, where walk lengths vary: lz_match +33 % on text, +10 % on the
+        // bitmap-like C2 files (profiles/match_overhead).
         // Measured and dropped (profiles/round2_notes.md): rounds of "walk until a candidate survives, then extend all survivors
         // together" (the walks of a tile then run one after the other: 36.2 ms against 29.8 ms per 512 MiB of text), and
         // inheriting after the first 1-4 candidates already, to raise the bar for the rest of the walk (+3 % on text, +10 % on
         // the near-incompressible C2 files, where tiles without any match pay for the shuffles).
+        uint32_t wmatch = 0; // positions of this warp's tiles that found a match
         for (;;) {
-            uint32_t tile = 0;
-            if (lane == 0) tile = atomicAdd(&ctl->next_tile, 1u);
-            tile = __shfl_sync(ZWZ_FULL, tile, 0);
-            if (tile >= ntiles) break;
-            if ((skipmask >> (tile >> 5)) & 1ull) { // noise: not searched, not written (the encoder reads the raw bytes)
-                if (lane == 0) atomicMax(&ctl->next_tile, ((tile >> 5) + 1u) << 5); // the rest of the stretch need not be handed out tile by tile
-                continue;
-            }
-
-            const uint32_t p = tile * 32u + lane;
-            uint32_t best_len = 2u, best_dist = 0u;
-            uint32_t maxlen = 0u;
-            if (p < nhash) {
-                maxlen = (n - p) < ZWZ_MAX_MATCH ? (n - p) : ZWZ_MAX_MATCH;
-                const uint32_t limit = p > ZWZ_MAX_DIST ? p - ZWZ_MAX_DIST : 0u;
-                const uint32_t span = p - limit;            // a candidate is usable iff 0 <= cand - limit < span (NIL fails)
-                uint32_t cand = lds16(sP + 2u * p);
-                if ((cand - limit) < span || (DICT && dwl != 0u && p < ZWZ_MAX_DIST)) {
-                    const uint32_t ap = sD + p;             // shared address of the scan position
-                    const uint32_t ka = ap & ~3u, sa = (ap & 3u) * 8u;
-                    const uint32_t a0 = lds32(ka), a1 = lds32(ka + 4u), a2 = lds32(ka + 8u), a3 = lds32(ka + 12u);
-                    const uint32_t S0 = __funnelshift_r(a0, a1, sa), S1 = __funnelshift_r(a1, a2, sa), S2 = __funnelshift_r(a2, a3, sa); // bytes [0, 12)
-                    uint32_t scan_end = (S0 >> 16) & 0xffu, scan_end1 = (S0 >> 8) & 0xffu; // bytes at best_len and best_len - 1
-                    uint32_t budget = job.depth;
-                    for (; budget != 0u && (cand - limit) < span; --budget) {
-                        const uint32_t ac = sD + cand;
-                        const uint32_t nxt = lds16(sP + 2u * cand); // next link is fetched while this candidate is examined
-                        if (lds8(ac + best_len) == scan_end && lds8(ac + best_len - 1u) == scan_end1) {
-                            const uint32_t kc = ac & ~3u, sc = (ac & 3u) * 8u;
-                            const uint32_t c0 = lds32(kc), c1 = lds32(kc + 4u), c2 = lds32(kc + 8u), c3 = lds32(kc + 12u);
-                            const uint32_t x0 = __funnelshift_r(c0, c1, sc) ^ S0, x1 = __funnelshift_r(c1, c2, sc) ^ S1,
-                                           x2 = __funnelshift_r(c2, c3, sc) ^ S2;
-                            uint32_t len;
-                            if (x0) {
-                                len = ((uint32_t) __ffs((int) x0) - 1u) >> 3; // < 3: a hash collision
-                            } else if (x1) {
-                                len = 4u + (((uint32_t) __ffs((int) x1) - 1u) >> 3);
-                            } else if (x2) {
-                                len = 8u + (((uint32_t) __ffs((int) x2) - 1u) >> 3);
-                            } else {
-                                len = 12u;
-                                while (len < maxlen) {
-                                    uint32_t y = lds32u(ac + len) ^ lds32u(ap + len);
-                                    if (y) {
-                                        len += ((uint32_t) __ffs((int) y) - 1u) >> 3;
-                                        break;
+            uint32_t i = 0;
+            if (lane == 0) i = atomicAdd(&ctl->next_tile, 1u);
+            i = __shfl_sync(ZWZ_FULL, i, 0);
+            if (i >= ntiles) break;
+            const uint32_t tile = ((uint32_t) slist[i >> 5] << 5) | (i & 31u);
+                const uint32_t p = tile * 32u + lane;
+                uint32_t best_len = 2u, best_dist = 0u;
+                uint32_t maxlen = 0u;
+                if (p < nhash) {
+                    maxlen = (n - p) < ZWZ_MAX_MATCH ? (n - p) : ZWZ_MAX_MATCH;
+                    const uint32_t limit = p > ZWZ_MAX_DIST ? p - ZWZ_MAX_DIST : 0u;
+                    const uint32_t span = p - limit;            // a candidate is usable iff 0 <= cand - limit < span (NIL fails)
+                    uint32_t cand = lds16(sP + 2u * p);
+                    if ((cand - limit) < span || (DICT && dwl != 0u && p < ZWZ_MAX_DIST)) {
+                        const uint32_t ap = sD + p;             // shared address of the scan position
+                        const uint32_t ka = ap & ~3u, sa = (ap & 3u) * 8u;
+                        const uint32_t a0 = lds32(ka), a1 = lds32(ka + 4u), a2 = lds32(ka + 8u), a3 = lds32(ka + 12u);
+                        const uint32_t S0 = __funnelshift_r(a0, a1, sa), S1 = __funnelshift_r(a1, a2, sa), S2 = __funnelshift_r(a2, a3, sa); // bytes [0, 12)
+                        uint32_t scan_end = (S0 >> 16) & 0xffu, scan_end1 = (S0 >> 8) & 0xffu; // bytes at best_len and best_len - 1
+                        uint32_t budget = job.depth;
+                        for (; budget != 0u && (cand - limit) < span; --budget) {
+                            const uint32_t ac = sD + cand;
+                            const uint32_t nxt = lds16(sP + 2u * cand); // next link is fetched while this candidate is examined
+                            if (lds8(ac + best_len) == scan_end && lds8(ac + best_len - 1u) == scan_end1) {
+                                const uint32_t kc = ac & ~3u, sc = (ac & 3u) * 8u;
+                                const uint32_t c0 = lds32(kc), c1 = lds32(kc + 4u), c2 = lds32(kc + 8u), c3 = lds32(kc + 12u);
+                                const uint32_t x0 = __funnelshift_r(c0, c1, sc) ^ S0, x1 = __funnelshift_r(c1, c2, sc) ^ S1,
+                                               x2 = __funnelshift_r(c2, c3, sc) ^ S2;
+                                uint32_t len;
+                                if (x0) {
+                                    len = ((uint32_t) __ffs((int) x0) - 1u) >> 3; // < 3: a hash collision
+                                } else if (x1) {
+                                    len = 4u + (((uint32_t) __ffs((int) x1) - 1u) >> 3);
+                                } else if (x2) {
+                                    len = 8u + (((uint32_t) __ffs((int) x2) - 1u) >> 3);
+                                } else {
+                                    len = 12u;
+                                    while (len < maxlen) {
+                                        uint32_t y = lds32u(ac + len) ^ lds32u(ap + len);
+                                        if (y) {
+                                            len += ((uint32_t) __ffs((int) y) - 1u) >> 3;
+                                            break;
+                                        }
+                                        len += 4u;
                                     }
-                                    len += 4u;
                                 }
-                            }
-                            if (len > maxlen) len = maxlen;
-                            if (len > best_len) {
-                                best_len = len;
-                                best_dist = p - cand;
-                                if (len >= job.nice || len >= maxlen) break;
-                                scan_end = lds8(ap + len);
-                                scan_end1 = lds8(ap + len - 1u);
-                            }
-                        }
-                        cand = nxt;
-                    }
-                    // The chunk's own chain is exhausted with budget left and no match of `nice` bytes: the walk goes on in the
-                    // dictionary's chain, most recent position first as in zlib (whose window holds the dictionary right before
-                    // the chunk), within the same budget. Window position q is at distance p + dwl - q. The 14-bit hash of the
-                    // scan position holds this class's hash in its top bits, so no candidate of a true match is lost. The
-                    // window is read from global memory (the record is L2-resident, read by every chunk of the call); a match
-                    // that starts in the window ends at its end — DEFLATE would let it run on into the chunk, zlib does.
-                    if (DICT && budget != 0u && best_len < job.nice && best_len < maxlen && dwl != 0u && p < ZWZ_MAX_DIST) {
-                        const uint16_t *dhead = (const uint16_t *) (drec + ZWZ_DICT_HEAD), *dprev = (const uint16_t *) (drec + ZWZ_DICT_PREV);
-                        const uint8_t *dwin = drec + ZWZ_DICT_WIN;
-                        const uint32_t dlim = p + dwl > ZWZ_MAX_DIST ? p + dwl - ZWZ_MAX_DIST : 0u; // oldest usable window position
-                        const uint32_t dspan = dwl - dlim;                                         // NIL fails (q - dlim) < dspan
-                        uint32_t q = __ldg(dhead + dm_hash3<ZWZ_DICT_HBITS>(S0 & 0xffu, (S0 >> 8) & 0xffu, (S0 >> 16) & 0xffu));
-                        for (; budget != 0u && (q - dlim) < dspan; --budget) {
-                            const uint32_t nxt = __ldg(dprev + q);
-                            const uint32_t dmax = dwl - q < maxlen ? dwl - q : maxlen;
-                            if (best_len < dmax && __ldg(dwin + q + best_len) == scan_end && __ldg(dwin + q + best_len - 1u) == scan_end1) {
-                                uint32_t len = 0;
-                                while (len < dmax) {
-                                    const uint32_t y = ld32u((const uint32_t *) dwin, q + len) ^ lds32u(ap + len);
-                                    if (y) {
-                                        len += ((uint32_t) __ffs((int) y) - 1u) >> 3;
-                                        break;
-                                    }
-                                    len += 4u;
-                                }
-                                if (len > dmax) len = dmax;
+                                if (len > maxlen) len = maxlen;
                                 if (len > best_len) {
                                     best_len = len;
-                                    best_dist = p + dwl - q;
+                                    best_dist = p - cand;
                                     if (len >= job.nice || len >= maxlen) break;
                                     scan_end = lds8(ap + len);
                                     scan_end1 = lds8(ap + len - 1u);
                                 }
                             }
-                            q = nxt;
+                            cand = nxt;
+                        }
+                        // The chunk's own chain is exhausted with budget left and no match of `nice` bytes: the walk goes on in the
+                        // dictionary's chain, most recent position first as in zlib (whose window holds the dictionary right before
+                        // the chunk), within the same budget. Window position q is at distance p + dwl - q. The 14-bit hash of the
+                        // scan position holds this class's hash in its top bits, so no candidate of a true match is lost. The
+                        // window is read from global memory (the record is L2-resident, read by every chunk of the call); a match
+                        // that starts in the window ends at its end — DEFLATE would let it run on into the chunk, zlib does.
+                        if (DICT && budget != 0u && best_len < job.nice && best_len < maxlen && dwl != 0u && p < ZWZ_MAX_DIST) {
+                            const uint16_t *dhead = (const uint16_t *) (drec + ZWZ_DICT_HEAD), *dprev = (const uint16_t *) (drec + ZWZ_DICT_PREV);
+                            const uint8_t *dwin = drec + ZWZ_DICT_WIN;
+                            const uint32_t dlim = p + dwl > ZWZ_MAX_DIST ? p + dwl - ZWZ_MAX_DIST : 0u; // oldest usable window position
+                            const uint32_t dspan = dwl - dlim;                                         // NIL fails (q - dlim) < dspan
+                            uint32_t q = __ldg(dhead + dm_hash3<ZWZ_DICT_HBITS>(S0 & 0xffu, (S0 >> 8) & 0xffu, (S0 >> 16) & 0xffu));
+                            for (; budget != 0u && (q - dlim) < dspan; --budget) {
+                                const uint32_t nxt = __ldg(dprev + q);
+                                const uint32_t dmax = dwl - q < maxlen ? dwl - q : maxlen;
+                                if (best_len < dmax && __ldg(dwin + q + best_len) == scan_end && __ldg(dwin + q + best_len - 1u) == scan_end1) {
+                                    uint32_t len = 0;
+                                    while (len < dmax) {
+                                        const uint32_t y = ld32u((const uint32_t *) dwin, q + len) ^ lds32u(ap + len);
+                                        if (y) {
+                                            len += ((uint32_t) __ffs((int) y) - 1u) >> 3;
+                                            break;
+                                        }
+                                        len += 4u;
+                                    }
+                                    if (len > dmax) len = dmax;
+                                    if (len > best_len) {
+                                        best_len = len;
+                                        best_dist = p + dwl - q;
+                                        if (len >= job.nice || len >= maxlen) break;
+                                        scan_end = lds8(ap + len);
+                                        scan_end1 = lds8(ap + len - 1u);
+                                    }
+                                }
+                                q = nxt;
+                            }
                         }
                     }
                 }
-            }
-            if (__any_sync(ZWZ_FULL, best_len >= 4u)) { // inherit (a 3-byte match has no tail worth passing on)
-                uint32_t key = best_len >= 3u ? best_len + lane : 0u, kd = best_dist;
-#pragma unroll
-                for (int d = 1; d < 32; d <<= 1) {
-                    const uint32_t ok = __shfl_up_sync(ZWZ_FULL, key, d), od = __shfl_up_sync(ZWZ_FULL, kd, d);
-                    if (lane >= (unsigned) d && ok > key) {
-                        key = ok;
-                        kd = od;
+                if (__any_sync(ZWZ_FULL, best_len >= 4u)) { // inherit (a 3-byte match has no tail worth passing on)
+                    uint32_t key = best_len >= 3u ? best_len + lane : 0u, kd = best_dist;
+    #pragma unroll
+                    for (int d = 1; d < 32; d <<= 1) {
+                        const uint32_t ok = __shfl_up_sync(ZWZ_FULL, key, d), od = __shfl_up_sync(ZWZ_FULL, kd, d);
+                        if (lane >= (unsigned) d && ok > key) {
+                            key = ok;
+                            kd = od;
+                        }
+                    }
+                    if (key >= lane + 3u && key - lane > best_len && key - lane <= maxlen) { // maxlen = 0: no hash here (last two bytes)
+                        best_len = key - lane;
+                        best_dist = kd;
                     }
                 }
-                if (key >= lane + 3u && key - lane > best_len && key - lane <= maxlen) { // maxlen = 0: no hash here (last two bytes)
-                    best_len = key - lane;
-                    best_dist = kd;
+                if (best_len == 3u && best_dist > 4096u) best_len = 2u; // zlib's TOO_FAR: such a match costs more than 3 literals
+                // a tile without a single match is not written at all: the encoder takes its literals from the raw bytes
+                const unsigned hit = __ballot_sync(ZWZ_FULL, best_len >= 3u);
+                if (hit) {
+                    if (p < n) mout[p] = tok_make(lds8(sD + p), best_len >= 3u ? best_len : 0u, best_dist);
+                    if (lane == 0) atomicOr(&tflags[tile >> 5], 1u << (tile & 31u));
+                    wmatch += (uint32_t) __popc(hit);
                 }
-            }
-            if (best_len == 3u && best_dist > 4096u) best_len = 2u; // zlib's TOO_FAR: such a match costs more than 3 literals
-            // a tile without a single match is not written at all: the encoder takes its literals from the raw bytes
-            const unsigned hit = __ballot_sync(ZWZ_FULL, best_len >= 3u);
-            if (hit) {
-                if (p < n) mout[p] = tok_make(lds8(sD + p), best_len >= 3u ? best_len : 0u, best_dist);
-                if (lane == 0) {
-                    atomicAdd(&ctl->nmatch, (uint32_t) __popc(hit));
-                    atomicOr(&tflags[tile >> 5], 1u << (tile & 31u));
-                }
-            }
         }
-        __syncthreads();
-        {
-            uint32_t *gflags = mout + scr_flag_offset(n);
-            const uint32_t used = (ntiles + 31u) >> 5;
-            for (uint32_t i = tid; i < ZWZ_SCR_FLAG_WORDS; i += T) gflags[i] = i < used ? tflags[i] : 0u;
-        }
+        if (lane == 0 && wmatch) atomicAdd(&ctl->nmatch, wmatch);
 
         // ---- 7. Adler-32 of the chunk ----
-        // Thread t takes the aligned words t, t + T, ... of the staging buffer (conflict-free; a contiguous byte range per
-        // thread put 32 lanes on two banks): a = sum of bytes, b = sum of (n - i) * byte_i, both by byte dot products.
+        // Each warp adds its part once it is out of tiles. Thread t takes the aligned words t, t + T, ... of the staging buffer
+        // (conflict-free; a contiguous byte range per thread put 32 lanes on two banks): a = sum of bytes, b = sum of
+        // (n - i) * byte_i, both by byte dot products.
+        AdlerPart part;
+        part.a = 0;
+        part.b = 0;
+        part.len = 0; // b is kept position-weighted from the start: parts add up without length terms
         {
-            AdlerPart part;
-            part.a = 0;
-            part.b = 0;
-            part.len = 0; // b is kept position-weighted from the start: parts add up without length terms
             const uint32_t nwords = (skew + n + 3u) >> 2;
             for (uint32_t j = tid; j < nwords; j += T) { // <= 17 words per thread: (n - pos0) * 1020 * 17 < 2^32
                 uint32_t wv = dataw[j];
@@ -627,28 +677,42 @@ ZWZ_KERNEL __launch_bounds__(MatchClass<CLS>::kThreads, MatchClass<CLS>::kCtasPe
                 ctl->adler_b[wid] = part.b;
                 ctl->adler_len[wid] = part.len;
             }
-            __syncthreads();
-            if (wid == 0) {
-                part.a = lane < NW ? ctl->adler_a[lane] : 0u;
-                part.b = lane < NW ? ctl->adler_b[lane] : 0u;
-                part.len = lane < NW ? ctl->adler_len[lane] : 0u;
+        }
+        __syncthreads();
+        ZWZ_DM_CLK(8);
+        // The lists are dead now. They were written and read back through L2 by this CTA alone: tell L2 to drop the lines instead
+        // of writing 2 bytes per input byte back to DRAM (profiles/round1: lz_match moved 6.9x its algorithmic bytes).
+        {
+            const uint32_t list_lines = (nhash * 2u + 127u) >> 7;
+            for (uint32_t i = tid; i < list_lines; i += T) discard_l2_line((const unsigned char *) list + 128u * i);
+        }
+        {
+            uint32_t *gflags = mout + scr_flag_offset(n);
+            const uint32_t used = (((n + 31u) >> 5) + 31u) >> 5;
+            for (uint32_t i = tid; i < ZWZ_SCR_FLAG_WORDS; i += T) gflags[i] = i < used ? tflags[i] : 0u;
+        }
+        if (wid == 0) {
+            part.a = lane < NW ? ctl->adler_a[lane] : 0u;
+            part.b = lane < NW ? ctl->adler_b[lane] : 0u;
+            part.len = lane < NW ? ctl->adler_len[lane] : 0u;
 #pragma unroll
-                for (int d = 1; d < 32; d <<= 1) {
-                    AdlerPart o;
-                    o.a = __shfl_down_sync(ZWZ_FULL, part.a, d);
-                    o.b = __shfl_down_sync(ZWZ_FULL, part.b, d);
-                    o.len = __shfl_down_sync(ZWZ_FULL, part.len, d);
-                    if ((lane & (2u * d - 1u)) == 0u) part = adler_combine(part, o);
-                }
-                if (lane == 0) {
-                    uint32_t a = (1u + part.a) % 65521u;
-                    uint32_t b = (n % 65521u + part.b) % 65521u;
-                    job.adler[c] = (b << 16) | a;
-                    job.nmatch[c] = ctl->nmatch;
-                }
+            for (int d = 1; d < 32; d <<= 1) {
+                AdlerPart o;
+                o.a = __shfl_down_sync(ZWZ_FULL, part.a, d);
+                o.b = __shfl_down_sync(ZWZ_FULL, part.b, d);
+                o.len = __shfl_down_sync(ZWZ_FULL, part.len, d);
+                if ((lane & (2u * d - 1u)) == 0u) part = adler_combine(part, o);
+            }
+            if (lane == 0) {
+                uint32_t a = (1u + part.a) % 65521u;
+                uint32_t b = (n % 65521u + part.b) % 65521u;
+                job.adler[c] = (b << 16) | a;
+                job.nmatch[c] = ctl->nmatch;
             }
         }
-        __syncthreads(); // smem is reused by the next chunk
+        ZWZ_DM_CLK(9);
+        // No barrier here: the next chunk's first writes to shared memory (staging, the control block) follow the barrier at the
+        // top of the loop, and every read of this chunk's data, flags and Adler parts precedes it.
     }
 }
 
