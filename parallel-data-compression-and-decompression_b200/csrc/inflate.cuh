@@ -238,6 +238,14 @@ struct InfBits {
     uint64_t fed;           // stream bits fed into hold so far (may run past 8 * nbytes: zero padding)
 };
 
+// a reader over p[0, nbytes); position it with infb_seek or infb_seek_bits
+ZWZ_DEV void infb_open(InfBits &b, const uint8_t *p, uint32_t nbytes) {
+    b.skew = (uint32_t) ((uintptr_t) p & 3u);
+    b.wbase = (const uint32_t *) (p - b.skew);
+    b.nbytes = nbytes;
+    b.nwords = (b.skew + nbytes + 3u) >> 2;
+    b.nfull = (b.skew + nbytes) >> 2;
+}
 ZWZ_DEV uint32_t infb_load(const InfBits &b, uint32_t k) {
     if (k >= b.nwords) return 0u;
     uint32_t w = __ldg(b.wbase + k);
@@ -296,6 +304,11 @@ ZWZ_DEV void infb_seek_bits(InfBits &b, uint64_t bit_pos) {
     infb_seek(b, (uint32_t) (bit_pos >> 3));
     infb_drop(b, (uint32_t) bit_pos & 7u); // <= 7 of the >= 8 bits the seek left in the buffer
 }
+// Everything already in `hold` is real stream data while only whole words of the stream have been fed; only the tail of a
+// stream (or a truncated one) needs the per-symbol availability checks that give zlib's exact stop position.
+ZWZ_DEV bool infb_inside(const InfBits &b) { return b.widx <= b.nfull; }
+// the next n bits (n <= the bits in `hold`) lie inside the stream
+ZWZ_DEV bool infb_need(const InfBits &b, uint32_t n) { return infb_inside(b) || infb_used(b) + n <= (uint64_t) b.nbytes * 8u; }
 
 } // namespace zwz
 #include "inflate_fast.cuh"
@@ -351,19 +364,173 @@ ZWZ_DEV_NOINLINE uint32_t inf_gzip_header(const uint8_t *comp, uint32_t comp_len
     return (p << 2) | ZWZ_STREAM_END;
 }
 
+// 32-bit values of the trailers: RFC 1950's Adler-32 is big-endian, RFC 1952's CRC-32 and ISIZE little-endian
+ZWZ_DEV uint32_t inf_be32(const uint8_t *p) { return ((uint32_t) p[0] << 24) | ((uint32_t) p[1] << 16) | ((uint32_t) p[2] << 8) | p[3]; }
+ZWZ_DEV uint32_t inf_le32(const uint8_t *p) { return (uint32_t) p[0] | ((uint32_t) p[1] << 8) | ((uint32_t) p[2] << 16) | ((uint32_t) p[3] << 24); }
+
+// The decoding steps below are shared by the batch decoder (inflate_stream), the span decoder and the block finder
+// (inflate_stream.cuh). Each returns ZWZ_STREAM_END when it succeeded, else the status zlib ends with there; all are warp-uniform.
+
+// RFC 1950 header (inflate.c HEAD) at the reader: consumes CMF and FLG and returns FLG in `flg`. FDICT is BAD unless fdict_ok:
+// without a dictionary it is zlib's Z_NEED_DICT, and nothing can be decoded.
+ZWZ_DEV uint32_t inf_zlib_header(InfBits &B, bool fdict_ok, uint32_t &flg) {
+    infb_refill(B);
+    if (!infb_need(B, 16)) return ZWZ_STREAM_TRUNCATED;
+    const uint32_t cmf = (uint32_t) B.hold & 0xffu;
+    flg = ((uint32_t) B.hold >> 8) & 0xffu;
+    if (((cmf << 8) + flg) % 31u != 0u || (cmf & 15u) != 8u || (cmf >> 4) + 8u > 15u || ((flg & 0x20u) && !fdict_ok)) return ZWZ_STREAM_BAD;
+    infb_drop(B, 16);
+    return ZWZ_STREAM_END;
+}
+
+// Stored block after its 3 header bits: skips to the byte boundary and reads LEN / NLEN. The block's bytes start at stream byte
+// `bpos`; `len` is LEN. The caller copies min(LEN, bytes left) and then seeks to bpos + len.
+ZWZ_DEV uint32_t inf_stored_header(InfBits &B, uint32_t &bpos, uint32_t &len) {
+    bpos = (uint32_t) ((infb_used(B) + 7u) >> 3);
+    if ((uint64_t) bpos + 4u > B.nbytes) return ZWZ_STREAM_TRUNCATED;
+    infb_seek(B, bpos);
+    infb_refill(B);
+    const uint32_t v = (uint32_t) B.hold;
+    if ((v & 0xffffu) != ((v >> 16) ^ 0xffffu)) return ZWZ_STREAM_BAD;
+    len = v & 0xffffu;
+    bpos += 4u;
+    return ZWZ_STREAM_END;
+}
+
+// the tables of a fixed-Huffman block (RFC 1951 §3.2.6)
+ZWZ_DEV void inf_fixed_tables(InflateWarpSmem &S, uint32_t &max_ll, uint32_t &max_d) {
+    const unsigned lane = lane_id();
+    for (uint32_t s = lane; s < 288u; s += 32u) S.lens[32u + s] = (uint8_t) (s < 144u ? 8 : (s < 256u ? 9 : (s < 280u ? 7 : 8)));
+    S.lens[320u + lane] = 5;
+    __syncwarp();
+    inf_build<1>(S.lens + 32, 288u, S.cnt_ll, S.sorted_ll, S.run, S.lit, ZWZ_INF_LBITS, max_ll);
+    inf_build<2>(S.lens + 320, 32u, S.cnt_d, S.sorted_d, S.run, S.dst, ZWZ_INF_DBITS, max_d);
+}
+
+// The tables of a dynamic block (RFC 1951 §3.2.7), read after its 3 header bits with at least 14 bits left in `hold` (what a
+// refill leaves behind them): HLIT / HDIST / HCLEN, the code-length code, the code lengths, then both codes built as inf_build
+// requires, with code 256 present. The block finder's candidates are the headers this accepts.
+ZWZ_DEV uint32_t inf_dyn_tables(InflateWarpSmem &S, InfBits &B, uint32_t &max_ll, uint32_t &max_d) {
+    const unsigned lane = lane_id();
+    if (!infb_need(B, 14)) return ZWZ_STREAM_TRUNCATED;
+    const uint32_t nlen = ((uint32_t) B.hold & 31u) + 257u;
+    const uint32_t ndist = (((uint32_t) B.hold >> 5) & 31u) + 1u;
+    const uint32_t ncode = (((uint32_t) B.hold >> 10) & 15u) + 4u;
+    infb_drop(B, 14);
+    if (nlen > 286u || ndist > 30u) return ZWZ_STREAM_BAD;
+    if (lane < 19u) S.lens[lane] = 0;
+    __syncwarp();
+    for (uint32_t i = 0; i < ncode; ++i) {
+        infb_refill(B);
+        if (!infb_need(B, 3)) return ZWZ_STREAM_TRUNCATED;
+        // permutation 16 17 18 0 8 7 9 6 10 5 11 4 12 3 13 2 14 1 15
+        const uint32_t slot = i < 3u ? 16u + i : (i == 3u ? 0u : ((i & 1u) ? 7u - ((i - 5u) >> 1) : 8u + ((i - 4u) >> 1)));
+        if (lane == 0) S.lens[slot] = (uint8_t) ((uint32_t) B.hold & 7u);
+        infb_drop(B, 3);
+    }
+    __syncwarp();
+    uint32_t max_cl = 0;
+    if (inf_build<0>(S.lens, 19u, S.cnt_cl, S.sorted_cl, S.run, S.clt, 7u, max_cl) != 0 || max_cl == 0u) return ZWZ_STREAM_BAD;
+    // code lengths for nlen + ndist symbols (warp-uniform decode, lane 0 stores)
+    uint32_t have = 0, prev_len = 0;
+    const uint32_t total = nlen + ndist;
+    while (have < total) {
+        infb_refill(B);
+        const uint32_t e = S.clt[(uint32_t) B.hold & 127u];
+        const uint32_t nb = e & 15u;
+        if (nb == 0u) return ZWZ_STREAM_BAD; // invalid pattern is impossible for a complete code; defensive
+        const uint32_t sym = e >> 4;
+        const uint32_t eb = sym < 16u ? 0u : (sym == 16u ? 2u : (sym == 17u ? 3u : 7u));
+        if (!infb_need(B, nb + eb)) return ZWZ_STREAM_TRUNCATED;
+        infb_drop(B, nb);
+        if (sym < 16u) {
+            if (lane == 0) S.lens[32u + have] = (uint8_t) sym;
+            prev_len = sym;
+            have++;
+            continue;
+        }
+        uint32_t rep, val = 0;
+        const uint32_t x = (uint32_t) B.hold & ((1u << eb) - 1u);
+        infb_drop(B, eb);
+        if (sym == 16u) {
+            if (have == 0u) return ZWZ_STREAM_BAD;
+            val = prev_len;
+            rep = 3u + x;
+        } else {
+            rep = (sym == 17u ? 3u : 11u) + x;
+        }
+        if (have + rep > total) return ZWZ_STREAM_BAD;
+        // Rolled on purpose: unrolled (five predicated stores), inflate_span_kernel spills 36 / 52 bytes instead of 28 / 44 and
+        // block_find_kernel needs 52 registers instead of 50.
+#pragma unroll 1
+        for (uint32_t r = lane; r < rep; r += 32u) S.lens[32u + have + r] = (uint8_t) val;
+        prev_len = val;
+        have += rep;
+    }
+    __syncwarp();
+    if (S.lens[32u + 256u] == 0) return ZWZ_STREAM_BAD; // missing end-of-block code
+    // S.lens[32 .. 32+nlen) literal/length, then ndist distance lengths. inf_build reads them in place; the two builds use
+    // disjoint outputs, and the distance lengths are read before anything overwrites them.
+    if (inf_build<1>(S.lens + 32, nlen, S.cnt_ll, S.sorted_ll, S.run, S.lit, ZWZ_INF_LBITS, max_ll) != 0 ||
+        inf_build<2>(S.lens + 32 + nlen, ndist, S.cnt_d, S.sorted_d, S.run, S.dst, ZWZ_INF_DBITS, max_d) != 0)
+        return ZWZ_STREAM_BAD;
+    return ZWZ_STREAM_END;
+}
+
+// what inf_token decoded, besides ZWZ_STREAM_TRUNCATED / ZWZ_STREAM_BAD; apart from every stream status and span result, so
+// that a token code passed on as a status by mistake cannot read as one
+enum { INF_TOK_LIT = 16, INF_TOK_EOB = 17, INF_TOK_MATCH = 18 };
+
+// One token of a Huffman block, from the literal/length entry `e` of the refilled reader's next bits. A code longer than the
+// table index is resolved by the canonical walk. A token is consumed only when it lies completely inside the input (zlib: a
+// literal needs its whole code, a match length + extra + distance + extra); an invalid code is BAD once its own bits are there.
+// INF_TOK_LIT: the byte in v. INF_TOK_MATCH: length v and distance dist, which the caller checks against its window.
+ZWZ_DEV uint32_t inf_token(const InflateWarpSmem &S, InfBits &B, uint32_t e, uint32_t max_ll, uint32_t max_d, uint32_t &v, uint32_t &dist) {
+    uint32_t nb = e & 15u;
+    if (ZWZ_LL_IS_LONG(e)) { // complete sets only get here
+        uint32_t len = 0;
+        const uint32_t sym = inf_canon_walk((uint32_t) B.hold, S.cnt_ll, S.sorted_ll, max_ll, len);
+        e = sym == 0xffffffffu ? ZWZ_LL_INVALID(max_ll) : inf_litlen_entry(sym, len);
+        nb = e & 15u;
+    }
+    if (ZWZ_LL_IS_INVALID(e)) return infb_need(B, nb) ? ZWZ_STREAM_BAD : ZWZ_STREAM_TRUNCATED; // zlib's invalid-code entry
+    if (!infb_need(B, nb)) return ZWZ_STREAM_TRUNCATED;
+    infb_drop(B, nb);
+    if (ZWZ_LL_IS_LIT(e)) {
+        v = e >> 7;
+        return INF_TOK_LIT;
+    }
+    if (ZWZ_LL_IS_EOB(e)) return INF_TOK_EOB;
+    // length (the code may have been the second one since the last refill: top up before the extra bits)
+    infb_refill(B);
+    const uint32_t eb = (e >> 4) & 7u;
+    v = (e >> 7) - 253u + ((uint32_t) B.hold & ((1u << eb) - 1u));
+    if (!infb_need(B, eb)) return ZWZ_STREAM_TRUNCATED;
+    infb_drop(B, eb);
+    infb_refill(B);
+    uint32_t d = S.dst[(uint32_t) B.hold & ((1u << ZWZ_INF_DBITS) - 1u)];
+    if (ZWZ_D_IS_LONG(d)) {
+        uint32_t len = 0;
+        const uint32_t sym = inf_canon_walk((uint32_t) B.hold, S.cnt_d, S.sorted_d, max_d, len);
+        d = sym == 0xffffffffu ? ZWZ_D_INVALID(max_d) : inf_dist_entry(sym, len);
+    }
+    const uint32_t dnb = d & 15u;
+    if (ZWZ_D_IS_SPECIAL(d)) return infb_need(B, dnb) ? ZWZ_STREAM_BAD : ZWZ_STREAM_TRUNCATED;
+    const uint32_t deb = (d >> 4) & 15u;
+    if (!infb_need(B, dnb + deb)) return ZWZ_STREAM_TRUNCATED;
+    dist = ZWZ_D_DM1(d, (uint32_t) B.hold) + 1u;
+    infb_drop(B, dnb + deb);
+    return INF_TOK_MATCH;
+}
+
 // One warp decodes stream `sid`. DICT: the stream may have a preset dictionary, whose window (dwl bytes at dwin, 0 = none) comes
 // before output position 0; a zlib stream asks for it with FDICT and names it by its DICTID (did), a raw stream just uses it.
 template <bool DICT>
 ZWZ_DEV void inflate_stream(InflateWarpSmem &S, const uint8_t *__restrict__ comp, uint32_t comp_len, uint8_t *out, uint32_t cap,
                             uint32_t flags, uint32_t &raw_len_out, uint32_t &status_out, const uint8_t *dwin, uint32_t dwl, uint32_t did) {
     const unsigned lane = lane_id();
-    const uint64_t total_bits = (uint64_t) comp_len * 8u;
     InfBits B;
-    B.skew = (uint32_t) ((uintptr_t) comp & 3u);
-    B.wbase = (const uint32_t *) (comp - B.skew);
-    B.nbytes = comp_len;
-    B.nwords = (B.skew + comp_len + 3u) >> 2;
-    B.nfull = (B.skew + comp_len) >> 2;
+    infb_open(B, comp, comp_len);
     infb_seek(B, 0);
 
     uint32_t pos = 0;       // bytes produced (counted past cap too)
@@ -379,10 +546,6 @@ ZWZ_DEV void inflate_stream(InflateWarpSmem &S, const uint8_t *__restrict__ comp
         if (q_ >= pend_lo && q_ < pos && q_ < cap) out[q_] = (uint8_t) mybyte;   \
         pend_lo = pos;                                                           \
     } while (0)
-// Everything already in `hold` is real stream data while fed <= total_bits; only the tail of a stream (or a truncated
-// one) needs the per-symbol availability checks that give zlib's exact stop position.
-#define INF_FAST() (B.widx <= B.nfull)
-#define INF_NEED(nbits_) (INF_FAST() || infb_used(B) + (uint64_t) (nbits_) <= total_bits)
 
     if (format == ZWZ_FORMAT_GZIP) {
         const uint32_t h = inf_gzip_header(comp, comp_len);
@@ -390,22 +553,13 @@ ZWZ_DEV void inflate_stream(InflateWarpSmem &S, const uint8_t *__restrict__ comp
         if (status != ZWZ_STREAM_END) goto done;
         infb_seek(B, h >> 2);
     } else if (format == ZWZ_FORMAT_ZLIB) {
-        // ---- RFC 1950 header (inflate.c HEAD) ----
-        infb_refill(B);
-        if (!INF_NEED(16)) {
-            status = ZWZ_STREAM_TRUNCATED;
-            goto done;
-        }
-        uint32_t cmf = (uint32_t) B.hold & 0xffu, flg = ((uint32_t) B.hold >> 8) & 0xffu;
-        if (((cmf << 8) + flg) % 31u != 0u || (cmf & 15u) != 8u || (cmf >> 4) + 8u > 15u || ((flg & 0x20u) && (!DICT || dwl == 0u))) {
-            status = ZWZ_STREAM_BAD; // FDICT without a dictionary is zlib's Z_NEED_DICT: nothing can be decoded
-            goto done;
-        }
-        infb_drop(B, 16);
+        uint32_t flg = 0;
+        status = inf_zlib_header(B, DICT && dwl != 0u, flg);
+        if (status != ZWZ_STREAM_END) goto done;
         if (DICT) {
             if (flg & 0x20u) { // DICTID (inflate.c DICTID): it must name the dictionary given, else inflateSetDictionary's Z_DATA_ERROR
                 infb_refill(B);
-                if (!INF_NEED(32)) {
+                if (!infb_need(B, 32)) {
                     status = ZWZ_STREAM_TRUNCATED;
                     goto done;
                 }
@@ -423,7 +577,7 @@ ZWZ_DEV void inflate_stream(InflateWarpSmem &S, const uint8_t *__restrict__ comp
 
     for (;;) {
         infb_refill(B);
-        if (!INF_NEED(3)) {
+        if (!infb_need(B, 3)) {
             status = ZWZ_STREAM_TRUNCATED;
             goto done;
         }
@@ -432,24 +586,10 @@ ZWZ_DEV void inflate_stream(InflateWarpSmem &S, const uint8_t *__restrict__ comp
         infb_drop(B, 3);
 
         if (type == 0u) {
-            // stored: skip to the byte boundary, LEN/NLEN, then a plain copy
-            uint64_t used = infb_used(B);
-            uint32_t bpos = (uint32_t) ((used + 7u) >> 3);
-            if ((uint64_t) bpos + 4u > comp_len) {
-                status = ZWZ_STREAM_TRUNCATED;
-                goto done;
-            }
-            infb_seek(B, bpos);
-            infb_refill(B);
-            uint32_t v = (uint32_t) B.hold;
-            if ((v & 0xffffu) != ((v >> 16) ^ 0xffffu)) {
-                status = ZWZ_STREAM_BAD;
-                goto done;
-            }
-            uint32_t len = v & 0xffffu;
-            bpos += 4u;
-            uint32_t avail = comp_len - bpos;
-            uint32_t ncopy = len < avail ? len : avail;
+            uint32_t bpos = 0, len = 0;
+            status = inf_stored_header(B, bpos, len);
+            if (status != ZWZ_STREAM_END) goto done;
+            const uint32_t ncopy = len < comp_len - bpos ? len : comp_len - bpos;
             INF_FLUSH_LITS();
             {
                 const uint32_t room = pos < cap ? cap - pos : 0u;
@@ -474,105 +614,10 @@ ZWZ_DEV void inflate_stream(InflateWarpSmem &S, const uint8_t *__restrict__ comp
         uint32_t max_ll = 0, max_d = 0;
         uint32_t min_ll = 1; // shortest literal/length code of this block: bounds how many codes fit a 32-bit window
         if (type == 1u) {
-            for (uint32_t s = lane; s < 288u; s += 32u) S.lens[32u + s] = (uint8_t) (s < 144u ? 8 : (s < 256u ? 9 : (s < 280u ? 7 : 8)));
-            S.lens[320u + lane] = 5;
-            __syncwarp();
-            inf_build<1>(S.lens + 32, 288u, S.cnt_ll, S.sorted_ll, S.run, S.lit, ZWZ_INF_LBITS, max_ll);
-            inf_build<2>(S.lens + 320, 32u, S.cnt_d, S.sorted_d, S.run, S.dst, ZWZ_INF_DBITS, max_d);
+            inf_fixed_tables(S, max_ll, max_d);
         } else {
-            if (!INF_NEED(14)) {
-                status = ZWZ_STREAM_TRUNCATED;
-                goto done;
-            }
-            uint32_t nlen = ((uint32_t) B.hold & 31u) + 257u;
-            uint32_t ndist = (((uint32_t) B.hold >> 5) & 31u) + 1u;
-            uint32_t ncode = (((uint32_t) B.hold >> 10) & 15u) + 4u;
-            infb_drop(B, 14);
-            if (nlen > 286u || ndist > 30u) {
-                status = ZWZ_STREAM_BAD;
-                goto done;
-            }
-            if (lane < 19u) S.lens[lane] = 0;
-            __syncwarp();
-            for (uint32_t i = 0; i < ncode; ++i) {
-                infb_refill(B);
-                if (!INF_NEED(3)) {
-                    status = ZWZ_STREAM_TRUNCATED;
-                    goto done;
-                }
-                // RFC 1951 §3.2.7 permutation 16 17 18 0 8 7 9 6 10 5 11 4 12 3 13 2 14 1 15
-                uint32_t slot = i < 3u ? 16u + i : (i == 3u ? 0u : ((i & 1u) ? 7u - ((i - 5u) >> 1) : 8u + ((i - 4u) >> 1)));
-                if (lane == 0) S.lens[slot] = (uint8_t) ((uint32_t) B.hold & 7u);
-                infb_drop(B, 3);
-            }
-            __syncwarp();
-            uint32_t max_cl = 0;
-            if (inf_build<0>(S.lens, 19u, S.cnt_cl, S.sorted_cl, S.run, S.clt, 7u, max_cl) != 0 || max_cl == 0u) {
-                status = ZWZ_STREAM_BAD;
-                goto done;
-            }
-            // code lengths for nlen + ndist symbols (warp-uniform decode, lane 0 stores)
-            uint32_t have = 0, total = nlen + ndist, prev_len = 0;
-            while (have < total) {
-                infb_refill(B);
-                uint32_t e = S.clt[(uint32_t) B.hold & 127u];
-                uint32_t nb = e & 15u;
-                if (nb == 0u) { // invalid pattern is impossible for a complete code; defensive
-                    status = ZWZ_STREAM_BAD;
-                    goto done;
-                }
-                uint32_t sym = e >> 4;
-                uint32_t eb = sym < 16u ? 0u : (sym == 16u ? 2u : (sym == 17u ? 3u : 7u));
-                if (!INF_NEED(nb + eb)) {
-                    status = ZWZ_STREAM_TRUNCATED;
-                    goto done;
-                }
-                infb_drop(B, nb);
-                if (sym < 16u) {
-                    if (lane == 0) S.lens[32u + have] = (uint8_t) sym;
-                    prev_len = sym;
-                    have++;
-                    continue;
-                }
-                uint32_t rep, val = 0;
-                uint32_t x = (uint32_t) B.hold & ((1u << eb) - 1u);
-                infb_drop(B, eb);
-                if (sym == 16u) {
-                    if (have == 0u) {
-                        status = ZWZ_STREAM_BAD;
-                        goto done;
-                    }
-                    val = prev_len;
-                    rep = 3u + x;
-                } else if (sym == 17u) {
-                    rep = 3u + x;
-                } else {
-                    rep = 11u + x;
-                }
-                if (have + rep > total) {
-                    status = ZWZ_STREAM_BAD;
-                    goto done;
-                }
-                if (lane < rep) S.lens[32u + have + lane] = (uint8_t) val;
-                if (lane + 32u < rep) S.lens[32u + have + lane + 32u] = (uint8_t) val;
-                if (lane + 64u < rep) S.lens[32u + have + lane + 64u] = (uint8_t) val;
-                if (lane + 96u < rep) S.lens[32u + have + lane + 96u] = (uint8_t) val;
-                if (lane + 128u < rep) S.lens[32u + have + lane + 128u] = (uint8_t) val;
-                prev_len = val;
-                have += rep;
-            }
-            __syncwarp();
-            if (S.lens[32u + 256u] == 0) { // missing end-of-block code
-                status = ZWZ_STREAM_BAD;
-                goto done;
-            }
-            // S.lens[32 .. 32+nlen) literal/length, then ndist distance lengths. inf_build reads them in place; the two
-            // builds use disjoint outputs, and the distance lengths are read before anything overwrites them.
-            if (inf_build<1>(S.lens + 32, nlen, S.cnt_ll, S.sorted_ll, S.run, S.lit, ZWZ_INF_LBITS, max_ll) != 0 ||
-                inf_build<2>(S.lens + 32 + nlen, ndist, S.cnt_d, S.sorted_d, S.run, S.dst, ZWZ_INF_DBITS, max_d) != 0) {
-                status = ZWZ_STREAM_BAD;
-                goto done;
-            }
+            status = inf_dyn_tables(S, B, max_ll, max_d);
+            if (status != ZWZ_STREAM_END) goto done;
         }
 
         for (min_ll = 1; min_ll < 15u && S.cnt_ll[min_ll] == 0u; ++min_ll) {}
@@ -598,7 +643,7 @@ ZWZ_DEV void inflate_stream(InflateWarpSmem &S, const uint8_t *__restrict__ comp
         for (;;) {
             infb_refill(B); // >= 33 valid bits
             uint32_t e;
-            if (INF_FAST()) {
+            if (infb_inside(B)) {
                 // Literal runs, 32 bit offsets at a time ("warp-ballot symbol decode"): lane l decodes the code that WOULD
                 // start at bit l of the buffer; the ballot says which offsets hold a complete literal; the offsets that
                 // really are code starts form the chain 0 -> nb(0) -> ..., recovered with 5 rounds of pointer doubling on
@@ -652,57 +697,19 @@ ZWZ_DEV void inflate_stream(InflateWarpSmem &S, const uint8_t *__restrict__ comp
             } else {
                 e = S.lit[(uint32_t) B.hold & ((1u << ZWZ_INF_LBITS) - 1u)];
             }
-            uint32_t nb = e & 15u;
-            if (ZWZ_LL_IS_LONG(e)) { // code longer than the table index: canonical walk (complete sets only get here)
-                uint32_t len = 0;
-                uint32_t sym = inf_canon_walk((uint32_t) B.hold, S.cnt_ll, S.sorted_ll, max_ll, len);
-                e = sym == 0xffffffffu ? ZWZ_LL_INVALID(max_ll) : inf_litlen_entry(sym, len);
-                nb = e & 15u;
-            }
-            if (ZWZ_LL_IS_INVALID(e)) { // zlib's invalid-code entry: it still has to see the code's bits first
-                status = INF_NEED(nb) ? ZWZ_STREAM_BAD : ZWZ_STREAM_TRUNCATED;
-                goto done;
-            }
-            if (!INF_NEED(nb)) {
-                status = ZWZ_STREAM_TRUNCATED;
-                goto done;
-            }
-            infb_drop(B, nb);
-            if (ZWZ_LL_IS_LIT(e)) {
-                if (lane == (pos & 31u)) mybyte = e >> 7;
+            uint32_t v = 0, dist = 0;
+            const uint32_t t = inf_token(S, B, e, max_ll, max_d, v, dist);
+            if (t == INF_TOK_LIT) {
+                if (lane == (pos & 31u)) mybyte = v;
                 pos++;
                 if ((pos & 31u) == 0u) INF_FLUSH_LITS();
                 continue;
             }
-            if (ZWZ_LL_IS_EOB(e)) break;
-            // length (the code may have been the second one since the last refill: top up before the extra bits)
-            infb_refill(B);
-            uint32_t eb = (e >> 4) & 7u;
-            uint32_t mlen = (e >> 7) - 253u + ((uint32_t) B.hold & ((1u << eb) - 1u));
-            if (!INF_NEED(eb)) {
-                status = ZWZ_STREAM_TRUNCATED;
+            if (t == INF_TOK_EOB) break;
+            if (t != INF_TOK_MATCH) {
+                status = t;
                 goto done;
             }
-            infb_drop(B, eb);
-            infb_refill(B);
-            uint32_t d = S.dst[(uint32_t) B.hold & ((1u << ZWZ_INF_DBITS) - 1u)];
-            if (ZWZ_D_IS_LONG(d)) {
-                uint32_t len = 0;
-                uint32_t sym = inf_canon_walk((uint32_t) B.hold, S.cnt_d, S.sorted_d, max_d, len);
-                d = sym == 0xffffffffu ? ZWZ_D_INVALID(max_d) : inf_dist_entry(sym, len);
-            }
-            const uint32_t dnb = d & 15u;
-            if (ZWZ_D_IS_SPECIAL(d)) {
-                status = INF_NEED(dnb) ? ZWZ_STREAM_BAD : ZWZ_STREAM_TRUNCATED;
-                goto done;
-            }
-            uint32_t deb = (d >> 4) & 15u;
-            if (!INF_NEED(dnb + deb)) {
-                status = ZWZ_STREAM_TRUNCATED;
-                goto done;
-            }
-            uint32_t dist = ZWZ_D_DM1(d, (uint32_t) B.hold) + 1u;
-            infb_drop(B, dnb + deb);
             if (dist > pos + dwl) { // "invalid distance too far back" (a preset dictionary's window counts as written)
                 status = ZWZ_STREAM_BAD;
                 goto done;
@@ -711,9 +718,9 @@ ZWZ_DEV void inflate_stream(InflateWarpSmem &S, const uint8_t *__restrict__ comp
             // written by other lanes of this warp moments ago and L1 is not coherent for that.
             INF_FLUSH_LITS();
             __syncwarp();
-            if (pos + mlen > cap) overflow = true;
-            inf_copy_match<DICT>(out, pos, mlen, dist, cap, dwin, dwl);
-            pos += mlen;
+            if (pos + v > cap) overflow = true;
+            inf_copy_match<DICT>(out, pos, v, dist, cap, dwin, dwl);
+            pos += v;
             pend_lo = pos;
         }
         if (last) break;
@@ -730,20 +737,16 @@ ZWZ_DEV void inflate_stream(InflateWarpSmem &S, const uint8_t *__restrict__ comp
         }
         if (format == ZWZ_FORMAT_ZLIB) {
             if (!(flags & 1u) && !overflow) {
-                uint32_t want = ((uint32_t) comp[bpos] << 24) | ((uint32_t) comp[bpos + 1] << 16) | ((uint32_t) comp[bpos + 2] << 8) | comp[bpos + 3];
                 const uint32_t have = inf_adler32(out, pos); // a = 1 + sum(byte), b = n + sum((n - j) * byte_j)  (mod 65521)
-                if (have != want) status = ZWZ_STREAM_BAD;
+                if (have != inf_be32(comp + bpos)) status = ZWZ_STREAM_BAD;
             }
         } else {
-            const uint32_t want = (uint32_t) comp[bpos] | ((uint32_t) comp[bpos + 1] << 8) | ((uint32_t) comp[bpos + 2] << 16) | ((uint32_t) comp[bpos + 3] << 24);
-            if (!(flags & 1u) && !overflow && inf_crc32(out, pos) != want) {
+            if (!(flags & 1u) && !overflow && inf_crc32(out, pos) != inf_le32(comp + bpos)) {
                 status = ZWZ_STREAM_BAD;
             } else if ((uint64_t) bpos + 8u > comp_len) {
                 status = ZWZ_STREAM_TRUNCATED;
-            } else {
-                const uint32_t isize = (uint32_t) comp[bpos + 4] | ((uint32_t) comp[bpos + 5] << 8) | ((uint32_t) comp[bpos + 6] << 16) |
-                                       ((uint32_t) comp[bpos + 7] << 24);
-                if (isize != pos) status = ZWZ_STREAM_BAD; // pos counts past the capacity too
+            } else if (inf_le32(comp + bpos + 4u) != pos) { // ISIZE; pos counts past the capacity too
+                status = ZWZ_STREAM_BAD;
             }
         }
     }
@@ -754,7 +757,6 @@ done:
     raw_len_out = pos;
     status_out = status;
 #undef INF_FLUSH_LITS
-#undef INF_NEED
 }
 
 // Persistent warps: every warp pulls the next stream from a global counter, so a CTA is never kept alive by one long stream

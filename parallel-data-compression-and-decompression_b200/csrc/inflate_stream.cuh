@@ -66,84 +66,6 @@ struct SpanMember {
     uint32_t pad;
 };
 
-#define SPAN_NEED(nbits_) ((B.widx <= B.nfull) || infb_used(B) + (uint64_t) (nbits_) <= total_bits)
-
-// The tables of a dynamic block, read after its 3 header bits: ZWZ_STREAM_END when both codes were built, else the status zlib
-// ends with. The block finder calls it too, so that "a candidate" means "a header the span decoder accepts". It is a copy of the
-// dynamic-header code of inflate_stream (inflate.cuh), kept apart so that inflate_kernel compiles exactly as before: a change to
-// either must be made to both (tests/test_inflate_stream.py compares both decoders with zlib on the same streams).
-ZWZ_DEV uint32_t inf_dyn_tables(InflateWarpSmem &S, InfBits &B, uint64_t total_bits, uint32_t &max_ll, uint32_t &max_d) {
-    const unsigned lane = lane_id();
-    infb_refill(B);
-    if (!SPAN_NEED(14)) return ZWZ_STREAM_TRUNCATED;
-    const uint32_t nlen = ((uint32_t) B.hold & 31u) + 257u;
-    const uint32_t ndist = (((uint32_t) B.hold >> 5) & 31u) + 1u;
-    const uint32_t ncode = (((uint32_t) B.hold >> 10) & 15u) + 4u;
-    infb_drop(B, 14);
-    if (nlen > 286u || ndist > 30u) return ZWZ_STREAM_BAD;
-    if (lane < 19u) S.lens[lane] = 0;
-    __syncwarp();
-    for (uint32_t i = 0; i < ncode; ++i) {
-        infb_refill(B);
-        if (!SPAN_NEED(3)) return ZWZ_STREAM_TRUNCATED;
-        const uint32_t slot = i < 3u ? 16u + i : (i == 3u ? 0u : ((i & 1u) ? 7u - ((i - 5u) >> 1) : 8u + ((i - 4u) >> 1)));
-        if (lane == 0) S.lens[slot] = (uint8_t) ((uint32_t) B.hold & 7u);
-        infb_drop(B, 3);
-    }
-    __syncwarp();
-    uint32_t max_cl = 0;
-    if (inf_build<0>(S.lens, 19u, S.cnt_cl, S.sorted_cl, S.run, S.clt, 7u, max_cl) != 0 || max_cl == 0u) return ZWZ_STREAM_BAD;
-    uint32_t have = 0, prev_len = 0;
-    const uint32_t total = nlen + ndist;
-    while (have < total) {
-        infb_refill(B);
-        const uint32_t e = S.clt[(uint32_t) B.hold & 127u];
-        const uint32_t nb = e & 15u;
-        if (nb == 0u) return ZWZ_STREAM_BAD;
-        const uint32_t sym = e >> 4;
-        const uint32_t eb = sym < 16u ? 0u : (sym == 16u ? 2u : (sym == 17u ? 3u : 7u));
-        if (!SPAN_NEED(nb + eb)) return ZWZ_STREAM_TRUNCATED;
-        infb_drop(B, nb);
-        if (sym < 16u) {
-            if (lane == 0) S.lens[32u + have] = (uint8_t) sym;
-            prev_len = sym;
-            have++;
-            continue;
-        }
-        uint32_t rep, val = 0;
-        const uint32_t x = (uint32_t) B.hold & ((1u << eb) - 1u);
-        infb_drop(B, eb);
-        if (sym == 16u) {
-            if (have == 0u) return ZWZ_STREAM_BAD;
-            val = prev_len;
-            rep = 3u + x;
-        } else {
-            rep = (sym == 17u ? 3u : 11u) + x;
-        }
-        if (have + rep > total) return ZWZ_STREAM_BAD;
-        for (uint32_t r = lane; r < rep; r += 32u) S.lens[32u + have + r] = (uint8_t) val;
-        prev_len = val;
-        have += rep;
-    }
-    __syncwarp();
-    if (S.lens[32u + 256u] == 0) return ZWZ_STREAM_BAD;
-    if (inf_build<1>(S.lens + 32, nlen, S.cnt_ll, S.sorted_ll, S.run, S.lit, ZWZ_INF_LBITS, max_ll) != 0 ||
-        inf_build<2>(S.lens + 32 + nlen, ndist, S.cnt_d, S.sorted_d, S.run, S.dst, ZWZ_INF_DBITS, max_d) != 0)
-        return ZWZ_STREAM_BAD;
-    return ZWZ_STREAM_END;
-}
-
-// a bit reader over comp[byte0, comp_len), positioned at bit `bit` of the stream
-ZWZ_DEV void span_reader(InfBits &B, const uint8_t *comp, uint64_t comp_len, uint64_t byte0, uint64_t bit) {
-    const uint8_t *c = comp + byte0;
-    B.skew = (uint32_t) ((uintptr_t) c & 3u);
-    B.wbase = (const uint32_t *) (c - B.skew);
-    B.nbytes = (uint32_t) (comp_len - byte0);
-    B.nwords = (B.skew + B.nbytes + 3u) >> 2;
-    B.nfull = (B.skew + B.nbytes) >> 2;
-    infb_seek_bits(B, bit - byte0 * 8u);
-}
-
 // element s of the span's output, s < pos (s < 0: the unknown window, as 256 + its index)
 ZWZ_DEV uint32_t span_src(const uint16_t *slot, uint64_t cap, int64_t s) {
     if (s < 0) return 256u + (uint32_t) (ZWZ_SPAN_WIN + s);
@@ -161,9 +83,9 @@ ZWZ_DEV void span_decode(InflateWarpSmem &S, const uint8_t *__restrict__ comp, u
     const uint64_t byte0 = bit0 >> 3;
     const uint32_t clen = (uint32_t) (comp_len - byte0); // bytes from byte0 on
     const uint8_t *c = comp + byte0;
-    const uint64_t total_bits = (uint64_t) clen * 8u;
     InfBits B;
-    span_reader(B, comp, comp_len, byte0, bit0);
+    infb_open(B, c, clen);
+    infb_seek_bits(B, bit0 - byte0 * 8u);
 
     uint64_t pos = 0, pend_lo = 0, mstart = 0, reset = at_header ? 0u : ~(uint64_t) 0;
     bool first = !at_header;
@@ -183,7 +105,7 @@ ZWZ_DEV void span_decode(InflateWarpSmem &S, const uint8_t *__restrict__ comp, u
     for (;;) {
         { // block boundary: stop here when this block is at or past the next span's start
             infb_refill(B);
-            if (!SPAN_NEED(3)) {
+            if (!infb_need(B, 3)) {
                 status = ZWZ_STREAM_TRUNCATED;
                 goto done;
             }
@@ -202,22 +124,10 @@ ZWZ_DEV void span_decode(InflateWarpSmem &S, const uint8_t *__restrict__ comp, u
             first = false;
             infb_drop(B, 3);
             if (type == 0u) {
-                uint32_t bpos = (uint32_t) ((infb_used(B) + 7u) >> 3);
-                if ((uint64_t) bpos + 4u > clen) {
-                    status = ZWZ_STREAM_TRUNCATED;
-                    goto done;
-                }
-                infb_seek(B, bpos);
-                infb_refill(B);
-                const uint32_t v = (uint32_t) B.hold;
-                if ((v & 0xffffu) != ((v >> 16) ^ 0xffffu)) {
-                    status = ZWZ_STREAM_BAD;
-                    goto done;
-                }
-                const uint32_t len = v & 0xffffu;
-                bpos += 4u;
-                const uint32_t avail = clen - bpos;
-                const uint32_t ncopy = len < avail ? len : avail;
+                uint32_t bpos = 0, len = 0;
+                status = inf_stored_header(B, bpos, len);
+                if (status != ZWZ_STREAM_END) goto done;
+                const uint32_t ncopy = len < clen - bpos ? len : clen - bpos;
                 SPAN_FLUSH_LITS();
                 for (uint32_t i = lane; i < ncopy; i += 32u)
                     if (pos + i < cap) slot[pos + i] = c[bpos + i];
@@ -237,71 +147,26 @@ ZWZ_DEV void span_decode(InflateWarpSmem &S, const uint8_t *__restrict__ comp, u
             }
             uint32_t max_ll = 0, max_d = 0;
             if (type == 1u) {
-                for (uint32_t s = lane; s < 288u; s += 32u) S.lens[32u + s] = (uint8_t) (s < 144u ? 8 : (s < 256u ? 9 : (s < 280u ? 7 : 8)));
-                S.lens[320u + lane] = 5;
-                __syncwarp();
-                inf_build<1>(S.lens + 32, 288u, S.cnt_ll, S.sorted_ll, S.run, S.lit, ZWZ_INF_LBITS, max_ll);
-                inf_build<2>(S.lens + 320, 32u, S.cnt_d, S.sorted_d, S.run, S.dst, ZWZ_INF_DBITS, max_d);
+                inf_fixed_tables(S, max_ll, max_d);
             } else {
-                const uint32_t st = inf_dyn_tables(S, B, total_bits, max_ll, max_d);
-                if (st != ZWZ_STREAM_END) {
-                    status = st;
-                    goto done;
-                }
+                status = inf_dyn_tables(S, B, max_ll, max_d);
+                if (status != ZWZ_STREAM_END) goto done;
             }
             for (;;) { // symbol loop
                 infb_refill(B);
-                uint32_t e = S.lit[(uint32_t) B.hold & ((1u << ZWZ_INF_LBITS) - 1u)];
-                uint32_t nb = e & 15u;
-                if (ZWZ_LL_IS_LONG(e)) {
-                    uint32_t l = 0;
-                    const uint32_t sym = inf_canon_walk((uint32_t) B.hold, S.cnt_ll, S.sorted_ll, max_ll, l);
-                    e = sym == 0xffffffffu ? ZWZ_LL_INVALID(max_ll) : inf_litlen_entry(sym, l);
-                    nb = e & 15u;
-                }
-                if (ZWZ_LL_IS_INVALID(e)) {
-                    status = SPAN_NEED(nb) ? ZWZ_STREAM_BAD : ZWZ_STREAM_TRUNCATED;
-                    goto done;
-                }
-                if (!SPAN_NEED(nb)) {
-                    status = ZWZ_STREAM_TRUNCATED;
-                    goto done;
-                }
-                infb_drop(B, nb);
-                if (ZWZ_LL_IS_LIT(e)) {
-                    if (lane == (uint32_t) (pos & 31u)) mybyte = e >> 7;
+                uint32_t v = 0, dist = 0;
+                const uint32_t t = inf_token(S, B, S.lit[(uint32_t) B.hold & ((1u << ZWZ_INF_LBITS) - 1u)], max_ll, max_d, v, dist);
+                if (t == INF_TOK_LIT) {
+                    if (lane == (uint32_t) (pos & 31u)) mybyte = v;
                     pos++;
                     if ((pos & 31u) == 0u) SPAN_FLUSH_LITS();
                     continue;
                 }
-                if (ZWZ_LL_IS_EOB(e)) break;
-                infb_refill(B);
-                const uint32_t eb = (e >> 4) & 7u;
-                const uint32_t mlen = (e >> 7) - 253u + ((uint32_t) B.hold & ((1u << eb) - 1u));
-                if (!SPAN_NEED(eb)) {
-                    status = ZWZ_STREAM_TRUNCATED;
+                if (t == INF_TOK_EOB) break;
+                if (t != INF_TOK_MATCH) {
+                    status = t;
                     goto done;
                 }
-                infb_drop(B, eb);
-                infb_refill(B);
-                uint32_t d = S.dst[(uint32_t) B.hold & ((1u << ZWZ_INF_DBITS) - 1u)];
-                if (ZWZ_D_IS_LONG(d)) {
-                    uint32_t l = 0;
-                    const uint32_t sym = inf_canon_walk((uint32_t) B.hold, S.cnt_d, S.sorted_d, max_d, l);
-                    d = sym == 0xffffffffu ? ZWZ_D_INVALID(max_d) : inf_dist_entry(sym, l);
-                }
-                const uint32_t dnb = d & 15u;
-                if (ZWZ_D_IS_SPECIAL(d)) {
-                    status = SPAN_NEED(dnb) ? ZWZ_STREAM_BAD : ZWZ_STREAM_TRUNCATED;
-                    goto done;
-                }
-                const uint32_t deb = (d >> 4) & 15u;
-                if (!SPAN_NEED(dnb + deb)) {
-                    status = ZWZ_STREAM_TRUNCATED;
-                    goto done;
-                }
-                const uint32_t dist = ZWZ_D_DM1(d, (uint32_t) B.hold) + 1u;
-                infb_drop(B, dnb + deb);
                 // "invalid distance too far back": exact once the member started in this span; before that the window is
                 // not known here, and a reference that lands before the member start resolves to INVALID in the gather
                 if (fresh && dist > pos - mstart) {
@@ -310,15 +175,15 @@ ZWZ_DEV void span_decode(InflateWarpSmem &S, const uint8_t *__restrict__ comp, u
                 }
                 SPAN_FLUSH_LITS();
                 __syncwarp();
-                // every source lies before pos: a run with period dist < mlen repeats the period already written
+                // every source lies before pos: a run with period dist < v repeats the period already written
                 const int64_t src0 = (int64_t) pos - (int64_t) dist;
-                for (uint32_t i = lane; i < mlen; i += 32u) {
+                for (uint32_t i = lane; i < v; i += 32u) {
                     const uint64_t q = pos + i;
-                    const uint32_t v = span_src(slot, cap, src0 + (int64_t) (i < dist ? i : i % dist));
-                    if (q < cap) slot[q] = (uint16_t) v;
+                    const uint32_t x = span_src(slot, cap, src0 + (int64_t) (i < dist ? i : i % dist));
+                    if (q < cap) slot[q] = (uint16_t) x;
                 }
                 __syncwarp();
-                pos += mlen;
+                pos += v;
                 pend_lo = pos;
             }
             if (!last) continue;
@@ -336,12 +201,11 @@ ZWZ_DEV void span_decode(InflateWarpSmem &S, const uint8_t *__restrict__ comp, u
             uint32_t have = 0, check = 0, isize = 0;
             if ((uint64_t) bpos + 4u <= clen) {
                 have = 1u;
-                check = format == ZWZ_FORMAT_ZLIB ? ((uint32_t) c[bpos] << 24) | ((uint32_t) c[bpos + 1] << 16) | ((uint32_t) c[bpos + 2] << 8) | c[bpos + 3]
-                                                  : (uint32_t) c[bpos] | ((uint32_t) c[bpos + 1] << 8) | ((uint32_t) c[bpos + 2] << 16) | ((uint32_t) c[bpos + 3] << 24);
+                check = format == ZWZ_FORMAT_ZLIB ? inf_be32(c + bpos) : inf_le32(c + bpos);
             }
             if (format == ZWZ_FORMAT_GZIP && (uint64_t) bpos + 8u <= clen) {
                 have |= 2u;
-                isize = (uint32_t) c[bpos + 4] | ((uint32_t) c[bpos + 5] << 8) | ((uint32_t) c[bpos + 6] << 16) | ((uint32_t) c[bpos + 7] << 24);
+                isize = inf_le32(c + bpos + 4u);
             }
             if (lane == 0) {
                 SpanMember m;
@@ -386,17 +250,9 @@ ZWZ_DEV void span_decode(InflateWarpSmem &S, const uint8_t *__restrict__ comp, u
             }
             infb_seek(B, hp + (h >> 2));
         } else if (format == ZWZ_FORMAT_ZLIB) {
-            infb_refill(B);
-            if (!SPAN_NEED(16)) {
-                status = ZWZ_STREAM_TRUNCATED;
-                goto done;
-            }
-            const uint32_t cmf = (uint32_t) B.hold & 0xffu, flg = ((uint32_t) B.hold >> 8) & 0xffu;
-            if (((cmf << 8) + flg) % 31u != 0u || (cmf & 15u) != 8u || (cmf >> 4) + 8u > 15u || (flg & 0x20u)) {
-                status = ZWZ_STREAM_BAD; // FDICT: this call takes no dictionary (zlib's Z_NEED_DICT)
-                goto done;
-            }
-            infb_drop(B, 16);
+            uint32_t flg = 0;
+            status = inf_zlib_header(B, false, flg); // this call takes no dictionary
+            if (status != ZWZ_STREAM_END) goto done;
         }
         fresh = true;
         mstart = pos;
@@ -495,10 +351,12 @@ ZWZ_KERNEL __launch_bounds__(32) block_find_kernel(const uint8_t *__restrict__ c
             bool ok = is_sto;
             if (!is_sto) {
                 InfBits B;
-                span_reader(B, comp, comp_len, pp >> 3, pp);
+                infb_open(B, comp + (pp >> 3), (uint32_t) (comp_len - (pp >> 3)));
+                infb_seek_bits(B, pp & 7u);
                 infb_drop(B, 3);
+                infb_refill(B);
                 uint32_t mll = 0, md = 0;
-                ok = inf_dyn_tables(S, B, (comp_len - (pp >> 3)) * 8u, mll, md) == ZWZ_STREAM_END;
+                ok = inf_dyn_tables(S, B, mll, md) == ZWZ_STREAM_END;
             }
             if (ok) {
                 const uint32_t bfinal = __shfl_sync(ZWZ_FULL, (uint32_t) v & 1u, l);
