@@ -178,6 +178,70 @@ int zwz_inflate_stream_device(zwz_ctx *ctx, const uint8_t *d_comp, uint64_t comp
 int zwz_inflate_stream(zwz_ctx *ctx, const uint8_t *comp, uint64_t comp_len, uint8_t *out, uint64_t out_cap,
                        uint64_t *raw_len, uint32_t *status, uint32_t flags);
 
+/* ---- random access into one long stream: a seek index (zlib's zran.c idea) -------------------------------------------------
+ * zwz_inflate_stream_index[_device] inflate exactly as zwz_inflate_stream[_device] (same output, *raw_len and *status for the same
+ * input, flags, tuning and out_cap) and keep what the span decoding already found: access points, each a confirmed span start
+ * with its resolved 32 KiB window (DESIGN.md §4.9).
+ *   out == NULL: index only; the library decodes into its own memory and writes nothing to the caller.
+ *   *index is set only with ZWZ_STREAM_END, else it is NULL (OUTPUT_FULL, truncated or bad streams, "too far back").
+ *   Access points: the stream start (point 0, empty window), then greedily the first confirmed span start whose output offset is
+ *   at least the previous point's + max(spacing, 1); spacing 0 = every confirmed span start that adds output. A point records its
+ *   output offset, the bit where decoding starts (a block header, a stored block's key = the bit 3 in front of its LEN field, or a
+ *   gzip member header's first bit), its mode (ZWZ_INDEX_MODE_*), BFINAL, and its window: the last wlen <= 32 768 output bytes
+ *   before it that lie inside the same gzip member (0 at the stream start and at member headers).
+ * A zwz_index belongs to the context that created or loaded it; free it with zwz_index_free before that context is destroyed.
+ * Its point table is host memory, its windows one device allocation. */
+typedef struct zwz_index zwz_index;
+#define ZWZ_INDEX_MODE_BLOCK 0   /* a block header                                                           */
+#define ZWZ_INDEX_MODE_START 1   /* the stream's first bit (zlib / gzip header, or the first raw block)      */
+#define ZWZ_INDEX_MODE_MEMBER 2  /* a following gzip member's header                                          */
+#define ZWZ_INDEX_MODE_STORED 3  /* a stored block's key: the block type is not read from the bits there      */
+int zwz_inflate_stream_index_device(zwz_ctx *ctx, const uint8_t *d_comp, uint64_t comp_len, uint8_t *d_out, uint64_t out_cap,
+                                    uint64_t *raw_len, uint32_t *status, uint32_t flags, uint64_t spacing, zwz_index **index,
+                                    void *stream);
+int zwz_inflate_stream_index(zwz_ctx *ctx, const uint8_t *comp, uint64_t comp_len, uint8_t *out, uint64_t out_cap,
+                             uint64_t *raw_len, uint32_t *status, uint32_t flags, uint64_t spacing, zwz_index **index);
+void zwz_index_free(zwz_index *ix);
+int zwz_index_info(const zwz_index *ix, uint64_t *comp_len, uint64_t *raw_len, uint32_t *format, uint64_t *npoints);
+/* Saved form, little-endian:
+ *    0  char[8]  "ZWZIDX\0\1"
+ *    8  u32      version = 1
+ *   12  u32      format (ZWZ_FORMAT_*)
+ *   16  u64      comp_len
+ *   24  u64      raw_len
+ *   32  u64      npoints
+ *   40  u64      spacing asked for
+ *   48  u32      CRC-32 (as zlib.crc32) of the whole blob with these four bytes read as zero
+ *   52  u32      0
+ *   56  npoints x { u64 out_off; u64 bit; u16 mode; u8 bfinal; u8 0; u32 wlen }   (24 bytes each)
+ *       then the windows of the points in point order, back to back (sum of wlen bytes)
+ * zwz_index_save: *len = the blob's size; buf == NULL asks for the size only; cap < *len is ZWZ_E_CAPACITY.
+ * zwz_index_load: the blob is outside input and is checked: magic, version, CRC; len == 56 + 24 npoints + sum(wlen); format <= RAW;
+ *   comp_len <= 0xffffff00; point 0 = {0, 0, START, bfinal 0, wlen 0}; out_off strictly increasing and <= raw_len; bit strictly
+ *   increasing and < 8 comp_len; mode in range (START at point 0 only, MEMBER in gzip only); header points byte-aligned and stored
+ *   keys 3 bits before a byte boundary; bfinal <= 1, pad bytes 0; wlen <= min(32 768, out_off), and 0 at START and MEMBER points.
+ *   Anything else is ZWZ_E_ARG. */
+int zwz_index_save(const zwz_index *ix, uint8_t *buf, uint64_t cap, uint64_t *len);
+int zwz_index_load(zwz_ctx *ctx, const uint8_t *buf, uint64_t len, zwz_index **out);
+/* zwz_index_extract[_device]: range i is bytes [off[i], off[i] + len[i]) of what zwz_inflate_stream decodes the stream to; they go to
+ * out + out_off[i]. On success status[i] = ZWZ_STREAM_END and got[i] = len[i]. Each range is cut at the access points inside it; a
+ * piece is decoded by one warp from the last point at or before its start, with that point's window, up to the first block
+ * boundary at or past its end (inflate_seek.cuh). Pieces that start at a point are decoded straight into the output; the others
+ * into scratch, from which the kept bytes are copied.
+ *   ZWZ_E_ARG: a range past raw_len, a comp_len other than the index's, an index of another context, NULL pointers, flags other
+ *   than ZWZ_INFLATE_CAREFUL (the careful decoder only, for tests and A/B runs), and a piece that would decode 4 GiB or more from
+ *   its point (the decoder's positions are 32-bit: two points more than 4 GiB of output apart, as in a stream of fixed blocks only).
+ *   Check values are not verified (as in zran.c). A stream of the same length that is not the one indexed may give another status
+ *   (got[i] = the bytes delivered before the piece that came up short) or wrong bytes; it never writes outside the ranges.
+ *   Device scratch: skip + want bytes per piece that does not start at a point, in batches of about ZWZ_TUNE_STREAM_SCRATCH_BYTES.
+ * The host form uploads comp on every call; random reads of a resident stream should use the device form. */
+int zwz_index_extract_device(zwz_ctx *ctx, const zwz_index *ix, const uint8_t *d_comp, uint64_t comp_len, uint32_t n,
+                             const uint64_t *off, const uint64_t *len, uint8_t *d_out, const uint64_t *out_off,
+                             uint64_t *got, uint32_t *status, uint32_t flags, void *stream);
+int zwz_index_extract(zwz_ctx *ctx, const zwz_index *ix, const uint8_t *comp, uint64_t comp_len, uint32_t n,
+                      const uint64_t *off, const uint64_t *len, uint8_t *out, const uint64_t *out_off,
+                      uint64_t *got, uint32_t *status, uint32_t flags);
+
 /* ---- preset dictionaries (zlib's deflateSetDictionary / inflateSetDictionary, Python's zdict=) ----------------------------
  * A table of dictionaries, and for every chunk / stream the one it uses. Dictionary k is data[off[k] .. off[k+1]) (at most
  * 2^30 bytes); only its last min(len, 32 768) bytes are the window a stream may refer into, as if they came just before the

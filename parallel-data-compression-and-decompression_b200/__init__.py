@@ -18,6 +18,7 @@ from __future__ import annotations
 
 import ctypes as C
 import os
+import weakref
 from typing import Optional, Tuple
 
 import numpy as np
@@ -29,6 +30,7 @@ __all__ = ["Context", "ZwzError", "load_library", "library_path", "CHUNK_SIZE", 
 CHUNK_SIZE = 65535  # process.hpp:12
 STREAM_END, STREAM_TRUNCATED, STREAM_BAD, STREAM_OUTPUT_FULL = 0, 1, 2, 3
 INFLATE_NO_ADLER = 1
+INFLATE_CAREFUL = 2  # the careful decoder only (A/B runs and tests)
 # stream formats (ZWZ_FORMAT_*): the wrapper around the DEFLATE body. The ``format=`` keywords take these names.
 FORMAT_ZLIB, FORMAT_GZIP, FORMAT_RAW = 0, 1, 2
 BGZF_BLOCK = 65280  # largest chunk in gzip format: one BGZF member each
@@ -155,6 +157,15 @@ def _declare(L):
     L.zwz_inflate_batch_dict.argtypes = [vp, vp, vp, vp, u32, vp, vp, vp, vp, u32, dp]
     L.zwz_inflate_stream_device.argtypes = [vp, vp, u64, vp, u64, vp, vp, u32, vp]
     L.zwz_inflate_stream.argtypes = [vp, vp, u64, vp, u64, vp, vp, u32]
+    L.zwz_inflate_stream_index_device.argtypes = [vp, vp, u64, vp, u64, vp, vp, u32, u64, C.POINTER(vp), vp]
+    L.zwz_inflate_stream_index.argtypes = [vp, vp, u64, vp, u64, vp, vp, u32, u64, C.POINTER(vp)]
+    L.zwz_index_free.argtypes = [vp]
+    L.zwz_index_free.restype = None
+    L.zwz_index_info.argtypes = [vp, vp, vp, vp, vp]
+    L.zwz_index_save.argtypes = [vp, vp, u64, vp]
+    L.zwz_index_load.argtypes = [vp, vp, u64, C.POINTER(vp)]
+    L.zwz_index_extract_device.argtypes = [vp, vp, vp, u64, u32, vp, vp, vp, vp, vp, vp, u32, vp]
+    L.zwz_index_extract.argtypes = [vp, vp, vp, u64, u32, vp, vp, vp, vp, vp, vp, u32]
     return L
 
 
@@ -209,6 +220,72 @@ def _u8(a) -> np.ndarray:
     return np.ascontiguousarray(a)
 
 
+class StreamIndex:
+    """A seek index of one long stream (zwz_index): access points with their windows, for random reads of the decoded bytes.
+    It belongs to its Context, which keeps it alive and frees it first when it is closed."""
+
+    def __init__(self, ctx: "Context", h):
+        self.ctx = ctx
+        self.h = h
+        cl, rl, fm, n = C.c_uint64(), C.c_uint64(), C.c_uint32(), C.c_uint64()
+        ctx._check(ctx.lib.zwz_index_info(h, C.byref(cl), C.byref(rl), C.byref(fm), C.byref(n)))
+        self.comp_len, self.raw_len, self.format, self.npoints = cl.value, rl.value, fm.value, n.value
+        ctx._indexes.add(self)
+
+    def close(self):
+        if getattr(self, "h", None):
+            self.ctx.lib.zwz_index_free(self.h)
+            self.h = None
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+    def __enter__(self):
+        return self
+
+    def __exit__(self, *a):
+        self.close()
+
+    def save(self) -> bytes:
+        n = C.c_uint64()
+        self.ctx._check(self.ctx.lib.zwz_index_save(self.h, None, 0, C.byref(n)))
+        buf = np.empty(n.value, dtype=np.uint8)
+        self.ctx._check(self.ctx.lib.zwz_index_save(self.h, buf.ctypes.data, n.value, C.byref(n)))
+        return buf.tobytes()
+
+    def extract(self, comp, off, length, flags: int = 0):
+        """Host buffers: ranges [off[i], off[i] + length[i]) of the decoded stream, from comp (the stream indexed). Returns
+        (data, out_off[n + 1], got[n], status[n]): range i is data[out_off[i] : out_off[i] + got[i]]."""
+        comp = _u8(comp)
+        off = np.ascontiguousarray(off, dtype=np.uint64)
+        length = np.ascontiguousarray(length, dtype=np.uint64)
+        n = len(off)
+        out_off = np.zeros(n + 1, dtype=np.uint64)
+        np.cumsum(length, out=out_off[1:])
+        data = np.zeros(max(int(out_off[n]), 1), dtype=np.uint8)
+        got = np.zeros(n, dtype=np.uint64)
+        st = np.zeros(n, dtype=np.uint32)
+        keep = comp if comp.size else np.zeros(1, dtype=np.uint8)
+        self.ctx._check(self.ctx.lib.zwz_index_extract(self.ctx.h, self.h, keep.ctypes.data, comp.size, n, _ptr(off), _ptr(length), data.ctypes.data,
+                                                       out_off.ctypes.data, _ptr(got), _ptr(st), flags))
+        return data[:int(out_off[n])], out_off, got, st
+
+    def extract_device(self, d_comp: int, comp_len: int, off, length, d_out: int, out_off, flags: int = 0, stream: int = 0):
+        """Device buffers: range i goes to d_out + out_off[i]. Returns (got[n], status[n])."""
+        off = np.ascontiguousarray(off, dtype=np.uint64)
+        length = np.ascontiguousarray(length, dtype=np.uint64)
+        out_off = np.ascontiguousarray(out_off, dtype=np.uint64)
+        n = len(off)
+        got = np.zeros(n, dtype=np.uint64)
+        st = np.zeros(n, dtype=np.uint32)
+        self.ctx._check(self.ctx.lib.zwz_index_extract_device(self.ctx.h, self.h, d_comp, comp_len, n, _ptr(off), _ptr(length), d_out, _ptr(out_off),
+                                                              _ptr(got), _ptr(st), flags, stream or None))
+        return got, st
+
+
 class Context:
     """One GPU's worth of streams and arenas (``zwz_ctx``)."""
 
@@ -220,9 +297,12 @@ class Context:
             raise ZwzError(rc, "zwz_init failed: no usable sm_100a device (this package has no CPU fallback)")
         self.h = h
         self.device = device
+        self._indexes = weakref.WeakSet()  # seek indexes of this context: freed before it
 
     def close(self):
         if getattr(self, "h", None):
+            for ix in list(getattr(self, "_indexes", ())):
+                ix.close()
             self.lib.zwz_destroy(self.h)
             self.h = None
 
@@ -403,6 +483,59 @@ class Context:
         self._check(self.lib.zwz_inflate_stream_device(self.h, d_comp, comp_len, d_out, out_cap, rl.ctypes.data, st.ctypes.data,
                                                        flags | (_format(format) << 8), stream or None))
         return int(rl[0]), int(st[0])
+
+    # ---- random access into one long stream: a seek index ----
+    def inflate_stream_index(self, comp, format: str = "gzip", spacing: int = 1 << 20, want_output: bool = True, out_cap: Optional[int] = None,
+                             flags: int = 0):
+        """inflate_stream that also builds a seek index: access points at least `spacing` output bytes apart (0 = every confirmed span
+        start), each with its 32 KiB window. Returns (out, status, StreamIndex or None); the index exists only with STREAM_END.
+        want_output=False: index only (out is empty, nothing is copied back)."""
+        comp = _u8(comp)
+        f = _format(format)
+        if not want_output:
+            out, st, _, ix = self._inflate_stream_index(comp, f, None, (1 << 64) - 1, flags, spacing)
+            return out, st, ix
+        cap = out_cap
+        if cap is None:
+            cap = 4 * len(comp) + 1024
+            if f == FORMAT_GZIP and len(comp) >= 4:
+                cap = min(int.from_bytes(comp[-4:].tobytes(), "little"), 1032 * len(comp) + 1024)
+        out, st, need, ix = self._inflate_stream_index(comp, f, max(cap, 1), cap, flags, spacing)
+        if st == STREAM_OUTPUT_FULL and out_cap is None:
+            out, st, need, ix = self._inflate_stream_index(comp, f, max(need, 1), need, flags, spacing)
+        self.last_needed = need
+        return out, st, ix
+
+    def _inflate_stream_index(self, comp, f: int, alloc: Optional[int], cap: int, flags: int, spacing: int):
+        out = np.empty(alloc, dtype=np.uint8) if alloc is not None else None
+        rl = np.zeros(1, dtype=np.uint64)
+        st = np.zeros(1, dtype=np.uint32)
+        h = C.c_void_p()
+        keep = comp if comp.size else np.zeros(1, dtype=np.uint8)
+        self._check(self.lib.zwz_inflate_stream_index(self.h, keep.ctypes.data, comp.size, None if out is None else out.ctypes.data, cap,
+                                                      rl.ctypes.data, st.ctypes.data, flags | (f << 8), spacing, C.byref(h)))
+        ix = StreamIndex(self, h) if h.value else None
+        if int(st[0]) == STREAM_OUTPUT_FULL or out is None:
+            return np.empty(0, dtype=np.uint8), int(st[0]), int(rl[0]), ix
+        return out[:int(rl[0])], int(st[0]), int(rl[0]), ix
+
+    def inflate_stream_index_device(self, d_comp: int, comp_len: int, d_out: Optional[int], out_cap: int, format: str = "gzip",
+                                    spacing: int = 1 << 20, flags: int = 0, stream: int = 0):
+        """Device form: d_out == 0 / None builds the index only. Returns (raw_len, status, StreamIndex or None)."""
+        rl = np.zeros(1, dtype=np.uint64)
+        st = np.zeros(1, dtype=np.uint32)
+        h = C.c_void_p()
+        self._check(self.lib.zwz_inflate_stream_index_device(self.h, d_comp, comp_len, d_out or None, out_cap, rl.ctypes.data, st.ctypes.data,
+                                                             flags | (_format(format) << 8), spacing, C.byref(h), stream or None))
+        return int(rl[0]), int(st[0]), (StreamIndex(self, h) if h.value else None)
+
+    def load_index(self, blob) -> "StreamIndex":
+        """A seek index saved with StreamIndex.save(); the blob is checked (ZwzError on anything malformed)."""
+        b = _u8(blob)
+        keep = b if b.size else np.zeros(1, dtype=np.uint8)
+        h = C.c_void_p()
+        self._check(self.lib.zwz_index_load(self.h, keep.ctypes.data, b.size, C.byref(h)))
+        return StreamIndex(self, h)
 
     def decompress_records(self, comp, off, length, rec_cap, rec_file, nf: int, out_cap: int, want_md5: bool = True, flags: int = 0):
         """Worker side of decompression.cpp:100-151 for a group of records (host buffers): inflate every record, concatenate the

@@ -12,6 +12,7 @@
 #include "inflate.cuh"
 #include "inflate_lanes.cuh"
 #include "inflate_stream.cuh"
+#include "inflate_seek.cuh"
 #include "deflate_match.cuh"
 #include "deflate_encode.cuh"
 
@@ -169,6 +170,7 @@ struct zwz_ctx {
     int inf_blocks_per_sm = 1; // resident inflate_kernel CTAs per SM
     int inf_dict_blocks_per_sm = 1; // the same for inflate_kernel<true>
     int span_blocks_per_sm = 1; // the same for inflate_span_kernel
+    int seek_blocks_per_sm = 1; // the same for inflate_seek_kernel
     uint64_t stream_span_bytes = 0; // ZWZ_TUNE_STREAM_SPAN_BYTES (0 = default)
     uint64_t stream_scratch_bytes = 0; // ZWZ_TUNE_STREAM_SCRATCH_BYTES (0 = default)
     zwz_stream_t stream = nullptr;
@@ -537,13 +539,15 @@ int zwz_init(int device, zwz_ctx **out) {
         zwz_rt::set_max_dyn_smem((const void *) zwz::inflate_kernel<false>, ZWZ_INF_SMEM) ||
         zwz_rt::set_max_dyn_smem((const void *) zwz::inflate_lanes_kernel, ZWZ_IL_SMEM) ||
         zwz_rt::set_max_dyn_smem((const void *) zwz::inflate_span_kernel, ZWZ_INF_SMEM) ||
-        zwz_rt::set_max_dyn_smem((const void *) zwz::block_find_kernel, ZWZ_INF_SMEM)) {
+        zwz_rt::set_max_dyn_smem((const void *) zwz::block_find_kernel, ZWZ_INF_SMEM) ||
+        zwz_rt::set_max_dyn_smem((const void *) zwz::inflate_seek_kernel, ZWZ_INF_SMEM)) {
         delete ctx;
         return ZWZ_E_NODEVICE;
     }
     if (zwz_rt::max_blocks_per_sm(&ctx->inf_blocks_per_sm, (const void *) zwz::inflate_kernel<false>, ZWZ_INF_WARPS * 32, ZWZ_INF_SMEM) ||
         zwz_rt::max_blocks_per_sm(&ctx->inf_dict_blocks_per_sm, (const void *) zwz::inflate_kernel<true>, ZWZ_INF_WARPS * 32, ZWZ_INF_SMEM) ||
-        zwz_rt::max_blocks_per_sm(&ctx->span_blocks_per_sm, (const void *) zwz::inflate_span_kernel, ZWZ_INF_WARPS * 32, ZWZ_INF_SMEM)) {
+        zwz_rt::max_blocks_per_sm(&ctx->span_blocks_per_sm, (const void *) zwz::inflate_span_kernel, ZWZ_INF_WARPS * 32, ZWZ_INF_SMEM) ||
+        zwz_rt::max_blocks_per_sm(&ctx->seek_blocks_per_sm, (const void *) zwz::inflate_seek_kernel, ZWZ_INF_WARPS * 32, ZWZ_INF_SMEM)) {
         delete ctx;
         return ZWZ_E_NODEVICE;
     }
@@ -1987,12 +1991,74 @@ static int span_decode_exact(zwz_ctx *ctx, zwz_stream_t st, StreamBufs &bufs, co
     return span_decode_round(ctx, st, bufs, d_comp, comp_len, flags, L, tail, over, true);
 }
 
+// ---- seek index (zwz_inflate_stream_index*): access points chosen from the confirmed span starts ----
+struct IndexPoint {
+    uint64_t out, bit;
+    uint32_t mode, bfinal, wlen;
+};
+struct IndexBuild {
+    uint64_t spacing;
+    std::vector<IndexPoint> pts;
+    std::vector<uint8_t> win; // the windows of the points, back to back
+};
+
+// The access points among the confirmed spans of one wave (W, output positions base + sw[i].base): span 0 of the stream, then
+// greedily the first span start at least `spacing` (at least 1) bytes of output past the previous point. A point's window is the
+// resolved window in front of its span: win_in for the wave's first span, w0 + ((i - 1) << 15) for span i. A wave with no output
+// has its windows unresolved; only its first span can be a point there.
+static int index_points(zwz_ctx *ctx, zwz_stream_t st, StreamBufs &wb, IndexBuild &ib, const std::vector<SpanEnt> &W, const std::vector<zwz::SpanWin> &sw,
+                        uint64_t base, uint64_t total, const uint16_t *win_in, const uint16_t *w0) {
+    std::vector<const uint16_t *> src;
+    std::vector<size_t> at;
+    const size_t ns = total ? W.size() : 1;
+    for (size_t i = 0; i < ns; ++i) {
+        const SpanEnt &e = W[i];
+        IndexPoint p{base + sw[i].base, 0, e.mode, 0, 0};
+        if (!ib.pts.empty() && p.out - ib.pts.back().out < std::max<uint64_t>(ib.spacing, 1u)) continue;
+        if (e.mode == zwz::SPAN_MODE_MEMBER) {
+            p.bit = (e.start >> 4) * 8u;
+        } else if (e.mode != zwz::SPAN_MODE_FIRST) {
+            p.bit = e.start >> 1;
+            p.bfinal = (uint32_t) (e.start & 1u);
+        }
+        const uint16_t *w = i ? w0 + ((size_t) (i - 1) << 15) : win_in;
+        if (w && e.mode != zwz::SPAN_MODE_MEMBER && e.mode != zwz::SPAN_MODE_FIRST) { // a member starts with an empty window
+            src.push_back(w);
+            at.push_back(ib.pts.size());
+        }
+        ib.pts.push_back(p);
+    }
+    if (src.empty()) return ZWZ_OK;
+    const size_t k = src.size();
+    uint8_t *dm = (uint8_t *) wb.get(k * (ZWZ_SPAN_WIN + 12) + 64);
+    if (!dm) return fail(ctx, ZWZ_E_NOMEM, "index scratch allocation failed");
+    uint8_t *d_win = dm;
+    const uint16_t **d_src = (const uint16_t **) (dm + k * ZWZ_SPAN_WIN);
+    uint32_t *d_inv = (uint32_t *) (dm + k * (ZWZ_SPAN_WIN + 8));
+    if (zwz_rt::memcpy_h2d(d_src, src.data(), k * 8, st) || zwz_rt::memset_device(d_inv, 0, k * 4, st)) return fail(ctx, ZWZ_E_CUDA, "index upload failed");
+    {
+        ProfSpan ps(ctx, ZWZ_PROF_PACK, st);
+        ZWZ_LAUNCH(zwz::index_pack_kernel, (uint32_t) (k * (ZWZ_SPAN_WIN / 256u)), 256, 0, st, (const uint16_t *const *) d_src, d_win, d_inv);
+    }
+    int rc;
+    if ((rc = check_launch(ctx, "index_pack_kernel"))) return rc;
+    std::vector<uint8_t> win(k * ZWZ_SPAN_WIN);
+    std::vector<uint32_t> inv(k);
+    if (zwz_rt::memcpy_d2h(win.data(), d_win, win.size(), st) || zwz_rt::memcpy_d2h(inv.data(), d_inv, k * 4, st) || zwz_rt::stream_sync(st))
+        return fail(ctx, ZWZ_E_CUDA, "index_pack_kernel failed");
+    for (size_t j = 0; j < k; ++j) {
+        ib.pts[at[j]].wlen = ZWZ_SPAN_WIN - inv[j];
+        ib.win.insert(ib.win.end(), win.begin() + j * ZWZ_SPAN_WIN + inv[j], win.begin() + (j + 1) * ZWZ_SPAN_WIN);
+    }
+    return ZWZ_OK;
+}
+
 // Waves: the spans are decoded, confirmed, resolved and gathered in order, a wave at a time, so that the u16 slots of one wave stay
 // near the scratch budget (ZWZ_TUNE_STREAM_SCRATCH_BYTES). A wave hands the next one the resolved window behind its last span, the
-// position where that span stopped and the running check value of the member still open. d_out == NULL (the host-buffer form):
-// every wave is gathered into grow_out and downloaded to h_out.
+// position where that span stopped and the running check value of the member still open. d_out == NULL: every wave is gathered into
+// grow_out, and downloaded to h_out when there is one. ib: the access points of a seek index are collected wave by wave.
 static int inflate_stream_impl(zwz_ctx *ctx, const uint8_t *d_comp, uint64_t comp_len, uint8_t *d_out, uint8_t *h_out, uint64_t out_cap,
-                               Arena *grow_out, uint64_t *raw_len, uint32_t *status, uint32_t flags, zwz_stream_t st) {
+                               Arena *grow_out, uint64_t *raw_len, uint32_t *status, uint32_t flags, zwz_stream_t st, IndexBuild *ib = nullptr) {
     const uint32_t format = (flags >> 8) & 0xffu;
     Trace tr(ctx, "inflate_stream", st);
     int rc;
@@ -2175,6 +2241,7 @@ static int inflate_stream_impl(zwz_ctx *ctx, const uint8_t *d_comp, uint64_t com
             if ((rc = check_launch(ctx, "stream_gather_kernel"))) return rc;
             if (zwz_rt::memcpy_d2h(&first_bad, d_bad, 8, st) || zwz_rt::stream_sync(st)) return fail(ctx, ZWZ_E_CUDA, "stream_gather_kernel failed");
         }
+        if (ib && (rc = index_points(ctx, st, *wb, *ib, W, sw, base, total, win_in, w0))) return rc;
         uint64_t wlen = total; // valid bytes of the wave
         if (first_bad < total) {
             wlen = first_bad;
@@ -2285,6 +2352,348 @@ int zwz_inflate_stream(zwz_ctx *ctx, const uint8_t *comp, uint64_t comp_len, uin
     if ((rc = reserve(ctx, ctx->bulk_in, (size_t) comp_len + 64, false))) return rc;
     if (zwz_rt::memcpy_h2d(ctx->bulk_in.p, comp, (size_t) comp_len, ctx->stream)) return fail(ctx, ZWZ_E_CUDA, "compressed upload failed");
     return inflate_stream_impl(ctx, (const uint8_t *) ctx->bulk_in.p, comp_len, nullptr, out, out_cap, &ctx->bulk_out, raw_len, status, flags, ctx->stream);
+}
+
+// ======================================================================================================================
+// seek index: random access into one long stream (inflate_seek.cuh)
+// ======================================================================================================================
+static_assert(ZWZ_INDEX_MODE_BLOCK == zwz::SPAN_MODE_BLOCK && ZWZ_INDEX_MODE_START == zwz::SPAN_MODE_FIRST &&
+                  ZWZ_INDEX_MODE_MEMBER == zwz::SPAN_MODE_MEMBER && ZWZ_INDEX_MODE_STORED == zwz::SPAN_MODE_STORED,
+              "the saved modes are the span modes");
+
+struct zwz_index {
+    zwz_ctx *ctx;
+    uint32_t format;
+    uint64_t comp_len, raw_len, spacing;
+    std::vector<IndexPoint> pts;
+    std::vector<uint64_t> woff; // where each point's window starts in d_win
+    uint8_t *d_win = nullptr;   // the windows of all points, back to back
+    uint64_t win_bytes = 0;
+};
+
+static const uint64_t kIndexHead = 56, kIndexPoint = 24;
+static const uint64_t kStreamLimit = 0xffffff00ull; // the largest comp_len zwz_inflate_stream takes
+
+static uint32_t crc32_host(uint32_t c, const uint8_t *p, size_t n) {
+    static const zwz::Crc32Tables T = zwz::crc32_make_tables();
+    c = ~c;
+    for (size_t i = 0; i < n; ++i) c = T.slice[0][(c ^ p[i]) & 0xffu] ^ (c >> 8);
+    return ~c;
+}
+static uint32_t blob_crc(const uint8_t *b, uint64_t len) { // CRC-32 of the blob with its CRC field read as zero
+    static const uint8_t zero[4] = {0, 0, 0, 0};
+    uint32_t c = crc32_host(0, b, 48);
+    c = crc32_host(c, zero, 4);
+    return crc32_host(c, b + 52, (size_t) (len - 52));
+}
+static uint64_t rd_le(const uint8_t *p, int n) {
+    uint64_t v = 0;
+    for (int i = n; i-- > 0;) v = (v << 8) | p[i];
+    return v;
+}
+static void wr_le(uint8_t *p, uint64_t v, int n) {
+    for (int i = 0; i < n; ++i, v >>= 8) p[i] = (uint8_t) v;
+}
+
+// takes the points and windows of `ib`: the windows go to one device allocation
+static int index_create(zwz_ctx *ctx, uint32_t format, uint64_t comp_len, uint64_t raw_len, uint64_t spacing, std::vector<IndexPoint> &&pts,
+                        const uint8_t *win, uint64_t win_bytes, zwz_index **out) {
+    std::unique_ptr<zwz_index> ix(new (std::nothrow) zwz_index());
+    if (!ix) return fail(ctx, ZWZ_E_NOMEM, "index allocation failed");
+    ix->ctx = ctx;
+    ix->format = format;
+    ix->comp_len = comp_len;
+    ix->raw_len = raw_len;
+    ix->spacing = spacing;
+    ix->pts = std::move(pts);
+    ix->woff.resize(ix->pts.size());
+    uint64_t o = 0;
+    for (size_t k = 0; k < ix->pts.size(); ++k) {
+        ix->woff[k] = o;
+        o += ix->pts[k].wlen;
+    }
+    ix->win_bytes = win_bytes;
+    if (zwz_rt::malloc_device((void **) &ix->d_win, win_bytes)) return fail(ctx, ZWZ_E_NOMEM, "index window allocation failed");
+    if (win_bytes && (zwz_rt::memcpy_h2d(ix->d_win, win, win_bytes, ctx->stream) || zwz_rt::stream_sync(ctx->stream))) {
+        zwz_rt::free_device(ix->d_win);
+        return fail(ctx, ZWZ_E_CUDA, "index window upload failed");
+    }
+    *out = ix.release();
+    return ZWZ_OK;
+}
+
+static int stream_index_impl(zwz_ctx *ctx, const uint8_t *d_comp, uint64_t comp_len, uint8_t *d_out, uint8_t *h_out, uint64_t out_cap, uint64_t *raw_len,
+                             uint32_t *status, uint32_t flags, uint64_t spacing, zwz_index **index, zwz_stream_t st) {
+    IndexBuild ib{spacing, {}, {}};
+    int rc = inflate_stream_impl(ctx, d_comp, comp_len, d_out, h_out, out_cap, d_out ? nullptr : &ctx->bulk_out, raw_len, status, flags, st, &ib);
+    if (rc || *status != ZWZ_STREAM_END) return rc;
+    return index_create(ctx, (flags >> 8) & 0xffu, comp_len, *raw_len, spacing, std::move(ib.pts), ib.win.data(), ib.win.size(), index);
+}
+
+static int stream_index_args(zwz_ctx *ctx, const uint8_t *comp, uint64_t *raw_len, uint32_t *status, uint32_t flags, uint64_t comp_len, zwz_index **index) {
+    if (index) *index = nullptr;
+    if (!comp || !raw_len || !status || !index) return fail(ctx, ZWZ_E_ARG, "null argument");
+    if (((flags >> 8) & 0xffu) > ZWZ_FORMAT_RAW) return fail(ctx, ZWZ_E_ARG, "unknown stream format");
+    if (comp_len > kStreamLimit) return fail(ctx, ZWZ_E_ARG, "compressed stream of 4 GiB or more");
+    return ZWZ_OK;
+}
+
+int zwz_inflate_stream_index_device(zwz_ctx *ctx, const uint8_t *d_comp, uint64_t comp_len, uint8_t *d_out, uint64_t out_cap, uint64_t *raw_len,
+                                    uint32_t *status, uint32_t flags, uint64_t spacing, zwz_index **index, void *stream_v) {
+    if (!ctx) return ZWZ_E_ARG;
+    int rc;
+    if ((rc = stream_index_args(ctx, d_comp, raw_len, status, flags, comp_len, index))) return rc;
+    zwz_rt::set_device(ctx->device);
+    return stream_index_impl(ctx, d_comp, comp_len, d_out, nullptr, out_cap, raw_len, status, flags, spacing, index,
+                             stream_v ? (zwz_stream_t) stream_v : ctx->stream);
+}
+
+int zwz_inflate_stream_index(zwz_ctx *ctx, const uint8_t *comp, uint64_t comp_len, uint8_t *out, uint64_t out_cap, uint64_t *raw_len, uint32_t *status,
+                             uint32_t flags, uint64_t spacing, zwz_index **index) {
+    if (!ctx) return ZWZ_E_ARG;
+    int rc;
+    if ((rc = stream_index_args(ctx, comp, raw_len, status, flags, comp_len, index))) return rc;
+    zwz_rt::set_device(ctx->device);
+    if ((rc = reserve(ctx, ctx->bulk_in, (size_t) comp_len + 64, false))) return rc;
+    if (zwz_rt::memcpy_h2d(ctx->bulk_in.p, comp, (size_t) comp_len, ctx->stream)) return fail(ctx, ZWZ_E_CUDA, "compressed upload failed");
+    return stream_index_impl(ctx, (const uint8_t *) ctx->bulk_in.p, comp_len, nullptr, out, out_cap, raw_len, status, flags, spacing, index, ctx->stream);
+}
+
+void zwz_index_free(zwz_index *ix) {
+    if (!ix) return;
+    zwz_rt::set_device(ix->ctx->device);
+    zwz_rt::stream_sync(ix->ctx->stream);
+    zwz_rt::free_device(ix->d_win);
+    delete ix;
+}
+
+int zwz_index_info(const zwz_index *ix, uint64_t *comp_len, uint64_t *raw_len, uint32_t *format, uint64_t *npoints) {
+    if (!ix) return ZWZ_E_ARG;
+    if (comp_len) *comp_len = ix->comp_len;
+    if (raw_len) *raw_len = ix->raw_len;
+    if (format) *format = ix->format;
+    if (npoints) *npoints = ix->pts.size();
+    return ZWZ_OK;
+}
+
+int zwz_index_save(const zwz_index *ix, uint8_t *buf, uint64_t cap, uint64_t *len) {
+    if (!ix || !len) return ZWZ_E_ARG;
+    const uint64_t n = ix->pts.size(), need = kIndexHead + kIndexPoint * n + ix->win_bytes;
+    *len = need;
+    if (!buf) return ZWZ_OK;
+    if (cap < need) return fail(ix->ctx, ZWZ_E_CAPACITY, "index buffer too small");
+    memset(buf, 0, kIndexHead + kIndexPoint * n);
+    memcpy(buf, "ZWZIDX\0\1", 8);
+    wr_le(buf + 8, 1, 4);
+    wr_le(buf + 12, ix->format, 4);
+    wr_le(buf + 16, ix->comp_len, 8);
+    wr_le(buf + 24, ix->raw_len, 8);
+    wr_le(buf + 32, n, 8);
+    wr_le(buf + 40, ix->spacing, 8);
+    for (uint64_t k = 0; k < n; ++k) {
+        uint8_t *p = buf + kIndexHead + kIndexPoint * k;
+        const IndexPoint &q = ix->pts[k];
+        wr_le(p, q.out, 8);
+        wr_le(p + 8, q.bit, 8);
+        wr_le(p + 16, q.mode, 2);
+        p[18] = (uint8_t) q.bfinal;
+        wr_le(p + 20, q.wlen, 4);
+    }
+    zwz_ctx *ctx = ix->ctx;
+    zwz_rt::set_device(ctx->device);
+    if (ix->win_bytes && (zwz_rt::memcpy_d2h(buf + kIndexHead + kIndexPoint * n, ix->d_win, ix->win_bytes, ctx->stream) || zwz_rt::stream_sync(ctx->stream)))
+        return fail(ctx, ZWZ_E_CUDA, "index window download failed");
+    wr_le(buf + 48, blob_crc(buf, need), 4);
+    return ZWZ_OK;
+}
+
+int zwz_index_load(zwz_ctx *ctx, const uint8_t *buf, uint64_t len, zwz_index **out) {
+    if (!ctx) return ZWZ_E_ARG;
+    if (out) *out = nullptr;
+    if (!buf || !out) return fail(ctx, ZWZ_E_ARG, "null argument");
+    auto bad = [&](const char *what) { return fail(ctx, ZWZ_E_ARG, what); };
+    if (len < kIndexHead || memcmp(buf, "ZWZIDX\0\1", 8) != 0 || rd_le(buf + 8, 4) != 1u) return bad("not a seek index of version 1");
+    if (rd_le(buf + 48, 4) != blob_crc(buf, len)) return bad("index CRC mismatch");
+    const uint32_t format = (uint32_t) rd_le(buf + 12, 4);
+    const uint64_t comp_len = rd_le(buf + 16, 8), raw_len = rd_le(buf + 24, 8), n = rd_le(buf + 32, 8), spacing = rd_le(buf + 40, 8);
+    if (format > ZWZ_FORMAT_RAW || comp_len > kStreamLimit || rd_le(buf + 52, 4) != 0u) return bad("index header out of range");
+    if (n == 0 || n > (len - kIndexHead) / kIndexPoint) return bad("index point table does not fit");
+    std::vector<IndexPoint> pts(n);
+    uint64_t wsum = 0;
+    for (uint64_t k = 0; k < n; ++k) {
+        const uint8_t *p = buf + kIndexHead + kIndexPoint * k;
+        IndexPoint &q = pts[k];
+        q.out = rd_le(p, 8);
+        q.bit = rd_le(p + 8, 8);
+        q.mode = (uint32_t) rd_le(p + 16, 2);
+        q.bfinal = p[18];
+        q.wlen = (uint32_t) rd_le(p + 20, 4);
+        const bool header = q.mode == ZWZ_INDEX_MODE_START || q.mode == ZWZ_INDEX_MODE_MEMBER;
+        bool ok = q.mode <= ZWZ_INDEX_MODE_STORED && q.bfinal <= 1u && p[19] == 0 && q.out <= raw_len && q.bit < comp_len * 8u &&
+                  q.wlen <= std::min<uint64_t>(ZWZ_SPAN_WIN, q.out) && (!header || (q.wlen == 0u && q.bfinal == 0u && (q.bit & 7u) == 0u)) &&
+                  (q.mode != ZWZ_INDEX_MODE_STORED || ((q.bit + 3u) & 7u) == 0u) && (q.mode != ZWZ_INDEX_MODE_MEMBER || format == ZWZ_FORMAT_GZIP);
+        if (k == 0) ok = ok && q.out == 0 && q.bit == 0 && q.mode == ZWZ_INDEX_MODE_START;
+        else ok = ok && q.mode != ZWZ_INDEX_MODE_START && q.out > pts[k - 1].out && q.bit > pts[k - 1].bit;
+        if (!ok) return bad("index point out of range");
+        wsum += q.wlen;
+    }
+    if (len != kIndexHead + kIndexPoint * n + wsum) return bad("index length does not match its points");
+    zwz_rt::set_device(ctx->device);
+    return index_create(ctx, format, comp_len, raw_len, spacing, std::move(pts), buf + kIndexHead + kIndexPoint * n, wsum, out);
+}
+
+// One piece of a range: decoded from point p, of which the first `skip` bytes are dropped and the next `want` kept.
+struct SeekPiece {
+    uint64_t skip, want, dst; // dst: offset in the caller's output
+    uint32_t point, range;
+};
+
+int zwz_index_extract_device(zwz_ctx *ctx, const zwz_index *ix, const uint8_t *d_comp, uint64_t comp_len, uint32_t n, const uint64_t *off,
+                             const uint64_t *len, uint8_t *d_out, const uint64_t *out_off, uint64_t *got, uint32_t *status, uint32_t flags,
+                             void *stream_v) {
+    if (!ctx) return ZWZ_E_ARG;
+    if (!ix || !d_comp || (n && (!off || !len || !d_out || !out_off || !got || !status))) return fail(ctx, ZWZ_E_ARG, "null argument");
+    if (ix->ctx != ctx) return fail(ctx, ZWZ_E_ARG, "index of another context");
+    if (comp_len != ix->comp_len) return fail(ctx, ZWZ_E_ARG, "compressed length differs from the index's");
+    if (flags & ~ZWZ_INFLATE_CAREFUL) return fail(ctx, ZWZ_E_ARG, "unknown extract flags");
+    // ---- pieces: every range cut at each point inside it ----
+    std::vector<SeekPiece> pcs;
+    const std::vector<IndexPoint> &P = ix->pts;
+    for (uint32_t i = 0; i < n; ++i) {
+        if (off[i] > ix->raw_len || len[i] > ix->raw_len - off[i]) return fail(ctx, ZWZ_E_ARG, "range past the end of the stream");
+        uint64_t a = off[i];
+        const uint64_t e = off[i] + len[i];
+        if (a == e) continue;
+        size_t p = (size_t) (std::upper_bound(P.begin(), P.end(), a, [](uint64_t v, const IndexPoint &q) { return v < q.out; }) - P.begin()) - 1;
+        for (; a < e; ++p) {
+            const uint64_t b = p + 1 < P.size() ? std::min(e, P[p + 1].out) : e;
+            const SeekPiece s{a - P[p].out, b - a, out_off[i] + (a - off[i]), (uint32_t) p, i};
+            // the decoder's positions are 32-bit
+            if (s.skip >= ((uint64_t) 1 << 32) || s.want >= ((uint64_t) 1 << 32) - s.skip)
+                return fail(ctx, ZWZ_E_ARG, "a piece decodes 4 GiB or more from its access point");
+            pcs.push_back(s);
+            a = b;
+        }
+    }
+    zwz_rt::set_device(ctx->device);
+    const zwz_stream_t st = stream_v ? (zwz_stream_t) stream_v : ctx->stream;
+    std::vector<size_t> ord(pcs.size());
+    for (size_t k = 0; k < ord.size(); ++k) ord[k] = k;
+    std::stable_sort(ord.begin(), ord.end(), [&](size_t x, size_t y) { return pcs[x].skip + pcs[x].want > pcs[y].skip + pcs[y].want; });
+    std::vector<zwz::SeekRes> res(pcs.size());
+    // ---- batches of pieces whose scratch (the pieces with skip > 0 decode skip + want bytes there) fits the budget ----
+    const uint64_t budget = ctx->stream_scratch_bytes ? ctx->stream_scratch_bytes : ((uint64_t) 4 << 30);
+    const uint32_t format = ix->format;
+    int rc;
+    for (size_t k0 = 0; k0 < ord.size();) {
+        size_t k1 = k0;
+        uint64_t scratch = 0;
+        for (; k1 < ord.size(); ++k1) {
+            const SeekPiece &s = pcs[ord[k1]];
+            const uint64_t need = s.skip ? align_up(s.skip + s.want, 16) : 0;
+            if (k1 > k0 && scratch + need > budget) break;
+            scratch += need;
+        }
+        const size_t m = k1 - k0;
+        StreamBufs bufs(st);
+        uint8_t *d_scr = (uint8_t *) bufs.get(scratch);
+        uint8_t *dj = (uint8_t *) bufs.get(m * (sizeof(zwz::SeekJob) + sizeof(zwz::SeekRes) + 20) + 64);
+        if (!d_scr || !dj) return fail(ctx, ZWZ_E_NOMEM, "extract scratch allocation failed");
+        std::vector<zwz::SeekJob> jobs(m);
+        std::vector<uint64_t> g_src, g_dst;
+        std::vector<uint32_t> g_len;
+        uint64_t so = 0;
+        for (size_t k = 0; k < m; ++k) {
+            const SeekPiece &s = pcs[ord[k0 + k]];
+            const IndexPoint &q = P[s.point];
+            zwz::SeekJob &J = jobs[k];
+            J.bit = q.bit;
+            J.win = ix->d_win + ix->woff[s.point];
+            J.wlen = q.wlen;
+            J.need = (uint32_t) (s.skip + s.want);
+            J.mode = q.mode;
+            J.bfinal = q.bfinal;
+            if (s.skip) {
+                J.out = d_scr + so;
+                g_src.push_back(so + s.skip);
+                g_dst.push_back(s.dst);
+                g_len.push_back((uint32_t) s.want);
+                so += align_up(s.skip + s.want, 16);
+            } else {
+                J.out = d_out + s.dst;
+            }
+        }
+        const size_t ng = g_len.size();
+        zwz::SeekJob *d_jobs = (zwz::SeekJob *) dj;
+        zwz::SeekRes *d_res = (zwz::SeekRes *) (dj + m * sizeof(zwz::SeekJob));
+        uint64_t *d_gs = (uint64_t *) (dj + m * (sizeof(zwz::SeekJob) + sizeof(zwz::SeekRes)));
+        uint64_t *d_gd = d_gs + m;
+        uint32_t *d_gl = (uint32_t *) (d_gd + m);
+        uint32_t *d_counter = d_gl + m;
+        if (zwz_rt::memcpy_h2d(d_jobs, jobs.data(), m * sizeof(zwz::SeekJob), st) || zwz_rt::memset_device(d_counter, 0, 4, st) ||
+            (ng && (zwz_rt::memcpy_h2d(d_gs, g_src.data(), ng * 8, st) || zwz_rt::memcpy_h2d(d_gd, g_dst.data(), ng * 8, st) ||
+                    zwz_rt::memcpy_h2d(d_gl, g_len.data(), ng * 4, st))))
+            return fail(ctx, ZWZ_E_CUDA, "piece upload failed");
+        {
+            ProfSpan ps(ctx, ZWZ_PROF_INFLATE, st);
+            const uint32_t grid = (uint32_t) std::min<size_t>(m, (size_t) ctx->sm_count * ctx->seek_blocks_per_sm);
+            ZWZ_LAUNCH(zwz::inflate_seek_kernel, grid, ZWZ_INF_WARPS * 32, ZWZ_INF_SMEM, st, d_comp, comp_len, (const zwz::SeekJob *) d_jobs, d_res,
+                       (uint32_t) m, flags | (format << 8), d_counter);
+        }
+        if ((rc = check_launch(ctx, "inflate_seek_kernel"))) return rc;
+        if (ng) { // the kept bytes of the pieces that decoded into scratch
+            ProfSpan ps(ctx, ZWZ_PROF_PACK, st);
+            ZWZ_LAUNCH(zwz::gather_records_kernel, (uint32_t) ((ng + 7) / 8), 256, 0, st, (const uint8_t *) d_scr, (const uint64_t *) d_gs,
+                       (const uint64_t *) d_gd, (const uint32_t *) d_gl, d_out, (uint32_t) ng);
+        }
+        if ((rc = check_launch(ctx, "gather_records_kernel"))) return rc;
+        std::vector<zwz::SeekRes> r(m);
+        if (zwz_rt::memcpy_d2h(r.data(), d_res, m * sizeof(zwz::SeekRes), st) || zwz_rt::stream_sync(st))
+            return fail(ctx, ZWZ_E_CUDA, "inflate_seek_kernel failed");
+        for (size_t k = 0; k < m; ++k) res[ord[k0 + k]] = r[k];
+        k0 = k1;
+    }
+    // ---- per range: the bytes delivered in order up to the first piece that came up short, and that piece's status ----
+    for (uint32_t i = 0; i < n; ++i) {
+        got[i] = 0;
+        status[i] = ZWZ_STREAM_END;
+    }
+    for (size_t k = 0; k < pcs.size(); ++k) {
+        const SeekPiece &s = pcs[k];
+        const uint32_t i = s.range;
+        if (status[i] != ZWZ_STREAM_END) continue;
+        const uint64_t have = res[k].nout > s.skip ? std::min(res[k].nout - s.skip, s.want) : 0;
+        got[i] += have;
+        // a piece that stopped short: the stream ended (TRUNCATED: not the stream indexed) or could not be decoded further
+        if (have < s.want) status[i] = res[k].status == ZWZ_STREAM_END ? ZWZ_STREAM_TRUNCATED : res[k].status;
+    }
+    return ZWZ_OK;
+}
+
+int zwz_index_extract(zwz_ctx *ctx, const zwz_index *ix, const uint8_t *comp, uint64_t comp_len, uint32_t n, const uint64_t *off, const uint64_t *len,
+                      uint8_t *out, const uint64_t *out_off, uint64_t *got, uint32_t *status, uint32_t flags) {
+    if (!ctx) return ZWZ_E_ARG;
+    if (!ix || !comp || (n && (!off || !len || !out || !out_off || !got || !status))) return fail(ctx, ZWZ_E_ARG, "null argument");
+    // the ranges are extracted back to back into device memory, downloaded in one copy and put in place here
+    std::vector<uint64_t> packed(n);
+    uint64_t total = 0;
+    for (uint32_t i = 0; i < n; ++i) {
+        packed[i] = total;
+        if (len[i] > ix->raw_len) return fail(ctx, ZWZ_E_ARG, "range past the end of the stream");
+        total += len[i];
+    }
+    zwz_rt::set_device(ctx->device);
+    int rc;
+    if ((rc = reserve(ctx, ctx->bulk_in, (size_t) comp_len + 64, false)) || (rc = reserve(ctx, ctx->bulk_out, (size_t) total + 64, false))) return rc;
+    if (zwz_rt::memcpy_h2d(ctx->bulk_in.p, comp, (size_t) comp_len, ctx->stream)) return fail(ctx, ZWZ_E_CUDA, "compressed upload failed");
+    if ((rc = zwz_index_extract_device(ctx, ix, (const uint8_t *) ctx->bulk_in.p, comp_len, n, off, len, (uint8_t *) ctx->bulk_out.p, packed.data(), got,
+                                       status, flags, nullptr)))
+        return rc;
+    std::vector<uint8_t> h(total);
+    if (total && (zwz_rt::memcpy_d2h(h.data(), ctx->bulk_out.p, total, ctx->stream) || zwz_rt::stream_sync(ctx->stream)))
+        return fail(ctx, ZWZ_E_CUDA, "range download failed");
+    for (uint32_t i = 0; i < n; ++i) memcpy(out + out_off[i], h.data() + packed[i], got[i]);
+    return ZWZ_OK;
 }
 
 } // extern "C"
