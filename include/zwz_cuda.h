@@ -167,16 +167,36 @@ int zwz_inflate_batch(zwz_ctx *ctx, const uint8_t *comp, const uint64_t *off, co
  *   Bytes and status are zlib's otherwise (ZWZ_STREAM_END / TRUNCATED / BAD, bytes before an error included); NO_ADLER skips
  *   CRC-32 / Adler-32 (ISIZE is still checked). Bytes of out past *raw_len may have been written.
  *   ZWZ_STREAM_OUTPUT_FULL: out_cap is smaller than what the stream decodes to (up to its end or first decoding error, check
- *   values aside); *raw_len is that size. Nothing is written when the stream fits one scratch wave (below); otherwise the waves
+ *   values and "too far back" aside); *raw_len is that size. It takes precedence over a check value or "too far back" error,
+ *   whatever the scratch waves (below), so the result does not depend on ZWZ_TUNE_STREAM_SCRATCH_BYTES. Nothing is written when the stream fits one scratch wave (below); otherwise the waves
  *   before the one that would pass out_cap have been written. (The batch calls instead fill up to the capacity.)
  *   NULL pointers and an unknown format are ZWZ_E_ARG.
- * Device scratch: u16 span slots (2 bytes per output byte) of one wave at a time, about ZWZ_TUNE_STREAM_SCRATCH_BYTES, plus 128 KiB
- * of window maps per span of the wave; allocated for the call and freed after it.
+ * Device scratch: u16 span slots (2 bytes per output byte) and 128 KiB of window maps for each span whose outgoing window a later
+ * span reads, of one wave at a time, about ZWZ_TUNE_STREAM_SCRATCH_BYTES; allocated for the call and freed after it.
  * Adversarial input with a false block start in every span costs one confirmation round per span; it still decodes exactly. */
 int zwz_inflate_stream_device(zwz_ctx *ctx, const uint8_t *d_comp, uint64_t comp_len, uint8_t *d_out, uint64_t out_cap,
                               uint64_t *raw_len, uint32_t *status, uint32_t flags, void *stream);
 int zwz_inflate_stream(zwz_ctx *ctx, const uint8_t *comp, uint64_t comp_len, uint8_t *out, uint64_t out_cap,
                        uint64_t *raw_len, uint32_t *status, uint32_t flags);
+
+/* zwz_inflate_stream_batch[_device]: many such streams (a set of .gz files, say) in one call, their spans sharing the GPU and
+ * their confirmation rounds sharing launches (DESIGN.md §4.10).
+ *   Stream i is comp[off[i] .. off[i] + len[i]) (ranges may overlap or repeat; they are only read) and decodes into
+ *   out[out_off[i] .. out_off[i + 1]). raw_len[i] and status[i] are exactly what zwz_inflate_stream returns for that stream alone
+ *   with out_cap = out_off[i + 1] - out_off[i] and the same flags, and so are the bytes up to raw_len[i]. One format per call, in
+ *   bits 8..15 of flags.
+ *   Nothing outside a stream's own region is written, whatever its status; an OUTPUT_FULL region's contents are unspecified. No
+ *   stream's result depends on the others: a bad stream leaves its neighbours alone, and no window reaches from one into the next.
+ *   ZWZ_E_ARG: NULL pointers with n > 0, an unknown format, len[i] > 0xffffff00, off[i] + len[i] past 2^64, a decreasing
+ *   out_off. n == 0 does nothing.
+ *   The host form uploads the extent [min off, max off + len) once and downloads every wave's output.
+ * Device scratch: that of zwz_inflate_stream for one wave of spans, which may hold spans of many streams; ZWZ_TUNE_STREAM_SCRATCH_BYTES
+ * counts slots and window maps. */
+int zwz_inflate_stream_batch_device(zwz_ctx *ctx, const uint8_t *d_comp, const uint64_t *off, const uint64_t *len, uint32_t n,
+                                    uint8_t *d_out, const uint64_t *out_off, uint64_t *raw_len, uint32_t *status,
+                                    uint32_t flags, void *stream);
+int zwz_inflate_stream_batch(zwz_ctx *ctx, const uint8_t *comp, const uint64_t *off, const uint64_t *len, uint32_t n,
+                             uint8_t *out, const uint64_t *out_off, uint64_t *raw_len, uint32_t *status, uint32_t flags);
 
 /* ---- random access into one long stream: a seek index (zlib's zran.c idea) -------------------------------------------------
  * zwz_inflate_stream_index[_device] inflate exactly as zwz_inflate_stream[_device] (same output, *raw_len and *status for the same
@@ -327,7 +347,8 @@ int zwz_decompress_records(zwz_ctx *ctx, const uint8_t *comp, const uint64_t *of
 /* ZWZ_TUNE_STREAM_SPAN_BYTES: compressed bytes per span of zwz_inflate_stream* (>= 1024; 0 = default: max(64 KiB, enough for two
  * spans per resident decoder warp)). */
 #define ZWZ_TUNE_STREAM_SPAN_BYTES 4
-/* ZWZ_TUNE_STREAM_SCRATCH_BYTES: u16 span slots of one wave of zwz_inflate_stream* (0 = default, 4 GiB). Larger streams are decoded
+/* ZWZ_TUNE_STREAM_SCRATCH_BYTES: u16 span slots and window maps (128 KiB for each span whose outgoing window a later span reads) of
+ * one wave of zwz_inflate_stream* (0 = default, 4 GiB). Larger streams are decoded
  * in waves of consecutive spans that hand on the resolved window and the running check value; a single span larger than the budget
  * still forms a wave of its own. */
 #define ZWZ_TUNE_STREAM_SCRATCH_BYTES 5

@@ -157,6 +157,8 @@ def _declare(L):
     L.zwz_inflate_batch_dict.argtypes = [vp, vp, vp, vp, u32, vp, vp, vp, vp, u32, dp]
     L.zwz_inflate_stream_device.argtypes = [vp, vp, u64, vp, u64, vp, vp, u32, vp]
     L.zwz_inflate_stream.argtypes = [vp, vp, u64, vp, u64, vp, vp, u32]
+    L.zwz_inflate_stream_batch_device.argtypes = [vp, vp, vp, vp, u32, vp, vp, vp, vp, u32, vp]
+    L.zwz_inflate_stream_batch.argtypes = [vp, vp, vp, vp, u32, vp, vp, vp, vp, u32]
     L.zwz_inflate_stream_index_device.argtypes = [vp, vp, u64, vp, u64, vp, vp, u32, u64, C.POINTER(vp), vp]
     L.zwz_inflate_stream_index.argtypes = [vp, vp, u64, vp, u64, vp, vp, u32, u64, C.POINTER(vp)]
     L.zwz_index_free.argtypes = [vp]
@@ -483,6 +485,68 @@ class Context:
         self._check(self.lib.zwz_inflate_stream_device(self.h, d_comp, comp_len, d_out, out_cap, rl.ctypes.data, st.ctypes.data,
                                                        flags | (_format(format) << 8), stream or None))
         return int(rl[0]), int(st[0])
+
+    def inflate_stream_batch(self, comp, off, length, format: str = "gzip", out_caps=None, flags: int = 0):
+        """Host buffer holding n streams, stream i = comp[off[i] .. off[i] + length[i]), each decoded as inflate_stream would decode
+        it alone, all in one call on the whole GPU. Returns (out uint8 array, out_off[n+1] u64, status[n]) packed like gunzip_files:
+        stream i's bytes are out[out_off[i] .. out_off[i+1]). Without out_caps each stream starts with the capacity inflate_stream
+        would guess, and the streams that report STREAM_OUTPUT_FULL run once more, in one more call, with the size they need. With
+        out_caps a STREAM_OUTPUT_FULL stream has no bytes; self.last_needed[i] is the size stream i needs."""
+        comp = _u8(comp)
+        f = _format(format)
+        off = np.ascontiguousarray(off, dtype=np.uint64)
+        length = np.ascontiguousarray(length, dtype=np.uint64)
+        n = len(off)
+        if out_caps is None:
+            caps = 4 * length.astype(np.int64) + 1024
+            if f == FORMAT_GZIP:
+                for i in np.nonzero(length >= 4)[0]:
+                    e = int(off[i] + length[i])
+                    caps[i] = min(int.from_bytes(comp[e - 4:e].tobytes(), "little"), 1032 * int(length[i]) + 1024)
+        else:
+            caps = np.ascontiguousarray(out_caps, dtype=np.int64)
+        out, out_off, rl, st = self._inflate_stream_batch(comp, f, off, length, caps, flags)
+        redo = np.nonzero(st == STREAM_OUTPUT_FULL)[0] if out_caps is None else np.zeros(0, dtype=np.int64)
+        if redo.size:
+            out2, off2, rl2, st2 = self._inflate_stream_batch(comp, f, off[redo], length[redo], rl[redo].astype(np.int64), flags)
+            rl[redo], st[redo] = rl2, st2
+        self.last_needed = rl.copy()
+        got = np.where(st == STREAM_OUTPUT_FULL, 0, rl).astype(np.uint64)
+        res_off = np.zeros(n + 1, dtype=np.uint64)
+        np.cumsum(got, out=res_off[1:])
+        res = np.empty(int(res_off[n]), dtype=np.uint8)
+        where = {int(i): k for k, i in enumerate(redo)}
+        for i in range(n):
+            if not got[i]:
+                continue
+            src, so = (out2, off2[where[i]]) if i in where else (out, out_off[i])
+            res[int(res_off[i]):int(res_off[i + 1])] = src[int(so):int(so) + int(got[i])]
+        return res, res_off, st
+
+    def _inflate_stream_batch(self, comp, f: int, off, length, caps, flags: int):
+        n = len(off)
+        out_off = np.zeros(n + 1, dtype=np.uint64)
+        np.cumsum(np.asarray(caps, dtype=np.uint64), out=out_off[1:])
+        out = np.empty(max(int(out_off[n]), 1), dtype=np.uint8)
+        rl = np.zeros(max(n, 1), dtype=np.uint64)
+        st = np.zeros(max(n, 1), dtype=np.uint32)
+        keep = comp if comp.size else np.zeros(1, dtype=np.uint8)
+        self._check(self.lib.zwz_inflate_stream_batch(self.h, keep.ctypes.data, off.ctypes.data, length.ctypes.data, n, out.ctypes.data,
+                                                      out_off.ctypes.data, rl.ctypes.data, st.ctypes.data, flags | (f << 8)))
+        return out, out_off, rl[:n], st[:n]
+
+    def inflate_stream_batch_device(self, d_comp: int, off, length, d_out: int, out_off, format: str = "gzip", flags: int = 0, stream: int = 0):
+        """Device buffers: stream i = d_comp[off[i] .. off[i] + length[i]) decodes into d_out[out_off[i] .. out_off[i+1]).
+        Returns (raw_len[n] u64, status[n]); with STREAM_OUTPUT_FULL raw_len[i] is the size stream i needs."""
+        off = np.ascontiguousarray(off, dtype=np.uint64)
+        length = np.ascontiguousarray(length, dtype=np.uint64)
+        out_off = np.ascontiguousarray(out_off, dtype=np.uint64)
+        n = len(off)
+        rl = np.zeros(max(n, 1), dtype=np.uint64)
+        st = np.zeros(max(n, 1), dtype=np.uint32)
+        self._check(self.lib.zwz_inflate_stream_batch_device(self.h, d_comp, off.ctypes.data, length.ctypes.data, n, d_out, out_off.ctypes.data,
+                                                             rl.ctypes.data, st.ctypes.data, flags | (_format(format) << 8), stream or None))
+        return rl[:n], st[:n]
 
     # ---- random access into one long stream: a seek index ----
     def inflate_stream_index(self, comp, format: str = "gzip", spacing: int = 1 << 20, want_output: bool = True, out_cap: Optional[int] = None,

@@ -15,11 +15,16 @@
 //   win_scan_kernel      window index, or ZWZ_SPAN_INVALID for what lies before the stream or before a member start). Composing
 //                        maps is a gather and associative: an inclusive scan over the spans (log2 N launches, double
 //                        buffered, no CTA waits for another) gives every span its resolved incoming window;
-//   stream_gather_kernel out[base + i] = v < 256 ? v : window[v - 256]; the first position whose value resolves to INVALID is
+//   stream_gather_kernel out[dst + i] = v < 256 ? v : window[v - 256]; the first position whose value resolves to INVALID is
 //                        where zlib stops with "invalid distance too far back".
 //
+// One call may inflate many streams (zwz_inflate_stream_batch*): every job carries the byte base and length of its stream, and
+// decodes exactly as it would in a call of its own. The first span of a stream starts at its header with an empty window, so its
+// window map holds no window reference and the scan needs no segment flags between streams (DESIGN.md §4.10).
+//
 // The host (zwz_cuda.cu) confirms the spans: span 0 starts at the stream's first byte, span j is confirmed when the confirmed span
-// j - 1 stopped exactly at its start; a span behind a false candidate is decoded again from where its predecessor stopped.
+// j - 1 of the same stream stopped exactly at its start; a span behind a false candidate is decoded again from where its
+// predecessor stopped.
 #pragma once
 #include "inflate.cuh"
 
@@ -49,7 +54,9 @@ struct SpanJob {
     uint64_t target;  // stop at the first block whose key64 >> 1 is >= target >> 1; ~0 = run to the end of the stream
     uint16_t *slot;
     uint64_t cap;     // slot elements; the decoder counts past it
-    uint32_t mode, pad;
+    uint64_t cbase;   // the stream's first byte in the compressed buffer; positions above are relative to it
+    uint32_t mode;
+    uint32_t clen;    // the stream's compressed bytes
 };
 struct SpanRes {
     uint64_t stop;    // SPAN_STOPPED: key64 it stopped at; SPAN_STOP_MEMBER: byte position << 4 of the next member header
@@ -73,7 +80,7 @@ ZWZ_DEV uint32_t span_src(const uint16_t *slot, uint64_t cap, int64_t s) {
 }
 
 // One warp decodes one span (the careful, warp-uniform decoder of inflate_stream, writing u16 elements).
-ZWZ_DEV void span_decode(InflateWarpSmem &S, const uint8_t *__restrict__ comp, uint64_t comp_len, const SpanJob &J, uint32_t format, uint32_t flags,
+ZWZ_DEV void span_decode(InflateWarpSmem &S, const uint8_t *__restrict__ comp_all, const SpanJob &J, uint32_t format, uint32_t flags,
                          SpanRes &R, SpanMember *mem) {
     const unsigned lane = lane_id();
     uint16_t *slot = J.slot;
@@ -81,8 +88,8 @@ ZWZ_DEV void span_decode(InflateWarpSmem &S, const uint8_t *__restrict__ comp, u
     const bool at_header = J.mode == SPAN_MODE_FIRST || J.mode == SPAN_MODE_MEMBER;
     const uint64_t bit0 = at_header ? (J.start >> 4) * 8u : J.start >> 1;
     const uint64_t byte0 = bit0 >> 3;
-    const uint32_t clen = (uint32_t) (comp_len - byte0); // bytes from byte0 on
-    const uint8_t *c = comp + byte0;
+    const uint32_t clen = (uint32_t) (J.clen - byte0); // bytes from byte0 on
+    const uint8_t *c = comp_all + J.cbase + byte0;
     InfBits B;
     infb_open(B, c, clen);
     infb_seek_bits(B, bit0 - byte0 * 8u);
@@ -273,9 +280,9 @@ done:
 }
 
 // Persistent warps over the span jobs of one round (spans differ in output length by orders of magnitude).
-ZWZ_KERNEL __launch_bounds__(ZWZ_INF_WARPS * 32, ZWZ_INF_MIN_CTAS) inflate_span_kernel(const uint8_t *__restrict__ comp, uint64_t comp_len,
-                                                                                     const SpanJob *__restrict__ jobs, SpanRes *res, SpanMember *mem,
-                                                                                     uint32_t n, uint32_t flags, uint32_t *work_counter) {
+ZWZ_KERNEL __launch_bounds__(ZWZ_INF_WARPS * 32, ZWZ_INF_MIN_CTAS) inflate_span_kernel(const uint8_t *__restrict__ comp, const SpanJob *__restrict__ jobs,
+                                                                                     SpanRes *res, SpanMember *mem, uint32_t n, uint32_t flags,
+                                                                                     uint32_t *work_counter) {
     ZWZ_DYN_SMEM(inf_raw);
     InflateWarpSmem *smem = (InflateWarpSmem *) inf_raw;
     const uint32_t format = (flags >> 8) & 0xffu;
@@ -285,7 +292,7 @@ ZWZ_KERNEL __launch_bounds__(ZWZ_INF_WARPS * 32, ZWZ_INF_MIN_CTAS) inflate_span_
         j = __shfl_sync(ZWZ_FULL, j, 0);
         if (j >= n) break;
         const SpanJob J = jobs[j];
-        span_decode(smem[warp_id()], comp, comp_len, J, format, flags, res[j], mem + (size_t) j * ZWZ_SPAN_MAXM);
+        span_decode(smem[warp_id()], comp, J, format, flags, res[j], mem + (size_t) j * ZWZ_SPAN_MAXM);
     }
 }
 
@@ -308,16 +315,26 @@ ZWZ_DEV uint64_t bf_peek64(const uint8_t *comp, uint64_t comp_len, uint64_t p) {
     return s ? (lo >> s) | ((uint64_t) w[2] << (64u - s)) : lo;
 }
 
-// One warp per span j = 1 .. n: cand[j - 1] = key64 of the first block header candidate inside bytes [j * S, (j + 1) * S), or ~0.
+// span j >= 1 of the stream comp[base .. base + len)
+struct FindJob {
+    uint64_t base;
+    uint32_t len, span;
+};
+
+// One warp per job: cand[job] = key64 (relative to its stream) of the first block header candidate inside bytes [j * S, (j + 1) * S)
+// of its stream, or ~0. Nothing past the stream's end is read, so a candidate is a header the decoder accepts there too.
 // 32 bit offsets per step, one per lane: the cheap tests (BTYPE, HLIT / HDIST, the precode's Kraft sum; a stored block's
 // LEN == ~NLEN) run on every lane, the few survivors get the full table check by the whole warp, in bit order.
-ZWZ_KERNEL __launch_bounds__(32) block_find_kernel(const uint8_t *__restrict__ comp, uint64_t comp_len, uint64_t span_bytes, uint64_t *cand,
-                                                   uint32_t n) {
+ZWZ_KERNEL __launch_bounds__(32) block_find_kernel(const uint8_t *__restrict__ comp_all, const FindJob *__restrict__ jobs, uint64_t span_bytes,
+                                                   uint64_t *cand, uint32_t n) {
     ZWZ_DYN_SMEM(inf_raw);
     InflateWarpSmem &S = *(InflateWarpSmem *) inf_raw;
     const unsigned lane = lane_id();
-    const uint32_t j = blockIdx.x + 1u;
-    if (j > n) return;
+    if (blockIdx.x >= n) return;
+    const FindJob fj = jobs[blockIdx.x];
+    const uint8_t *comp = comp_all + fj.base;
+    const uint64_t comp_len = fj.len;
+    const uint32_t j = fj.span;
     const uint64_t lo = (uint64_t) j * span_bytes * 8u;
     const uint64_t hi_byte = (uint64_t) (j + 1u) * span_bytes;
     const uint64_t hi = (hi_byte < comp_len ? hi_byte : comp_len) * 8u;
@@ -360,12 +377,12 @@ ZWZ_KERNEL __launch_bounds__(32) block_find_kernel(const uint8_t *__restrict__ c
             }
             if (ok) {
                 const uint32_t bfinal = __shfl_sync(ZWZ_FULL, (uint32_t) v & 1u, l);
-                if (lane == 0) cand[j - 1u] = (pp << 1) | bfinal | (is_sto ? ZWZ_SPAN_CAND_STORED : 0ull);
+                if (lane == 0) cand[blockIdx.x] = (pp << 1) | bfinal | (is_sto ? ZWZ_SPAN_CAND_STORED : 0ull);
                 return;
             }
         }
     }
-    if (lane == 0) cand[j - 1u] = ~(uint64_t) 0;
+    if (lane == 0) cand[blockIdx.x] = ~(uint64_t) 0;
 }
 
 // ---- window resolution and gather ----
@@ -373,11 +390,15 @@ struct SpanWin {
     const uint16_t *slot;
     uint64_t nout;
     uint64_t reset; // ~0: no member starts inside the span
-    uint64_t base;  // output position of its first element
+    uint64_t base;  // output position of its first element in its stream's part of the wave
+    uint64_t dst;   // where that element goes in the gather's output
+    const uint16_t *win; // the resolved window in front of the span (nullptr: none, the span starts its stream)
+    uint32_t sid, pad;   // the stream's index in the wave (its first_bad entry)
 };
 
-// map[i][k] (i < m): what the k-th byte of the window behind span i is, in terms of the window in front of it
-// win_in: the resolved window in front of span 0 (the previous wave's last), nullptr = nothing comes before it
+// map[i][k] (i < m): what the k-th byte of the window behind span sp[i] is, in terms of the window in front of it (sp: the spans of
+// the wave whose outgoing window a later span reads, in order)
+// win_in: the resolved window in front of sp[0] when it goes on from the previous wave, nullptr = nothing comes before it
 ZWZ_KERNEL win_map_kernel(const SpanWin *__restrict__ sp, const uint16_t *__restrict__ win_in, uint16_t *map, uint32_t m) {
     const uint64_t t = (uint64_t) blockIdx.x * blockDim.x + threadIdx.x;
     const uint32_t i = (uint32_t) (t >> 15), k = (uint32_t) (t & (ZWZ_SPAN_WIN - 1u));
@@ -403,10 +424,8 @@ ZWZ_KERNEL win_scan_kernel(const uint16_t *__restrict__ cur, uint16_t *nxt, uint
 }
 
 #define ZWZ_GATHER_TILE 65536u
-// one CTA per tile of ZWZ_GATHER_TILE elements of one span; win = the resolved windows (window behind span i at i << 15)
-ZWZ_KERNEL stream_gather_kernel(const SpanWin *__restrict__ sp, const uint64_t *__restrict__ tiles, const uint16_t *__restrict__ win,
-                                const uint16_t *__restrict__ win_in, uint8_t *out,
-                                unsigned long long *first_bad) {
+// one CTA per tile of ZWZ_GATHER_TILE elements of one span; first_bad: one entry per stream of the wave
+ZWZ_KERNEL stream_gather_kernel(const SpanWin *__restrict__ sp, const uint64_t *__restrict__ tiles, uint8_t *out, unsigned long long *first_bad) {
     const uint64_t tl = tiles[blockIdx.x];
     const uint32_t i = (uint32_t) (tl >> 40);
     const uint64_t e0 = tl & ((1ull << 40) - 1u);
@@ -414,9 +433,9 @@ ZWZ_KERNEL stream_gather_kernel(const SpanWin *__restrict__ sp, const uint64_t *
     const uint64_t e1 = e0 + ZWZ_GATHER_TILE < s.nout ? e0 + ZWZ_GATHER_TILE : s.nout;
     for (uint64_t e = e0 + threadIdx.x; e < e1; e += blockDim.x) {
         uint32_t v = s.slot[e];
-        if (v >= 256u && v != ZWZ_SPAN_INVALID) v = i ? win[((uint64_t) (i - 1u) << 15) | (v - 256u)] : (win_in ? win_in[v - 256u] : ZWZ_SPAN_INVALID);
-        if (v == ZWZ_SPAN_INVALID) atomicMin(first_bad, (unsigned long long) (s.base + e));
-        else out[s.base + e] = (uint8_t) v;
+        if (v >= 256u && v != ZWZ_SPAN_INVALID) v = s.win ? s.win[v - 256u] : ZWZ_SPAN_INVALID;
+        if (v == ZWZ_SPAN_INVALID) atomicMin(first_bad + s.sid, (unsigned long long) (s.base + e));
+        else out[s.dst + e] = (uint8_t) v;
     }
 }
 

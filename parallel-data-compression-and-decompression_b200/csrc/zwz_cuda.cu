@@ -1904,6 +1904,7 @@ struct StreamBufs {
 struct SpanEnt {
     uint64_t start;     // SpanJob::start
     uint32_t mode;
+    uint32_t sid = 0;   // the stream it belongs to
     bool decoded = false;
     zwz::SpanRes r{};
     std::vector<zwz::SpanMember> mem;
@@ -1923,24 +1924,49 @@ static uint64_t span_estimate(uint64_t start, uint64_t target, uint64_t comp_len
     const uint64_t b0 = (start >> 1) >> 3, b1 = target == ~(uint64_t) 0 ? comp_len : std::min<uint64_t>(comp_len, (target >> 1) >> 3);
     return (b1 > b0 ? b1 - b0 : 0) * 4u + 4096u;
 }
+// a span's window map, double-buffered for the scan: scratch of every span whose outgoing window a later span reads
+static const uint64_t kSpanMapBytes = 2u * 2u * ZWZ_SPAN_WIN;
 
-// Decode the entries `todo` of L in one launch, each up to the start of its successor (the last one of L up to `tail`); `exact`:
-// slots of exactly the size the previous decode of the entry reported.
-static int span_decode_round(zwz_ctx *ctx, zwz_stream_t st, StreamBufs &bufs, const uint8_t *d_comp, uint64_t comp_len, uint32_t flags,
-                             std::vector<SpanEnt> &L, uint64_t tail, const std::vector<size_t> &todo, bool exact) {
+// one stream of an inflate_stream_impl call: where it is, and where its decoding stands
+struct StreamCall {
+    uint64_t off, len;              // its compressed bytes: d_comp[off .. off + len)
+    uint64_t out_off, cap;          // its output region
+    uint32_t open_val = 0;          // check value of the open member so far
+    uint64_t open_start = 0;        // where it started
+    uint64_t base = 0, outlen = 0;  // output position of its next wave; bytes valid in the end
+    uint32_t stat = ZWZ_STREAM_END;
+    bool full = false;
+    // an error was found before the stream's end: its status and length are fixed, and its remaining spans are decoded for their
+    // size only, so that OUTPUT_FULL is decided from the whole size wherever the waves split the stream
+    bool bad = false;
+};
+// the stream whose spans go on past the wave (sid ~0: none) and the start of its next candidate
+struct SpanTail {
+    uint32_t sid;
+    uint64_t start;
+};
+
+// Decode the entries `todo` of L in one launch, each up to the start of its successor in the same stream (a stream's last entry in
+// L up to tail.start when it is tail's stream, else to its end); `exact`: slots of exactly the size the previous decode of the
+// entry reported.
+static int span_decode_round(zwz_ctx *ctx, zwz_stream_t st, StreamBufs &bufs, const uint8_t *d_comp, const std::vector<StreamCall> &S, uint32_t flags,
+                             std::vector<SpanEnt> &L, SpanTail tail, const std::vector<size_t> &todo, bool exact) {
     const size_t n = todo.size();
     if (!n) return ZWZ_OK;
     std::vector<zwz::SpanJob> jobs(n);
     size_t elems = 0;
     for (size_t k = 0; k < n; ++k) {
         SpanEnt &e = L[todo[k]];
-        const uint64_t target = todo[k] + 1 < L.size() ? L[todo[k] + 1].start : tail;
-        const uint64_t cap = exact ? e.r.nout : span_estimate(e.start, target, comp_len);
+        const StreamCall &sc = S[e.sid];
+        const size_t i = todo[k];
+        const uint64_t target = i + 1 < L.size() && L[i + 1].sid == e.sid ? L[i + 1].start : (tail.sid == e.sid ? tail.start : ~(uint64_t) 0);
+        const uint64_t cap = exact ? e.r.nout : span_estimate(e.start, target, sc.len);
         jobs[k].start = e.start;
         jobs[k].target = target;
         jobs[k].cap = cap;
+        jobs[k].cbase = sc.off;
         jobs[k].mode = e.mode;
-        jobs[k].pad = 0;
+        jobs[k].clen = (uint32_t) sc.len;
         elems += align_up(cap, 64);
     }
     uint16_t *slab = (uint16_t *) bufs.get(elems * 2);
@@ -1959,7 +1985,7 @@ static int span_decode_round(zwz_ctx *ctx, zwz_stream_t st, StreamBufs &bufs, co
     {
         ProfSpan ps(ctx, ZWZ_PROF_INFLATE, st);
         const uint32_t grid = (uint32_t) std::min<size_t>(n, (size_t) ctx->sm_count * ctx->span_blocks_per_sm);
-        ZWZ_LAUNCH(zwz::inflate_span_kernel, grid, ZWZ_INF_WARPS * 32, ZWZ_INF_SMEM, st, d_comp, comp_len, (const zwz::SpanJob *) d_jobs, d_res, d_mem,
+        ZWZ_LAUNCH(zwz::inflate_span_kernel, grid, ZWZ_INF_WARPS * 32, ZWZ_INF_SMEM, st, d_comp, (const zwz::SpanJob *) d_jobs, d_res, d_mem,
                    (uint32_t) n, flags, d_counter);
     }
     int rc;
@@ -1982,13 +2008,13 @@ static int span_decode_round(zwz_ctx *ctx, zwz_stream_t st, StreamBufs &bufs, co
 }
 
 // the slots that overflowed, decoded again with their exact size
-static int span_decode_exact(zwz_ctx *ctx, zwz_stream_t st, StreamBufs &bufs, const uint8_t *d_comp, uint64_t comp_len, uint32_t flags,
-                             std::vector<SpanEnt> &L, uint64_t tail, const std::vector<size_t> &todo) {
+static int span_decode_exact(zwz_ctx *ctx, zwz_stream_t st, StreamBufs &bufs, const uint8_t *d_comp, const std::vector<StreamCall> &S, uint32_t flags,
+                             std::vector<SpanEnt> &L, SpanTail tail, const std::vector<size_t> &todo) {
     std::vector<size_t> over;
     for (size_t i : todo)
         if (L[i].r.nout > L[i].cap) over.push_back(i);
     ZWZ_STREAM_STAT(3, over.size());
-    return span_decode_round(ctx, st, bufs, d_comp, comp_len, flags, L, tail, over, true);
+    return span_decode_round(ctx, st, bufs, d_comp, S, flags, L, tail, over, true);
 }
 
 // ---- seek index (zwz_inflate_stream_index*): access points chosen from the confirmed span starts ----
@@ -2004,10 +2030,10 @@ struct IndexBuild {
 
 // The access points among the confirmed spans of one wave (W, output positions base + sw[i].base): span 0 of the stream, then
 // greedily the first span start at least `spacing` (at least 1) bytes of output past the previous point. A point's window is the
-// resolved window in front of its span: win_in for the wave's first span, w0 + ((i - 1) << 15) for span i. A wave with no output
-// has its windows unresolved; only its first span can be a point there.
+// resolved window in front of its span, sw[i].win. A wave with no output has its windows unresolved; only its first span can be a
+// point there.
 static int index_points(zwz_ctx *ctx, zwz_stream_t st, StreamBufs &wb, IndexBuild &ib, const std::vector<SpanEnt> &W, const std::vector<zwz::SpanWin> &sw,
-                        uint64_t base, uint64_t total, const uint16_t *win_in, const uint16_t *w0) {
+                        uint64_t base, uint64_t total) {
     std::vector<const uint16_t *> src;
     std::vector<size_t> at;
     const size_t ns = total ? W.size() : 1;
@@ -2021,7 +2047,7 @@ static int index_points(zwz_ctx *ctx, zwz_stream_t st, StreamBufs &wb, IndexBuil
             p.bit = e.start >> 1;
             p.bfinal = (uint32_t) (e.start & 1u);
         }
-        const uint16_t *w = i ? w0 + ((size_t) (i - 1) << 15) : win_in;
+        const uint16_t *w = sw[i].win;
         if (w && e.mode != zwz::SPAN_MODE_MEMBER && e.mode != zwz::SPAN_MODE_FIRST) { // a member starts with an empty window
             src.push_back(w);
             at.push_back(ib.pts.size());
@@ -2053,281 +2079,387 @@ static int index_points(zwz_ctx *ctx, zwz_stream_t st, StreamBufs &wb, IndexBuil
     return ZWZ_OK;
 }
 
-// Waves: the spans are decoded, confirmed, resolved and gathered in order, a wave at a time, so that the u16 slots of one wave stay
-// near the scratch budget (ZWZ_TUNE_STREAM_SCRATCH_BYTES). A wave hands the next one the resolved window behind its last span, the
-// position where that span stopped and the running check value of the member still open. d_out == NULL: every wave is gathered into
-// grow_out, and downloaded to h_out when there is one. ib: the access points of a seek index are collected wave by wave.
-static int inflate_stream_impl(zwz_ctx *ctx, const uint8_t *d_comp, uint64_t comp_len, uint8_t *d_out, uint8_t *h_out, uint64_t out_cap,
-                               Arena *grow_out, uint64_t *raw_len, uint32_t *status, uint32_t flags, zwz_stream_t st, IndexBuild *ib = nullptr) {
+// Inflate the streams S (n >= 1) with one set of launches: the spans of all streams share the decoder warps and the confirmation
+// rounds. Waves: the spans are decoded, confirmed, resolved and gathered in stream order, a wave at a time, so that the u16 slots and
+// window maps of one wave stay near the scratch budget (ZWZ_TUNE_STREAM_SCRATCH_BYTES). Only the stream that straddles a wave's end
+// goes on in the next wave, which gets the resolved window behind its last span, the position where that span stopped and the
+// running check value of its open member; every other stream of the wave ends in it. d_out == NULL: every wave is gathered into
+// grow_out, and downloaded to h_out when there is one. ib (one stream): the access points of a seek index are collected wave by wave.
+static int inflate_stream_impl(zwz_ctx *ctx, const uint8_t *d_comp, std::vector<StreamCall> &S, uint8_t *d_out, uint8_t *h_out, Arena *grow_out,
+                               uint32_t flags, zwz_stream_t st, IndexBuild *ib = nullptr) {
     const uint32_t format = (flags >> 8) & 0xffu;
+    const uint32_t n = (uint32_t) S.size();
     Trace tr(ctx, "inflate_stream", st);
     int rc;
     // ---- spans and their candidate starts ----
+    uint64_t comp_total = 0;
+    for (const StreamCall &s : S) comp_total += s.len;
     const uint64_t warps = (uint64_t) ctx->sm_count * ctx->span_blocks_per_sm * ZWZ_INF_WARPS;
-    const uint64_t S = ctx->stream_span_bytes ? ctx->stream_span_bytes : std::max<uint64_t>(65536u, (comp_len + 2 * warps - 1) / (2 * warps));
-    const uint64_t nspan = std::max<uint64_t>(1u, (comp_len + S - 1) / S);
+    const uint64_t SB = ctx->stream_span_bytes ? ctx->stream_span_bytes : std::max<uint64_t>(65536u, (comp_total + 2 * warps - 1) / (2 * warps));
     const uint64_t budget = ctx->stream_scratch_bytes ? ctx->stream_scratch_bytes : ((uint64_t) 4 << 30);
-    std::deque<SpanEnt> Q; // candidate starts not decoded yet, in stream order
-    if (nspan > 1) {
+    std::vector<zwz::FindJob> fj; // span j >= 1 of every stream
+    for (uint32_t s = 0; s < n; ++s)
+        for (uint64_t j = 1; j * SB < S[s].len; ++j) fj.push_back(zwz::FindJob{S[s].off, (uint32_t) S[s].len, (uint32_t) j});
+    std::vector<uint64_t> cand(fj.size());
+    if (!fj.empty()) {
         StreamBufs fb(st);
-        uint64_t *d_cand = (uint64_t *) fb.get((nspan - 1) * 8);
-        if (!d_cand) return fail(ctx, ZWZ_E_NOMEM, "stream scratch allocation failed");
+        uint8_t *dm = (uint8_t *) fb.get(fj.size() * (sizeof(zwz::FindJob) + 8));
+        if (!dm) return fail(ctx, ZWZ_E_NOMEM, "stream scratch allocation failed");
+        uint64_t *d_cand = (uint64_t *) (dm + fj.size() * sizeof(zwz::FindJob));
+        if (zwz_rt::memcpy_h2d(dm, fj.data(), fj.size() * sizeof(zwz::FindJob), st)) return fail(ctx, ZWZ_E_CUDA, "span upload failed");
         {
             ProfSpan ps(ctx, ZWZ_PROF_INFLATE, st);
-            ZWZ_LAUNCH(zwz::block_find_kernel, (uint32_t) (nspan - 1), 32, ZWZ_INF_SMEM, st, d_comp, comp_len, S, d_cand, (uint32_t) (nspan - 1));
+            ZWZ_LAUNCH(zwz::block_find_kernel, (uint32_t) fj.size(), 32, ZWZ_INF_SMEM, st, d_comp, (const zwz::FindJob *) dm, SB, d_cand, (uint32_t) fj.size());
         }
         if ((rc = check_launch(ctx, "block_find_kernel"))) return rc;
-        std::vector<uint64_t> cand(nspan - 1);
         if (zwz_rt::memcpy_d2h(cand.data(), d_cand, cand.size() * 8, st) || zwz_rt::stream_sync(st)) return fail(ctx, ZWZ_E_CUDA, "block_find_kernel failed");
-        for (uint64_t c : cand)
-            if (c != ~(uint64_t) 0)
-                Q.push_back(SpanEnt{c & ~ZWZ_SPAN_CAND_STORED, (c & ZWZ_SPAN_CAND_STORED) ? (uint32_t) zwz::SPAN_MODE_STORED : (uint32_t) zwz::SPAN_MODE_BLOCK});
-        ZWZ_STREAM_STAT(4, Q.size());
+    }
+    // spans not decoded yet, in stream order: each stream's start (span 0, or where its previous wave stopped), then its candidates
+    std::deque<SpanEnt> P;
+    {
+        size_t k = 0, ncand = 0;
+        for (uint32_t s = 0; s < n; ++s) {
+            P.push_back(SpanEnt{0, zwz::SPAN_MODE_FIRST, s});
+            for (uint64_t j = 1; j * SB < S[s].len; ++j) {
+                const uint64_t c = cand[k++];
+                if (c == ~(uint64_t) 0) continue;
+                P.push_back(SpanEnt{c & ~ZWZ_SPAN_CAND_STORED, (c & ZWZ_SPAN_CAND_STORED) ? (uint32_t) zwz::SPAN_MODE_STORED : (uint32_t) zwz::SPAN_MODE_BLOCK, s});
+                ncand++;
+            }
+        }
+        ZWZ_STREAM_STAT(4, ncand);
     }
     tr.mark("find");
-    SpanEnt cur{0, zwz::SPAN_MODE_FIRST};
     std::unique_ptr<StreamBufs> prevb; // keeps the window handed on by the previous wave alive
     const uint16_t *win_in = nullptr;
     const bool sums = format != ZWZ_FORMAT_RAW && !(flags & ZWZ_INFLATE_NO_ADLER);
     const uint32_t init = format == ZWZ_FORMAT_GZIP ? 0u : 1u;
-    uint32_t open_val = init;     // check value of the open member so far
-    uint64_t open_start = 0;      // where it started
-    uint64_t base = 0, len = 0;   // output position of the wave; bytes valid in the end
-    uint32_t stat = ZWZ_STREAM_END;
-    bool full = false;
+    for (StreamCall &s : S) s.open_val = init;
     size_t rounds = 0, reruns = 0, nspans = 0, waves = 0;
-    for (bool finished = false; !finished;) {
+    while (!P.empty()) {
         waves++;
         std::unique_ptr<StreamBufs> wb(new StreamBufs(st));
-        // ---- the wave: the spans from `cur` on whose estimated slots fit the budget (one at least) ----
-        while (!Q.empty() && (Q.front().start >> 1) <= (cur.start >> 1)) Q.pop_front();
-        std::vector<SpanEnt> W;
-        W.push_back(std::move(cur));
-        auto tail = [&]() { return Q.empty() ? ~(uint64_t) 0 : Q.front().start; };
-        {
-            uint64_t est = 2 * span_estimate(W[0].start, tail(), comp_len);
-            while (!Q.empty()) {
-                const uint64_t nxt = Q.size() > 1 ? Q[1].start : ~(uint64_t) 0;
-                const uint64_t e = 2 * span_estimate(Q.front().start, nxt, comp_len);
-                if (est + e > budget) break;
-                est += e;
-                W.push_back(std::move(Q.front()));
-                Q.pop_front();
-            }
+        // ---- the wave: the spans from the front of P whose estimated slots and maps fit the budget (one at least) ----
+        while (P.size() > 1 && P[1].sid == P[0].sid && (P[1].start >> 1) <= (P[0].start >> 1)) { // candidates behind the start
+            SpanEnt h = std::move(P[0]);
+            P.pop_front();
+            P.pop_front();
+            P.push_front(std::move(h));
         }
+        std::vector<SpanEnt> W;
+        {
+            uint64_t est = 0;
+            do {
+                const bool more = P.size() > 1 && P[1].sid == P[0].sid;
+                const uint64_t e = 2 * span_estimate(P[0].start, more ? P[1].start : ~(uint64_t) 0, S[P[0].sid].len) + (more ? kSpanMapBytes : 0);
+                if (!W.empty() && est + e > budget) break;
+                est += e;
+                W.push_back(std::move(P.front()));
+                P.pop_front();
+            } while (!P.empty());
+        }
+        auto tail = [&]() { return P.empty() ? SpanTail{~0u, ~(uint64_t) 0} : SpanTail{P.front().sid, P.front().start}; };
+        // spans whose outgoing window a later span of the same stream reads (in this wave or, from W's last span, in the next)
+        auto mapped = [&](size_t i) {
+            return i + 1 < W.size() ? W[i + 1].sid == W[i].sid : (!P.empty() && P.front().sid == W[i].sid);
+        };
         std::vector<size_t> all(W.size());
         for (size_t i = 0; i < all.size(); ++i) all[i] = i;
-        if ((rc = span_decode_round(ctx, st, *wb, d_comp, comp_len, flags, W, tail(), all, false))) return rc;
-        // the slots they really need: spans past the budget go back to the queue (one span stays, whatever it needs)
+        if ((rc = span_decode_round(ctx, st, *wb, d_comp, S, flags, W, tail(), all, false))) return rc;
+        // the slots they really need: spans past the budget go back to P (one span stays, whatever it needs)
         {
             size_t keep = 1;
-            uint64_t acc = 2 * W[0].r.nout;
-            while (keep < W.size() && acc + 2 * W[keep].r.nout <= budget) acc += 2 * W[keep++].r.nout;
-            for (size_t i = W.size(); i-- > keep;) Q.push_front(SpanEnt{W[i].start, W[i].mode});
+            uint64_t acc = 2 * W[0].r.nout + (mapped(0) ? kSpanMapBytes : 0);
+            for (; keep < W.size(); ++keep) {
+                const uint64_t e = 2 * W[keep].r.nout + (mapped(keep) ? kSpanMapBytes : 0);
+                if (acc + e > budget) break;
+                acc += e;
+            }
+            for (size_t i = W.size(); i-- > keep;) P.push_front(SpanEnt{W[i].start, W[i].mode, W[i].sid});
             W.resize(keep);
             all.resize(keep);
         }
-        if ((rc = span_decode_exact(ctx, st, *wb, d_comp, comp_len, flags, W, tail(), all))) return rc;
-        // ---- confirmation: W[0] is real; W[i + 1] is when W[i] (real) stopped exactly at its start. Every round decodes again each
-        // span whose decoded predecessor stopped elsewhere, from that stop; the confirmed prefix grows by one span at least. The
-        // last span's stop is where the next wave starts ----
-        size_t f = 0;
+        if ((rc = span_decode_exact(ctx, st, *wb, d_comp, S, flags, W, tail(), all))) return rc;
+        // ---- confirmation, per stream: its first span in W is real; the next is when the real one stopped exactly at its start.
+        // Every round decodes again, for all streams at once, each span whose decoded predecessor stopped elsewhere, from that
+        // stop; every stream's confirmed prefix grows by one span at least. A terminal span ends its stream's part of W. The last
+        // span of W's last stream stops where the next wave starts; any other stream's part runs to the stream's end ----
         for (;;) {
-            bool settled = false;
-            for (;;) {
-                const SpanEnt &e = W[f];
-                if (span_terminal(e)) {
-                    W.resize(f + 1);
-                    finished = settled = true;
-                    break;
-                }
-                if (f + 1 == W.size()) {
-                    settled = true;
-                    break;
-                }
-                if (W[f + 1].decoded && W[f + 1].start == e.r.stop && W[f + 1].mode == span_stop_mode(e)) {
-                    f++;
-                    continue;
-                }
-                break;
-            }
-            if (settled) break;
-            std::vector<SpanEnt> nl(W.begin(), W.begin() + (ptrdiff_t) f + 1);
-            for (size_t j = f + 1; j < W.size(); ++j) {
-                const SpanEnt &p = nl.back();
-                if (p.decoded && !span_terminal(p)) {
-                    const uint64_t b = p.r.stop;
-                    const uint32_t m = span_stop_mode(p);
-                    if ((W[j].start >> 1) < (b >> 1)) continue; // overrun by its predecessor
-                    if (W[j].start != b || W[j].mode != m) {
-                        nl.push_back(SpanEnt{b, m}); // decode from where the predecessor stopped
-                        reruns++;
-                        if ((W[j].start >> 1) == (b >> 1)) continue; // same position, other BFINAL / mode: replaced
+            bool settled = true;
+            std::vector<SpanEnt> nl;
+            nl.reserve(W.size());
+            for (size_t a = 0; a < W.size();) {
+                size_t b = a + 1;
+                while (b < W.size() && W[b].sid == W[a].sid) ++b;
+                size_t f = a;
+                while (!span_terminal(W[f]) && f + 1 < b && W[f + 1].decoded && W[f + 1].start == W[f].r.stop && W[f + 1].mode == span_stop_mode(W[f])) f++;
+                for (size_t j = a; j <= f; ++j) nl.push_back(std::move(W[j]));
+                const SpanEnt &e = nl.back();
+                if (span_terminal(e) || (f + 1 == b && b == W.size())) {
+                    // settled: candidates behind a terminal span (trailing garbage, say) are dropped
+                } else if (f + 1 == b) { // it stopped before its stream's end (a span records at most ZWZ_SPAN_MAXM members)
+                    nl.push_back(SpanEnt{e.r.stop, span_stop_mode(e), e.sid});
+                    reruns++;
+                    settled = false;
+                } else {
+                    settled = false;
+                    for (size_t j = f + 1; j < b; ++j) {
+                        const SpanEnt &p = nl.back();
+                        if (p.decoded && !span_terminal(p)) {
+                            const uint64_t bs = p.r.stop;
+                            const uint32_t m = span_stop_mode(p);
+                            if ((W[j].start >> 1) < (bs >> 1)) continue; // overrun by its predecessor
+                            if (W[j].start != bs || W[j].mode != m) {
+                                nl.push_back(SpanEnt{bs, m, p.sid}); // decode from where the predecessor stopped
+                                reruns++;
+                                if ((W[j].start >> 1) == (bs >> 1)) continue; // same position, other BFINAL / mode: replaced
+                            }
+                        }
+                        nl.push_back(std::move(W[j]));
                     }
                 }
-                nl.push_back(std::move(W[j]));
+                a = b;
             }
             W.swap(nl);
+            if (settled) break;
             std::vector<size_t> todo;
-            for (size_t i = f; i < W.size(); ++i)
+            for (size_t i = 0; i < W.size(); ++i)
                 if (!W[i].decoded) todo.push_back(i);
             rounds++;
-            if ((rc = span_decode_round(ctx, st, *wb, d_comp, comp_len, flags, W, tail(), todo, false)) ||
-                (rc = span_decode_exact(ctx, st, *wb, d_comp, comp_len, flags, W, tail(), todo)))
+            if ((rc = span_decode_round(ctx, st, *wb, d_comp, S, flags, W, tail(), todo, false)) ||
+                (rc = span_decode_exact(ctx, st, *wb, d_comp, S, flags, W, tail(), todo)))
                 return rc;
         }
         nspans += W.size();
-        if (!finished) cur = SpanEnt{W.back().r.stop, span_stop_mode(W.back())};
-        // ---- lengths and members of the wave ----
+        // ---- the streams of the wave: lengths, members, and where their bytes go ----
         const size_t ns = W.size();
-        std::vector<zwz::SpanWin> sw(ns);
         struct Member {
-            uint64_t end; // in the wave
+            uint64_t end; // in the stream's part of the wave
             zwz::SpanMember t;
         };
-        std::vector<Member> members;
-        uint64_t total = 0;
-        for (size_t i = 0; i < ns; ++i) {
-            sw[i].slot = W[i].slot;
-            sw[i].nout = W[i].r.nout;
-            sw[i].reset = W[i].r.reset;
-            sw[i].base = total;
-            for (const zwz::SpanMember &m : W[i].mem) members.push_back(Member{total + m.end, m});
-            total += W[i].r.nout;
+        struct Seg {
+            uint32_t sid;
+            size_t a, b;          // its spans W[a .. b)
+            uint64_t total, dst;  // output elements; where its first goes in the wave's output
+            bool fin, gather;     // its stream ends in the wave; its bytes are resolved (it fits its region)
+            std::vector<Member> members;
+        };
+        std::vector<Seg> G;
+        std::vector<zwz::SpanWin> sw(ns);
+        uint64_t wave_bytes = 0; // host form: the gathered streams packed back to back in grow_out
+        for (size_t a = 0; a < ns;) {
+            Seg g{W[a].sid, a, a + 1, 0, 0, false, false, {}};
+            while (g.b < ns && W[g.b].sid == g.sid) g.b++;
+            for (size_t i = a; i < g.b; ++i) {
+                sw[i] = zwz::SpanWin{W[i].slot, W[i].r.nout, W[i].r.reset, g.total, 0, nullptr, (uint32_t) G.size(), 0};
+                for (const zwz::SpanMember &m : W[i].mem) g.members.push_back(Member{g.total + m.end, m});
+                g.total += W[i].r.nout;
+            }
+            g.fin = span_terminal(W[g.b - 1]);
+            StreamCall &sc = S[g.sid];
+            if (!sc.full && sc.base + g.total > sc.cap) sc.full = true; // from here on only the size needed
+            g.gather = !sc.full && !sc.bad;
+            if (g.gather) {
+                g.dst = d_out ? sc.out_off + sc.base : wave_bytes;
+                wave_bytes += g.total;
+            }
+            a = g.b;
+            G.push_back(std::move(g));
         }
-        if (!full && base + total > out_cap) full = true;
-        if (full) { // only the size needed from here on
-            base += total;
-            continue;
-        }
-        uint8_t *wdst = d_out ? d_out + base : nullptr;
+        uint8_t *wdst = d_out;
         if (!wdst) {
-            if ((rc = reserve(ctx, *grow_out, total + 64, false))) return rc;
+            if ((rc = reserve(ctx, *grow_out, wave_bytes + 64, false))) return rc;
             wdst = (uint8_t *) grow_out->p;
         }
-        // ---- windows: map per span, inclusive scan of the compositions, then the gather ----
-        unsigned long long first_bad = ~0ull;
-        const uint32_t m = (uint32_t) (finished ? ns - 1 : ns); // spans whose outgoing window someone reads
+        // ---- windows: a map per span whose outgoing window is read, inclusive scan of the compositions, then the gather. A stream's
+        // first span in the wave reads win_in (the stream went on from the previous wave) or nothing (it starts its stream) ----
+        std::vector<size_t> mp;              // the spans with a map, in order
+        std::vector<uint32_t> mix(ns, ~0u);  // a span's map
+        for (const Seg &g : G) {
+            if (!g.gather) continue;
+            for (size_t i = g.a; i < g.b; ++i)
+                if (i + 1 < g.b || (i + 1 == ns && !g.fin)) {
+                    mix[i] = (uint32_t) mp.size();
+                    mp.push_back(i);
+                }
+        }
+        const uint32_t m = (uint32_t) mp.size();
         uint16_t *w0 = nullptr, *w1 = nullptr;
         if (m) {
             w0 = (uint16_t *) wb->get((size_t) m * ZWZ_SPAN_WIN * 2);
             w1 = (uint16_t *) wb->get((size_t) m * ZWZ_SPAN_WIN * 2);
+            if (!w0 || !w1) return fail(ctx, ZWZ_E_NOMEM, "stream scratch allocation failed");
         }
-        if (total) {
-            std::vector<uint64_t> tiles;
-            for (size_t i = 0; i < ns; ++i)
+        uint32_t steps = 0;
+        for (uint32_t d = 1; d < m; d <<= 1) steps++;
+        uint16_t *wres = (steps & 1u) ? w1 : w0; // where the scan leaves the resolved windows
+        for (const Seg &g : G)
+            for (size_t i = g.a; i < g.b; ++i) {
+                sw[i].dst = g.dst + sw[i].base;
+                sw[i].win = i > g.a ? wres + ((size_t) mix[i - 1] << 15) : (i == 0 ? win_in : nullptr);
+            }
+        std::vector<unsigned long long> first_bad(G.size(), ~0ull);
+        std::vector<uint64_t> tiles;
+        for (const Seg &g : G) {
+            if (!g.gather) continue;
+            for (size_t i = g.a; i < g.b; ++i)
                 for (uint64_t e = 0; e < sw[i].nout; e += ZWZ_GATHER_TILE) tiles.push_back(((uint64_t) i << 40) | e);
-            uint8_t *dm = (uint8_t *) wb->get(ns * sizeof(zwz::SpanWin) + tiles.size() * 8 + 64);
-            if ((m && (!w0 || !w1)) || !dm) return fail(ctx, ZWZ_E_NOMEM, "stream scratch allocation failed");
-            zwz::SpanWin *d_sw = (zwz::SpanWin *) dm;
-            uint64_t *d_tiles = (uint64_t *) (dm + ns * sizeof(zwz::SpanWin));
-            unsigned long long *d_bad = (unsigned long long *) (dm + ns * sizeof(zwz::SpanWin) + tiles.size() * 8);
-            if (zwz_rt::memcpy_h2d(d_sw, sw.data(), ns * sizeof(zwz::SpanWin), st) || zwz_rt::memcpy_h2d(d_tiles, tiles.data(), tiles.size() * 8, st) ||
-                zwz_rt::memcpy_h2d(d_bad, &first_bad, 8, st))
+        }
+        if (m || !tiles.empty()) {
+            std::vector<zwz::SpanWin> msw(m);
+            for (uint32_t k = 0; k < m; ++k) msw[k] = sw[mp[k]];
+            const size_t bad_at = (ns + m) * sizeof(zwz::SpanWin) + tiles.size() * 8;
+            uint8_t *dm = (uint8_t *) wb->get(bad_at + G.size() * 8 + 64);
+            if (!dm) return fail(ctx, ZWZ_E_NOMEM, "stream scratch allocation failed");
+            zwz::SpanWin *d_sw = (zwz::SpanWin *) dm, *d_msw = d_sw + ns;
+            uint64_t *d_tiles = (uint64_t *) (dm + (ns + m) * sizeof(zwz::SpanWin));
+            unsigned long long *d_bad = (unsigned long long *) (dm + bad_at);
+            if (zwz_rt::memcpy_h2d(d_sw, sw.data(), ns * sizeof(zwz::SpanWin), st) || zwz_rt::memcpy_h2d(d_msw, msw.data(), m * sizeof(zwz::SpanWin), st) ||
+                zwz_rt::memcpy_h2d(d_tiles, tiles.data(), tiles.size() * 8, st) || zwz_rt::memcpy_h2d(d_bad, first_bad.data(), G.size() * 8, st))
                 return fail(ctx, ZWZ_E_CUDA, "window upload failed");
             {
                 ProfSpan ps(ctx, ZWZ_PROF_PACK, st);
                 if (m) {
                     const uint32_t grid = m * (ZWZ_SPAN_WIN / 256u);
-                    ZWZ_LAUNCH(zwz::win_map_kernel, grid, 256, 0, st, (const zwz::SpanWin *) d_sw, win_in, w0, m);
+                    ZWZ_LAUNCH(zwz::win_map_kernel, grid, 256, 0, st, (const zwz::SpanWin *) d_msw, win_in, w0, m);
                     for (uint32_t d = 1; d < m; d <<= 1) {
                         ZWZ_LAUNCH(zwz::win_scan_kernel, grid, 256, 0, st, (const uint16_t *) w0, w1, m, d);
                         std::swap(w0, w1);
                     }
                 }
-                ZWZ_LAUNCH(zwz::stream_gather_kernel, (uint32_t) tiles.size(), 256, 0, st, (const zwz::SpanWin *) d_sw, (const uint64_t *) d_tiles,
-                           (const uint16_t *) w0, win_in, wdst, d_bad);
+                if (!tiles.empty())
+                    ZWZ_LAUNCH(zwz::stream_gather_kernel, (uint32_t) tiles.size(), 256, 0, st, (const zwz::SpanWin *) d_sw, (const uint64_t *) d_tiles, wdst, d_bad);
             }
             if ((rc = check_launch(ctx, "stream_gather_kernel"))) return rc;
-            if (zwz_rt::memcpy_d2h(&first_bad, d_bad, 8, st) || zwz_rt::stream_sync(st)) return fail(ctx, ZWZ_E_CUDA, "stream_gather_kernel failed");
+            if (zwz_rt::memcpy_d2h(first_bad.data(), d_bad, G.size() * 8, st) || zwz_rt::stream_sync(st)) return fail(ctx, ZWZ_E_CUDA, "stream_gather_kernel failed");
         }
-        if (ib && (rc = index_points(ctx, st, *wb, *ib, W, sw, base, total, win_in, w0))) return rc;
-        uint64_t wlen = total; // valid bytes of the wave
-        if (first_bad < total) {
-            wlen = first_bad;
-            stat = ZWZ_STREAM_BAD;
-            finished = true;
-        } else if (finished) {
-            stat = W.back().r.status;
-        }
+        if (ib && G[0].gather && (rc = index_points(ctx, st, *wb, *ib, W, sw, S[0].base, G[0].total))) return rc;
         // ---- check values: the members that ended in the wave (before an error), and the open member's running value; pieces of
-        // <= 1 MiB, combined in order ----
-        size_t nm = 0;
-        while (nm < members.size() && members[nm].end <= wlen) nm++;
-        if (format != ZWZ_FORMAT_RAW) {
-            std::vector<uint64_t> poff;
-            std::vector<uint32_t> plen, pseg;
-            uint64_t s0 = open_start > base ? open_start - base : 0;
-            for (size_t k = 0; k <= nm && sums; ++k) {
-                const uint64_t e = k < nm ? members[k].end : (finished ? s0 : wlen); // k == nm: the open member
+        // <= 1 MiB of every stream, one launch, combined in order per stream ----
+        std::vector<uint64_t> wlen(G.size());
+        std::vector<uint8_t> done(G.size());
+        std::vector<size_t> nm(G.size());
+        std::vector<uint64_t> poff;
+        std::vector<uint32_t> plen;
+        std::vector<std::pair<uint32_t, uint32_t>> pseg; // (stream of the wave, member)
+        for (size_t gi = 0; gi < G.size(); ++gi) {
+            const Seg &g = G[gi];
+            StreamCall &sc = S[g.sid];
+            if (!g.gather) continue;
+            wlen[gi] = g.total; // valid bytes of the stream's part
+            done[gi] = g.fin;
+            if (first_bad[gi] < g.total) {
+                wlen[gi] = first_bad[gi];
+                sc.stat = ZWZ_STREAM_BAD;
+                done[gi] = 1;
+            } else if (g.fin) {
+                sc.stat = W[g.b - 1].r.status;
+            }
+            while (nm[gi] < g.members.size() && g.members[nm[gi]].end <= wlen[gi]) nm[gi]++;
+            if (!sums) continue;
+            uint64_t s0 = sc.open_start > sc.base ? sc.open_start - sc.base : 0;
+            for (size_t k = 0; k <= nm[gi]; ++k) {
+                const uint64_t e = k < nm[gi] ? g.members[k].end : (done[gi] ? s0 : wlen[gi]); // k == nm: the open member
                 for (uint64_t a = s0; a < e; a += (1u << 20)) {
-                    poff.push_back(a);
+                    poff.push_back(g.dst + a);
                     plen.push_back((uint32_t) std::min<uint64_t>(1u << 20, e - a));
-                    pseg.push_back((uint32_t) k);
+                    pseg.push_back({(uint32_t) gi, (uint32_t) k});
                 }
-                if (k < nm) s0 = members[k].end;
-            }
-            std::vector<uint32_t> pv(poff.size());
-            if (!poff.empty()) {
-                const size_t np = poff.size();
-                uint8_t *dm = (uint8_t *) wb->get(np * 16 + 64);
-                if (!dm) return fail(ctx, ZWZ_E_NOMEM, "stream scratch allocation failed");
-                if (zwz_rt::memcpy_h2d(dm, poff.data(), np * 8, st) || zwz_rt::memcpy_h2d(dm + np * 8, plen.data(), np * 4, st))
-                    return fail(ctx, ZWZ_E_CUDA, "check upload failed");
-                {
-                    ProfSpan ps(ctx, ZWZ_PROF_ADLER, st);
-                    if (format == ZWZ_FORMAT_GZIP)
-                        ZWZ_LAUNCH(zwz::crc32_kernel, (uint32_t) ((np + 7) / 8), 256, 0, st, wdst, (const uint64_t *) dm, (const uint32_t *) (dm + np * 8),
-                                   (uint32_t *) (dm + np * 12), (uint32_t) np);
-                    else
-                        ZWZ_LAUNCH(zwz::adler32_kernel, (uint32_t) ((np + 7) / 8), 256, 0, st, wdst, (const uint64_t *) dm, (const uint32_t *) (dm + np * 8),
-                                   (uint32_t *) (dm + np * 12), (uint32_t) np);
-                }
-                if ((rc = check_launch(ctx, "stream check kernel"))) return rc;
-                if (zwz_rt::memcpy_d2h(pv.data(), dm + np * 12, np * 4, st) || zwz_rt::stream_sync(st)) return fail(ctx, ZWZ_E_CUDA, "check kernel failed");
-            }
-            size_t q = 0;
-            for (size_t k = 0; k <= nm; ++k) {
-                for (; q < pseg.size() && pseg[q] == k; ++q)
-                    open_val = format == ZWZ_FORMAT_GZIP ? crc32_combine_host(open_val, pv[q], plen[q]) : adler32_combine_host(open_val, pv[q], plen[q]);
-                if (k == nm) break;
-                const Member &mb = members[k];
-                bool bad = sums && (mb.t.have & 1u) && open_val != mb.t.check;
-                if (!bad && (mb.t.have & 2u)) bad = (uint32_t) (base + mb.end - open_start) != mb.t.isize;
-                open_val = init;
-                open_start = base + mb.end;
-                if (bad) {
-                    wlen = mb.end;
-                    stat = ZWZ_STREAM_BAD;
-                    finished = true;
-                    break;
-                }
+                if (k < nm[gi]) s0 = g.members[k].end;
             }
         }
-        if (h_out && wlen && (zwz_rt::memcpy_d2h(h_out + base, wdst, (size_t) wlen, st) || zwz_rt::stream_sync(st)))
-            return fail(ctx, ZWZ_E_CUDA, "raw download failed");
-        len = base + wlen;
-        base += total;
-        win_in = m && !finished ? w0 + (size_t) (ns - 1) * ZWZ_SPAN_WIN : nullptr;
+        std::vector<uint32_t> pv(poff.size());
+        if (!poff.empty()) {
+            const size_t np = poff.size();
+            uint8_t *dm = (uint8_t *) wb->get(np * 16 + 64);
+            if (!dm) return fail(ctx, ZWZ_E_NOMEM, "stream scratch allocation failed");
+            if (zwz_rt::memcpy_h2d(dm, poff.data(), np * 8, st) || zwz_rt::memcpy_h2d(dm + np * 8, plen.data(), np * 4, st))
+                return fail(ctx, ZWZ_E_CUDA, "check upload failed");
+            {
+                ProfSpan ps(ctx, ZWZ_PROF_ADLER, st);
+                if (format == ZWZ_FORMAT_GZIP)
+                    ZWZ_LAUNCH(zwz::crc32_kernel, (uint32_t) ((np + 7) / 8), 256, 0, st, wdst, (const uint64_t *) dm, (const uint32_t *) (dm + np * 8),
+                               (uint32_t *) (dm + np * 12), (uint32_t) np);
+                else
+                    ZWZ_LAUNCH(zwz::adler32_kernel, (uint32_t) ((np + 7) / 8), 256, 0, st, wdst, (const uint64_t *) dm, (const uint32_t *) (dm + np * 8),
+                               (uint32_t *) (dm + np * 12), (uint32_t) np);
+            }
+            if ((rc = check_launch(ctx, "stream check kernel"))) return rc;
+            if (zwz_rt::memcpy_d2h(pv.data(), dm + np * 12, np * 4, st) || zwz_rt::stream_sync(st)) return fail(ctx, ZWZ_E_CUDA, "check kernel failed");
+        }
+        bool dl = false;
+        for (size_t gi = 0, q = 0; gi < G.size(); ++gi) {
+            const Seg &g = G[gi];
+            StreamCall &sc = S[g.sid];
+            if (!g.gather) {
+                sc.base += g.total;
+                continue;
+            }
+            if (format != ZWZ_FORMAT_RAW) {
+                for (size_t k = 0; k <= nm[gi]; ++k) {
+                    for (; q < pseg.size() && pseg[q].first == gi && pseg[q].second == k; ++q)
+                        sc.open_val = format == ZWZ_FORMAT_GZIP ? crc32_combine_host(sc.open_val, pv[q], plen[q]) : adler32_combine_host(sc.open_val, pv[q], plen[q]);
+                    if (k == nm[gi]) break;
+                    const Member &mb = g.members[k];
+                    bool bad = sums && (mb.t.have & 1u) && sc.open_val != mb.t.check;
+                    if (!bad && (mb.t.have & 2u)) bad = (uint32_t) (sc.base + mb.end - sc.open_start) != mb.t.isize;
+                    sc.open_val = init;
+                    sc.open_start = sc.base + mb.end;
+                    if (bad) {
+                        wlen[gi] = mb.end;
+                        sc.stat = ZWZ_STREAM_BAD;
+                        done[gi] = 1;
+                        break;
+                    }
+                }
+                while (q < pseg.size() && pseg[q].first == gi) ++q;
+            }
+            if (h_out && wlen[gi]) {
+                if (zwz_rt::memcpy_d2h(h_out + sc.out_off + sc.base, wdst + g.dst, (size_t) wlen[gi], st)) return fail(ctx, ZWZ_E_CUDA, "raw download failed");
+                dl = true;
+            }
+            sc.outlen = sc.base + wlen[gi];
+            sc.base += g.total;
+            sc.bad = done[gi] && !g.fin;
+        }
+        if (dl && zwz_rt::stream_sync(st)) return fail(ctx, ZWZ_E_CUDA, "raw download failed");
+        // ---- the stream W ends with goes on in the next wave, from where its last span stopped, unless it ended ----
+        const Seg &gl = G.back();
+        if (gl.fin) {
+            while (!P.empty() && P.front().sid == gl.sid) P.pop_front();
+        } else {
+            P.push_front(SpanEnt{W.back().r.stop, span_stop_mode(W.back()), gl.sid});
+        }
+        win_in = !gl.fin && gl.gather && !S[gl.sid].bad ? wres + ((size_t) mix[ns - 1] << 15) : nullptr;
         prevb = std::move(wb); // the previous wave's buffers go; this wave's window stays for the next
     }
     ZWZ_STREAM_STAT(1, rounds);
     ZWZ_STREAM_STAT(2, reruns);
     ZWZ_STREAM_STAT(5, waves);
     if (ctx->trace) {
-        char buf[128];
-        snprintf(buf, sizeof buf, " spans %zu rounds %zu reruns %zu waves %zu,", nspans, rounds, reruns, waves);
+        char buf[160];
+        snprintf(buf, sizeof buf, " streams %u spans %zu rounds %zu reruns %zu waves %zu,", n, nspans, rounds, reruns, waves);
         tr.line += buf;
     }
     tr.mark("waves");
-    if (full) {
-        *raw_len = base;
-        *status = ZWZ_STREAM_OUTPUT_FULL;
-    } else {
-        *raw_len = len;
-        *status = stat;
-    }
     return ZWZ_OK;
+}
+
+// the one-stream calls
+static void stream_result(const StreamCall &s, uint64_t *raw_len, uint32_t *status) {
+    *raw_len = s.full ? s.base : s.outlen;
+    *status = s.full ? (uint32_t) ZWZ_STREAM_OUTPUT_FULL : s.stat;
+}
+static int inflate_one(zwz_ctx *ctx, const uint8_t *d_comp, uint64_t comp_len, uint8_t *d_out, uint8_t *h_out, uint64_t out_cap, uint64_t *raw_len,
+                       uint32_t *status, uint32_t flags, zwz_stream_t st, IndexBuild *ib = nullptr) {
+    std::vector<StreamCall> S(1);
+    S[0].off = 0;
+    S[0].len = comp_len;
+    S[0].out_off = 0;
+    S[0].cap = out_cap;
+    const int rc = inflate_stream_impl(ctx, d_comp, S, d_out, h_out, d_out ? nullptr : &ctx->bulk_out, flags, st, ib);
+    if (!rc) stream_result(S[0], raw_len, status);
+    return rc;
 }
 
 int zwz_inflate_stream_device(zwz_ctx *ctx, const uint8_t *d_comp, uint64_t comp_len, uint8_t *d_out, uint64_t out_cap, uint64_t *raw_len,
@@ -2337,8 +2469,7 @@ int zwz_inflate_stream_device(zwz_ctx *ctx, const uint8_t *d_comp, uint64_t comp
     if (((flags >> 8) & 0xffu) > ZWZ_FORMAT_RAW) return fail(ctx, ZWZ_E_ARG, "unknown stream format");
     if (comp_len > 0xffffff00ull) return fail(ctx, ZWZ_E_ARG, "compressed stream of 4 GiB or more");
     zwz_rt::set_device(ctx->device);
-    return inflate_stream_impl(ctx, d_comp, comp_len, d_out, nullptr, out_cap, nullptr, raw_len, status, flags,
-                               stream_v ? (zwz_stream_t) stream_v : ctx->stream);
+    return inflate_one(ctx, d_comp, comp_len, d_out, nullptr, out_cap, raw_len, status, flags, stream_v ? (zwz_stream_t) stream_v : ctx->stream);
 }
 
 int zwz_inflate_stream(zwz_ctx *ctx, const uint8_t *comp, uint64_t comp_len, uint8_t *out, uint64_t out_cap, uint64_t *raw_len, uint32_t *status,
@@ -2351,7 +2482,60 @@ int zwz_inflate_stream(zwz_ctx *ctx, const uint8_t *comp, uint64_t comp_len, uin
     int rc;
     if ((rc = reserve(ctx, ctx->bulk_in, (size_t) comp_len + 64, false))) return rc;
     if (zwz_rt::memcpy_h2d(ctx->bulk_in.p, comp, (size_t) comp_len, ctx->stream)) return fail(ctx, ZWZ_E_CUDA, "compressed upload failed");
-    return inflate_stream_impl(ctx, (const uint8_t *) ctx->bulk_in.p, comp_len, nullptr, out, out_cap, &ctx->bulk_out, raw_len, status, flags, ctx->stream);
+    return inflate_one(ctx, (const uint8_t *) ctx->bulk_in.p, comp_len, nullptr, out, out_cap, raw_len, status, flags, ctx->stream);
+}
+
+// ---- many streams in one call ----
+static int stream_batch_args(zwz_ctx *ctx, const void *comp, const uint64_t *off, const uint64_t *len, uint32_t n, const void *out, const uint64_t *out_off,
+                             const uint64_t *raw_len, const uint32_t *status, uint32_t flags, std::vector<StreamCall> &S) {
+    if (n && (!comp || !off || !len || !out || !out_off || !raw_len || !status)) return fail(ctx, ZWZ_E_ARG, "null argument");
+    if (((flags >> 8) & 0xffu) > ZWZ_FORMAT_RAW) return fail(ctx, ZWZ_E_ARG, "unknown stream format");
+    S.resize(n);
+    for (uint32_t i = 0; i < n; ++i) {
+        if (len[i] > 0xffffff00ull) return fail(ctx, ZWZ_E_ARG, "compressed stream of 4 GiB or more");
+        if (off[i] + len[i] < off[i]) return fail(ctx, ZWZ_E_ARG, "stream range wraps around");
+        if (out_off[i + 1] < out_off[i]) return fail(ctx, ZWZ_E_ARG, "out_off decreases");
+        S[i].off = off[i];
+        S[i].len = len[i];
+        S[i].out_off = out_off[i];
+        S[i].cap = out_off[i + 1] - out_off[i];
+    }
+    return ZWZ_OK;
+}
+
+int zwz_inflate_stream_batch_device(zwz_ctx *ctx, const uint8_t *d_comp, const uint64_t *off, const uint64_t *len, uint32_t n, uint8_t *d_out,
+                                    const uint64_t *out_off, uint64_t *raw_len, uint32_t *status, uint32_t flags, void *stream_v) {
+    if (!ctx) return ZWZ_E_ARG;
+    std::vector<StreamCall> S;
+    int rc;
+    if ((rc = stream_batch_args(ctx, d_comp, off, len, n, d_out, out_off, raw_len, status, flags, S))) return rc;
+    if (!n) return ZWZ_OK;
+    zwz_rt::set_device(ctx->device);
+    if ((rc = inflate_stream_impl(ctx, d_comp, S, d_out, nullptr, nullptr, flags, stream_v ? (zwz_stream_t) stream_v : ctx->stream))) return rc;
+    for (uint32_t i = 0; i < n; ++i) stream_result(S[i], raw_len + i, status + i);
+    return ZWZ_OK;
+}
+
+int zwz_inflate_stream_batch(zwz_ctx *ctx, const uint8_t *comp, const uint64_t *off, const uint64_t *len, uint32_t n, uint8_t *out,
+                             const uint64_t *out_off, uint64_t *raw_len, uint32_t *status, uint32_t flags) {
+    if (!ctx) return ZWZ_E_ARG;
+    std::vector<StreamCall> S;
+    int rc;
+    if ((rc = stream_batch_args(ctx, comp, off, len, n, out, out_off, raw_len, status, flags, S))) return rc;
+    if (!n) return ZWZ_OK;
+    zwz_rt::set_device(ctx->device);
+    // the extent of the inputs goes up once
+    uint64_t lo = ~(uint64_t) 0, hi = 0;
+    for (const StreamCall &s : S) {
+        lo = std::min(lo, s.off);
+        hi = std::max(hi, s.off + s.len);
+    }
+    for (StreamCall &s : S) s.off -= lo;
+    if ((rc = reserve(ctx, ctx->bulk_in, (size_t) (hi - lo) + 64, false))) return rc;
+    if (hi > lo && zwz_rt::memcpy_h2d(ctx->bulk_in.p, comp + lo, (size_t) (hi - lo), ctx->stream)) return fail(ctx, ZWZ_E_CUDA, "compressed upload failed");
+    if ((rc = inflate_stream_impl(ctx, (const uint8_t *) ctx->bulk_in.p, S, nullptr, out, &ctx->bulk_out, flags, ctx->stream))) return rc;
+    for (uint32_t i = 0; i < n; ++i) stream_result(S[i], raw_len + i, status + i);
+    return ZWZ_OK;
 }
 
 // ======================================================================================================================
@@ -2425,7 +2609,7 @@ static int index_create(zwz_ctx *ctx, uint32_t format, uint64_t comp_len, uint64
 static int stream_index_impl(zwz_ctx *ctx, const uint8_t *d_comp, uint64_t comp_len, uint8_t *d_out, uint8_t *h_out, uint64_t out_cap, uint64_t *raw_len,
                              uint32_t *status, uint32_t flags, uint64_t spacing, zwz_index **index, zwz_stream_t st) {
     IndexBuild ib{spacing, {}, {}};
-    int rc = inflate_stream_impl(ctx, d_comp, comp_len, d_out, h_out, out_cap, d_out ? nullptr : &ctx->bulk_out, raw_len, status, flags, st, &ib);
+    int rc = inflate_one(ctx, d_comp, comp_len, d_out, h_out, out_cap, raw_len, status, flags, st, &ib);
     if (rc || *status != ZWZ_STREAM_END) return rc;
     return index_create(ctx, (flags >> 8) & 0xffu, comp_len, *raw_len, spacing, std::move(ib.pts), ib.win.data(), ib.win.size(), index);
 }
