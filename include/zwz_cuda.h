@@ -54,6 +54,7 @@ extern "C" {
 #define ZWZ_STREAM_TRUNCATED 1   /* input ran out first; everything decodable was produced        (zlib: Z_OK/Z_BUF_ERROR) */
 #define ZWZ_STREAM_BAD 2         /* invalid stream / check value mismatch; output up to the error (zlib: Z_DATA_ERROR)  */
 #define ZWZ_STREAM_OUTPUT_FULL 3 /* would produce more than the capacity given; raw_len = size needed */
+#define ZWZ_STREAM_MORE 4        /* zwz_inflater: not ended; feed more input, or call again to drain queued output   (zlib: Z_OK) */
 
 /* per-chunk deflate result */
 typedef struct zwz_deflate_result {
@@ -156,7 +157,8 @@ int zwz_inflate_batch(zwz_ctx *ctx, const uint8_t *comp, const uint64_t *off, co
  * searching (dynamic and stored blocks; a stream made of fixed blocks only decodes as one span), are decoded in parallel with
  * their 32 KiB window still unknown, confirmed against each other (a false start is decoded again), and the windows are then
  * resolved by a log-depth scan (DESIGN.md §4.8).
- *   comp[0 .. comp_len) is ONE stream, comp_len < 4 GiB; the output may be larger than 4 GiB. flags are the inflate flags with
+ *   comp[0 .. comp_len) is ONE stream, comp_len < 4 GiB; the output may be larger than 4 GiB. A stream of 4 GiB or more, one that
+ *   arrives in pieces (a pipe, a socket) or one whose output does not fit in memory at once goes through zwz_inflater (below). flags are the inflate flags with
  *   the format in bits 8..15, whatever ZWZ_INFLATE_MODE says:
  *     GZIP : every member, as gzip -d: a member follows where the previous trailer ends when the next two bytes are 1f 8b; any
  *            other bytes behind a trailer are ignored. The result is that of zlib 1.3 (windowBits 31) decoding the members one
@@ -197,6 +199,42 @@ int zwz_inflate_stream_batch_device(zwz_ctx *ctx, const uint8_t *d_comp, const u
                                     uint32_t flags, void *stream);
 int zwz_inflate_stream_batch(zwz_ctx *ctx, const uint8_t *comp, const uint64_t *off, const uint64_t *len, uint32_t n,
                              uint8_t *out, const uint64_t *out_off, uint64_t *raw_len, uint32_t *status, uint32_t flags);
+
+/* ---- one stream fed piece by piece: the streaming inflater (zlib's inflate() on successive buffers, Python's decompressobj) ----
+ * zwz_inflater_new: an inflater for one stream; flags are those of zwz_inflate_stream (the format in bits 8..15, NO_ADLER; other
+ *   bits are ignored). An unknown format or a NULL out is ZWZ_E_ARG.
+ * zwz_inflater_feed[_device](f, in, in_len, final, out, out_cap, &produced, &status): appends in[0 .. in_len) to the pending input.
+ *   When no decoded output is queued, it decodes everything the pending input allows (on the whole GPU, as zwz_inflate_stream does)
+ *   into the inflater's output queue. Then it hands out min(queued, out_cap) bytes to out and sets *produced to that count.
+ *   final != 0 says no input follows (it may come with the last bytes or in an empty call).
+ *   Equivalence: the bytes produced over all calls, concatenated, and the terminal status equal zwz_inflate_stream on the
+ *   concatenated input with the same flags (END, TRUNCATED or BAD, bytes before an error included), for every way of cutting the
+ *   input into calls, every out_cap and any number of empty calls. OUTPUT_FULL does not occur, and there is no limit on the
+ *   stream's total length, compressed or decoded.
+ *   *status: ZWZ_STREAM_MORE until the stream has ended and its queue is drained, then the terminal status, which stays.
+ *   TRUNCATED needs final. A zlib or raw stream ends with its last block (and trailer); a gzip stream ends when two bytes other
+ *   than 1f 8b follow a trailer, or at final. Once the stream has ended, further input is ignored, as zwz_inflate_stream ignores
+ *   bytes behind the end.
+ *   ZWZ_E_ARG, with the inflater unchanged: NULL f, produced or status; NULL in with in_len > 0 or NULL out with out_cap > 0; input
+ *   after final; pending input that would reach 0xffffff00 bytes. Pending input is what the decoder could not use yet: the bytes
+ *   from the last complete block (or member header) on. A caller that keeps feeding without ever draining the queue stops the
+ *   decoding, so its pending input grows until this refusal.
+ *   The _device form takes device pointers and a cudaStream_t as void* (NULL = the context's stream); both forms return after the
+ *   bytes are in out. After a ZWZ_E_CUDA or ZWZ_E_NOMEM the inflater only takes zwz_inflater_free.
+ * Memory, on the context's device: the pending input, a 64 KiB window and the output queue, which holds the output of one decode:
+ *   what the input of one call (plus the pending bytes) decodes to. Decoding has the fixed cost of a zwz_inflate_stream call (a few
+ *   launches and synchronisations): feeds of hundreds of MiB approach its rate, 64 MiB feeds reach about half of it and feeds of
+ *   1 MiB a few percent (DESIGN.md §4.11).
+ * zwz_inflater_info: bytes given (total_in), bytes handed out (total_out), pending input and queued output; NULL fields are skipped.
+ * An inflater belongs to its context; free it with zwz_inflater_free before the context is destroyed. */
+typedef struct zwz_inflater zwz_inflater;
+int zwz_inflater_new(zwz_ctx *ctx, uint32_t flags, zwz_inflater **out);
+void zwz_inflater_free(zwz_inflater *f);
+int zwz_inflater_feed_device(zwz_inflater *f, const uint8_t *d_in, uint64_t in_len, int final, uint8_t *d_out, uint64_t out_cap,
+                             uint64_t *produced, uint32_t *status, void *stream);
+int zwz_inflater_feed(zwz_inflater *f, const uint8_t *in, uint64_t in_len, int final, uint8_t *out, uint64_t out_cap,
+                      uint64_t *produced, uint32_t *status);
+int zwz_inflater_info(const zwz_inflater *f, uint64_t *total_in, uint64_t *total_out, uint64_t *pending_in, uint64_t *queued_out);
 
 /* ---- random access into one long stream: a seek index (zlib's zran.c idea) -------------------------------------------------
  * zwz_inflate_stream_index[_device] inflate exactly as zwz_inflate_stream[_device] (same output, *raw_len and *status for the same

@@ -23,12 +23,13 @@ from typing import Optional, Tuple
 
 import numpy as np
 
-__all__ = ["Context", "ZwzError", "load_library", "library_path", "CHUNK_SIZE", "deflate_bound", "chunk_table",
-           "STREAM_END", "STREAM_TRUNCATED", "STREAM_BAD", "STREAM_OUTPUT_FULL", "RESULT_DTYPE",
+__all__ = ["Context", "ZwzError", "StreamInflater", "load_library", "library_path", "CHUNK_SIZE", "deflate_bound", "chunk_table",
+           "STREAM_END", "STREAM_TRUNCATED", "STREAM_BAD", "STREAM_OUTPUT_FULL", "STREAM_MORE", "RESULT_DTYPE",
            "FORMAT_ZLIB", "FORMAT_GZIP", "FORMAT_RAW", "BGZF_BLOCK", "NO_DICT"]
 
 CHUNK_SIZE = 65535  # process.hpp:12
 STREAM_END, STREAM_TRUNCATED, STREAM_BAD, STREAM_OUTPUT_FULL = 0, 1, 2, 3
+STREAM_MORE = 4  # a streaming inflater that has not ended: feed more input, or call again for queued output
 INFLATE_NO_ADLER = 1
 INFLATE_CAREFUL = 2  # the careful decoder only (A/B runs and tests)
 # stream formats (ZWZ_FORMAT_*): the wrapper around the DEFLATE body. The ``format=`` keywords take these names.
@@ -168,6 +169,12 @@ def _declare(L):
     L.zwz_index_load.argtypes = [vp, vp, u64, C.POINTER(vp)]
     L.zwz_index_extract_device.argtypes = [vp, vp, vp, u64, u32, vp, vp, vp, vp, vp, vp, u32, vp]
     L.zwz_index_extract.argtypes = [vp, vp, vp, u64, u32, vp, vp, vp, vp, vp, vp, u32]
+    L.zwz_inflater_new.argtypes = [vp, u32, C.POINTER(vp)]
+    L.zwz_inflater_free.argtypes = [vp]
+    L.zwz_inflater_free.restype = None
+    L.zwz_inflater_feed_device.argtypes = [vp, vp, u64, i32, vp, u64, vp, vp, vp]
+    L.zwz_inflater_feed.argtypes = [vp, vp, u64, i32, vp, u64, vp, vp]
+    L.zwz_inflater_info.argtypes = [vp, vp, vp, vp, vp]
     return L
 
 
@@ -288,6 +295,95 @@ class StreamIndex:
         return got, st
 
 
+class StreamInflater:
+    """One gzip, zlib or raw DEFLATE stream fed piece by piece (zwz_inflater), as zlib.decompressobj reads it: any length, input
+    from a pipe or socket, output taken as it comes. It belongs to its Context, which frees it first when it is closed."""
+
+    def __init__(self, ctx: "Context", format: str = "gzip", flags: int = 0):
+        self.ctx = ctx
+        self.h = None
+        h = C.c_void_p()
+        ctx._check(ctx.lib.zwz_inflater_new(ctx.h, flags | (_format(format) << 8), C.byref(h)))
+        self.h = h
+        self.status = STREAM_MORE
+        self._n = np.zeros(1, dtype=np.uint64)
+        self._st = np.zeros(1, dtype=np.uint32)
+        ctx._inflaters.add(self)
+
+    def close(self):
+        if getattr(self, "h", None):
+            self.ctx.lib.zwz_inflater_free(self.h)
+            self.h = None
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+    def __enter__(self):
+        return self
+
+    def __exit__(self, *a):
+        self.close()
+
+    @property
+    def eof(self) -> bool:
+        """The stream has ended and everything it decoded has been handed out."""
+        return self.status != STREAM_MORE
+
+    def _info(self):
+        v = np.zeros(4, dtype=np.uint64)
+        self.ctx._check(self.ctx.lib.zwz_inflater_info(self.h, v[0:].ctypes.data, v[1:].ctypes.data, v[2:].ctypes.data, v[3:].ctypes.data))
+        return [int(x) for x in v]
+
+    @property
+    def total_in(self) -> int:
+        return self._info()[0]
+
+    @property
+    def total_out(self) -> int:
+        return self._info()[1]
+
+    @property
+    def pending_in(self) -> int:
+        return self._info()[2]
+
+    @property
+    def queued_out(self) -> int:
+        return self._info()[3]
+
+    def _feed(self, data, final: bool) -> np.ndarray:
+        data = _u8(data)
+        parts = []
+        while True:  # the call that decodes hands out up to 1 MiB; the rest of the queue follows in one more call
+            out = np.empty(max(self.queued_out, 1 << 20), dtype=np.uint8)
+            self.ctx._check(self.ctx.lib.zwz_inflater_feed(self.h, data.ctypes.data if data.size else None, data.size, 1 if final else 0,
+                                                           out.ctypes.data, out.size, self._n.ctypes.data, self._st.ctypes.data))
+            data = data[:0]
+            self.status = int(self._st[0])
+            if self._n[0]:
+                parts.append(out[:int(self._n[0])])
+            if self.status != STREAM_MORE or not self.queued_out:
+                break
+        return np.concatenate(parts) if parts else np.empty(0, dtype=np.uint8)
+
+    def decompress(self, data) -> np.ndarray:
+        """Feed data; returns every byte it (with what came before) decodes to so far, the queue drained."""
+        return self._feed(data, False)
+
+    def flush(self) -> np.ndarray:
+        """The final call: no more input. Returns the rest; afterwards status is END, TRUNCATED or BAD."""
+        return self._feed(b"", True)
+
+    def feed_device(self, d_in: int, n: int, d_out: int, out_cap: int, final: bool = False, stream: int = 0):
+        """zwz_inflater_feed_device: d_in[0 .. n) appended, at most out_cap bytes to d_out. Returns (produced, status)."""
+        self.ctx._check(self.ctx.lib.zwz_inflater_feed_device(self.h, d_in or None, n, 1 if final else 0, d_out or None, out_cap, self._n.ctypes.data,
+                                                              self._st.ctypes.data, stream or None))
+        self.status = int(self._st[0])
+        return int(self._n[0]), self.status
+
+
 class Context:
     """One GPU's worth of streams and arenas (``zwz_ctx``)."""
 
@@ -300,11 +396,14 @@ class Context:
         self.h = h
         self.device = device
         self._indexes = weakref.WeakSet()  # seek indexes of this context: freed before it
+        self._inflaters = weakref.WeakSet()  # streaming inflaters: the same
 
     def close(self):
         if getattr(self, "h", None):
             for ix in list(getattr(self, "_indexes", ())):
                 ix.close()
+            for f in list(getattr(self, "_inflaters", ())):
+                f.close()
             self.lib.zwz_destroy(self.h)
             self.h = None
 
@@ -592,6 +691,11 @@ class Context:
         self._check(self.lib.zwz_inflate_stream_index_device(self.h, d_comp, comp_len, d_out or None, out_cap, rl.ctypes.data, st.ctypes.data,
                                                              flags | (_format(format) << 8), spacing, C.byref(h), stream or None))
         return int(rl[0]), int(st[0]), (StreamIndex(self, h) if h.value else None)
+
+    def decompressobj(self, format: str = "gzip", flags: int = 0) -> StreamInflater:
+        """A streaming inflater for one stream fed piece by piece, as zlib.decompressobj: decompress(data) returns the bytes decoded
+        so far, flush() ends the input. Equal to inflate_stream on the concatenated input, with no limit on its length."""
+        return StreamInflater(self, format, flags)
 
     def load_index(self, blob) -> "StreamIndex":
         """A seek index saved with StreamIndex.save(); the blob is checked (ZwzError on anything malformed)."""

@@ -39,6 +39,11 @@ namespace zwz {
 enum { SPAN_MODE_BLOCK = 0, SPAN_MODE_FIRST = 1, SPAN_MODE_MEMBER = 2, SPAN_MODE_STORED = 3 };
 // span results besides ZWZ_STREAM_END / TRUNCATED / BAD (which end the stream)
 enum { SPAN_STOPPED = 4, SPAN_STOP_MEMBER = 5, SPAN_STOPPED_STORED = 6 }; // stopped at a block, a member header, a stored block
+// SpanJob::mode flag: more input may follow the stream's last byte (zwz_inflater). Where the input runs out, the span reports the
+// last point it passed where decoding can resume (a block key or a member header, its own start when it passed none) with the
+// stop result and nout / nmem / reset as they were there, and sets SpanRes::more, instead of ZWZ_STREAM_TRUNCATED. Exact because
+// a prefix that runs out is never ZWZ_STREAM_BAD: every other result stays what it is.
+#define ZWZ_SPAN_PARTIAL 0x100u
 
 // Where a span starts and stops is a block "key": the bit position of the block header, except for a stored block, whose key is
 // the bit 3 in front of its LEN field (the header may sit anywhere in the padding before it, and decodes the same from there).
@@ -64,6 +69,8 @@ struct SpanRes {
     uint64_t reset;   // position of the last member start inside the span (~0: none; 0 for FIRST / MEMBER spans)
     uint32_t status;
     uint32_t nmem;    // member trailers recorded
+    uint32_t more;    // ZWZ_SPAN_PARTIAL: the input ran out, the fields above describe the last resume point passed
+    uint32_t pad;
 };
 struct SpanMember {
     uint64_t end;     // output position (in the span) where the member ended
@@ -85,7 +92,9 @@ ZWZ_DEV void span_decode(InflateWarpSmem &S, const uint8_t *__restrict__ comp_al
     const unsigned lane = lane_id();
     uint16_t *slot = J.slot;
     const uint64_t cap = J.cap;
-    const bool at_header = J.mode == SPAN_MODE_FIRST || J.mode == SPAN_MODE_MEMBER;
+    const uint32_t mode = J.mode & 3u;
+    const bool partial = (J.mode & ZWZ_SPAN_PARTIAL) != 0u;
+    const bool at_header = mode == SPAN_MODE_FIRST || mode == SPAN_MODE_MEMBER;
     const uint64_t bit0 = at_header ? (J.start >> 4) * 8u : J.start >> 1;
     const uint64_t byte0 = bit0 >> 3;
     const uint32_t clen = (uint32_t) (J.clen - byte0); // bytes from byte0 on
@@ -100,6 +109,19 @@ ZWZ_DEV void span_decode(InflateWarpSmem &S, const uint8_t *__restrict__ comp_al
     uint32_t mybyte = 0, status = ZWZ_STREAM_END, nmem = 0;
     uint64_t stop = 0;
     uint32_t hp = 0; // member header position (bytes from byte0)
+    // partial: lane 0 keeps the last resume point in R itself (no registers held across the decode loop); done leaves it there
+    // when the input ran out
+#define SPAN_RESUME_AT(stop_, status_)         \
+    do {                                       \
+        if (partial && lane == 0) {            \
+            R.stop = (stop_);                  \
+            R.status = (status_);              \
+            R.nout = pos;                      \
+            R.reset = reset;                   \
+            R.nmem = nmem;                     \
+        }                                      \
+    } while (0)
+    SPAN_RESUME_AT(J.start, mode == SPAN_MODE_BLOCK ? (uint32_t) SPAN_STOPPED : (mode == SPAN_MODE_STORED ? (uint32_t) SPAN_STOPPED_STORED : (uint32_t) SPAN_STOP_MEMBER));
 
 #define SPAN_FLUSH_LITS()                                                          \
     do {                                                                           \
@@ -122,12 +144,14 @@ ZWZ_DEV void span_decode(InflateWarpSmem &S, const uint8_t *__restrict__ comp_al
                 stop = key;
                 goto done;
             }
+            // the span's first block resumes from its own key and mode (a stored key's bits may be padding)
+            if (!first) SPAN_RESUME_AT(key, (((uint32_t) B.hold >> 1) & 3u) == 0u ? (uint32_t) SPAN_STOPPED_STORED : (uint32_t) SPAN_STOPPED);
         }
         {
             // a span that starts at a stored block's key may sit in the padding behind the real header (RFC 1951 leaves padding
             // bits arbitrary): BFINAL comes from the key and the type from the mode
             const uint32_t last = first ? (uint32_t) (J.start & 1u) : (uint32_t) B.hold & 1u;
-            const uint32_t type = first && J.mode == SPAN_MODE_STORED ? 0u : ((uint32_t) B.hold >> 1) & 3u;
+            const uint32_t type = first && mode == SPAN_MODE_STORED ? 0u : ((uint32_t) B.hold >> 1) & 3u;
             first = false;
             infb_drop(B, 3);
             if (type == 0u) {
@@ -232,8 +256,14 @@ ZWZ_DEV void span_decode(InflateWarpSmem &S, const uint8_t *__restrict__ comp_al
                 status = ZWZ_STREAM_END;
                 goto done;
             }
-            // gzip: another member follows when the next two bytes are its magic; anything else behind a trailer is ignored
+            // gzip: another member follows when the next two bytes are its magic; anything else behind a trailer is ignored.
+            // Partial: fewer than two bytes do not tell yet, so decoding resumes at the header position.
             hp = bpos + 8u;
+            SPAN_RESUME_AT((byte0 + hp) << 4, (uint32_t) SPAN_STOP_MEMBER);
+            if (partial && clen - hp < 2u) {
+                status = ZWZ_STREAM_TRUNCATED;
+                goto done;
+            }
             if (clen - hp < 2u || c[hp] != 0x1fu || c[hp + 1u] != 0x8bu) {
                 status = ZWZ_STREAM_END;
                 goto done;
@@ -246,8 +276,8 @@ ZWZ_DEV void span_decode(InflateWarpSmem &S, const uint8_t *__restrict__ comp_al
         }
     header:
         if (format == ZWZ_FORMAT_GZIP) {
-            if (J.mode == SPAN_MODE_MEMBER && nmem == 0u && (clen < 2u || c[0] != 0x1fu || c[1] != 0x8bu)) {
-                status = ZWZ_STREAM_END;
+            if (mode == SPAN_MODE_MEMBER && nmem == 0u && (clen < 2u || c[0] != 0x1fu || c[1] != 0x8bu)) {
+                status = partial && clen < 2u ? ZWZ_STREAM_TRUNCATED : ZWZ_STREAM_END;
                 goto done;
             }
             const uint32_t h = inf_gzip_header(c + hp, clen - hp);
@@ -269,13 +299,18 @@ done:
     SPAN_FLUSH_LITS();
     __syncwarp();
     if (lane == 0) {
-        R.stop = stop;
-        R.nout = pos;
-        R.reset = reset;
-        R.status = status;
-        R.nmem = nmem;
+        const bool more = partial && status == ZWZ_STREAM_TRUNCATED;
+        if (!more) {
+            R.stop = stop;
+            R.nout = pos;
+            R.reset = reset;
+            R.status = status;
+            R.nmem = nmem;
+        }
+        R.more = more ? 1u : 0u;
     }
     __syncwarp();
+#undef SPAN_RESUME_AT
 #undef SPAN_FLUSH_LITS
 }
 

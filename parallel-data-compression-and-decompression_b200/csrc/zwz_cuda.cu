@@ -1901,6 +1901,22 @@ struct StreamBufs {
     }
 };
 
+// grow a device arena from the stream-ordered pool to at least `bytes`, keeping its first `keep` bytes
+static int grow_keep(zwz_ctx *ctx, Arena &a, size_t bytes, size_t keep, zwz_stream_t st) {
+    if (a.p && a.cap >= bytes) return ZWZ_OK;
+    void *q = nullptr;
+    const size_t want = std::max(bytes + bytes / 4 + 4096, a.cap * 2);
+    if (zwz_rt::malloc_arena(&q, want, st)) return fail(ctx, ZWZ_E_NOMEM, "device allocation failed");
+    if (keep && zwz_rt::memcpy_d2d(q, a.p, keep, st)) {
+        zwz_rt::free_arena(q, st);
+        return fail(ctx, ZWZ_E_CUDA, "device copy failed");
+    }
+    if (a.p) zwz_rt::free_arena(a.p, st);
+    a.p = q;
+    a.cap = want;
+    return ZWZ_OK;
+}
+
 struct SpanEnt {
     uint64_t start;     // SpanJob::start
     uint32_t mode;
@@ -1914,8 +1930,12 @@ struct SpanEnt {
 static bool span_terminal(const SpanEnt &e) {
     return e.r.status != zwz::SPAN_STOPPED && e.r.status != zwz::SPAN_STOP_MEMBER && e.r.status != zwz::SPAN_STOPPED_STORED;
 }
-// the mode a span starting where e stopped decodes in
+// the stream's decoding ends with e in this call: e ended the stream, or (partial spans) the input ran out inside it
+static bool span_end(const SpanEnt &e) { return span_terminal(e) || e.r.more; }
+// the mode a span starting where e stopped decodes in (a partial span that passed no resume point stopped at its own start, in
+// its own mode: FIRST included)
 static uint32_t span_stop_mode(const SpanEnt &e) {
+    if (e.r.more && e.r.stop == e.start && e.r.nout == 0) return e.mode;
     return e.r.status == zwz::SPAN_STOP_MEMBER ? zwz::SPAN_MODE_MEMBER : (e.r.status == zwz::SPAN_STOPPED_STORED ? zwz::SPAN_MODE_STORED : zwz::SPAN_MODE_BLOCK);
 }
 // slot elements a span gets at first: about 4x its compressed bytes (enough for text); a span that needs more is decoded again
@@ -1939,6 +1959,16 @@ struct StreamCall {
     // an error was found before the stream's end: its status and length are fixed, and its remaining spans are decoded for their
     // size only, so that OUTPUT_FULL is decided from the whole size wherever the waves split the stream
     bool bad = false;
+    // streaming (zwz_inflater, one-stream calls): decoding starts at `start` in `mode` (SpanJob::start / SPAN_MODE_*), with the
+    // resolved window `win` in front of it (BLOCK / STORED starts), and check values and positions going on from open_val,
+    // open_start and base. partial: more input may follow, so every span is decoded with ZWZ_SPAN_PARTIAL; when the input runs out
+    // the stream waits (`more`), start / mode are where decoding resumes and the resolved window in front of that point is copied
+    // to win_out.
+    uint64_t start = 0;
+    uint32_t mode = zwz::SPAN_MODE_FIRST;
+    const uint16_t *win = nullptr;
+    uint16_t *win_out = nullptr;
+    bool partial = false, more = false;
 };
 // the stream whose spans go on past the wave (sid ~0: none) and the start of its next candidate
 struct SpanTail {
@@ -1965,7 +1995,7 @@ static int span_decode_round(zwz_ctx *ctx, zwz_stream_t st, StreamBufs &bufs, co
         jobs[k].target = target;
         jobs[k].cap = cap;
         jobs[k].cbase = sc.off;
-        jobs[k].mode = e.mode;
+        jobs[k].mode = e.mode | (sc.partial ? ZWZ_SPAN_PARTIAL : 0u);
         jobs[k].clen = (uint32_t) sc.len;
         elems += align_up(cap, 64);
     }
@@ -2084,9 +2114,10 @@ static int index_points(zwz_ctx *ctx, zwz_stream_t st, StreamBufs &wb, IndexBuil
 // window maps of one wave stay near the scratch budget (ZWZ_TUNE_STREAM_SCRATCH_BYTES). Only the stream that straddles a wave's end
 // goes on in the next wave, which gets the resolved window behind its last span, the position where that span stopped and the
 // running check value of its open member; every other stream of the wave ends in it. d_out == NULL: every wave is gathered into
-// grow_out, and downloaded to h_out when there is one. ib (one stream): the access points of a seek index are collected wave by wave.
+// grow_out, and downloaded to h_out when there is one; `append` (the inflater's queue): the waves are appended in grow_out, which
+// keeps what earlier waves put there. ib (one stream): the access points of a seek index are collected wave by wave.
 static int inflate_stream_impl(zwz_ctx *ctx, const uint8_t *d_comp, std::vector<StreamCall> &S, uint8_t *d_out, uint8_t *h_out, Arena *grow_out,
-                               uint32_t flags, zwz_stream_t st, IndexBuild *ib = nullptr) {
+                               uint32_t flags, zwz_stream_t st, IndexBuild *ib = nullptr, bool append = false) {
     const uint32_t format = (flags >> 8) & 0xffu;
     const uint32_t n = (uint32_t) S.size();
     Trace tr(ctx, "inflate_stream", st);
@@ -2119,7 +2150,7 @@ static int inflate_stream_impl(zwz_ctx *ctx, const uint8_t *d_comp, std::vector<
     {
         size_t k = 0, ncand = 0;
         for (uint32_t s = 0; s < n; ++s) {
-            P.push_back(SpanEnt{0, zwz::SPAN_MODE_FIRST, s});
+            P.push_back(SpanEnt{S[s].start, S[s].mode, s});
             for (uint64_t j = 1; j * SB < S[s].len; ++j) {
                 const uint64_t c = cand[k++];
                 if (c == ~(uint64_t) 0) continue;
@@ -2131,10 +2162,12 @@ static int inflate_stream_impl(zwz_ctx *ctx, const uint8_t *d_comp, std::vector<
     }
     tr.mark("find");
     std::unique_ptr<StreamBufs> prevb; // keeps the window handed on by the previous wave alive
-    const uint16_t *win_in = nullptr;
+    const uint16_t *win_in = S[0].win;
     const bool sums = format != ZWZ_FORMAT_RAW && !(flags & ZWZ_INFLATE_NO_ADLER);
     const uint32_t init = format == ZWZ_FORMAT_GZIP ? 0u : 1u;
-    for (StreamCall &s : S) s.open_val = init;
+    for (StreamCall &s : S)
+        if (s.mode == zwz::SPAN_MODE_FIRST) s.open_val = init;
+    uint64_t appended = 0; // bytes earlier waves left in grow_out (append)
     size_t rounds = 0, reruns = 0, nspans = 0, waves = 0;
     while (!P.empty()) {
         waves++;
@@ -2192,11 +2225,11 @@ static int inflate_stream_impl(zwz_ctx *ctx, const uint8_t *d_comp, std::vector<
                 size_t b = a + 1;
                 while (b < W.size() && W[b].sid == W[a].sid) ++b;
                 size_t f = a;
-                while (!span_terminal(W[f]) && f + 1 < b && W[f + 1].decoded && W[f + 1].start == W[f].r.stop && W[f + 1].mode == span_stop_mode(W[f])) f++;
+                while (!span_end(W[f]) && f + 1 < b && W[f + 1].decoded && W[f + 1].start == W[f].r.stop && W[f + 1].mode == span_stop_mode(W[f])) f++;
                 for (size_t j = a; j <= f; ++j) nl.push_back(std::move(W[j]));
                 const SpanEnt &e = nl.back();
-                if (span_terminal(e) || (f + 1 == b && b == W.size())) {
-                    // settled: candidates behind a terminal span (trailing garbage, say) are dropped
+                if (span_end(e) || (f + 1 == b && b == W.size())) {
+                    // settled: candidates behind a terminal span (trailing garbage, say) or behind the end of the input are dropped
                 } else if (f + 1 == b) { // it stopped before its stream's end (a span records at most ZWZ_SPAN_MAXM members)
                     nl.push_back(SpanEnt{e.r.stop, span_stop_mode(e), e.sid});
                     reruns++;
@@ -2205,7 +2238,7 @@ static int inflate_stream_impl(zwz_ctx *ctx, const uint8_t *d_comp, std::vector<
                     settled = false;
                     for (size_t j = f + 1; j < b; ++j) {
                         const SpanEnt &p = nl.back();
-                        if (p.decoded && !span_terminal(p)) {
+                        if (p.decoded && !span_end(p)) {
                             const uint64_t bs = p.r.stop;
                             const uint32_t m = span_stop_mode(p);
                             if ((W[j].start >> 1) < (bs >> 1)) continue; // overrun by its predecessor
@@ -2267,7 +2300,11 @@ static int inflate_stream_impl(zwz_ctx *ctx, const uint8_t *d_comp, std::vector<
             G.push_back(std::move(g));
         }
         uint8_t *wdst = d_out;
-        if (!wdst) {
+        if (append) {
+            if ((rc = grow_keep(ctx, *grow_out, appended + wave_bytes + 64, appended, st))) return rc;
+            wdst = (uint8_t *) grow_out->p + appended;
+            appended += wave_bytes;
+        } else if (!wdst) {
             if ((rc = reserve(ctx, *grow_out, wave_bytes + 64, false))) return rc;
             wdst = (uint8_t *) grow_out->p;
         }
@@ -2424,13 +2461,22 @@ static int inflate_stream_impl(zwz_ctx *ctx, const uint8_t *d_comp, std::vector<
         }
         if (dl && zwz_rt::stream_sync(st)) return fail(ctx, ZWZ_E_CUDA, "raw download failed");
         // ---- the stream W ends with goes on in the next wave, from where its last span stopped, unless it ended ----
+        // A partial stream whose input ran out waits for more: where it resumes and the window in front of that point are kept ----
         const Seg &gl = G.back();
-        if (gl.fin) {
+        StreamCall &sl = S[gl.sid];
+        const bool waits = W.back().r.more != 0;
+        if (gl.fin || waits) {
             while (!P.empty() && P.front().sid == gl.sid) P.pop_front();
         } else {
             P.push_front(SpanEnt{W.back().r.stop, span_stop_mode(W.back()), gl.sid});
         }
-        win_in = !gl.fin && gl.gather && !S[gl.sid].bad ? wres + ((size_t) mix[ns - 1] << 15) : nullptr;
+        win_in = !gl.fin && gl.gather && !sl.bad ? wres + ((size_t) mix[ns - 1] << 15) : nullptr;
+        if (waits && !sl.bad) {
+            sl.more = true;
+            sl.start = W.back().r.stop;
+            sl.mode = span_stop_mode(W.back());
+            if (zwz_rt::memcpy_d2d(sl.win_out, win_in, ZWZ_SPAN_WIN * 2, st) || zwz_rt::stream_sync(st)) return fail(ctx, ZWZ_E_CUDA, "window copy failed");
+        }
         prevb = std::move(wb); // the previous wave's buffers go; this wave's window stays for the next
     }
     ZWZ_STREAM_STAT(1, rounds);
@@ -2535,6 +2581,183 @@ int zwz_inflate_stream_batch(zwz_ctx *ctx, const uint8_t *comp, const uint64_t *
     if (hi > lo && zwz_rt::memcpy_h2d(ctx->bulk_in.p, comp + lo, (size_t) (hi - lo), ctx->stream)) return fail(ctx, ZWZ_E_CUDA, "compressed upload failed");
     if ((rc = inflate_stream_impl(ctx, (const uint8_t *) ctx->bulk_in.p, S, nullptr, out, &ctx->bulk_out, flags, ctx->stream))) return rc;
     for (uint32_t i = 0; i < n; ++i) stream_result(S[i], raw_len + i, status + i);
+    return ZWZ_OK;
+}
+
+// ======================================================================================================================
+// streaming inflater: one stream fed piece by piece (zlib's inflate() on successive buffers)
+// ======================================================================================================================
+struct zwz_inflater {
+    zwz_ctx *ctx;
+    uint32_t flags;
+    Arena pend;                     // device: the pending compressed bytes are pend[pend_off .. pend_off + pend_len)
+    uint64_t pend_off = 0, pend_len = 0;
+    uint16_t *win = nullptr;        // device: the resolved 32 KiB window in front of `start` (u16, as the span decoder keeps it)
+    Arena queue;                    // device: decoded bytes queue[q_head .. q_len) not handed out yet
+    uint64_t q_head = 0, q_len = 0;
+    uint64_t start = 0;             // where decoding resumes in pend (SpanJob::start, relative to pend_off), and in which mode
+    uint32_t mode = zwz::SPAN_MODE_FIRST;
+    bool has_win = false;
+    uint32_t open_val = 0;          // check value and start of the open member
+    uint64_t open_start = 0;
+    uint64_t decoded = 0;           // bytes decoded so far (the stream's output position)
+    uint64_t total_in = 0, total_out = 0;
+    bool final = false, fresh = false, ended = false, broken = false;
+    uint32_t status = ZWZ_STREAM_END; // once ended
+};
+
+static void inflater_release(zwz_inflater *f) {
+    zwz_rt::stream_sync(f->ctx->stream);
+    if (f->pend.p) zwz_rt::free_arena(f->pend.p, f->ctx->stream);
+    if (f->queue.p) zwz_rt::free_arena(f->queue.p, f->ctx->stream);
+    if (f->win) zwz_rt::free_arena(f->win, f->ctx->stream);
+    zwz_rt::stream_sync(f->ctx->stream);
+}
+
+int zwz_inflater_new(zwz_ctx *ctx, uint32_t flags, zwz_inflater **out) {
+    if (!ctx) return ZWZ_E_ARG;
+    if (!out) return fail(ctx, ZWZ_E_ARG, "null argument");
+    *out = nullptr;
+    if (((flags >> 8) & 0xffu) > ZWZ_FORMAT_RAW) return fail(ctx, ZWZ_E_ARG, "unknown stream format");
+    zwz_rt::set_device(ctx->device);
+    std::unique_ptr<zwz_inflater> f(new (std::nothrow) zwz_inflater());
+    if (!f) return fail(ctx, ZWZ_E_NOMEM, "inflater allocation failed");
+    f->ctx = ctx;
+    f->flags = flags & (ZWZ_INFLATE_NO_ADLER | 0xff00u);
+    if (zwz_rt::malloc_arena((void **) &f->win, ZWZ_SPAN_WIN * 2, ctx->stream)) return fail(ctx, ZWZ_E_NOMEM, "inflater allocation failed");
+    *out = f.release();
+    return ZWZ_OK;
+}
+
+void zwz_inflater_free(zwz_inflater *f) {
+    if (!f) return;
+    zwz_rt::set_device(f->ctx->device);
+    inflater_release(f);
+    delete f;
+}
+
+// everything the pending input allows, into the (empty) queue
+static int inflater_decode(zwz_inflater *f, zwz_stream_t st) {
+    zwz_ctx *ctx = f->ctx;
+    std::vector<StreamCall> S(1);
+    StreamCall &s = S[0];
+    s.off = f->pend_off;
+    s.len = f->pend_len;
+    s.out_off = 0;
+    s.cap = ~(uint64_t) 0;
+    s.open_val = f->open_val;
+    s.open_start = f->open_start;
+    s.base = f->decoded;
+    s.start = f->start;
+    s.mode = f->mode;
+    s.win = f->has_win ? f->win : nullptr;
+    s.partial = !f->final;
+    s.win_out = s.partial ? f->win : nullptr;
+    f->q_head = f->q_len = 0;
+    const uint8_t *d_comp = (const uint8_t *) (f->pend.p ? f->pend.p : f->win); // any device address for an empty input
+    int rc = inflate_stream_impl(ctx, d_comp, S, nullptr, nullptr, &f->queue, f->flags, st, nullptr, true);
+    if (rc) {
+        f->broken = true;
+        return rc;
+    }
+    f->fresh = false;
+    if (!s.more) { // END, TRUNCATED (final only) or BAD: bytes up to the error
+        f->q_len = s.outlen - f->decoded;
+        f->decoded = s.outlen;
+        f->ended = true;
+        f->status = s.stat;
+        f->pend_len = 0;
+        return ZWZ_OK;
+    }
+    f->q_len = s.base - f->decoded;
+    f->decoded = s.base;
+    f->open_val = s.open_val;
+    f->open_start = s.open_start;
+    f->has_win = true;
+    // the compressed tail is kept from the byte of the resume point on
+    const uint64_t bit = s.mode == zwz::SPAN_MODE_FIRST || s.mode == zwz::SPAN_MODE_MEMBER ? (s.start >> 4) * 8u : s.start >> 1;
+    const uint64_t drop = bit >> 3;
+    f->pend_off += drop;
+    f->pend_len -= drop;
+    f->start = s.start - (drop << 4);
+    f->mode = s.mode;
+    return ZWZ_OK;
+}
+
+// append in[0 .. n) (host or device memory) to the pending input, moving the pending bytes to the front of a new buffer when
+// they do not fit behind the ones there
+static int inflater_append(zwz_inflater *f, const uint8_t *in, uint64_t n, bool device, zwz_stream_t st) {
+    zwz_ctx *ctx = f->ctx;
+    if (!n) return ZWZ_OK;
+    const uint64_t need = f->pend_len + n + 64; // the block finder reads whole words up to 3 bytes past the end
+    if (!f->pend.p || f->pend_off + need > f->pend.cap) {
+        void *q = nullptr;
+        const size_t want = std::max<size_t>(need + need / 4 + 4096, f->pend.cap);
+        if (zwz_rt::malloc_arena(&q, want, st)) return fail(ctx, ZWZ_E_NOMEM, "device allocation failed");
+        if (f->pend_len && zwz_rt::memcpy_d2d(q, (uint8_t *) f->pend.p + f->pend_off, f->pend_len, st)) {
+            zwz_rt::free_arena(q, st);
+            return fail(ctx, ZWZ_E_CUDA, "device copy failed");
+        }
+        if (f->pend.p) zwz_rt::free_arena(f->pend.p, st);
+        f->pend.p = q;
+        f->pend.cap = want;
+        f->pend_off = 0;
+    }
+    uint8_t *dst = (uint8_t *) f->pend.p + f->pend_off + f->pend_len;
+    if (device ? zwz_rt::memcpy_d2d(dst, in, n, st) : zwz_rt::memcpy_h2d(dst, in, n, st)) return fail(ctx, ZWZ_E_CUDA, "input copy failed");
+    f->pend_len += n;
+    f->fresh = true;
+    return ZWZ_OK;
+}
+
+static int inflater_feed(zwz_inflater *f, const uint8_t *in, uint64_t in_len, int final, uint8_t *out, uint64_t out_cap, uint64_t *produced,
+                         uint32_t *status, bool device, zwz_stream_t st) {
+    zwz_ctx *ctx = f->ctx;
+    if (!produced || !status || (!in && in_len) || (!out && out_cap)) return fail(ctx, ZWZ_E_ARG, "null argument");
+    if (f->broken) return fail(ctx, ZWZ_E_CUDA, "inflater unusable after an earlier failure");
+    if (f->final && in_len) return fail(ctx, ZWZ_E_ARG, "input after the final call");
+    if (!f->ended && f->pend_len + in_len >= 0xffffff00ull) return fail(ctx, ZWZ_E_ARG, "pending input would reach 0xffffff00 bytes");
+    zwz_rt::set_device(ctx->device);
+    *produced = 0;
+    int rc;
+    if (!f->ended && (rc = inflater_append(f, in, in_len, device, st))) return rc;
+    f->total_in += in_len;
+    if (final && !f->final) {
+        f->final = true;
+        f->fresh = true;
+    }
+    if (f->q_head == f->q_len && !f->ended && f->fresh && (rc = inflater_decode(f, st))) return rc;
+    const uint64_t k = std::min(f->q_len - f->q_head, out_cap);
+    if (k) {
+        const uint8_t *src = (const uint8_t *) f->queue.p + f->q_head;
+        if ((device ? zwz_rt::memcpy_d2d(out, src, k, st) : zwz_rt::memcpy_d2h(out, src, k, st)) || zwz_rt::stream_sync(st))
+            return fail(ctx, ZWZ_E_CUDA, "output copy failed");
+        f->q_head += k;
+        f->total_out += k;
+        *produced = k;
+    }
+    *status = f->ended && f->q_head == f->q_len ? f->status : (uint32_t) ZWZ_STREAM_MORE;
+    return ZWZ_OK;
+}
+
+int zwz_inflater_feed_device(zwz_inflater *f, const uint8_t *d_in, uint64_t in_len, int final, uint8_t *d_out, uint64_t out_cap, uint64_t *produced,
+                             uint32_t *status, void *stream_v) {
+    if (!f) return ZWZ_E_ARG;
+    return inflater_feed(f, d_in, in_len, final, d_out, out_cap, produced, status, true, stream_v ? (zwz_stream_t) stream_v : f->ctx->stream);
+}
+
+int zwz_inflater_feed(zwz_inflater *f, const uint8_t *in, uint64_t in_len, int final, uint8_t *out, uint64_t out_cap, uint64_t *produced,
+                      uint32_t *status) {
+    if (!f) return ZWZ_E_ARG;
+    return inflater_feed(f, in, in_len, final, out, out_cap, produced, status, false, f->ctx->stream);
+}
+
+int zwz_inflater_info(const zwz_inflater *f, uint64_t *total_in, uint64_t *total_out, uint64_t *pending_in, uint64_t *queued_out) {
+    if (!f) return ZWZ_E_ARG;
+    if (total_in) *total_in = f->total_in;
+    if (total_out) *total_out = f->total_out;
+    if (pending_in) *pending_in = f->ended ? 0 : f->pend_len;
+    if (queued_out) *queued_out = f->q_len - f->q_head;
     return ZWZ_OK;
 }
 

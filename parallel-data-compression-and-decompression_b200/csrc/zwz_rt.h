@@ -43,6 +43,7 @@ inline int stream_destroy(zwz_stream_t) { return 0; }
 inline int stream_sync(zwz_stream_t) { return 0; }
 inline int memcpy_h2d(void *d, const void *s, size_t n, zwz_stream_t) { if (n) memcpy(d, s, n); return 0; }
 inline int memcpy_d2h(void *d, const void *s, size_t n, zwz_stream_t) { if (n) memcpy(d, s, n); return 0; }
+inline int memcpy_d2d(void *d, const void *s, size_t n, zwz_stream_t) { if (n) memmove(d, s, n); return 0; }
 inline int memset_device(void *d, int v, size_t n, zwz_stream_t) { if (n) memset(d, v, n); return 0; }
 inline int last_error(std::string &) { return 0; }
 inline int set_max_dyn_smem(const void *, size_t) { return 0; }
@@ -127,6 +128,9 @@ inline int memcpy_h2d(void *d, const void *s, size_t n, zwz_stream_t st) {
 }
 inline int memcpy_d2h(void *d, const void *s, size_t n, zwz_stream_t st) {
     return n == 0 || cudaMemcpyAsync(d, s, n, cudaMemcpyDeviceToHost, st) == cudaSuccess ? 0 : 1;
+}
+inline int memcpy_d2d(void *d, const void *s, size_t n, zwz_stream_t st) {
+    return n == 0 || cudaMemcpyAsync(d, s, n, cudaMemcpyDeviceToDevice, st) == cudaSuccess ? 0 : 1;
 }
 inline int memset_device(void *d, int v, size_t n, zwz_stream_t st) { return n == 0 || cudaMemsetAsync(d, v, n, st) == cudaSuccess ? 0 : 1; }
 inline int last_error(std::string &msg) {
