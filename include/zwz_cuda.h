@@ -236,6 +236,64 @@ int zwz_inflater_feed(zwz_inflater *f, const uint8_t *in, uint64_t in_len, int f
                       uint64_t *produced, uint32_t *status);
 int zwz_inflater_info(const zwz_inflater *f, uint64_t *total_in, uint64_t *total_out, uint64_t *pending_in, uint64_t *queued_out);
 
+/* ---- one long input into one gzip, zlib or raw DEFLATE stream on the whole GPU (what gzip, zlib.compress and compressobj write) ----
+ * The batch calls write one complete stream per chunk of at most 64 KiB. These calls write ONE stream of any length: the input is cut
+ * into chunks of C bytes (ZWZ_TUNE_DEFLATE_STREAM_CHUNK_BYTES, default 65 535), counted from the stream start or the last flush point,
+ * and every chunk is compressed by the batch kernels as a piece of the stream, its window being the <= 32 KiB of input in front of it
+ * (back to the stream start or the last full flush). A piece that is not the last has no header or trailer, BFINAL 0 on all its blocks,
+ * and ends on a byte boundary with an empty stored block (00 00 ff ff after three zero bits, as zlib's Z_SYNC_FLUSH), so the pieces
+ * are joined byte for byte; the last piece ends the stream (DESIGN.md §4.12). Limits of the window search: a match that starts in the
+ * window ends at the window's end, noise stretches are not searched against the window, and its last two positions are not chained.
+ *   Wrappers: gzip = one member, header 1f 8b 08 00, MTIME 0, XFL 0, OS ff, trailer CRC-32 and ISIZE (length mod 2^32) little-endian;
+ *   zlib = 78 9c, trailer Adler-32 big-endian; raw = the bare blocks. An empty input gives zlib's bytes: 03 00 in raw, 78 9c 03 00 00 00
+ *   00 01 in zlib, a 20-byte member in gzip.
+ * zwz_deflate_stream[_device]: d_raw[0 .. raw_len) (any length; passes of ZWZ_TUNE_DEFLATE_SUBBATCH_BYTES bound the device memory) into
+ *   out[0 .. *comp_len). level as in zwz_deflate_batch. ZWZ_E_CAPACITY: out_cap is smaller than the stream, *comp_len is the size needed
+ *   (bytes up to out_cap may have been written). ZWZ_E_ARG: NULL comp_len, NULL raw with raw_len > 0, NULL out with out_cap > 0, an
+ *   unknown format. The host form feeds a zwz_deflater in passes of up to 1 GiB; its bytes are those of the device form.
+ * zwz_deflate_stream_bound(raw_len): out_cap >= this always suffices for one call, whatever the format, level and chunk size. */
+uint64_t zwz_deflate_stream_bound(uint64_t raw_len);
+int zwz_deflate_stream_device(zwz_ctx *ctx, const uint8_t *d_raw, uint64_t raw_len, uint8_t *d_out, uint64_t out_cap, uint64_t *comp_len,
+                              int level, int format, void *stream);
+int zwz_deflate_stream(zwz_ctx *ctx, const uint8_t *raw, uint64_t raw_len, uint8_t *out, uint64_t out_cap, uint64_t *comp_len, int level,
+                       int format);
+
+/* ---- one stream written piece by piece: the streaming deflater (zlib's deflate() on successive buffers, Python's compressobj) ----
+ * zwz_deflater_new: a deflater for one stream in `format` at `level` (as zwz_deflate_stream); it keeps the chunk size C the context
+ *   has when it is made. An unknown format or a NULL out is ZWZ_E_ARG.
+ * zwz_deflater_feed[_device](f, in, in_len, flush, out, out_cap, &produced): appends in[0 .. in_len) to the pending input. When no
+ *   compressed output is queued, it compresses as `flush` says (numbered as zlib's, so Python may pass zlib.Z_*):
+ *     ZWZ_NO_FLUSH   every whole chunk behind which at least one more pending byte follows; at most C bytes stay pending (the stream's
+ *                    last chunk must stay pending to become its final piece). The last <= 32 KiB compressed is kept as the next window.
+ *     ZWZ_SYNC_FLUSH everything pending: the output so far ends with the empty stored block (written also when nothing is pending).
+ *     ZWZ_FULL_FLUSH the same, and the window is dropped: the next chunk refers to nothing before it, so a decoder can start there.
+ *     ZWZ_FINISH     everything pending, the final piece and the trailer. Later input is ZWZ_E_ARG; later calls only drain the queue.
+ *   Then it hands out min(queued, out_cap) bytes to out and sets *produced to that count. A flush asked for while output is queued is
+ *   done once the queue is empty: a call that empties the queue compresses again, so a call that returns with nothing queued has done
+ *   every flush asked for. Until then call again, as with zlib, without input: input given then is ZWZ_E_ARG.
+ *   Equivalence: chunk cuts are counted from the last flush point, so the output depends only on the input bytes and on where and which
+ *   flushes were asked for. NO_FLUSH feeds and one FINISH give, concatenated, exactly the bytes of zwz_deflate_stream on the concatenated
+ *   input, for every way of cutting it and every out_cap.
+ *   ZWZ_E_ARG: NULL f or produced; NULL in with in_len > 0 or NULL out with out_cap > 0; an unknown flush; pending input that would reach
+ *   0xffffff00 bytes. The _device form takes device pointers and a cudaStream_t as void* (NULL = the context's stream); both forms return
+ *   after the bytes are in out. After a ZWZ_E_CUDA or ZWZ_E_NOMEM the deflater only takes zwz_deflater_free.
+ * Memory, on the context's device: the pending input with its 32 KiB window in front, and the output queue, which holds what one
+ *   compression wrote (at most zwz_deflate_stream_bound of the pending input). The running check value and length stay on the host.
+ *   Each compression has the fixed cost of a zwz_deflate_stream call; feeds of tens of MiB or more amortise it (DESIGN.md §4.12).
+ * zwz_deflater_info: bytes given (total_in), bytes handed out (total_out), pending input and queued output; NULL fields are skipped.
+ * A deflater belongs to its context; free it with zwz_deflater_free before the context is destroyed. */
+#define ZWZ_NO_FLUSH 0
+#define ZWZ_SYNC_FLUSH 2
+#define ZWZ_FULL_FLUSH 3
+#define ZWZ_FINISH 4
+typedef struct zwz_deflater zwz_deflater;
+int zwz_deflater_new(zwz_ctx *ctx, int level, int format, zwz_deflater **out);
+void zwz_deflater_free(zwz_deflater *f);
+int zwz_deflater_feed_device(zwz_deflater *f, const uint8_t *d_in, uint64_t in_len, int flush, uint8_t *d_out, uint64_t out_cap,
+                             uint64_t *produced, void *stream);
+int zwz_deflater_feed(zwz_deflater *f, const uint8_t *in, uint64_t in_len, int flush, uint8_t *out, uint64_t out_cap, uint64_t *produced);
+int zwz_deflater_info(const zwz_deflater *f, uint64_t *total_in, uint64_t *total_out, uint64_t *pending_in, uint64_t *queued_out);
+
 /* ---- random access into one long stream: a seek index (zlib's zran.c idea) -------------------------------------------------
  * zwz_inflate_stream_index[_device] inflate exactly as zwz_inflate_stream[_device] (same output, *raw_len and *status for the same
  * input, flags, tuning and out_cap) and keep what the span decoding already found: access points, each a confirmed span start
@@ -390,6 +448,9 @@ int zwz_decompress_records(zwz_ctx *ctx, const uint8_t *comp, const uint64_t *of
  * in waves of consecutive spans that hand on the resolved window and the running check value; a single span larger than the budget
  * still forms a wave of its own. */
 #define ZWZ_TUNE_STREAM_SCRATCH_BYTES 5
+/* ZWZ_TUNE_DEFLATE_STREAM_CHUNK_BYTES: the chunk size C of zwz_deflate_stream* and of the deflaters made afterwards (1 024 .. 65 535;
+ * 0 = default, 65 535). Small values let tests cross many chunk boundaries, and windows that span several chunks, with small inputs. */
+#define ZWZ_TUNE_DEFLATE_STREAM_CHUNK_BYTES 6
 int zwz_ctx_tune(zwz_ctx *ctx, int what, uint64_t value);
 
 /* ---- asynchronous forms: the digests are DEFERRED ----------------------------------------------------------------------

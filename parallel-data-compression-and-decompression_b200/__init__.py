@@ -23,9 +23,10 @@ from typing import Optional, Tuple
 
 import numpy as np
 
-__all__ = ["Context", "ZwzError", "StreamInflater", "load_library", "library_path", "CHUNK_SIZE", "deflate_bound", "chunk_table",
+__all__ = ["Context", "ZwzError", "StreamInflater", "StreamDeflater", "load_library", "library_path", "CHUNK_SIZE", "deflate_bound", "chunk_table",
            "STREAM_END", "STREAM_TRUNCATED", "STREAM_BAD", "STREAM_OUTPUT_FULL", "STREAM_MORE", "RESULT_DTYPE",
-           "FORMAT_ZLIB", "FORMAT_GZIP", "FORMAT_RAW", "BGZF_BLOCK", "NO_DICT"]
+           "FORMAT_ZLIB", "FORMAT_GZIP", "FORMAT_RAW", "BGZF_BLOCK", "NO_DICT", "NO_FLUSH", "SYNC_FLUSH", "FULL_FLUSH", "FINISH",
+           "TUNE_DEFLATE_STREAM_CHUNK_BYTES", "deflate_stream_bound"]
 
 CHUNK_SIZE = 65535  # process.hpp:12
 STREAM_END, STREAM_TRUNCATED, STREAM_BAD, STREAM_OUTPUT_FULL = 0, 1, 2, 3
@@ -36,6 +37,9 @@ INFLATE_CAREFUL = 2  # the careful decoder only (A/B runs and tests)
 FORMAT_ZLIB, FORMAT_GZIP, FORMAT_RAW = 0, 1, 2
 BGZF_BLOCK = 65280  # largest chunk in gzip format: one BGZF member each
 _FORMATS = {"zlib": FORMAT_ZLIB, "gzip": FORMAT_GZIP, "raw": FORMAT_RAW}
+# flush modes of the streaming deflater (ZWZ_*_FLUSH, ZWZ_FINISH): zlib's numbering, so zlib.Z_SYNC_FLUSH etc. may be passed as well
+NO_FLUSH, SYNC_FLUSH, FULL_FLUSH, FINISH = 0, 2, 3, 4
+TUNE_DEFLATE_STREAM_CHUNK_BYTES = 6  # chunk size of compress_stream / compressobj (1 024 .. 65 535; 0 = 65 535)
 
 
 def _format(name: str) -> int:
@@ -175,6 +179,16 @@ def _declare(L):
     L.zwz_inflater_feed_device.argtypes = [vp, vp, u64, i32, vp, u64, vp, vp, vp]
     L.zwz_inflater_feed.argtypes = [vp, vp, u64, i32, vp, u64, vp, vp]
     L.zwz_inflater_info.argtypes = [vp, vp, vp, vp, vp]
+    L.zwz_deflate_stream_bound.argtypes = [u64]
+    L.zwz_deflate_stream_bound.restype = u64
+    L.zwz_deflate_stream_device.argtypes = [vp, vp, u64, vp, u64, vp, i32, i32, vp]
+    L.zwz_deflate_stream.argtypes = [vp, vp, u64, vp, u64, vp, i32, i32]
+    L.zwz_deflater_new.argtypes = [vp, i32, i32, C.POINTER(vp)]
+    L.zwz_deflater_free.argtypes = [vp]
+    L.zwz_deflater_free.restype = None
+    L.zwz_deflater_feed_device.argtypes = [vp, vp, u64, i32, vp, u64, vp, vp]
+    L.zwz_deflater_feed.argtypes = [vp, vp, u64, i32, vp, u64, vp]
+    L.zwz_deflater_info.argtypes = [vp, vp, vp, vp, vp]
     return L
 
 
@@ -196,6 +210,11 @@ def load_library(path: Optional[str] = None):
 def deflate_bound(raw_len) -> np.ndarray:
     """zwz_deflate_bound(): capacity a chunk's output slot must have."""
     return ((np.asarray(raw_len, dtype=np.uint64) + np.uint64(48 + 15)) & ~np.uint64(15)).astype(np.uint64)
+
+
+def deflate_stream_bound(raw_len: int) -> int:
+    """zwz_deflate_stream_bound(): an output capacity that always suffices for compress_stream of raw_len bytes."""
+    return raw_len + raw_len // 100 + 64
 
 
 def chunk_table(file_offs) -> Tuple[np.ndarray, np.ndarray, np.ndarray, np.ndarray]:
@@ -384,6 +403,92 @@ class StreamInflater:
         return int(self._n[0]), self.status
 
 
+class StreamDeflater:
+    """One gzip, zlib or raw DEFLATE stream written from input given piece by piece (zwz_deflater), as zlib.compressobj writes it: any
+    length, input from a pipe or a growing file. With compress() calls and one flush() the bytes are exactly those of
+    Context.compress_stream on the concatenated input. It belongs to its Context, which frees it first when it is closed."""
+
+    def __init__(self, ctx: "Context", format: str = "gzip", level: int = 0):
+        self.ctx = ctx
+        self.h = None
+        h = C.c_void_p()
+        ctx._check(ctx.lib.zwz_deflater_new(ctx.h, level, _format(format), C.byref(h)))
+        self.h = h
+        self.eof = False  # FINISH has been asked for and everything it wrote has been handed out
+        self._n = np.zeros(1, dtype=np.uint64)
+        ctx._deflaters.add(self)
+
+    def close(self):
+        if getattr(self, "h", None):
+            self.ctx.lib.zwz_deflater_free(self.h)
+            self.h = None
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+    def __enter__(self):
+        return self
+
+    def __exit__(self, *a):
+        self.close()
+
+    def _info(self):
+        v = np.zeros(4, dtype=np.uint64)
+        self.ctx._check(self.ctx.lib.zwz_deflater_info(self.h, v[0:].ctypes.data, v[1:].ctypes.data, v[2:].ctypes.data, v[3:].ctypes.data))
+        return [int(x) for x in v]
+
+    @property
+    def total_in(self) -> int:
+        return self._info()[0]
+
+    @property
+    def total_out(self) -> int:
+        return self._info()[1]
+
+    @property
+    def pending_in(self) -> int:
+        return self._info()[2]
+
+    @property
+    def queued_out(self) -> int:
+        return self._info()[3]
+
+    def _feed(self, data, mode: int) -> bytes:
+        data = _u8(data)
+        parts = []
+        while True:  # the call that compresses hands out up to 1 MiB; the rest of the queue follows in one more call
+            out = np.empty(max(self.queued_out, 1 << 20), dtype=np.uint8)
+            self.ctx._check(self.ctx.lib.zwz_deflater_feed(self.h, data.ctypes.data if data.size else None, data.size, mode, out.ctypes.data,
+                                                           out.size, self._n.ctypes.data))
+            data = data[:0]
+            if self._n[0]:
+                parts.append(out[:int(self._n[0])].tobytes())
+            if not self.queued_out:
+                break
+        if mode == FINISH:
+            self.eof = True
+        return b"".join(parts)
+
+    def compress(self, data) -> bytes:
+        """Feed data (NO_FLUSH); returns the compressed bytes it completed, possibly none."""
+        return self._feed(data, NO_FLUSH)
+
+    def flush(self, mode: int = FINISH) -> bytes:
+        """SYNC_FLUSH, FULL_FLUSH or FINISH (zlib.Z_* are the same numbers): compress everything pending; FINISH ends the stream."""
+        return self._feed(b"", mode)
+
+    def feed_device(self, d_in: int, n: int, d_out: int, out_cap: int, flush: int = NO_FLUSH, stream: int = 0) -> int:
+        """zwz_deflater_feed_device: d_in[0 .. n) appended, at most out_cap bytes to d_out. Returns the bytes produced."""
+        self.ctx._check(self.ctx.lib.zwz_deflater_feed_device(self.h, d_in or None, n, flush, d_out or None, out_cap, self._n.ctypes.data,
+                                                              stream or None))
+        if flush == FINISH and not self.queued_out:
+            self.eof = True
+        return int(self._n[0])
+
+
 class Context:
     """One GPU's worth of streams and arenas (``zwz_ctx``)."""
 
@@ -397,12 +502,15 @@ class Context:
         self.device = device
         self._indexes = weakref.WeakSet()  # seek indexes of this context: freed before it
         self._inflaters = weakref.WeakSet()  # streaming inflaters: the same
+        self._deflaters = weakref.WeakSet()  # streaming deflaters: the same
 
     def close(self):
         if getattr(self, "h", None):
             for ix in list(getattr(self, "_indexes", ())):
                 ix.close()
             for f in list(getattr(self, "_inflaters", ())):
+                f.close()
+            for f in list(getattr(self, "_deflaters", ())):
                 f.close()
             self.lib.zwz_destroy(self.h)
             self.h = None
@@ -434,6 +542,7 @@ class Context:
     TUNE_HOST_PARALLEL_MIN = 3
     TUNE_STREAM_SPAN_BYTES = 4
     TUNE_STREAM_SCRATCH_BYTES = 5
+    TUNE_DEFLATE_STREAM_CHUNK_BYTES = TUNE_DEFLATE_STREAM_CHUNK_BYTES
 
     def tune(self, what: int, value: int):
         """zwz_ctx_tune: e.g. TUNE_DEFLATE_SUBBATCH_BYTES (raw bytes per internal deflate pass; the scratch is 6 bytes per raw byte of one pass),
@@ -696,6 +805,32 @@ class Context:
         """A streaming inflater for one stream fed piece by piece, as zlib.decompressobj: decompress(data) returns the bytes decoded
         so far, flush() ends the input. Equal to inflate_stream on the concatenated input, with no limit on its length."""
         return StreamInflater(self, format, flags)
+
+    # ---- one long input into one stream ----
+    def compress_stream(self, data, format: str = "gzip", level: int = 0) -> bytes:
+        """data -> one gzip member, zlib stream or raw DEFLATE stream of any length, compressed on the whole GPU with a window carried
+        across its chunks (what gzip.compress / zlib.compress write; the bytes are this library's own)."""
+        data = _u8(data)
+        cap = deflate_stream_bound(data.size)
+        out = np.empty(cap, dtype=np.uint8)
+        n = C.c_uint64()
+        self._check(self.lib.zwz_deflate_stream(self.h, data.ctypes.data if data.size else None, data.size, out.ctypes.data, cap, C.byref(n), level,
+                                                _format(format)))
+        return out[:n.value].tobytes()
+
+    def compress_stream_device(self, d_raw: int, raw_len: int, d_out: int, out_cap: int, format: str = "gzip", level: int = 0,
+                               stream: int = 0) -> int:
+        """Device buffers: d_raw[0 .. raw_len) -> d_out; returns the stream's length (ZwzError with ZWZ_E_CAPACITY when out_cap is short;
+        deflate_stream_bound(raw_len) always suffices)."""
+        n = C.c_uint64()
+        self._check(self.lib.zwz_deflate_stream_device(self.h, d_raw or None, raw_len, d_out or None, out_cap, C.byref(n), level, _format(format),
+                                                       stream or None))
+        return n.value
+
+    def compressobj(self, format: str = "gzip", level: int = 0) -> StreamDeflater:
+        """A streaming deflater for one stream written from input given piece by piece, as zlib.compressobj: compress(data) returns the
+        bytes completed so far, flush(mode) with SYNC_FLUSH, FULL_FLUSH or FINISH (the default) as zlib's."""
+        return StreamDeflater(self, format, level)
 
     def load_index(self, blob) -> "StreamIndex":
         """A seek index saved with StreamIndex.save(); the blob is checked (ZwzError on anything malformed)."""

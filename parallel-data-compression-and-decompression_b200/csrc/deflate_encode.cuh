@@ -302,6 +302,13 @@ ZWZ_DEV_NOINLINE uint32_t enc_adler_global(const uint8_t *p, uint32_t n) {
 // ZWZ_WRAP_ZLIB_DICT: the wrapper of a zlib chunk with a preset dictionary, 78 BB (FDICT set) + DICTID in front. It has no split
 // rule and no 65 535-byte limit (neither has GZIP or RAW): the split rule serves .zwz records, which never have a dictionary.
 #define ZWZ_WRAP_ZLIB_DICT 3u
+// Pieces of one longer stream (zwz_deflate_stream, zwz_deflater), always launched with the DICT kernels: the chunks' windows are
+// their "dictionaries". ZWZ_WRAP_PIECES: every chunk is a non-final piece: no header, no trailer, BFINAL = 0 on every block, and
+// an empty stored block behind the body (3 zero bits, padding, 00 00 ff ff: zlib's Z_SYNC_FLUSH marker), so that pieces join byte
+// for byte. ZWZ_WRAP_PIECES_LAST: the same, but the launch's last chunk is the stream's final piece, written as a RAW body.
+#define ZWZ_WRAP_PIECES 4u
+#define ZWZ_WRAP_PIECES_LAST 5u
+#define ZWZ_WRAP_PIECE 6u // per chunk: a non-final piece
 ZWZ_DEV uint32_t enc_head_bytes(uint32_t format) {
     return format == ZWZ_FORMAT_GZIP ? 18u : (format == ZWZ_FORMAT_ZLIB ? 2u : (format == ZWZ_WRAP_ZLIB_DICT ? 6u : 0u));
 }
@@ -354,6 +361,28 @@ ZWZ_DEV_NOINLINE uint32_t enc_stored_stream(uint8_t *out, const uint8_t *src, ui
     __syncwarp();
     inf_copy_plain(out + h + 5u, src, n);
     return n + 5u + enc_wrap_bytes(format);
+}
+
+// a non-final piece as one stored block (BFINAL 0) followed by the empty stored block; returns its size, n + 10
+ZWZ_DEV_NOINLINE uint32_t enc_stored_piece(uint8_t *out, const uint8_t *src, uint32_t n) {
+    const uint32_t l = enc_stored_stream(out, src, n, 0u, ZWZ_FORMAT_RAW, 0u);
+    if (lane_id() == 0) {
+        out[0] = 0x00;
+        out[l] = out[l + 1u] = out[l + 2u] = 0x00;
+        out[l + 3u] = out[l + 4u] = 0xff;
+    }
+    __syncwarp();
+    return l + 5u;
+}
+
+// the end of a non-final Huffman-coded piece: the empty stored block (3 zero bits, padding to a byte, LEN 0000, NLEN ffff)
+ZWZ_DEV_NOINLINE void enc_piece_tail(BitSink *kp) {
+    EncWarpSmem &S = enc_smem();
+    const unsigned lane = lane_id();
+    BitSink k = *kp;
+    const uint32_t hb = 3u + ((8u - ((k.nwords * 32u + k.fill + 3u) & 7u)) & 7u);
+    sink_put(S, k, lane == 1u ? 0xffff0000ull : 0ull, lane == 0 ? hb : (lane == 1u ? 32u : 0u));
+    *kp = k;
 }
 
 // histogram of the tokens [t0, t1) into freq[0..320) (literal/length at 0, distance at 288); returns their extra bits
@@ -793,12 +822,15 @@ template <bool DICT> ZWZ_DEV void enc_chunk(EncWarpSmem &S, const DeflateJob &jo
     // the wrapper of this chunk: a zlib chunk with a preset dictionary names it in its header (RAW streams do not)
     uint32_t fmt = job.format, dictid = 0;
     if (DICT) {
+        if (fmt == ZWZ_WRAP_PIECES || fmt == ZWZ_WRAP_PIECES_LAST)
+            fmt = fmt == ZWZ_WRAP_PIECES_LAST && c + 1u == job.n ? ZWZ_FORMAT_RAW : ZWZ_WRAP_PIECE;
         const uint32_t di = job.dict.idx[c];
         if (di != ZWZ_NO_DICT && fmt == ZWZ_FORMAT_ZLIB) {
             fmt = ZWZ_WRAP_ZLIB_DICT;
             dictid = job.dict.id[di];
         }
     }
+    const bool piece = DICT && fmt == ZWZ_WRAP_PIECE; // compile-time false in the kernels of the calls without dictionaries
     const uint8_t *src = job.raw + job.raw_off[c];
     uint32_t *m = job.scratch + job.scr_off[c];
     uint8_t *out = job.out + job.out_off[c];
@@ -819,7 +851,7 @@ template <bool DICT> ZWZ_DEV void enc_chunk(EncWarpSmem &S, const DeflateJob &jo
         const float hb = enc_entropy_bits(0u, &nu);
         const float bound_bytes = hb * 0.125f + 7.f + (float) (nu >> 2);
         if (bound_bytes * 0.9995f >= (float) (n + 11u) - (float) (n >> 8) && (fmt != ZWZ_FORMAT_ZLIB || n + 11u <= ZWZ_CHUNK)) {
-            uint32_t l0 = enc_stored_stream(out, src, n, job.adler[c], fmt, dictid);
+            uint32_t l0 = piece ? enc_stored_piece(out, src, n) : enc_stored_stream(out, src, n, job.adler[c], fmt, dictid);
             if (lane == 0) {
                 job.res[4u * c + 0u] = l0;
                 job.res[4u * c + 1u] = 0u;
@@ -942,7 +974,7 @@ template <bool DICT> ZWZ_DEV void enc_chunk(EncWarpSmem &S, const DeflateJob &jo
     // n/256 bytes the three Huffman constructions below are skipped altogether.
     // The estimates are compared with the zlib-wrapped stored size in every format, so that the choice (and the body) does not
     // depend on the wrapper; the 65 535-byte record limit applies to zlib streams only.
-    const uint32_t sto_bytes = n + 5u + enc_wrap_bytes(fmt);
+    const uint32_t sto_bytes = n + 5u + (piece ? 5u : enc_wrap_bytes(fmt));
     const uint32_t zsto_bytes = n + 11u;
     const uint32_t sto_slack = n >> 8;
     bool force_stored = false;
@@ -973,7 +1005,7 @@ template <bool DICT> ZWZ_DEV void enc_chunk(EncWarpSmem &S, const DeflateJob &jo
                        n >= 512u;
     }
     if (force_stored) {
-        uint32_t l0 = enc_stored_stream(out, src, n, job.adler[c], fmt, dictid);
+        uint32_t l0 = piece ? enc_stored_piece(out, src, n) : enc_stored_stream(out, src, n, job.adler[c], fmt, dictid);
         if (lane == 0) {
             job.res[4u * c + 0u] = l0;
             job.res[4u * c + 1u] = 0u;
@@ -999,19 +1031,20 @@ template <bool DICT> ZWZ_DEV void enc_chunk(EncWarpSmem &S, const DeflateJob &jo
     __syncwarp();
     const uint32_t nreg = enc_find_stored_regions(m, n, ntok);
     if (nreg == 0u) {
-        enc_emit_range(&k, m, 0, ntok, extra_bits, true, true); // S.freq still holds the whole-chunk histogram from the parse
+        enc_emit_range(&k, m, 0, ntok, extra_bits, !piece, true); // S.freq still holds the whole-chunk histogram from the parse
     } else {
         uint32_t t = 0;
         for (uint32_t r = 0; r < nreg; ++r) {
             const uint32_t r0 = S.region[4u * r], r1 = S.region[4u * r + 1u], p0 = S.region[4u * r + 2u], p1 = S.region[4u * r + 3u];
             if (r0 > t) enc_emit_range(&k, m, t, r0, 0, false, false);
-            enc_emit_stored_block(&k, src + p0, p1 - p0, r1 == ntok);
+            enc_emit_stored_block(&k, src + p0, p1 - p0, !piece && r1 == ntok);
             t = r1;
         }
-        if (t < ntok) enc_emit_range(&k, m, t, ntok, 0, true, false);
+        if (t < ntok) enc_emit_range(&k, m, t, ntok, 0, !piece, false);
     }
     const uint32_t adler = job.adler[c];
-    enc_wrap_tail(&k, fmt, adler, n);
+    if (piece) enc_piece_tail(&k);
+    else enc_wrap_tail(&k, fmt, adler, n);
     const uint32_t huff_bytes = sink_finish(S, k);
     __syncwarp();
 
@@ -1026,7 +1059,7 @@ template <bool DICT> ZWZ_DEV void enc_chunk(EncWarpSmem &S, const DeflateJob &jo
             len0 = enc_stored_stream(out, src, raw0, a0, ZWZ_FORMAT_ZLIB, 0u);
             len1 = enc_stored_stream(out + len0, src + raw0, n - raw0, a1, ZWZ_FORMAT_ZLIB, 0u);
         } else {
-            len0 = enc_stored_stream(out, src, n, adler, fmt, dictid);
+            len0 = piece ? enc_stored_piece(out, src, n) : enc_stored_stream(out, src, n, adler, fmt, dictid);
         }
     }
     if (lane == 0) {

@@ -173,6 +173,7 @@ struct zwz_ctx {
     int seek_blocks_per_sm = 1; // the same for inflate_seek_kernel
     uint64_t stream_span_bytes = 0; // ZWZ_TUNE_STREAM_SPAN_BYTES (0 = default)
     uint64_t stream_scratch_bytes = 0; // ZWZ_TUNE_STREAM_SCRATCH_BYTES (0 = default)
+    uint64_t stream_chunk_bytes = 0; // ZWZ_TUNE_DEFLATE_STREAM_CHUNK_BYTES (0 = default, 65 535)
     zwz_stream_t stream = nullptr;
     zwz_stream_t md5_stream = nullptr; // deferred digests (DigestSlot)
     zwz::DigestSlot slot[2];
@@ -640,6 +641,11 @@ int zwz_ctx_tune(zwz_ctx *ctx, int what, uint64_t value) {
         ctx->stream_scratch_bytes = value;
         return ZWZ_OK;
     }
+    if (what == ZWZ_TUNE_DEFLATE_STREAM_CHUNK_BYTES) {
+        if (value != 0 && (value < 1024 || value > ZWZ_CHUNK_SIZE)) return fail(ctx, ZWZ_E_ARG, "stream chunk outside 1 024 .. 65 535 bytes");
+        ctx->stream_chunk_bytes = value;
+        return ZWZ_OK;
+    }
     return fail(ctx, ZWZ_E_ARG, "unknown tuning knob");
 }
 
@@ -730,15 +736,59 @@ int zwz_deflate_batch_device_ex(zwz_ctx *ctx, const uint8_t *d_raw, const uint64
     return zwz_deflate_batch_device_dict(ctx, d_raw, off, len, n, d_out, out_off, res, level, format, nullptr, stream_v);
 }
 
-int zwz_deflate_batch_device_dict(zwz_ctx *ctx, const uint8_t *d_raw, const uint64_t *off, const uint32_t *len, uint32_t n, uint8_t *d_out,
-                                  const uint64_t *out_off, zwz_deflate_result *res, int level, int format, const zwz_dicts *dicts, void *stream_v) {
-    if (!ctx) return ZWZ_E_ARG;
-    if (format < ZWZ_FORMAT_ZLIB || format > ZWZ_FORMAT_RAW) return fail(ctx, ZWZ_E_ARG, "unknown stream format");
-    if (n == 0) return ZWZ_OK;
-    if (!off || !len || !out_off || !res || !d_out) return fail(ctx, ZWZ_E_ARG, "null argument");
-    zwz_rt::set_device(ctx->device);
-    zwz_stream_t st = stream_v ? (zwz_stream_t) stream_v : ctx->stream;
-    Trace tr(ctx, "deflate_device", st);
+} // extern "C"
+
+namespace {
+
+// The chunks of one deflate call written as pieces of one longer stream (deflate_stream_impl): chunk i's window is the wlen[i] bytes
+// of d_raw in front of it, chained by dict_chain_kernel into one dictionary record per chunk that has a window. The call runs as one
+// sub-batch (the caller sizes it) and launches the DICT kernels, the encoder in ZWZ_WRAP_PIECES(_LAST) mode.
+struct PieceCall {
+    bool last;             // the call's last chunk is the stream's final piece
+    bool crc;              // per-chunk check value: CRC-32 (gzip), else the match kernel's Adler-32
+    const uint32_t *wlen;  // [n] host: window length of chunk i (0 = none)
+    uint32_t *check;       // [n] host, out: check value of chunk i
+};
+
+// dict_chain_kernel over the windows of a PieceCall; every chunk gets an entry in out->idx (ZWZ_NO_DICT without a window), so the
+// DICT kernels run even when no chunk has one. No DICTID: nothing in a piece names its window.
+int stage_windows(zwz_ctx *ctx, const uint8_t *d_raw, const uint64_t *off, const PieceCall &pc, uint32_t n, zwz_stream_t st, zwz::DictTable *out) {
+    uint32_t nw = 0;
+    for (uint32_t i = 0; i < n; ++i) nw += pc.wlen[i] != 0;
+    const size_t m_woff = align_up((size_t) n * 4, 256), m_wlen = m_woff + (size_t) nw * 8, m_end = m_wlen + (size_t) nw * 4;
+    int rc;
+    if ((rc = reserve(ctx, ctx->pin_dict, m_end, true))) return rc;
+    if ((rc = reserve(ctx, ctx->dict_meta, m_end + 256, false))) return rc;
+    if (nw && (rc = reserve(ctx, ctx->dict_arena, (size_t) nw * ZWZ_DICT_STRIDE, false))) return rc;
+    uint8_t *hp = (uint8_t *) ctx->pin_dict.p;
+    uint32_t k = 0;
+    for (uint32_t i = 0; i < n; ++i) {
+        ((uint32_t *) hp)[i] = pc.wlen[i] ? k : ZWZ_NO_DICT;
+        if (!pc.wlen[i]) continue;
+        ((uint64_t *) (hp + m_woff))[k] = off[i] - pc.wlen[i];
+        ((uint32_t *) (hp + m_wlen))[k++] = pc.wlen[i];
+    }
+    uint8_t *dm = (uint8_t *) ctx->dict_meta.p;
+    if (zwz_rt::memcpy_h2d(dm, hp, m_end, st)) return fail(ctx, ZWZ_E_CUDA, "window descriptor upload failed");
+    if (nw) {
+        {
+            ProfSpan ps(ctx, ZWZ_PROF_ADLER, st);
+            ZWZ_LAUNCH(zwz::dict_chain_kernel, nw, 1024, ZWZ_DICT_SMEM, st, d_raw, (const uint64_t *) (dm + m_woff), (const uint32_t *) (dm + m_wlen),
+                       (uint8_t *) ctx->dict_arena.p);
+        }
+        if ((rc = check_launch(ctx, "dict_chain_kernel"))) return rc;
+    }
+    out->idx = (const uint32_t *) dm;
+    out->arena = (const uint8_t *) ctx->dict_arena.p;
+    out->wlen = (const uint32_t *) (dm + m_wlen);
+    out->id = nullptr;
+    return ZWZ_OK;
+}
+
+int deflate_device_impl(zwz_ctx *ctx, const uint8_t *d_raw, const uint64_t *off, const uint32_t *len, uint32_t n, uint8_t *d_out,
+                        const uint64_t *out_off, zwz_deflate_result *res, int level, int format, const zwz_dicts *dicts, const PieceCall *pc,
+                        zwz_stream_t st) {
+    Trace tr(ctx, pc ? "deflate_pieces" : "deflate_device", st);
     ctx->keep_n = 0;
     // uint32 scratch entries of a chunk: best match per position (+ pad so the parser may peek one past the end), then the u16
     // position lists of lz_match_kernel (deflate_match.cuh: dm_scratch_match_words; zwz_common.cuh: scratch layout)
@@ -770,7 +820,7 @@ int zwz_deflate_batch_device_dict(zwz_ctx *ctx, const uint8_t *d_raw, const uint
     if (total_raw && !d_raw) return fail(ctx, ZWZ_E_ARG, "null raw buffer");
     zwz::DictTable dict{};
     int rc;
-    if ((rc = stage_dicts(ctx, dicts, n, format == ZWZ_FORMAT_GZIP, st, &dict))) return rc;
+    if ((rc = pc ? stage_windows(ctx, d_raw, off, *pc, n, st, &dict) : stage_dicts(ctx, dicts, n, format == ZWZ_FORMAT_GZIP, st, &dict))) return rc;
     tr.mark("validate");
 
     // descriptors: [raw_off u64][scr_off u64][raw_len u32][order u32] per chunk, then Adler-32 + match counts on the device;
@@ -931,7 +981,7 @@ int zwz_deflate_batch_device_dict(zwz_ctx *ctx, const uint8_t *d_raw, const uint
         }
         if ((rc = check_launch(ctx, "lz_match_kernel"))) return rc;
         ctx->launches--; // check_launch counted one more
-        if (format == ZWZ_FORMAT_GZIP) { // the CRC-32 replaces the Adler-32 the match kernel left in job.adler
+        if (format == ZWZ_FORMAT_GZIP || (pc && pc->crc)) { // the CRC-32 replaces the Adler-32 the match kernel left in job.adler
             {
                 ProfSpan ps(ctx, ZWZ_PROF_ADLER, st);
                 ZWZ_LAUNCH(zwz::crc32_kernel, (job.n + 7) / 8, 256, 0, st, d_raw, job.raw_off, job.raw_len, job.adler, job.n);
@@ -953,12 +1003,29 @@ int zwz_deflate_batch_device_dict(zwz_ctx *ctx, const uint8_t *d_raw, const uint
     tr.mark("kernels");
     // results come back behind the slot offsets in pin_keep, which then holds what zwz_pack_streams_device compares with
     uint8_t *h_res = (uint8_t *) ctx->pin_keep.p + keep_res_off(n);
-    if (zwz_rt::memcpy_d2h(h_res, d_res, (size_t) n * 16, st) || zwz_rt::stream_sync(st)) return fail(ctx, ZWZ_E_CUDA, "deflate kernels failed");
+    if (zwz_rt::memcpy_d2h(h_res, d_res, (size_t) n * 16, st)) return fail(ctx, ZWZ_E_CUDA, "deflate kernels failed");
+    if (pc && zwz_rt::memcpy_d2h(pc->check, d_adler, (size_t) n * 4, st)) return fail(ctx, ZWZ_E_CUDA, "deflate kernels failed");
+    if (zwz_rt::stream_sync(st)) return fail(ctx, ZWZ_E_CUDA, "deflate kernels failed");
     tr.mark("download");
     host_copy(ctx, res, h_res, (size_t) n * 16, n);
     ctx->keep_n = n;
     tr.mark("copy-out");
     return ZWZ_OK;
+}
+
+} // namespace
+
+extern "C" {
+
+int zwz_deflate_batch_device_dict(zwz_ctx *ctx, const uint8_t *d_raw, const uint64_t *off, const uint32_t *len, uint32_t n, uint8_t *d_out,
+                                  const uint64_t *out_off, zwz_deflate_result *res, int level, int format, const zwz_dicts *dicts, void *stream_v) {
+    if (!ctx) return ZWZ_E_ARG;
+    if (format < ZWZ_FORMAT_ZLIB || format > ZWZ_FORMAT_RAW) return fail(ctx, ZWZ_E_ARG, "unknown stream format");
+    if (n == 0) return ZWZ_OK;
+    if (!off || !len || !out_off || !res || !d_out) return fail(ctx, ZWZ_E_ARG, "null argument");
+    zwz_rt::set_device(ctx->device);
+    return deflate_device_impl(ctx, d_raw, off, len, n, d_out, out_off, res, level, format, dicts, nullptr,
+                               stream_v ? (zwz_stream_t) stream_v : ctx->stream);
 }
 
 static int md5_launch(zwz_ctx *ctx, uint32_t *state, const uint8_t *d_data, const uint64_t *off, const uint64_t *len, const uint64_t *total_len,
@@ -2759,6 +2826,304 @@ int zwz_inflater_info(const zwz_inflater *f, uint64_t *total_in, uint64_t *total
     if (pending_in) *pending_in = f->ended ? 0 : f->pend_len;
     if (queued_out) *queued_out = f->q_len - f->q_head;
     return ZWZ_OK;
+}
+
+// ======================================================================================================================
+// one long input into one gzip, zlib or raw DEFLATE stream: chunks written as pieces with windows (zwz_deflate_stream*, zwz_deflater)
+// ======================================================================================================================
+// What a stream being written carries from one call to the next.
+struct DeflateState {
+    int level = 0;
+    int format = ZWZ_FORMAT_GZIP;
+    uint64_t chunk = ZWZ_CHUNK_SIZE; // C: the input is cut every C bytes, counted from the stream start or the last flush point
+    bool head = false;               // the header has been written
+    uint32_t check = 0;              // CRC-32 (gzip) or Adler-32 (zlib) of the input compressed so far
+    uint64_t total = 0;              // input bytes compressed so far
+};
+
+// Level 0 of the stream calls is level 4's search. Like the batch default (level_params), it is the cheapest search inside the
+// project's 3 % size tolerance, but measured against zlib -6 over the whole input, which has a window across the chunks: the batch
+// default's search lands at 1.030 x on text there (DESIGN.md §4.12).
+static DeflateState deflate_state(const zwz_ctx *ctx, int level, int format) {
+    DeflateState s;
+    s.level = level >= 1 && level <= 9 ? level : 4;
+    s.format = format;
+    s.chunk = ctx->stream_chunk_bytes ? ctx->stream_chunk_bytes : ZWZ_CHUNK_SIZE;
+    s.check = format == ZWZ_FORMAT_ZLIB ? 1u : 0u;
+    return s;
+}
+
+// Compresses d_data[win .. win + len) as the next part of stream s. d_data[0 .. win) is the input in front of it, back to the stream
+// start or the last full flush: chunk k's window is the <= 32 KiB in front of it, a slice of the same buffer.
+//   flush: ZWZ_NO_FLUSH compresses the whole chunks behind which at least one more byte follows, so that the stream's last chunk can
+//   still become its final piece; the flushes compress everything, ZWZ_FINISH with the final piece and the trailer.
+//   The part goes to d_out. *out_len is its size, also when that is more than cap: then nothing past cap is written. *used = input
+//   bytes compressed.
+// Passes: chunks are taken while their raw bytes plus ZWZ_DICT_STRIDE / 6 per window record stay within the sub-batch size
+// (ZWZ_TUNE_DEFLATE_SUBBATCH_BYTES; the scratch is 6 bytes per raw byte, so the records count as the scratch does). A pass is one
+// deflate_device_impl call; its pieces are packed behind the previous pass's, and its check values are downloaded and combined here.
+static int deflate_stream_impl(zwz_ctx *ctx, DeflateState &s, const uint8_t *d_data, uint64_t win, uint64_t len, int flush, uint8_t *d_out,
+                               uint64_t cap, uint64_t *out_len, uint64_t *used, zwz_stream_t st) {
+    const uint64_t C = s.chunk;
+    const uint64_t nfull = flush == ZWZ_NO_FLUSH ? (len ? (len - 1) / C : 0) : len / C;
+    const uint64_t tail = flush == ZWZ_NO_FLUSH ? 0 : len - nfull * C;
+    const uint64_t nchunk = nfull + (tail ? 1u : 0u);
+    uint64_t pos = 0;
+    int rc;
+    auto put = [&](const uint8_t *b, uint32_t k) -> int { // bytes written by the host: header, markers, trailer
+        if (pos + k <= cap && zwz_rt::memcpy_h2d(d_out + pos, b, k, st)) return fail(ctx, ZWZ_E_CUDA, "stream bytes upload failed");
+        pos += k;
+        return ZWZ_OK;
+    };
+    if (!s.head) {
+        static const uint8_t gz[10] = {0x1f, 0x8b, 8, 0, 0, 0, 0, 0, 0, 0xff}, zl[2] = {0x78, 0x9c};
+        if (s.format == ZWZ_FORMAT_GZIP && (rc = put(gz, 10))) return rc;
+        if (s.format == ZWZ_FORMAT_ZLIB && (rc = put(zl, 2))) return rc;
+        s.head = true;
+    }
+    std::vector<uint64_t> off, slot, poff;
+    std::vector<uint32_t> clen, wlen, chk;
+    std::vector<zwz_deflate_result> res;
+    for (uint64_t c0 = 0; c0 < nchunk;) {
+        uint64_t c1 = c0, cost = 0;
+        while (c1 < nchunk) {
+            const uint64_t k = (c1 < nfull ? C : tail) + (win + c1 * C ? ZWZ_DICT_STRIDE / 6 : 0);
+            if (c1 > c0 && cost + k > ctx->batch_raw_bytes) break;
+            cost += k;
+            ++c1;
+        }
+        const uint32_t m = (uint32_t) (c1 - c0);
+        off.resize(m);
+        clen.resize(m);
+        wlen.resize(m);
+        chk.resize(m);
+        res.resize(m);
+        slot.resize(m + 1);
+        poff.resize(m + 1);
+        slot[0] = 0;
+        for (uint32_t i = 0; i < m; ++i) {
+            const uint64_t at = (c0 + i) * C;
+            off[i] = win + at;
+            clen[i] = (uint32_t) (c0 + i < nfull ? C : tail);
+            wlen[i] = (uint32_t) std::min<uint64_t>(ZWZ_MAX_DIST, win + at);
+            slot[i + 1] = slot[i] + zwz_deflate_bound(clen[i]);
+        }
+        if ((rc = reserve(ctx, ctx->bulk_out, (size_t) slot[m] + 64, false))) return rc;
+        PieceCall pc{flush == ZWZ_FINISH && c1 == nchunk, s.format == ZWZ_FORMAT_GZIP, wlen.data(), chk.data()};
+        if ((rc = deflate_device_impl(ctx, d_data, off.data(), clen.data(), m, (uint8_t *) ctx->bulk_out.p, slot.data(), res.data(), s.level,
+                                      pc.last ? ZWZ_WRAP_PIECES_LAST : ZWZ_WRAP_PIECES, nullptr, &pc, st)))
+            return rc;
+        poff[0] = pos;
+        for (uint32_t i = 0; i < m; ++i) {
+            poff[i + 1] = poff[i] + res[i].len0;
+            if (s.format == ZWZ_FORMAT_GZIP) s.check = crc32_combine_host(s.check, chk[i], clen[i]);
+            else if (s.format == ZWZ_FORMAT_ZLIB) s.check = adler32_combine_host(s.check, chk[i], clen[i]);
+            s.total += clen[i];
+        }
+        if (poff[m] <= cap) { // the pieces behind what is there (slot offsets and results are still in ctx->keep)
+            if ((rc = reserve(ctx, ctx->packed, (size_t) (m + 1) * 8, false))) return rc;
+            if (zwz_rt::memcpy_h2d(ctx->packed.p, poff.data(), (size_t) (m + 1) * 8, st)) return fail(ctx, ZWZ_E_CUDA, "offset upload failed");
+            {
+                ProfSpan ps(ctx, ZWZ_PROF_PACK, st);
+                ZWZ_LAUNCH(zwz::pack_streams_kernel, (m + 7) / 8, 256, 0, st, (const uint8_t *) ctx->bulk_out.p, (const uint64_t *) ctx->keep.p,
+                           (const uint32_t *) ((const uint8_t *) ctx->keep.p + keep_res_off(m)), d_out, (const uint64_t *) ctx->packed.p, m);
+            }
+            if ((rc = check_launch(ctx, "pack_streams_kernel"))) return rc;
+        }
+        pos = poff[m];
+        c0 = c1;
+    }
+    if (flush == ZWZ_SYNC_FLUSH || flush == ZWZ_FULL_FLUSH) {
+        static const uint8_t mark[5] = {0, 0, 0, 0xff, 0xff}; // nothing was pending: the empty stored block alone, as zlib writes it
+        if (!len && (rc = put(mark, 5))) return rc;
+    } else if (flush == ZWZ_FINISH) {
+        static const uint8_t empty[2] = {0x03, 0x00}; // an empty final block (fixed codes, end-of-block only)
+        if (!len && (rc = put(empty, 2))) return rc;
+        uint8_t t[8];
+        const uint32_t c = s.check, isize = (uint32_t) s.total;
+        for (int i = 0; i < 4; ++i) {
+            t[i] = (uint8_t) (c >> (8 * i));
+            t[4 + i] = (uint8_t) (isize >> (8 * i));
+        }
+        const uint8_t be[4] = {(uint8_t) (c >> 24), (uint8_t) (c >> 16), (uint8_t) (c >> 8), (uint8_t) c};
+        if (s.format == ZWZ_FORMAT_GZIP && (rc = put(t, 8))) return rc;
+        if (s.format == ZWZ_FORMAT_ZLIB && (rc = put(be, 4))) return rc;
+    }
+    *out_len = pos;
+    *used = nfull * C + tail;
+    return ZWZ_OK;
+}
+
+uint64_t zwz_deflate_stream_bound(uint64_t raw_len) { return raw_len + raw_len / 100 + 64; }
+
+static int stream_format_ok(int format) { return format >= ZWZ_FORMAT_ZLIB && format <= ZWZ_FORMAT_RAW; }
+
+int zwz_deflate_stream_device(zwz_ctx *ctx, const uint8_t *d_raw, uint64_t raw_len, uint8_t *d_out, uint64_t out_cap, uint64_t *comp_len, int level,
+                              int format, void *stream_v) {
+    if (!ctx) return ZWZ_E_ARG;
+    if (!comp_len || (!d_raw && raw_len) || (!d_out && out_cap)) return fail(ctx, ZWZ_E_ARG, "null argument");
+    if (!stream_format_ok(format)) return fail(ctx, ZWZ_E_ARG, "unknown stream format");
+    zwz_rt::set_device(ctx->device);
+    zwz_stream_t st = stream_v ? (zwz_stream_t) stream_v : ctx->stream;
+    DeflateState s = deflate_state(ctx, level, format);
+    uint64_t used = 0;
+    int rc = deflate_stream_impl(ctx, s, d_raw, 0, raw_len, ZWZ_FINISH, d_out, out_cap, comp_len, &used, st);
+    if (rc) return rc;
+    if (zwz_rt::stream_sync(st)) return fail(ctx, ZWZ_E_CUDA, "deflate stream failed");
+    return *comp_len > out_cap ? fail(ctx, ZWZ_E_CAPACITY, "output buffer too small") : ZWZ_OK;
+}
+
+// ---- the streaming deflater ----
+struct zwz_deflater {
+    zwz_ctx *ctx;
+    DeflateState s;
+    Arena buf[2];                 // device: buf[cur] holds the window (win bytes) and behind it the pending input (pend bytes)
+    int cur = 0;
+    uint64_t win = 0, pend = 0;
+    Arena queue;                  // device: compressed bytes queue[q_head .. q_len) not handed out yet
+    uint64_t q_head = 0, q_len = 0;
+    uint64_t total_in = 0, total_out = 0;
+    int asked = ZWZ_NO_FLUSH;     // a flush asked for while output was queued: done once the queue is empty
+    bool finished = false, broken = false;
+};
+
+int zwz_deflater_new(zwz_ctx *ctx, int level, int format, zwz_deflater **out) {
+    if (!ctx) return ZWZ_E_ARG;
+    if (!out) return fail(ctx, ZWZ_E_ARG, "null argument");
+    *out = nullptr;
+    if (!stream_format_ok(format)) return fail(ctx, ZWZ_E_ARG, "unknown stream format");
+    zwz_deflater *f = new (std::nothrow) zwz_deflater();
+    if (!f) return fail(ctx, ZWZ_E_NOMEM, "deflater allocation failed");
+    f->ctx = ctx;
+    f->s = deflate_state(ctx, level, format);
+    *out = f;
+    return ZWZ_OK;
+}
+
+void zwz_deflater_free(zwz_deflater *f) {
+    if (!f) return;
+    zwz_ctx *ctx = f->ctx;
+    zwz_rt::set_device(ctx->device);
+    zwz_rt::stream_sync(ctx->stream);
+    for (Arena *a : {&f->buf[0], &f->buf[1], &f->queue})
+        if (a->p) zwz_rt::free_arena(a->p, ctx->stream);
+    zwz_rt::stream_sync(ctx->stream);
+    delete f;
+}
+
+// the pending input as far as `mode` says, into the (empty) queue; the window in front of what stays pending is kept with it
+static int deflater_compress(zwz_deflater *f, int mode, zwz_stream_t st) {
+    zwz_ctx *ctx = f->ctx;
+    int rc;
+    if ((rc = grow_keep(ctx, f->queue, (size_t) zwz_deflate_stream_bound(f->pend), 0, st))) return rc;
+    uint64_t used = 0;
+    f->q_head = 0;
+    if ((rc = deflate_stream_impl(ctx, f->s, (const uint8_t *) f->buf[f->cur].p, f->win, f->pend, mode, (uint8_t *) f->queue.p, f->queue.cap, &f->q_len,
+                                  &used, st)))
+        return rc;
+    const uint64_t nwin = mode == ZWZ_FULL_FLUSH || mode == ZWZ_FINISH ? 0 : std::min<uint64_t>(ZWZ_MAX_DIST, f->win + used);
+    const uint64_t from = f->win + used - nwin, keep = nwin + f->pend - used;
+    if (from && keep) { // the window and the rest to the front of the other buffer
+        Arena &o = f->buf[f->cur ^ 1];
+        if ((rc = grow_keep(ctx, o, (size_t) keep + 64, 0, st))) return rc;
+        if (zwz_rt::memcpy_d2d(o.p, (const uint8_t *) f->buf[f->cur].p + from, (size_t) keep, st)) return fail(ctx, ZWZ_E_CUDA, "device copy failed");
+        f->cur ^= 1;
+    }
+    f->win = nwin;
+    f->pend -= used;
+    f->finished = mode == ZWZ_FINISH;
+    return ZWZ_OK;
+}
+
+static int deflater_feed(zwz_deflater *f, const uint8_t *in, uint64_t in_len, int flush, uint8_t *out, uint64_t out_cap, uint64_t *produced,
+                         bool device, zwz_stream_t st) {
+    zwz_ctx *ctx = f->ctx;
+    if (!produced || (!in && in_len) || (!out && out_cap)) return fail(ctx, ZWZ_E_ARG, "null argument");
+    if (flush != ZWZ_NO_FLUSH && flush != ZWZ_SYNC_FLUSH && flush != ZWZ_FULL_FLUSH && flush != ZWZ_FINISH) return fail(ctx, ZWZ_E_ARG, "unknown flush mode");
+    if (f->broken) return fail(ctx, ZWZ_E_CUDA, "deflater unusable after an earlier failure");
+    if (in_len && (f->finished || f->asked == ZWZ_FINISH)) return fail(ctx, ZWZ_E_ARG, "input after ZWZ_FINISH");
+    if (in_len && f->asked != ZWZ_NO_FLUSH) return fail(ctx, ZWZ_E_ARG, "input while a flush waits for the queued output to be taken");
+    if (f->pend + in_len >= 0xffffff00ull) return fail(ctx, ZWZ_E_ARG, "pending input would reach 0xffffff00 bytes");
+    zwz_rt::set_device(ctx->device);
+    *produced = 0;
+    int rc = ZWZ_OK;
+    if (in_len) {
+        Arena &b = f->buf[f->cur];
+        if ((rc = grow_keep(ctx, b, (size_t) (f->win + f->pend + in_len + 64), (size_t) (f->win + f->pend), st))) return rc;
+        uint8_t *dst = (uint8_t *) b.p + f->win + f->pend;
+        if (device ? zwz_rt::memcpy_d2d(dst, in, in_len, st) : zwz_rt::memcpy_h2d(dst, in, in_len, st)) return fail(ctx, ZWZ_E_CUDA, "input copy failed");
+        f->pend += in_len;
+        f->total_in += in_len;
+    }
+    if (!f->finished) f->asked = std::max(f->asked, flush);
+    // compress into an empty queue, hand out; when that emptied the queue, once more: so a call that returns with nothing queued has
+    // done every flush asked for
+    for (int round = 0; round < 2; ++round) {
+        if (f->q_head == f->q_len && !f->finished && (f->asked != ZWZ_NO_FLUSH || f->pend > f->s.chunk)) {
+            if ((rc = deflater_compress(f, f->asked, st))) {
+                f->broken = true;
+                return rc;
+            }
+            f->asked = ZWZ_NO_FLUSH;
+        }
+        const uint64_t k = std::min(f->q_len - f->q_head, out_cap - *produced);
+        if (k) {
+            const uint8_t *src = (const uint8_t *) f->queue.p + f->q_head;
+            if (device ? zwz_rt::memcpy_d2d(out + *produced, src, k, st) : zwz_rt::memcpy_d2h(out + *produced, src, k, st))
+                return fail(ctx, ZWZ_E_CUDA, "output copy failed");
+            f->q_head += k;
+            f->total_out += k;
+            *produced += k;
+        }
+        if (f->q_head != f->q_len) break;
+    }
+    if (zwz_rt::stream_sync(st)) return fail(ctx, ZWZ_E_CUDA, "deflater failed");
+    return ZWZ_OK;
+}
+
+int zwz_deflater_feed_device(zwz_deflater *f, const uint8_t *d_in, uint64_t in_len, int flush, uint8_t *d_out, uint64_t out_cap, uint64_t *produced,
+                             void *stream_v) {
+    if (!f) return ZWZ_E_ARG;
+    return deflater_feed(f, d_in, in_len, flush, d_out, out_cap, produced, true, stream_v ? (zwz_stream_t) stream_v : f->ctx->stream);
+}
+
+int zwz_deflater_feed(zwz_deflater *f, const uint8_t *in, uint64_t in_len, int flush, uint8_t *out, uint64_t out_cap, uint64_t *produced) {
+    if (!f) return ZWZ_E_ARG;
+    return deflater_feed(f, in, in_len, flush, out, out_cap, produced, false, f->ctx->stream);
+}
+
+int zwz_deflater_info(const zwz_deflater *f, uint64_t *total_in, uint64_t *total_out, uint64_t *pending_in, uint64_t *queued_out) {
+    if (!f) return ZWZ_E_ARG;
+    if (total_in) *total_in = f->total_in;
+    if (total_out) *total_out = f->total_out;
+    if (pending_in) *pending_in = f->pend;
+    if (queued_out) *queued_out = f->q_len - f->q_head;
+    return ZWZ_OK;
+}
+
+// The host form is the deflater fed in passes of up to 1 GiB (NO_FLUSH, then FINISH with the last one), so that its device memory
+// stays bounded whatever raw_len is; by the deflater's equivalence its bytes are those of zwz_deflate_stream_device.
+int zwz_deflate_stream(zwz_ctx *ctx, const uint8_t *raw, uint64_t raw_len, uint8_t *out, uint64_t out_cap, uint64_t *comp_len, int level, int format) {
+    if (!ctx) return ZWZ_E_ARG;
+    if (!comp_len || (!raw && raw_len) || (!out && out_cap)) return fail(ctx, ZWZ_E_ARG, "null argument");
+    zwz_deflater *fp = nullptr;
+    int rc = zwz_deflater_new(ctx, level, format, &fp);
+    if (rc) return rc;
+    std::unique_ptr<zwz_deflater, void (*)(zwz_deflater *)> f(fp, zwz_deflater_free);
+    const uint64_t step = std::min<uint64_t>(ctx->batch_raw_bytes, (uint64_t) 1 << 30);
+    uint64_t done = 0, pos = 0;
+    do {
+        const uint64_t k = std::min(step, raw_len - done);
+        const int fl = done + k == raw_len ? ZWZ_FINISH : ZWZ_NO_FLUSH;
+        uint64_t got = 0;
+        if ((rc = deflater_feed(fp, raw + done, k, fl, pos < out_cap ? out + pos : nullptr, pos < out_cap ? out_cap - pos : 0, &got, false, ctx->stream)))
+            return rc;
+        pos += got + (fp->q_len - fp->q_head); // what does not fit is counted, not written
+        fp->q_head = fp->q_len;
+        done += k;
+    } while (done < raw_len);
+    *comp_len = pos;
+    return pos > out_cap ? fail(ctx, ZWZ_E_CAPACITY, "output buffer too small") : ZWZ_OK;
 }
 
 // ======================================================================================================================
